@@ -9,6 +9,7 @@ aggregation -> count table.  Weak scaling: every rank owns 10 M reads of its own
 
   python bench.py [--gpus N --steps K --warmup W]            # CUDA path (one JSON line)
   python bench.py --impl reference [...]                      # CPU arm (oracle, all host threads)
+  python bench.py --dump-outputs DIR [...]                    # also writes the last timed step's count table (.npy)
 """
 from __future__ import annotations
 
@@ -153,6 +154,35 @@ def make_workload(n_reads, rank, world, n_cells=10000, kind="cfg2", transcripts=
     key = (pool[np.arange(len(cells)) % len(pool)][inv] << np.uint64(32)) | (key & np.uint64(0xFFFFFFFF))
     log("[rank %d] workload %s: %d reads generated in %.1fs" % (rank, kind, n_reads, time.time() - t0))
     return lib, asc, None, key
+
+
+DUMP_BYTES = 64_000_000         # all files of one --dump-outputs, .npy headers included
+
+
+def dump_outputs(out_dir, table, limit=DUMP_BYTES, prefix=""):
+    """Writes the count table of the last timed step, as a caller of the timed path receives it, to out_dir/<name>.npy
+    in float64 (exact for its uint32 values): cell, count, feat_off, feat_ids and the 0-d dropped_empty, n_called,
+    n_umis.  A table larger than `limit` bytes is written as a sample of its rows drawn with a fixed seed from the row
+    count alone: rows.npy holds the sampled row indices (ascending), feat_off / feat_ids describe those rows only."""
+    n = len(table.cell)
+    off = table.feat_off.astype(np.int64)
+    out = {"cell": table.cell, "count": table.count, "feat_off": off, "feat_ids": table.feat_ids}
+    nbytes = lambda d: sum(128 + 8 * v.size for v in d.values()) + 3 * (128 + 8)      # 128 B header per .npy file
+    m = n
+    while nbytes(out) > limit:
+        m = int(m * 0.95 * limit / nbytes(out))
+        rows = np.sort(np.random.default_rng(0).choice(n, size=m, replace=False))
+        nf = off[rows + 1] - off[rows]
+        ends = np.cumsum(nf)
+        ids = np.repeat(off[rows] - (ends - nf), nf) + np.arange(int(ends[-1]) if m else 0)
+        out = {"rows": rows, "cell": table.cell[rows], "count": table.count[rows],
+               "feat_off": np.concatenate([[0], ends]), "feat_ids": table.feat_ids[ids]}
+    for k_ in ("dropped_empty", "n_called", "n_umis"):
+        out[k_] = np.array(getattr(table, k_))
+    os.makedirs(out_dir, exist_ok=True)
+    for k_, v in out.items():
+        np.save(os.path.join(out_dir, prefix + k_ + ".npy"), np.asarray(v, np.float64))
+    log("[dump] %d of %d count rows -> %s" % (m, n, out_dir))
 
 
 def host_threads():
@@ -416,6 +446,8 @@ def run_report(args, rank, world, local):
         ms += t["agg_ms"]; launches += t["launches"]
     wall_ms = 1e3 * (time.perf_counter() - w0) / args.steps
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, table)
     ms /= args.steps
     same = np.array_equal(table.cell, table0.cell) and np.array_equal(table.count, table0.count) and np.array_equal(table.feat_ids, table0.feat_ids)
     peak, peak_src = peaks()
@@ -539,7 +571,7 @@ def hbm_pass(eng, args, threads, peak, peak_src, ra_hbm):
     for _ in range(2):
         eng.align_resident(lg, fetch_counts=False)
     eng.set_overlap(False)
-    acc, K = {}, 3
+    acc, K = {}, args.steps
     for _ in range(K):
         eng.align_resident(lg, fetch_counts=False)
         for k_, v in eng.timing().items():
@@ -579,7 +611,14 @@ def main():
                     help="default run: transcripts of the appended HBM-resident pass (0 = skip)")
     ap.add_argument("--hbm-reads", type=int, default=4_000_000)
     ap.add_argument("--hbm-parity", type=int, default=20_000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the count table of the last one to DIR/<name>.npy (float64, at most 64 MB: "
+                         "a seeded sample of the rows beyond that) to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "fastq-to-bam"):
+        ap.error("--dump-outputs: the timed path of --impl reference and --workload fastq-to-bam returns no count table")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
@@ -746,6 +785,8 @@ def main():
     clocks = sampler.stop()                                               # sampled over both timed regions
     same = (np.array_equal(table.cell, table_e.cell) and np.array_equal(table.count, table_e.count)
             and np.array_equal(table.feat_ids, table_e.feat_ids))     # `table` (resident arm) is a copy
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, table, DUMP_BYTES // world, "rank%d_" % rank if world > 1 else "")
 
     log("[rank %d] resident arm: %.2f ms/step (probe %.2f sw %.2f call %.2f agg %.2f gather %.2f)"
         % (rank, ms_per_step, tim_acc["probe_ms"] / args.steps, tim_acc["sw_ms"] / args.steps, tim_acc["call_ms"] / args.steps,
