@@ -215,6 +215,31 @@ int32_t nb200_align_files_multi(const int32_t *devices, int32_t n_devices, int32
                                 const char *const *library_json, int32_t n_libs, const char *strand_filter, int32_t k,
                                 const char *const *outputs, const char *trim, char *err, size_t err_cap, double *stats4);
 
+/* `align` (nimble/__main__.py:153-211) followed by `report` (nimble/__main__.py:254-293) in one streaming pass: BAM with
+ * CB / UB tags in, one counts TSV `feature<TAB>count<TAB>cell_barcode` per library out, byte-identical to
+ * nb200_align_files + nb200_report_file on the same input.  The called rows never leave the device: each slab appends the
+ * rows report would keep (a call, valid CB and UB, not one feature named like a pandas NA token) to a row store behind its
+ * calling kernels; after the last slab the rows are gathered in per-read TSV order, cells ranked by CB bytes, and the
+ * UMI stage (nb200_umi_counts, score 1 per row) runs on them.
+ * per_read_outputs may be NULL (no per-read TSV); otherwise the per-read TSVs are written in the same pass, identical to
+ * nb200_align_files'.  counts_outputs: one path per library.
+ * out3 (may be NULL): per library 3 values = rows used, count rows written, UMIs dropped (as nb200_report_file).
+ * FASTQ input or a BAM without any CB / UB tag fails (NB200_EINVAL); so does a library feature name containing
+ * ',', TAB, LF or CR (the per-read TSV cannot carry it).  More than 2^31 rows of one library: NB200_ELIMIT. */
+int32_t nb200_align_files_counts(nb200_ctx *ctx, const char *const *inputs, int32_t n_inputs, const int32_t *lib_ids,
+                                 const char *const *per_read_outputs, const char *const *counts_outputs, int32_t n_libs,
+                                 double umi_threshold, int32_t disable_thresholding, uint64_t *out3);
+/* The same over several GPUs (as nb200_align_files_multi): slabs go to whichever device has a free lane, each device
+ * keeps its own row store, the cell dictionary is shared, and the rows are gathered on devices[0] (cudaMemcpyPeerAsync,
+ * peer access where the devices allow it).  devices may repeat an index ({0, 0}: two contexts on one GPU).  Outputs are
+ * byte-identical to a one-GPU run. */
+int32_t nb200_align_files_counts_multi(const int32_t *devices, int32_t n_devices, int32_t host_threads,
+                                       const char *const *inputs, int32_t n_inputs, const char *const *library_json,
+                                       int32_t n_libs, const char *strand_filter, int32_t k, const char *trim,
+                                       const char *const *per_read_outputs, const char *const *counts_outputs,
+                                       double umi_threshold, int32_t disable_thresholding,
+                                       uint64_t *out3, char *err, size_t err_cap, double *stats4);
+
 /* Same computation with inputs already resident in HBM: upload once, then time repeated passes. */
 int32_t nb200_upload(nb200_ctx *ctx, const nb200_reads *r1, const nb200_reads *r2, const uint64_t *key);
 int32_t nb200_align_resident(nb200_ctx *ctx, int32_t lib_id, double umi_threshold,

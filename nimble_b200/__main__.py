@@ -24,7 +24,7 @@ def main(argv=None):
 
     a = sub.add_parser("align")
     a.add_argument("--reference", help="The reference genome to align to.", type=str, required=True)
-    a.add_argument("--output", help="The path to the output file.", type=str, required=True)
+    a.add_argument("--output", help="The path to the output file (per-read TSV; optional with --counts).", type=str, default=None)
     a.add_argument("--input", help="The input reads.", type=str, required=True, nargs="+")
     a.add_argument("-c", "--num_cores", help="The number of cores to use for alignment.", type=int, default=1)
     a.add_argument("--strand_filter", help="Filter reads based on strand information.", type=str, default="unstranded")
@@ -36,6 +36,12 @@ def main(argv=None):
     a.add_argument("--gpus", help="(extension) GPUs of this node to spread the reads over (default 1; also $NB200_GPUS)", type=int, default=None)
     a.add_argument("--cb-length", type=int, default=16)
     a.add_argument("--umi-length", type=int, default=12)
+    a.add_argument("--counts", help="(extension) also write the counts TSV `report` would write, in the same pass (BAM with CB/UB tags); "
+                                    "--output becomes optional", type=str, default=None)
+    a.add_argument("--threshold", help="with --counts: proportional count threshold for filtering features (default: 0.05), as for report",
+                   type=float, default=0.05)
+    a.add_argument("--disable_thresholding", help="with --counts: disable the per-UMI proportional count thresholding algorithm",
+                   action="store_true", default=False)
 
     r = sub.add_parser("report")
     r.add_argument("-i", "--input", help="The input file.", type=str, required=True)
@@ -64,7 +70,11 @@ def main(argv=None):
         print("nimble_b200: the aligner is the in-tree CUDA library (libnimble_b200.so); nothing to download.")
     elif args.subcommand == "generate":
         generate(args.file, args.opt_file, args.output_path)
+    elif args.subcommand == "align" and args.output is None and args.counts is None:
+        parser.error("align needs --output, --counts or both")
     elif args.subcommand == "align" and args.map:
+        if args.counts is not None:
+            parser.error("--counts does not combine with --map: run align --map, then report on its per-read TSV")
         if len(args.input) != 2:
             parser.error("--map needs exactly two --input files (R1 and R2 FASTQ)")
         if args.trim:
@@ -74,7 +84,8 @@ def main(argv=None):
                            args.cb_length, args.umi_length, k=args.kmer))
     elif args.subcommand == "align":
         sys.exit(align(args.reference, args.output, args.input, args.num_cores, args.strand_filter, args.trim,
-                       args.tmpdir, k=args.kmer, gpus=args.gpus))
+                       args.tmpdir, k=args.kmer, gpus=args.gpus, counts=args.counts, threshold=args.threshold,
+                       disable_thresholding=args.disable_thresholding))
     elif args.subcommand == "report":
         cols = args.summarize.split(",") if args.summarize else None
         report(args.input, args.output, cols, args.threshold, args.disable_thresholding)

@@ -552,4 +552,64 @@ __global__ void emit_ids_kernel(uint32_t n_out, const uint32_t *__restrict__ sta
     for (uint32_t j = a; j < b; j++) o_ids[j] = (uint32_t)l[j - a];
 }
 
+// ---- counts from files (nb200_align_files_counts): the row store ---------------------------------------------------
+// A slab's rows that reach the UMI stage are appended to the library's row store behind its calling kernels; the rows
+// are the ones `report` keeps of the per-read TSV: a call, a cell and a UMI (no NB200_NO_BARCODE), and not a single
+// feature whose name pandas reads as NaN (na_name[f], pandas_na.hpp).
+
+// read i -> (1 << 32 | names) when its row counts, else 0; entry n = 0 (the exclusive scan's total); *called += reads with
+// a call
+__global__ void __launch_bounds__(256)
+row_flag_kernel(uint32_t n, const uint64_t *__restrict__ key, const nb200_read_result *__restrict__ res, const int32_t *__restrict__ feats,
+                uint32_t mh, const uint8_t *__restrict__ na_name, uint64_t *__restrict__ val, unsigned long long *__restrict__ called) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    int c = 0;
+    if (i < n) {
+        const uint32_t k = res[i].n_feat;
+        c = k > 0;
+        bool keep = k > 0 && key[i] != NB200_NO_BARCODE;
+        if (keep && k == 1 && na_name[feats[(uint64_t)i * mh]]) keep = false;
+        val[i] = keep ? ((1ull << 32) | k) : 0ull;
+    } else if (i == n) {
+        val[i] = 0ull;
+    }
+    c = __syncthreads_count(c);
+    if (threadIdx.x == 0 && c) atomicAdd(called, (unsigned long long)c);
+}
+
+// pos = exclusive scan of row_flag_kernel's values: (row, id) offsets of read i inside the slab's segment; the segment
+// starts where the store ends (hdr[0] rows, hdr[1] ids: device-side, so that no host round trip sits between slabs)
+__global__ void __launch_bounds__(256)
+row_scatter_kernel(uint32_t n, const uint64_t *__restrict__ key, const int32_t *__restrict__ feats, uint32_t mh,
+                   const uint64_t *__restrict__ pos, const unsigned long long *__restrict__ hdr,
+                   uint64_t *__restrict__ s_key, uint32_t *__restrict__ s_nf, int32_t *__restrict__ s_ids) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint64_t a = pos[i], b = pos[i + 1];
+    if ((a >> 32) == (b >> 32)) return;
+    const uint64_t r = hdr[0] + (a >> 32), p = hdr[1] + (a & 0xFFFFFFFFull);
+    const uint32_t k = (uint32_t)(b - a);                  // (1 << 32 | k) apart
+    s_key[r] = key[i];
+    s_nf[r] = k;
+    const int32_t *f = feats + (uint64_t)i * mh;
+    for (uint32_t j = 0; j < k; j++) s_ids[p + j] = f[j];
+}
+
+// segment record seg = {first row, rows, first id, ids, (called)}; the store's end moves past it
+__global__ void row_advance_kernel(const uint64_t *__restrict__ total, unsigned long long *__restrict__ hdr, unsigned long long *__restrict__ seg) {
+    const uint64_t t = *total, rows = t >> 32, ids = t & 0xFFFFFFFFull;
+    seg[0] = hdr[0]; seg[1] = rows; seg[2] = hdr[1]; seg[3] = ids;
+    hdr[0] += rows; hdr[1] += ids;
+}
+
+// cell id (first-seen order of the host dictionary) -> rank of its CB string: the UMI stage orders cells by key, and
+// the counts TSV orders them by CB bytes
+__global__ void __launch_bounds__(256)
+cell_rank_kernel(uint64_t n, uint64_t *__restrict__ key, const uint32_t *__restrict__ rank) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint64_t k = key[i];
+    key[i] = ((uint64_t)rank[k >> 32] << 32) | (k & 0xFFFFFFFFull);
+}
+
 }  // namespace nb200

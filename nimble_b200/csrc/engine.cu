@@ -23,6 +23,7 @@
 #include "kernels.cuh"
 #include "ingest.hpp"
 #include "library.hpp"
+#include "pandas_na.hpp"
 #include "slab_api.hpp"
 #include "stream.hpp"
 #include "trim.hpp"
@@ -111,7 +112,23 @@ struct nb200_ctx {
         std::vector<int32_t> libs;
         std::vector<nb200_read_result *> out_res;
         std::vector<int32_t *> out_feats;
+        // counts mode: the slab's keys, the segment record per library (device / pinned: row0, rows, id0, ids, called)
+        DevBuf key, seg;
+        unsigned long long *h_seg = nullptr;
+        size_t h_seg_cap = 0;
+        const uint64_t *hkey = nullptr;           // what was submitted (an overflow re-runs it)
+        uint64_t n_rows_max = 0;                  // reads of the slab in flight: bound on the rows it appends
     } lane[kFileLanes];
+    // counts mode (slab_api.hpp): per library of the call, the rows that count, appended slab by slab on s_copy[1]
+    struct RowStore {
+        DevBuf key, nf, ids, hdr, na;             // hdr: rows / ids used (device); na: per feature, name is a pandas NA token
+        uint64_t cap_rows = 0, cap_ids = 0;
+        uint64_t hi_rows = 0, hi_ids = 0;         // store end as of the last segment the host has seen
+        std::vector<DevBuf> old;                  // outgrown buffers: freed when the call is done with the store
+        uint32_t mh = 1;
+    };
+    std::vector<RowStore> rs;
+    DevBuf rs_val, rs_pos, rs_tmp, rs_rank;
     cudaStream_t s_tail = nullptr;
     int overlap = 1, stats = 0, defer_fetch = 0;
     bool fetch_pending = false, fetch_started = false;   // a count table waits on the device for nb200_fetch_counts / its copies are in flight
@@ -887,10 +904,54 @@ bool lane_trim(nb200_ctx *c, int32_t lib_id, int *target, double *strictness) {
     return h.trim_on;
 }
 
+// Counts mode: append the slab's rows of store li behind its calling kernels, on s_copy[1] (the stream every lane's
+// result copies use, so that the appends of the two lanes follow one another).  The store grows geometrically; what it
+// must hold is known on the host without a synchronise: its end as of the last segment seen (lane_wait) plus, at most,
+// the reads of the other lane's slab in flight and of this one.
+static void append_rows(nb200_ctx *c, nb200_ctx::FileLane &F, int li, uint64_t n, const nb200_read_result *res, const int32_t *feats, uint32_t mh) {
+    cudaStream_t sd = c->s_copy[1];
+    nb200_ctx::RowStore &S = c->rs[(size_t)li];
+    uint64_t other = 0;
+    for (auto &G : c->lane) if (&G != &F && G.busy && G.hkey) other += G.n_rows_max;
+    const uint64_t live_r = S.hi_rows + other, live_i = S.hi_ids + other * S.mh;
+    const uint64_t need_r = live_r + n, need_i = live_i + n * mh;
+    if (need_r > S.cap_rows || need_i > S.cap_ids) {
+        const uint64_t cr = std::max(need_r, 2 * S.cap_rows), ci = std::max(need_i, 2 * S.cap_ids);
+        DevBuf k, f, d;
+        k.ensure(cr * 8); f.ensure(cr * 4); d.ensure(ci * 4);
+        const uint64_t keep_r = std::min(live_r, S.cap_rows), keep_i = std::min(live_i, S.cap_ids);
+        if (keep_r) {
+            CK(cudaMemcpyAsync(k.p, S.key.p, keep_r * 8, cudaMemcpyDeviceToDevice, sd));
+            CK(cudaMemcpyAsync(f.p, S.nf.p, keep_r * 4, cudaMemcpyDeviceToDevice, sd));
+        }
+        if (keep_i) CK(cudaMemcpyAsync(d.p, S.ids.p, keep_i * 4, cudaMemcpyDeviceToDevice, sd));
+        // the old buffers may still be read by work queued on sd: freed only when the call is done with the store
+        for (DevBuf *b : {&S.key, &S.nf, &S.ids}) if (b->p) S.old.push_back(*b);
+        S.key = k; S.nf = f; S.ids = d;
+        S.cap_rows = cr; S.cap_ids = ci;
+    }
+    c->rs_val.ensure((n + 1) * 8); c->rs_pos.ensure((n + 1) * 8);
+    unsigned long long *seg = F.seg.as<unsigned long long>() + 5 * (size_t)li;
+    CK(cudaMemsetAsync(seg, 0, 5 * 8, sd));
+    row_flag_kernel<<<nblk(n + 1, 256), 256, 0, sd>>>((uint32_t)n, F.key.as<uint64_t>(), res, feats, mh, S.na.as<uint8_t>(),
+                                                      c->rs_val.as<uint64_t>(), seg + 4);
+    size_t bytes = 0;
+    CK(cub::DeviceScan::ExclusiveSum(nullptr, bytes, c->rs_val.as<uint64_t>(), c->rs_pos.as<uint64_t>(), (int)(n + 1), sd));
+    c->rs_tmp.ensure(bytes);
+    CK(cub::DeviceScan::ExclusiveSum(c->rs_tmp.p, bytes, c->rs_val.as<uint64_t>(), c->rs_pos.as<uint64_t>(), (int)(n + 1), sd));
+    if (n) row_scatter_kernel<<<nblk(n, 256), 256, 0, sd>>>((uint32_t)n, F.key.as<uint64_t>(), feats, mh, c->rs_pos.as<uint64_t>(),
+                                                     S.hdr.as<unsigned long long>(), S.key.as<uint64_t>(), S.nf.as<uint32_t>(), S.ids.as<int32_t>());
+    row_advance_kernel<<<1, 1, 0, sd>>>(c->rs_pos.as<uint64_t>() + n, S.hdr.as<unsigned long long>(), seg);
+    CK(cudaMemcpyAsync(F.h_seg + 5 * (size_t)li, seg, 5 * 8, cudaMemcpyDeviceToHost, sd));
+    c->launches += 4;
+}
+
 void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_reads *r2, const int32_t *lib_ids, int n_libs,
-                 nb200_read_result *const *out_res, int32_t *const *out_feats, uint16_t *const *len1, uint16_t *const *len2) {
+                 nb200_read_result *const *out_res, int32_t *const *out_feats, uint16_t *const *len1, uint16_t *const *len2,
+                 const uint64_t *key) {
     nb200_ctx::FileLane &F = c->lane[lane];
     if (F.busy) throw std::runtime_error("lane is busy");
+    if (key && c->rs.size() < (size_t)n_libs) throw std::runtime_error("counts mode without lane_rows_begin");
     validate_reads(r1, "r1");
     if (r2) { validate_reads(r2, "r2"); if (r2->n != r1->n) throw std::runtime_error("r1 and r2 differ in read count"); }
     const uint64_t n = r1->n;
@@ -904,7 +965,16 @@ void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_read
     }
     F.hr1 = *r1; F.paired = r2 != nullptr; if (r2) F.hr2 = *r2;
     F.libs.assign(lib_ids, lib_ids + n_libs);
-    F.out_res.assign(out_res, out_res + n_libs); F.out_feats.assign(out_feats, out_feats + n_libs);
+    F.out_res.clear(); F.out_feats.clear();
+    if (out_res) F.out_res.assign(out_res, out_res + n_libs);
+    if (out_feats) F.out_feats.assign(out_feats, out_feats + n_libs);
+    F.hkey = key; F.n_rows_max = key ? n : 0;
+    if (key && (size_t)n_libs > F.h_seg_cap) {
+        if (F.h_seg) cudaFreeHost(F.h_seg);
+        F.h_seg = nullptr; F.h_seg_cap = 0;
+        CK(cudaMallocHost(&F.h_seg, 5 * 8 * (size_t)n_libs));
+        F.h_seg_cap = (size_t)n_libs;
+    }
     F.hlen1.clear(); F.hlen2.clear();
     if (len1) F.hlen1.assign(len1, len1 + n_libs);
     if (len2 && r2) F.hlen2.assign(len2, len2 + n_libs);
@@ -927,6 +997,10 @@ void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_read
             CK(cudaMemcpyAsync(F.l2.p, r2->len, n * 2, cudaMemcpyHostToDevice, sh));
         }
         io.r2 = ReadsDev{F.r2.as<uint8_t>(), F.l2.as<uint16_t>(), r2->stride, r2->words};
+    }
+    if (key) {
+        F.key.ensure(n * 8 + 16); F.seg.ensure(5 * 8 * (size_t)n_libs);
+        if (n) CK(cudaMemcpyAsync(F.key.p, key, n * 8, cudaMemcpyHostToDevice, sh));
     }
     if (len1 && n) {      // per-library lengths: all up before the first kernel
         F.l1v.resize(std::max<size_t>(F.l1v.size(), (size_t)n_libs)); F.l2v.resize(F.l1v.size());
@@ -977,9 +1051,10 @@ void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_read
         // results down, behind the tail of this library's kernels
         CK(cudaStreamWaitEvent(sd, B.tail_done, 0));
         if (n) {
-            CK(cudaMemcpyAsync(out_res[li], io.res, n * sizeof(nb200_read_result), cudaMemcpyDeviceToHost, sd));
-            CK(cudaMemcpyAsync(out_feats[li], io.feats, n * (size_t)mh * 4, cudaMemcpyDeviceToHost, sd));
+            if (out_res && out_res[li]) CK(cudaMemcpyAsync(out_res[li], io.res, n * sizeof(nb200_read_result), cudaMemcpyDeviceToHost, sd));
+            if (out_feats && out_feats[li]) CK(cudaMemcpyAsync(out_feats[li], io.feats, n * (size_t)mh * 4, cudaMemcpyDeviceToHost, sd));
         }
+        if (key) append_rows(c, F, li, n, io.res, io.feats, mh);
         CK(cudaMemcpyAsync(&F.h_ctr[li], B.ctr, sizeof(Counters), cudaMemcpyDeviceToHost, sd));
         // the next library (or the next slab on this lane) resets B.ctr: not before this copy has read it
         CK(cudaEventRecord(F.done, sd));
@@ -995,6 +1070,13 @@ void lane_wait(nb200_ctx *c, int lane) {
     for (int attempt = 0;; attempt++) {
         CK(cudaEventSynchronize(F.done));
         F.busy = false;
+        if (F.hkey)                                     // counts mode: where the stores end now (a re-run appends anew)
+            for (size_t li = 0; li < F.libs.size(); li++) {
+                const unsigned long long *s = F.h_seg + 5 * li;
+                nb200_ctx::RowStore &S = c->rs[li];
+                S.hi_rows = std::max<uint64_t>(S.hi_rows, s[0] + s[1]);
+                S.hi_ids = std::max<uint64_t>(S.hi_ids, s[2] + s[3]);
+            }
         unsigned long long need = 0;
         for (size_t li = 0; li < F.libs.size(); li++)
             if (F.h_ctr[li].overflow) need = std::max(need, F.h_ctr[li].items_max);
@@ -1007,9 +1089,122 @@ void lane_wait(nb200_ctx *c, int lane) {
         const std::vector<nb200_read_result *> orr = F.out_res;
         const std::vector<int32_t *> of = F.out_feats;
         const std::vector<uint16_t *> h1 = F.hlen1, h2 = F.hlen2;
-        lane_submit(c, lane, &r1, F.paired ? &r2 : nullptr, libs.data(), (int)libs.size(), orr.data(), of.data(),
-                    h1.empty() ? nullptr : h1.data(), h2.empty() ? nullptr : h2.data());
+        lane_submit(c, lane, &r1, F.paired ? &r2 : nullptr, libs.data(), (int)libs.size(), orr.empty() ? nullptr : orr.data(),
+                    of.empty() ? nullptr : of.data(), h1.empty() ? nullptr : h1.data(), h2.empty() ? nullptr : h2.data(), F.hkey);
     }
+}
+
+void lane_rows_begin(nb200_ctx *c, const int32_t *lib_ids, int n_libs) {
+    CK(cudaSetDevice(c->device));
+    for (auto &S : c->rs) {                         // (a previous call's stores)
+        for (DevBuf *b : {&S.key, &S.nf, &S.ids}) b->release();
+        for (auto &b : S.old) b.release();
+        S.old.clear();
+    }
+    c->rs.resize((size_t)n_libs);
+    for (int li = 0; li < n_libs; li++) {
+        const HostLibrary &h = lane_lib(c, lib_ids[li]).host;
+        nb200_ctx::RowStore &S = c->rs[(size_t)li];
+        S.cap_rows = S.cap_ids = S.hi_rows = S.hi_ids = 0;
+        S.mh = (uint32_t)std::max(1, h.cfg.max_hits_to_report);
+        std::vector<uint8_t> na(h.feature_names.size() + 1, 0);
+        for (size_t f = 0; f < h.feature_names.size(); f++) {
+            const std::string &nm = h.feature_names[f];
+            // a name the per-read TSV cannot carry as one token: `report` would read other names (or other rows)
+            if (nm.find_first_of(",\t\n\r") != std::string::npos)
+                throw std::runtime_error("feature name \"" + nm + "\" contains a comma, tab or line break: counts need names the per-read TSV can carry");
+            na[f] = pandas_na(nm) ? 1 : 0;
+        }
+        S.na.ensure(na.size());
+        CK(cudaMemcpy(S.na.p, na.data(), na.size(), cudaMemcpyHostToDevice));
+        S.hdr.ensure(16);
+        CK(cudaMemset(S.hdr.p, 0, 16));
+    }
+    c->rs_val.ensure(((size_t)1 << 17) * 8 + 64); c->rs_pos.ensure(((size_t)1 << 17) * 8 + 64);
+    CK(cudaDeviceSynchronize());                    // (flags and store ends in place before the lanes' streams read them)
+}
+
+void lane_rows_segments(nb200_ctx *c, int lane, RowSeg *out) {
+    const nb200_ctx::FileLane &F = c->lane[lane];
+    for (size_t li = 0; li < F.libs.size(); li++) {
+        const unsigned long long *s = F.h_seg + 5 * li;
+        out[li].row0 = s[0]; out[li].rows = s[1]; out[li].id0 = s[2]; out[li].ids = s[3]; out[li].called = s[4];
+    }
+}
+
+void lane_rows_count(const std::vector<nb200_ctx *> &ctxs, int li, int32_t lib_id, const std::vector<RowSeg> &segs,
+                     const std::vector<uint32_t> &cell_rank, double threshold, int disable, nb200_counts *counts, uint64_t *rows) {
+    nb200_ctx *c = ctxs[0];
+    for (nb200_ctx *x : ctxs) { CK(cudaSetDevice(x->device)); CK(cudaStreamSynchronize(x->s_copy[1])); }
+    CK(cudaSetDevice(c->device));
+    DevLibrary &L = lane_lib(c, lib_id);
+    uint64_t R = 0, I = 0;
+    for (const RowSeg &s : segs) { R += s.rows; I += s.ids; }
+    *rows = R;
+    if (R > 0x7FFFFFF0ull) throw LimitError("more than 2^31 rows for one library (CUB item counts are int)");
+    if (I > 0xFFFFFFF0ull) throw LimitError("more than 2^32 feature names in the rows of one library");
+    c->timing = nb200_timing{};
+    c->launches = 0;
+    c->gen_key.ensure(R * 8 + 16); c->gen_nf.ensure((R + 1) * 4 + 16); c->gen_off.ensure((R + 1) * 4 + 16); c->gen_feats.ensure(I * 4 + 16);
+    // peer access where the devices allow it (cudaMemcpyPeerAsync stages through the host otherwise)
+    for (nb200_ctx *x : ctxs)
+        if (x->device != c->device) {
+            int can = 0;
+            CK(cudaDeviceCanAccessPeer(&can, c->device, x->device));
+            if (can) {
+                const cudaError_t e = cudaDeviceEnablePeerAccess(x->device, 0);
+                if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) CK(e);
+                cudaGetLastError();
+            }
+        }
+    // gather in slab order (= per-read TSV order); runs of segments that lie back to back in one store go as one copy
+    cudaStream_t s = c->s_compute;
+    uint64_t at_r = 0, at_i = 0;
+    for (size_t a = 0; a < segs.size();) {
+        size_t b = a + 1;
+        while (b < segs.size() && segs[b].ctx == segs[a].ctx && segs[b].row0 == segs[b - 1].row0 + segs[b - 1].rows &&
+               segs[b].id0 == segs[b - 1].id0 + segs[b - 1].ids) b++;
+        uint64_t nr = 0, ni = 0;
+        for (size_t j = a; j < b; j++) { nr += segs[j].rows; ni += segs[j].ids; }
+        const nb200_ctx *x = ctxs[(size_t)segs[a].ctx];
+        const nb200_ctx::RowStore &S = x->rs[(size_t)li];
+        auto copy = [&](void *dst, const void *src, size_t bytes) {
+            if (!bytes) return;
+            if (x->device == c->device) CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, s));
+            else CK(cudaMemcpyPeerAsync(dst, c->device, src, x->device, bytes, s));
+        };
+        copy(c->gen_key.as<uint64_t>() + at_r, S.key.as<uint64_t>() + segs[a].row0, nr * 8);
+        copy(c->gen_nf.as<uint32_t>() + at_r, S.nf.as<uint32_t>() + segs[a].row0, nr * 4);
+        copy(c->gen_feats.as<int32_t>() + at_i, S.ids.as<int32_t>() + segs[a].id0, ni * 4);
+        at_r += nr; at_i += ni;
+        a = b;
+    }
+    CK(cudaMemsetAsync(c->gen_nf.as<uint32_t>() + R, 0, 4, s));
+    excl_scan_u32(c, c->gen_nf.as<uint32_t>(), c->gen_off.as<uint32_t>(), (uint32_t)(R + 1));
+    if (R) {
+        c->rs_rank.ensure(cell_rank.size() * 4 + 16);
+        CK(cudaMemcpyAsync(c->rs_rank.p, cell_rank.data(), cell_rank.size() * 4, cudaMemcpyHostToDevice, s));
+        cell_rank_kernel<<<nblk(R, 256), 256, 0, s>>>(R, c->gen_key.as<uint64_t>(), c->rs_rank.as<uint32_t>());
+        c->launches++;
+    }
+    CK(cudaMemsetAsync(c->d_ctr, 0, sizeof(Counters), s));
+    // the aligner writes nimble_score = 1 for every row: score NULL
+    aggregate(c, L, R, c->gen_key.as<uint64_t>(), Rows{c->gen_feats.as<int32_t>(), c->gen_off.as<uint32_t>(), nullptr, nullptr, 0}, nullptr,
+              0, threshold, disable, counts);
+    CK(cudaStreamSynchronize(s));
+    Counters h2;
+    CK(cudaMemcpy(&h2, c->d_ctr, sizeof(h2), cudaMemcpyDeviceToHost));
+    counts->dropped_empty = h2.dropped_empty;
+    // the stores of this library are done with
+    for (nb200_ctx *x : ctxs) {
+        CK(cudaSetDevice(x->device));
+        nb200_ctx::RowStore &S = x->rs[(size_t)li];
+        for (DevBuf *b : {&S.key, &S.nf, &S.ids}) b->release();
+        for (auto &b : S.old) b.release();
+        S.old.clear();
+        S.cap_rows = S.cap_ids = 0;
+    }
+    CK(cudaSetDevice(c->device));
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1299,7 +1494,14 @@ void nb200_destroy(nb200_ctx *c) {
         if (F.h2d_done) cudaEventDestroy(F.h2d_done);
         if (F.done) cudaEventDestroy(F.done);
         if (F.h_ctr) cudaFreeHost(F.h_ctr);
+        F.key.release(); F.seg.release();
+        if (F.h_seg) cudaFreeHost(F.h_seg);
     }
+    for (auto &S : c->rs) {
+        for (DevBuf *b : {&S.key, &S.nf, &S.ids, &S.hdr, &S.na}) b->release();
+        for (auto &b : S.old) b.release();
+    }
+    for (DevBuf *b : {&c->rs_val, &c->rs_pos, &c->rs_tmp, &c->rs_rank}) b->release();
     c->wls.clear();
     if (c->d_cbctr) cudaFree(c->d_cbctr);
     if (c->d_ctr) cudaFree(c->d_ctr);
@@ -1732,12 +1934,69 @@ int32_t nb200_align_files(nb200_ctx *c, const char *const *inputs, int32_t n_inp
 
 // The same pipeline over several GPUs of one node, in ONE process: libraries are loaded on every device (index
 // replicated), the reader deals slabs of reads to whichever GPU has a free lane, the writer restores input order
-// (SURVEY.md §8e: reads are independent up to the per-read TSV; the UMI stage that needs cell locality is `report`).
+// (SURVEY.md §8e: reads are independent up to the per-read TSV).  With counts outputs the rows of the UMI stage stay in
+// each device's row store and are gathered on the first device at the end (lane_rows_count).
+static int32_t files_multi(const int32_t *devices, int32_t n_devices, int32_t host_threads, const char *const *inputs, int32_t n_inputs,
+                           const char *const *library_json, int32_t n_libs, const char *strand_filter, int32_t k, const char *trim,
+                           const char *const *outputs, const char *const *counts_outputs, double umi_threshold, int32_t disable_thresholding,
+                           uint64_t *out3, char *err, size_t err_cap, double *stats4);
+
 int32_t nb200_align_files_multi(const int32_t *devices, int32_t n_devices, int32_t host_threads, const char *const *inputs, int32_t n_inputs,
                                 const char *const *library_json, int32_t n_libs, const char *strand_filter, int32_t k,
                                 const char *const *outputs, const char *trim, char *err, size_t err_cap, double *stats4) {
+    if (!outputs) { if (err && err_cap) snprintf(err, err_cap, "bad arguments"); return NB200_EINVAL; }
+    return files_multi(devices, n_devices, host_threads, inputs, n_inputs, library_json, n_libs, strand_filter, k, trim, outputs, nullptr,
+                       0.0, 0, nullptr, err, err_cap, stats4);
+}
+
+int32_t nb200_align_files_counts_multi(const int32_t *devices, int32_t n_devices, int32_t host_threads,
+                                       const char *const *inputs, int32_t n_inputs, const char *const *library_json,
+                                       int32_t n_libs, const char *strand_filter, int32_t k, const char *trim,
+                                       const char *const *per_read_outputs, const char *const *counts_outputs,
+                                       double umi_threshold, int32_t disable_thresholding,
+                                       uint64_t *out3, char *err, size_t err_cap, double *stats4) {
+    if (!counts_outputs) { if (err && err_cap) snprintf(err, err_cap, "bad arguments"); return NB200_EINVAL; }
+    return files_multi(devices, n_devices, host_threads, inputs, n_inputs, library_json, n_libs, strand_filter, k, trim, per_read_outputs,
+                       counts_outputs, umi_threshold, disable_thresholding, out3, err, err_cap, stats4);
+}
+
+int32_t nb200_align_files_counts(nb200_ctx *c, const char *const *inputs, int32_t n_inputs, const int32_t *lib_ids,
+                                 const char *const *per_read_outputs, const char *const *counts_outputs, int32_t n_libs,
+                                 double umi_threshold, int32_t disable_thresholding, uint64_t *out3) {
+    API_BEGIN(c)
+    if (!inputs || n_inputs < 1 || n_inputs > 2 || !lib_ids || !counts_outputs || n_libs < 1) throw std::runtime_error("bad arguments");
+    if (out3) for (int i = 0; i < 3 * n_libs; i++) out3[i] = 0;
+    try {
+        FileJob job;
+        for (int i = 0; i < n_inputs; i++) job.inputs.emplace_back(inputs[i]);
+        job.ctxs.push_back(c);
+        job.lib_ids.assign(lib_ids, lib_ids + n_libs);
+        for (int i = 0; i < n_libs; i++) {
+            get_lib(c, lib_ids[i]);
+            if (per_read_outputs) job.outputs.emplace_back(per_read_outputs[i]);
+            job.counts_outputs.emplace_back(counts_outputs[i]);
+        }
+        job.host_threads = c->host_threads;
+        job.umi_threshold = umi_threshold;
+        job.disable_thresholding = disable_thresholding;
+        FileStats st;
+        run_file_pipeline(job, &st);
+        if (out3) for (size_t i = 0; i < st.counts3.size(); i++) out3[i] = st.counts3[i];
+        if (getenv("NB200_TRACE"))
+            fprintf(stderr, "[nb200 trace] file pipeline (counts): %llu reads in %llu slabs, %.3f s (%.2f M reads/s), %d host threads\n",
+                    (unsigned long long)st.n_reads, (unsigned long long)st.n_slabs, st.seconds, st.n_reads / std::max(st.seconds, 1e-9) / 1e6, c->host_threads);
+    } catch (const IoError &e) { c->err = e.what(); return NB200_EIO; }
+    API_END(c)
+}
+
+static int32_t files_multi(const int32_t *devices, int32_t n_devices, int32_t host_threads, const char *const *inputs, int32_t n_inputs,
+                           const char *const *library_json, int32_t n_libs, const char *strand_filter, int32_t k, const char *trim,
+                           const char *const *outputs, const char *const *counts_outputs, double umi_threshold, int32_t disable_thresholding,
+                           uint64_t *out3, char *err, size_t err_cap, double *stats4) {
     auto fail = [&](int32_t rc, const std::string &w) { if (err && err_cap) { snprintf(err, err_cap, "%s", w.c_str()); } return rc; };
-    if (!devices || n_devices < 1 || !inputs || n_inputs < 1 || n_inputs > 2 || !library_json || n_libs < 1 || !outputs) return fail(NB200_EINVAL, "bad arguments");
+    if (!devices || n_devices < 1 || !inputs || n_inputs < 1 || n_inputs > 2 || !library_json || n_libs < 1 || (!outputs && !counts_outputs))
+        return fail(NB200_EINVAL, "bad arguments");
+    if (out3 && counts_outputs) for (int i = 0; i < 3 * n_libs; i++) out3[i] = 0;
     std::vector<std::pair<int, double>> trims;
     try { trims = parse_trim_arg(trim, (size_t)n_libs); } catch (const std::exception &e) { return fail(NB200_EINVAL, e.what()); }
     std::vector<nb200_ctx *> ctxs;
@@ -1772,13 +2031,20 @@ int32_t nb200_align_files_multi(const int32_t *devices, int32_t n_devices, int32
             for (int i = 0; i < n_inputs; i++) job.inputs.emplace_back(inputs[i]);
             job.ctxs = ctxs;
             job.lib_ids = ids;
-            for (int i = 0; i < n_libs; i++) job.outputs.emplace_back(outputs[i]);
+            for (int i = 0; i < n_libs; i++) {
+                if (outputs) job.outputs.emplace_back(outputs[i]);
+                if (counts_outputs) job.counts_outputs.emplace_back(counts_outputs[i]);
+            }
             job.host_threads = ctxs[0]->host_threads;
+            job.umi_threshold = umi_threshold;
+            job.disable_thresholding = disable_thresholding;
             FileStats st;
             run_file_pipeline(job, &st);
             if (stats4) { stats4[0] = (double)st.n_reads; stats4[1] = st.seconds; stats4[2] = (double)st.called; stats4[3] = (double)st.n_slabs; }
+            if (out3) for (size_t i = 0; i < st.counts3.size(); i++) out3[i] = st.counts3[i];
         } catch (const IoError &e) { rc = NB200_EIO; what = e.what(); }
         catch (const nb200::CudaError &e) { rc = NB200_ECUDA; what = e.what(); }
+        catch (const nb200::LimitError &e) { rc = NB200_ELIMIT; what = e.what(); }
         catch (const std::exception &e) { rc = NB200_EINVAL; what = e.what(); }
     }
     for (nb200_ctx *c : ctxs) nb200_destroy(c);

@@ -2,6 +2,7 @@
 // UMI stage (agg.cuh) -> counts TSV.  The arithmetic (merge, thresholding, intersection, counting)
 // runs on the GPU; this file only parses, interns strings and writes.
 #include "ingest.hpp"
+#include "pandas_na.hpp"
 
 #include <algorithm>
 #include <array>
@@ -17,14 +18,6 @@
 namespace nb200 {
 
 void slurp_maybe_gz(const std::string &path, std::string &out);   // ingest.cpp
-
-// what pandas.read_csv turns into NaN by default (check_df_from_input, __main__.py:219)
-static bool pandas_na(std::string_view v) {
-    static const char *na[] = {"", "#N/A", "#N/A N/A", "#NA", "-1.#IND", "-1.#QNAN", "-NaN", "-nan", "1.#IND", "1.#QNAN", "<NA>",
-                               "N/A", "NA", "NULL", "NaN", "None", "n/a", "nan", "null"};
-    for (const char *s : na) if (v == s) return true;
-    return false;
-}
 
 // strings -> dense ids in ascending byte order (pandas groupby order == output order of the counts TSV)
 static void intern_sorted(const std::vector<std::string_view> &vals, std::vector<uint32_t> &ids, std::vector<std::string> &uniq) {

@@ -3,6 +3,7 @@
 #pragma once
 #include <cstddef>
 #include <cstdint>
+#include <vector>
 
 #include "../../include/nimble_b200.h"
 
@@ -17,9 +18,12 @@ void lane_bind_thread(nb200_ctx *c);
 // Asynchronous; throws std::exception on error.
 // len1 / len2 (may be null): per library, the read lengths that library's kernels use instead of r1->len / r2->len
 // (--trim keeps a per-library prefix of every read; the packed records are shared).
+// out_res / out_feats may be null (counts only: no per-read results come back).
+// key (counts mode, after lane_rows_begin): per read cell << 32 | umi or NB200_NO_BARCODE, PINNED; it goes up with the
+// reads and every library's rows that count are appended to that library's row store on the device.
 void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_reads *r2, const int32_t *lib_ids, int n_libs,
                  nb200_read_result *const *out_res, int32_t *const *out_feats, uint16_t *const *len1 = nullptr,
-                 uint16_t *const *len2 = nullptr);
+                 uint16_t *const *len2 = nullptr, const uint64_t *key = nullptr);
 // --trim setting of a library (nb200_library_set_trim); false = none
 bool lane_trim(nb200_ctx *c, int32_t lib_id, int *target, double *strictness);
 // Block until the slab of this lane is done and its outputs are in the host buffers (re-runs it with a larger
@@ -32,5 +36,24 @@ int lane_host_threads(nb200_ctx *c);
 // page-lock / release an existing host range for every context of the process (cudaHostRegisterPortable); false = not pinned
 bool lane_pin(void *p, size_t bytes);
 void lane_unpin(void *p);
+
+// ---- counts mode: the rows of the UMI stage never leave the device --------------------------------------------
+// One row store per library and context: key u64, names per row u32, feature ids (CSR without offsets).  A slab
+// appends one segment per library behind its calling kernels; segments are gathered in slab order at the end.
+struct RowSeg {
+    uint64_t seq = 0;            // slab sequence number (per-read TSV order)
+    int ctx = 0;                 // index of the context in the call
+    uint64_t row0 = 0, rows = 0, id0 = 0, ids = 0;   // where the segment lies in that context's store
+    uint64_t called = 0;         // reads of the slab with a feature call (every read, not only rows that count)
+};
+// Empty the row stores of the libraries of this call and upload each library's "name is a pandas NA token" flags.
+void lane_rows_begin(nb200_ctx *c, const int32_t *lib_ids, int n_libs);
+// After lane_wait: the segment the lane's slab appended, per library (seq / ctx are the caller's to fill).
+void lane_rows_segments(nb200_ctx *c, int lane, RowSeg *out);
+// Gather the segments (in the order given) of library li from every context into ctxs[0], map the cell ids to ranks
+// (cell_rank[id], so that cell order is byte order), run the UMI stage.  *counts is the context's table as
+// nb200_umi_counts returns it; *rows = rows that reached the UMI stage.  Throws LimitError beyond 2^31 rows.
+void lane_rows_count(const std::vector<nb200_ctx *> &ctxs, int li, int32_t lib_id, const std::vector<RowSeg> &segs,
+                     const std::vector<uint32_t> &cell_rank, double threshold, int disable, nb200_counts *counts, uint64_t *rows);
 
 }  // namespace nb200

@@ -18,6 +18,7 @@
 #include <zlib.h>
 
 #include <algorithm>
+#include <array>
 #include <atomic>
 #include <chrono>
 #include <condition_variable>
@@ -29,11 +30,14 @@
 #include <memory>
 #include <mutex>
 #include <stdexcept>
+#include <string_view>
 #include <thread>
 #include <unordered_map>
 
 #include "fast_inflate.hpp"
 #include "ingest.hpp"
+#include "library.hpp"
+#include "pandas_na.hpp"
 #include "slab_api.hpp"
 #include "trim.hpp"
 
@@ -54,7 +58,7 @@ static bool ends_with_ci(const std::string &s, const char *suf) {
 // ---- shared failure state -------------------------------------------------------------------------
 static double g_wait_block = 0.0, g_wait_slab = 0.0;          // walker-thread waits of the last run (NB200_TRACE)
 static std::atomic<uint64_t> g_ns_inflate{0}, g_ns_parse{0}, g_ns_format{0};   // summed over the pool threads
-static std::atomic<uint64_t> g_ns_gpu_wait{0}, g_ns_gpu_submit{0}, g_ns_write{0};
+static std::atomic<uint64_t> g_ns_gpu_wait{0}, g_ns_gpu_submit{0}, g_ns_write{0}, g_ns_intern{0};
 static inline double now_s() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
 struct Abort {
@@ -471,7 +475,98 @@ struct Slab {
     std::vector<std::string> out;                                        // per library: rows (a gzip member for .gz)
     std::vector<std::unordered_map<std::string, uint64_t>> bulk;         // per library, untagged input: id list -> reads
     uint64_t bases1 = 0, bases2 = 0, called = 0;
+    uint64_t *key = nullptr;                                             // counts mode: cell << 32 | umi per read
+    uint64_t tagged = 0;                                                 // counts mode: reads with a CB or UB value
 };
+
+// ---- counts mode: CB / UB strings -> key = cell << 32 | umi -------------------------------------------------------
+// Cells: one dictionary for the call, shared by every context (ids agree across GPUs), ids in first-seen order; the
+// ranks by CB bytes are computed once at the end (lane_rows_count).  UMIs: only equality matters (report groups rows by
+// it, nimble/__main__.py:254-293): an ACGTN string of up to 13 bases is its bijective base-5 value (< 2^31, injective
+// across lengths, no dictionary), anything else is interned with bit 31 set.  A pool thread looks a CB up in a map of
+// its own first (CellCache) and takes a shard's lock only for the CB's first sight on that thread.
+class BarcodeDict {
+public:
+    BarcodeDict() { static std::atomic<uint64_t> calls{0}; gen_ = ++calls; }
+    uint64_t gen() const { return gen_; }        // tells the per-thread caches of one call from those of another
+    uint32_t cell(std::string_view s) { return get(cells_, n_cells_, s); }
+    uint32_t umi(std::string_view s) { return get(umis_, n_umis_, s) | 0x80000000u; }
+    std::vector<std::string> cell_names() const {                        // id -> CB
+        std::vector<std::string> v(n_cells_.load());
+        for (const Shard &S : cells_) for (const auto &kv : S.map) v[kv.second] = kv.first;
+        return v;
+    }
+private:
+    static constexpr size_t kShards = 64;
+    struct Shard { std::mutex m; std::unordered_map<std::string, uint32_t> map; };
+    static uint32_t get(Shard *sh, std::atomic<uint32_t> &ctr, std::string_view s) {
+        Shard &S = sh[std::hash<std::string_view>()(s) % kShards];
+        std::lock_guard<std::mutex> g(S.m);
+        std::string k(s);
+        auto it = S.map.find(k);
+        if (it != S.map.end()) return it->second;
+        const uint32_t id = ctr++;
+        if (id >= 0x7FFFFFFFu) throw LimitError("more than 2^31 distinct cell barcodes or UMIs");
+        S.map.emplace(std::move(k), id);
+        return id;
+    }
+    Shard cells_[kShards], umis_[kShards];
+    std::atomic<uint32_t> n_cells_{0}, n_umis_{0};
+    uint64_t gen_ = 0;
+};
+
+// CB -> cell id for one pool thread, kept across the slabs of a call: a slab holds most cells of a large sample once,
+// so a per-slab map sends nearly every read to the shared dictionary (its lock, a string copy); a thread's own map
+// stops doing so after its first slabs.  Bounded: beyond kMax cells the rest go to the shared dictionary.
+struct CellCache {
+    static constexpr size_t kMax = 1u << 18;
+    uint64_t gen = 0;
+    std::unordered_map<size_t, std::pair<uint32_t, std::string>> ids;      // hash of the CB -> (id, CB)
+};
+
+// bijective base 5 (A C G T N = 1..5) of an ACGTN string of 1..13 bases; false for anything else
+static inline bool umi_code(std::string_view s, uint32_t &x) {
+    static const auto digit = [] { std::array<uint8_t, 256> d{}; d['A'] = 1; d['C'] = 2; d['G'] = 3; d['T'] = 4; d['N'] = 5; return d; }();
+    if (s.size() > 13) return false;
+    x = 0;
+    for (char ch : s) {
+        const uint32_t d = digit[(unsigned char)ch];
+        if (!d) return false;
+        x = x * 5u + d;
+    }
+    return true;
+}
+
+// keys of a parsed slab (runs on the pool, inside the parse task): invalid barcodes (absent, empty, a pandas NA token:
+// `report` drops those rows, nimble/__main__.py:244-245) -> NB200_NO_BARCODE
+static void slab_keys(Slab &S, BarcodeDict &bc) {
+    const double t_in = now_s();
+    static thread_local CellCache cc;
+    if (cc.gen != bc.gen()) { cc.ids.clear(); cc.gen = bc.gen(); }
+    std::unordered_map<std::string_view, uint32_t> umis;
+    S.tagged = 0;
+    for (size_t i = 0; i < S.n; i++) {
+        const std::string_view cb(S.cb.ptr(i), S.cb.len(i)), ub(S.ub.ptr(i), S.ub.len(i));
+        S.tagged += !cb.empty() || !ub.empty();
+        if (pandas_na(cb) || pandas_na(ub)) { S.key[i] = NB200_NO_BARCODE; continue; }
+        const size_t h = std::hash<std::string_view>()(cb);
+        auto c = cc.ids.find(h);
+        uint32_t cid;
+        if (c != cc.ids.end() && c->second.second == cb) cid = c->second.first;
+        else {
+            cid = bc.cell(cb);
+            if (c == cc.ids.end() && cc.ids.size() < CellCache::kMax) cc.ids.emplace(h, std::make_pair(cid, std::string(cb)));
+        }
+        uint32_t u;
+        if (!umi_code(ub, u)) {
+            auto v = umis.find(ub);
+            if (v == umis.end()) v = umis.emplace(ub, bc.umi(ub)).first;
+            u = v->second;
+        }
+        S.key[i] = ((uint64_t)cid << 32) | u;
+    }
+    g_ns_intern += (uint64_t)((now_s() - t_in) * 1e9);
+}
 
 struct Entry {                                   // one read (pair) as the walker found it
     const char *a = nullptr, *b = nullptr;       // BAM: record bodies of mate 1 / mate 2; FASTQ: the two sequences
@@ -493,6 +588,7 @@ struct Task {
     size_t n_seg_records = 0, seg_bytes_of_last = 0;    // (bytes of the last run so far: the next record extends it when it starts right there)
     Slab *slab = nullptr;
     const std::vector<TrimTable> *trims = nullptr;   // per library (--trim), or nullptr
+    BarcodeDict *bc = nullptr;                   // counts mode
 };
 
 static inline uint32_t le32(const unsigned char *p) { return p[0] | (p[1] << 8) | (p[2] << 16) | ((uint32_t)p[3] << 24); }
@@ -689,6 +785,7 @@ static void parse_task(Task &t) {
             if (t.paired) { pack_ascii(e.b, e.lb, S.p2 + i * (size_t)s2, w2, s2); S.l2[i] = (uint16_t)e.lb; S.bases2 += e.lb; }
         }
     }
+    if (t.bc) slab_keys(S, *t.bc);
 }
 
 // ---- output ----------------------------------------------------------------------------------------------
@@ -787,6 +884,12 @@ struct Pipeline {
     std::thread committer;
     FileStats stats;
     bool dry = false;
+    bool per_read = true;                          // per-read TSVs are written
+    bool counts = false;                           // counts TSVs: keys per read, rows kept on the devices
+    BarcodeDict bc;
+    std::mutex seg_m;
+    std::vector<std::vector<RowSeg>> segs;         // counts mode, per library: the segments of every slab on every context
+    uint64_t tagged = 0;
 
     explicit Pipeline(const FileJob &j) : job(j) {}
 
@@ -798,10 +901,11 @@ struct Pipeline {
         const size_t n_libs = dry ? 0 : job.lib_ids.size();
         auto S = std::make_unique<Slab>();
         S->p1 = (uint8_t *)S->grab(kSlabSeqBytes + 256); S->l1 = (uint16_t *)S->grab(kSlabReads * 2 + 64);
-        for (size_t li = 0; li < n_libs; li++) {
+        for (size_t li = 0; li < (per_read ? n_libs : 0); li++) {       // (counts only: the per-read results stay on the device)
             S->res.push_back((nb200_read_result *)S->grab(kSlabReads * sizeof(nb200_read_result) + 64));
             S->feats.push_back((int32_t *)S->grab(kSlabReads * (size_t)libs[li].max_hits * 4 + 64));
         }
+        if (counts) S->key = (uint64_t *)S->grab(kSlabReads * 8 + 64);
         if (!trims.empty())
             for (size_t li = 0; li < n_libs; li++) S->lt1.push_back((uint16_t *)S->grab(kSlabReads * 2 + 64));
         S->out.resize(n_libs); S->bulk.resize(n_libs);
@@ -821,6 +925,7 @@ struct Pipeline {
         std::vector<int> g;
         if (!dry) for (const LibOut &lo : libs) g.push_back(lo.max_hits);
         g.push_back(trims.empty() ? 0 : 1);
+        g.push_back((per_read ? 1 : 0) | (counts ? 2 : 0));
         return g;
     }
     void start_pool(size_t count, nb200_ctx *bind) {
@@ -863,6 +968,7 @@ struct Pipeline {
     void after_parse(Slab *S) { if (dry) to_commit.push(S); else to_gpu.push(S); }
     // a slab with results: format every library's rows on the pool, then commit
     void after_gpu(Slab *S) {
+        if (!per_read) { to_commit.push(S); return; }
         auto left = std::make_shared<std::atomic<size_t>>(libs.size());
         for (size_t li = 0; li < libs.size(); li++)
             pool->push(Pool::FORMAT, [this, S, li, left] {
@@ -873,12 +979,23 @@ struct Pipeline {
             });
     }
 
-    void gpu_main(nb200_ctx *c) {
+    void gpu_main(nb200_ctx *c, int ctx_index) {
         Slab *fly[kFileLanes] = {nullptr, nullptr};
         try {
             lane_bind_thread(c);
             int lane = 0;                                   // next lane to fill; when both are busy it holds the older slab
-            auto finish = [&](int l) { const double t_in = now_s(); lane_wait(c, l); g_ns_gpu_wait += (uint64_t)((now_s() - t_in) * 1e9); Slab *S = fly[l]; fly[l] = nullptr; after_gpu(S); };
+            std::vector<RowSeg> sg(job.lib_ids.size());
+            auto finish = [&](int l) {
+                const double t_in = now_s(); lane_wait(c, l); g_ns_gpu_wait += (uint64_t)((now_s() - t_in) * 1e9);
+                Slab *S = fly[l]; fly[l] = nullptr;
+                if (counts) {                               // the segments this slab appended to the row stores
+                    lane_rows_segments(c, l, sg.data());
+                    std::lock_guard<std::mutex> g(seg_m);
+                    for (size_t li = 0; li < sg.size(); li++) { sg[li].seq = S->seq; sg[li].ctx = ctx_index; segs[li].push_back(sg[li]); }
+                    if (!per_read) S->called = sg[0].called;
+                }
+                after_gpu(S);
+            };
             for (;;) {
                 Slab *S = nullptr;
                 if (fly[0] || fly[1]) {
@@ -888,8 +1005,10 @@ struct Pipeline {
                 if (fly[lane]) finish(lane);
                 fly[lane] = S;
                 const double t_in = now_s();
-                lane_submit(c, lane, &S->r1, S->paired ? &S->r2 : nullptr, job.lib_ids.data(), (int)job.lib_ids.size(), S->res.data(), S->feats.data(),
-                            S->lt1.empty() ? nullptr : S->lt1.data(), (S->paired && !S->lt2.empty()) ? S->lt2.data() : nullptr);
+                lane_submit(c, lane, &S->r1, S->paired ? &S->r2 : nullptr, job.lib_ids.data(), (int)job.lib_ids.size(),
+                            S->res.empty() ? nullptr : S->res.data(), S->feats.empty() ? nullptr : S->feats.data(),
+                            S->lt1.empty() ? nullptr : S->lt1.data(), (S->paired && !S->lt2.empty()) ? S->lt2.data() : nullptr,
+                            counts ? S->key : nullptr);
                 g_ns_gpu_submit += (uint64_t)((now_s() - t_in) * 1e9);
                 lane ^= 1;
             }
@@ -930,7 +1049,7 @@ struct Pipeline {
                             if (T->has_tags) {
                                 const double t_in = now_s();
                                 struct Acc { double t; ~Acc() { g_ns_write += (uint64_t)((now_s() - t) * 1e9); } } acc{t_in};
-                                if (!T->out[li].empty() && fwrite(T->out[li].data(), 1, T->out[li].size(), lo.f) != T->out[li].size()) throw IoError("write failed: " + lo.tmp);
+                                if (lo.f && !T->out[li].empty() && fwrite(T->out[li].data(), 1, T->out[li].size(), lo.f) != T->out[li].size()) throw IoError("write failed: " + lo.tmp);
                             } else {
                                 for (auto &kv : T->bulk[li]) lo.bulk[kv.first] += kv.second;
                             }
@@ -938,6 +1057,7 @@ struct Pipeline {
                         }
                         stats.n_reads += T->n; stats.bases1 += T->bases1; stats.bases2 += T->bases2; stats.called += T->called;
                         stats.paired |= T->paired; stats.has_tags |= T->has_tags; stats.n_slabs++;
+                        tagged += T->tagged;
                         if (dry && !getenv("NB200_INGEST_NOSUM"))      // reader statistics (nb200_host_ingest_stats): same checksum as readset_checksum
                             for (size_t i = 0; i < T->n; i++) {
                                 mix(T->names.ptr(i), T->names.len(i));
@@ -968,6 +1088,7 @@ struct Pipeline {
         S->seq = issued++;
         t->slab = S;
         t->trims = trims.empty() ? nullptr : &trims;
+        t->bc = counts ? &bc : nullptr;
         pool->push(Pool::PARSE, [this, t] {
             const double t_in = now_s();
             try { parse_task(*t); } catch (...) { to_commit.push(t->slab); throw; }
@@ -1221,22 +1342,33 @@ namespace nb200 {
 
 void run_file_pipeline(const FileJob &job, FileStats *stats_out) {
     if (job.inputs.empty() || job.inputs.size() > 2) throw std::runtime_error("expected one or two --input files");
-    if (!job.ctxs.empty() && (job.lib_ids.empty() || job.lib_ids.size() != job.outputs.size())) throw std::runtime_error("bad arguments");
+    const bool counts = !job.counts_outputs.empty();
+    if (!job.ctxs.empty() && (job.lib_ids.empty() || (!job.outputs.empty() && job.lib_ids.size() != job.outputs.size()) ||
+                              (job.outputs.empty() && !counts) || (counts && job.counts_outputs.size() != job.lib_ids.size())))
+        throw std::runtime_error("bad arguments");
     const auto t0 = std::chrono::steady_clock::now();
     Pipeline P(job);
     P.dry = job.ctxs.empty();
+    P.counts = counts && !P.dry;
+    P.per_read = !job.outputs.empty();
     g_wait_block = g_wait_slab = 0.0;
-    g_ns_inflate = 0; g_ns_parse = 0; g_ns_format = 0; g_ns_gpu_wait = 0; g_ns_gpu_submit = 0; g_ns_write = 0;
-    double t_alloc = 0.0, t_walk = 0.0, t_drain = 0.0, t_finish = 0.0, t_free = 0.0;
+    g_ns_inflate = 0; g_ns_parse = 0; g_ns_format = 0; g_ns_gpu_wait = 0; g_ns_gpu_submit = 0; g_ns_write = 0; g_ns_intern = 0;
+    double t_alloc = 0.0, t_walk = 0.0, t_drain = 0.0, t_finish = 0.0, t_free = 0.0, t_counts = 0.0;
     const int T = std::max(1, job.host_threads);
     const bool bam = ends_with_ci(job.inputs[0], ".bam");
     if (bam && job.inputs.size() != 1) throw std::runtime_error("one BAM file expected");
+    if (P.counts && !bam)
+        throw std::runtime_error("counts need cell barcodes and UMIs (CB / UB tags of a BAM file); " + job.inputs[0] + " is FASTQ: write the per-read TSV instead");
+    if (P.counts) {                                    // (feature names the per-read TSV cannot carry fail here, before any work)
+        for (nb200_ctx *c : job.ctxs) lane_rows_begin(c, job.lib_ids.data(), (int)job.lib_ids.size());
+        P.segs.resize(job.lib_ids.size());
+    }
     // outputs
     for (size_t li = 0; li < (P.dry ? 0 : job.lib_ids.size()); li++) {
         LibOut lo;
         lo.lib_id = job.lib_ids[li];
         lo.max_hits = lane_max_hits(job.ctxs[0], lo.lib_id);
-        lo.path = job.outputs[li]; lo.tmp = lo.path + ".tmp";
+        if (P.per_read) { lo.path = job.outputs[li]; lo.tmp = lo.path + ".tmp"; }
         lo.gz = ends_with_ci(lo.path, ".gz");
         const uint32_t nf = lane_n_features(job.ctxs[0], lo.lib_id);
         lo.names.resize(nf);
@@ -1257,6 +1389,7 @@ void run_file_pipeline(const FileJob &job, FileStats *stats_out) {
         const size_t n_slabs = (P.dry ? 2 : 3 * job.ctxs.size()) + (size_t)std::min(T, 64) + 2;
         { const double ta = now_s(); P.start_pool(n_slabs, P.dry ? nullptr : job.ctxs[0]); t_alloc = now_s() - ta; }
         for (LibOut &lo : P.libs) {
+            if (!P.per_read) break;
             lo.f = fopen(lo.tmp.c_str(), "wb");
             if (!lo.f) throw IoError("cannot write " + lo.tmp);
             if (bam) {                                      // per-read TSV: the header leads (its own gzip member for .gz)
@@ -1266,7 +1399,7 @@ void run_file_pipeline(const FileJob &job, FileStats *stats_out) {
                 if (fwrite(w.data(), 1, w.size(), lo.f) != w.size()) throw IoError("write failed: " + lo.tmp);
             }
         }
-        for (nb200_ctx *c : job.ctxs) P.gpu_threads.emplace_back([&P, c] { P.gpu_main(c); });
+        for (size_t d = 0; d < job.ctxs.size(); d++) P.gpu_threads.emplace_back([&P, &job, d] { P.gpu_main(job.ctxs[d], (int)d); });
         P.committer = std::thread([&P] { P.commit_main(); });
         std::string walk_err; bool walk_io = false;
         const double tw = now_s();
@@ -1309,8 +1442,11 @@ void run_file_pipeline(const FileJob &job, FileStats *stats_out) {
             if (P.ab.io) throw IoError(P.ab.what);
             throw std::runtime_error(P.ab.what);
         }
+        if (P.counts && P.stats.n_reads && !P.tagged)
+            throw std::runtime_error("no read of " + job.inputs[0] + " carries a CB or UB tag: counts need cell barcodes and UMIs");
         // finish the files: per-read outputs are complete, bulk tables are written now
         for (LibOut &lo : P.libs) {
+            if (!lo.f) continue;
             if (!bam) {
                 // `features<TAB>count` for untagged input (nimble/parse.py:39-57), rows in ascending feature-string order
                 std::vector<std::pair<std::string, uint64_t>> rows;
@@ -1334,6 +1470,30 @@ void run_file_pipeline(const FileJob &job, FileStats *stats_out) {
             if (rename(lo.tmp.c_str(), lo.path.c_str()) != 0) throw IoError("cannot rename " + lo.tmp);
         }
         t_finish = now_s() - t_fin0;
+        if (P.counts) {
+            // counts TSVs (nimble/__main__.py:254-293): every library's rows gathered in slab order on the first context,
+            // cells ranked by CB bytes, the UMI stage on the device
+            const double tc = now_s();
+            std::vector<std::string> cell_names = P.bc.cell_names();
+            std::vector<uint32_t> order(cell_names.size()), rank(cell_names.size());
+            for (uint32_t i = 0; i < order.size(); i++) order[i] = i;
+            std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return cell_names[a] < cell_names[b]; });
+            std::vector<std::string> cells(cell_names.size());
+            for (uint32_t r = 0; r < order.size(); r++) { rank[order[r]] = r; cells[r] = std::move(cell_names[order[r]]); }
+            for (size_t li = 0; li < P.libs.size(); li++) {
+                std::vector<RowSeg> &sg = P.segs[li];
+                std::sort(sg.begin(), sg.end(), [](const RowSeg &a, const RowSeg &b) { return a.seq < b.seq; });
+                nb200_counts table{};
+                uint64_t rows = 0;
+                lane_rows_count(job.ctxs, (int)li, job.lib_ids[li], sg, rank, job.umi_threshold, job.disable_thresholding, &table, &rows);
+                std::vector<std::string> names(P.libs[li].names.size());
+                for (size_t f = 0; f < names.size(); f++) names[f].assign(P.libs[li].names[f].first, P.libs[li].names[f].second);
+                write_counts_tsv(job.counts_outputs[li], table.n_rows ? &table : nullptr, names, cells);
+                P.stats.counts3.push_back(rows); P.stats.counts3.push_back(table.n_rows); P.stats.counts3.push_back(table.dropped_empty);
+            }
+            lane_bind_thread(job.ctxs[0]);
+            t_counts = now_s() - tc;
+        }
         const double t_free0 = now_s();
         P.free_all();
         t_free = now_s() - t_free0;
@@ -1352,10 +1512,10 @@ void run_file_pipeline(const FileJob &job, FileStats *stats_out) {
     P.stats.seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
     if (getenv("NB200_TRACE"))
         fprintf(stderr, "[nb200 trace] pipeline: %.3f s total | slab pool %.3f | walker %.3f (waiting for blocks %.3f, for slabs %.3f) | drain %.3f | close+rename %.3f | free slabs %.3f | %llu slabs | "
-                        "pool thread-seconds: inflate %.3f parse %.3f format %.3f | gpu threads: submit %.3f wait %.3f | writer %.3f\n",
+                        "pool thread-seconds: inflate %.3f parse %.3f (barcode keys %.3f) format %.3f | gpu threads: submit %.3f wait %.3f | writer %.3f | counts %.3f\n",
                 P.stats.seconds, t_alloc, t_walk, g_wait_block, g_wait_slab, t_drain, t_finish, t_free, (unsigned long long)P.stats.n_slabs,
-                g_ns_inflate.load() * 1e-9, g_ns_parse.load() * 1e-9, g_ns_format.load() * 1e-9, g_ns_gpu_submit.load() * 1e-9,
-                g_ns_gpu_wait.load() * 1e-9, g_ns_write.load() * 1e-9);
+                g_ns_inflate.load() * 1e-9, g_ns_parse.load() * 1e-9, g_ns_intern.load() * 1e-9, g_ns_format.load() * 1e-9, g_ns_gpu_submit.load() * 1e-9,
+                g_ns_gpu_wait.load() * 1e-9, g_ns_write.load() * 1e-9, t_counts);
     if (stats_out) *stats_out = P.stats;
 }
 

@@ -16,13 +16,18 @@ struct FileJob {
     std::vector<std::string> inputs;      // one or two FASTQ(.gz), or one BAM
     std::vector<nb200_ctx *> ctxs;        // one context per GPU; empty = dry run (no device stage, reader statistics only)
     std::vector<int32_t> lib_ids;         // the same ids on every context (libraries loaded in the same order)
-    std::vector<std::string> outputs;     // one per library
+    std::vector<std::string> outputs;     // one per library (per-read TSV); empty in counts-only mode
     int host_threads = 1;
+    // counts mode (nb200_align_files_counts): one counts TSV per library, the UMI stage on the device
+    std::vector<std::string> counts_outputs;
+    double umi_threshold = 0.05;
+    int disable_thresholding = 0;
 };
 
 struct FileStats {
     uint64_t n_reads = 0, paired = 0, has_tags = 0, bases1 = 0, bases2 = 0, checksum = 0, n_slabs = 0, called = 0;
     double seconds = 0.0;
+    std::vector<uint64_t> counts3;        // counts mode: per library rows used, count rows written, UMIs dropped
 };
 
 // throws IoError / std::exception

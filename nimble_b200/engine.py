@@ -310,6 +310,19 @@ class Engine:
         outs = (ct.c_char_p * len(outputs))(*[os.fspath(p).encode() for p in outputs])
         self._ck(self.L.nb200_align_files(self.ctx, ins, len(inputs), ids, outs, len(libs)))
 
+    def align_files_counts(self, inputs, libs, counts_outputs, outputs=None, threshold=0.05, disable_thresholding=False):
+        """`align` + `report` in one pass (nb200_align_files_counts): BAM with CB/UB tags in, one counts TSV per library
+        out (outputs: per-read TSVs written in the same pass, or None).  Returns per library (rows used, count rows,
+        dropped UMIs), as report_file does."""
+        ins = (ct.c_char_p * len(inputs))(*[os.fspath(p).encode() for p in inputs])
+        ids = (ct.c_int32 * len(libs))(*[l.id for l in libs])
+        cnt = (ct.c_char_p * len(counts_outputs))(*[os.fspath(p).encode() for p in counts_outputs])
+        outs = (ct.c_char_p * len(outputs))(*[os.fspath(p).encode() for p in outputs]) if outputs else None
+        out3 = (ct.c_uint64 * (3 * len(libs)))()
+        self._ck(self.L.nb200_align_files_counts(self.ctx, ins, len(inputs), ids, outs, cnt, len(libs), float(threshold),
+                                                 int(bool(disable_thresholding)), out3))
+        return [(int(out3[3 * i]), int(out3[3 * i + 1]), int(out3[3 * i + 2])) for i in range(len(libs))]
+
     def report_file(self, in_tsv, out_tsv, threshold=0.05, disable_thresholding=False):
         """report() file to file (nb200_report_file).  Returns (rows used, count rows, dropped UMIs)."""
         out = (ct.c_uint64 * 3)()

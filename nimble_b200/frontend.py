@@ -331,65 +331,109 @@ def parse_trim(trim, n_libs):
     return out
 
 
-def align_multi_gpu(reference, output, input, num_cores, strand_filter, k, gpus, trim=""):
+def _per_library_paths(path, library_list):
+    """nimble/__main__.py:184-189: with several libraries, OUT + "." + library stem (append_path_string)."""
+    if path is None:
+        return None
+    return [append_path_string(path, "." + os.path.splitext(os.path.basename(l))[0] if len(library_list) > 1 else "")
+            for l in library_list]
+
+
+def _print_counts_summary(counts_paths, out3):
+    """What `report` prints after writing its counts TSV (nimble/__main__.py:279, write_empty_df)."""
+    for path, (used, _n_rows, dropped) in zip(counts_paths, out3):
+        if used == 0:
+            print("No data to parse from input file, writing empty output.")
+        else:
+            print(f"Dropped {dropped} UMIs due to empty intersections")
+        print("nimble_b200: wrote %s" % path)
+
+
+def align_multi_gpu(reference, output, input, num_cores, strand_filter, k, gpus, trim="", counts=None, threshold=0.05,
+                    disable_thresholding=False):
     """`align` over several GPUs of the node from this one process (nb200_align_files_multi): every library is loaded on
     every GPU, the reader deals slabs of reads to the GPUs, the writer restores input order (outputs byte-identical to a
-    one-GPU run).  gpus: a count (devices 0..N-1) or a list of device indices."""
+    one-GPU run).  gpus: a count (devices 0..N-1) or a list of device indices.  counts: the counts TSV path
+    (nb200_align_files_counts_multi; output may then be None)."""
     import ctypes as ct
     from . import _lib
     L = _lib.load()
     devs = list(range(int(gpus))) if isinstance(gpus, int) else [int(g) for g in gpus]
     library_list = reference.split(",")
-    outs = [append_path_string(output, "." + os.path.splitext(os.path.basename(l))[0] if len(library_list) > 1 else "")
-            for l in library_list]
+    outs = _per_library_paths(output, library_list)
+    cnts = _per_library_paths(counts, library_list)
     d = (ct.c_int32 * len(devs))(*devs)
     ins = (ct.c_char_p * len(input))(*[os.fspath(p).encode() for p in input])
     libs = (ct.c_char_p * len(library_list))(*[os.fspath(p).encode() for p in library_list])
-    out_c = (ct.c_char_p * len(outs))(*[os.fspath(p).encode() for p in outs])
+    out_c = (ct.c_char_p * len(outs))(*[os.fspath(p).encode() for p in outs]) if outs else None
     err = ct.create_string_buffer(1024)
     st = (ct.c_double * 4)()
-    rc = L.nb200_align_files_multi(d, len(devs), int(num_cores or 0), ins, len(input), libs, len(library_list), strand_filter.encode(), int(k),
-                                   out_c, (trim or "").encode(), err, len(err), st)
+    if cnts is None:
+        rc = L.nb200_align_files_multi(d, len(devs), int(num_cores or 0), ins, len(input), libs, len(library_list), strand_filter.encode(), int(k),
+                                       out_c, (trim or "").encode(), err, len(err), st)
+    else:
+        cnt_c = (ct.c_char_p * len(cnts))(*[os.fspath(p).encode() for p in cnts])
+        out3 = (ct.c_uint64 * (3 * len(cnts)))()
+        rc = L.nb200_align_files_counts_multi(d, len(devs), int(num_cores or 0), ins, len(input), libs, len(library_list), strand_filter.encode(),
+                                              int(k), (trim or "").encode(), out_c, cnt_c, float(threshold), int(bool(disable_thresholding)),
+                                              out3, err, len(err), st)
     if rc != 0:
         print("nimble_b200 aligner error: %s" % err.value.decode(errors="replace"), file=sys.stderr)
         return 2 if rc == -2 else 1
     print("nimble_b200: %d reads on %d GPUs in %.2f s (%.1f M reads/s), %d with a feature call" % (st[0], len(devs), st[1], st[0] / max(st[1], 1e-9) / 1e6, st[2]))
-    for o in outs:
+    for o in outs or []:
         print("nimble_b200: wrote %s" % o)
+    if cnts is not None:
+        _print_counts_summary(cnts, [tuple(out3[3 * i:3 * i + 3]) for i in range(len(cnts))])
     return 0
 
 
-def align(reference, output, input, num_cores, strand_filter, trim, tmpdir, k=20, engine=None, native=True, gpus=None):
+def align(reference, output, input, num_cores, strand_filter, trim, tmpdir, k=20, engine=None, native=True, gpus=None, counts=None,
+          threshold=0.05, disable_thresholding=False):
     """Drop-in for nimble/__main__.py:153-211.  Returns the aligner's return code (0 = success).
     gpus (extension; also $NB200_GPUS): a count or list of devices -> the streaming pipeline over all of them.
     One pass over the reads per library; OUT naming follows __main__.py:184-189.
     native=True (default) hands the files to nb200_align_files (multi-threaded native readers and TSV
     writer, what the `aligner` executable does); native=False keeps file parsing and TSV writing in Python
-    around the same GPU calls (the tests use it to cross-check the native file code)."""
+    around the same GPU calls (the tests use it to cross-check the native file code).
+    counts (extension): also write the counts TSV `report` would write from the per-read TSV (threshold /
+    disable_thresholding as for report), in the same pass, the rows kept on the GPU; output may then be None (no per-read
+    TSV).  Several libraries: one counts file per library, named like the outputs."""
     from .engine import Engine
     from ._lib import NimbleB200Error
     print("Aligning input data to the reference libraries")
     sys.stdout.flush()
+    if output is None and counts is None:
+        print("nimble_b200 aligner error: align needs --output, --counts or both", file=sys.stderr)
+        return 1
+    if counts is not None and not native:
+        print("nimble_b200 aligner error: counts are written by the native file pipeline only (native=True)", file=sys.stderr)
+        return 1
     if trim and not native:
         print("nimble_b200: --trim is applied by the native file pipeline only; ignored with native=False")
     if gpus is None and os.environ.get("NB200_GPUS"):
         gpus = int(os.environ["NB200_GPUS"])
     if gpus and engine is None and native and (not isinstance(gpus, int) or gpus > 1):
-        return align_multi_gpu(reference, output, list(input), num_cores, strand_filter, k, gpus, trim)
+        return align_multi_gpu(reference, output, list(input), num_cores, strand_filter, k, gpus, trim, counts, threshold, disable_thresholding)
     own = engine is None
     try:
         eng = engine or Engine(int(os.environ.get("LOCAL_RANK", 0)), int(num_cores or 0))
         if native:
             library_list = reference.split(",")
-            outs = [append_path_string(output, "." + os.path.splitext(os.path.basename(l))[0] if len(library_list) > 1 else "")
-                    for l in library_list]
+            outs = _per_library_paths(output, library_list)
+            cnts = _per_library_paths(counts, library_list)
             trims = parse_trim(trim, len(library_list))
             libs = [eng.load_library(l, strand_filter=strand_filter, k=k) for l in library_list]
             for lg, (t_len, t_strict) in zip(libs, trims):
                 lg.set_trim(t_len, t_strict)
-            eng.align_files(list(input), libs, outs)
-            for o in outs:
+            if cnts is None:
+                eng.align_files(list(input), libs, outs)
+            else:
+                out3 = eng.align_files_counts(list(input), libs, cnts, outs, threshold, disable_thresholding)
+            for o in outs or []:
                 print("nimble_b200: wrote %s" % o)
+            if cnts is not None:
+                _print_counts_summary(cnts, out3)
             if own:
                 eng.close()
             return 0

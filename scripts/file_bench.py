@@ -102,6 +102,46 @@ def write_bam_chunked(path, codes, n_reads, n_cells, chunk=4_000_000, seed=2, le
     return total + len(BGZF_EOF)
 
 
+def gpu_info():
+    """GPU name and power limit (read-only nvidia-smi query): part of every number this script prints."""
+    import subprocess
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True, text=True, timeout=30).stdout
+        first = out.strip().splitlines()[0].split(",")
+        return {"gpu_name": first[0].strip(), "gpu_power_limit": first[1].strip()}
+    except Exception as e:                      # noqa: BLE001 (recorded, not fatal)
+        return {"gpu_info_error": str(e)}
+
+
+def counts_bench(args, eng, kw, lib_path, bam, tsv, nbytes):
+    """Two-step route (align -> per-read TSV -> report) against the fused `align --counts` (counts only), alternating
+    them, two repetitions each; the counts files of the two routes must be byte-identical."""
+    import filecmp
+    two_counts, fused_counts = os.path.join(args.out_dir, "counts_two_step.tsv"), os.path.join(args.out_dir, "counts_fused.tsv")
+    frontend.align(lib_path, tsv, [bam], args.cores, "unstranded", "", None, **kw)            # warm-up (CUDA context, page cache)
+    frontend.align(lib_path, None, [bam], args.cores, "unstranded", "", None, counts=fused_counts, **kw)
+    out = {"workload": args.workload, "reads": args.reads, "gpus": args.gpus, "host_threads": args.cores or os.cpu_count(),
+           "bam_mb": nbytes / 1e6, "two_step_align_s": [], "two_step_report_s": [], "two_step_s": [], "fused_s": [], "rc": []}
+    out.update(gpu_info())
+    for _rep in range(2):
+        os.remove(tsv)
+        t0 = time.perf_counter()
+        rc1 = frontend.align(lib_path, tsv, [bam], args.cores, "unstranded", "", None, **kw)
+        t1 = time.perf_counter()
+        frontend.report(tsv, two_counts, None, 0.05, False, engine=eng)
+        t2 = time.perf_counter()
+        rc2 = frontend.align(lib_path, None, [bam], args.cores, "unstranded", "", None, counts=fused_counts, **kw)
+        t3 = time.perf_counter()
+        out["two_step_align_s"].append(t1 - t0); out["two_step_report_s"].append(t2 - t1); out["two_step_s"].append(t2 - t0)
+        out["fused_s"].append(t3 - t2); out["rc"] += [rc1, rc2]
+    out["counts_identical"] = filecmp.cmp(two_counts, fused_counts, shallow=False)
+    out["count_rows"] = sum(1 for _ in open(fused_counts))
+    out["fused_reads_per_s"] = args.reads / min(out["fused_s"])
+    print(json.dumps(out))
+    if not out["counts_identical"] or any(out["rc"]):
+        sys.exit(4)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reads", type=int, default=2_000_000)
@@ -113,6 +153,8 @@ def main():
     ap.add_argument("--skip-report", action="store_true")
     ap.add_argument("--rss", action="store_true", help="run the `aligner` executable as a child process on the same input and report its peak RSS "
                                                        "(the streaming pipeline holds a fixed pool of slabs, not the file)")
+    ap.add_argument("--counts", action="store_true", help="time the two-step route (align + report) against the fused `align --counts`, "
+                                                          "alternating, two repetitions each, and compare the counts files")
     args = ap.parse_args()
     os.makedirs(args.out_dir, exist_ok=True)
     if args.workload == "cfg4":
@@ -125,13 +167,26 @@ def main():
     with open(lib_path, "w") as f:
         json.dump(lib, f)
     bam = os.path.join(args.out_dir, "in.bam")
+    made = {"workload": args.workload, "reads": args.reads}
+    try:                                    # the same input as an earlier run into this directory: not written again
+        reuse = json.load(open(bam + ".json")) == made and os.path.exists(bam)
+    except (OSError, ValueError):
+        reuse = False
     t0 = time.time()
-    nbytes = write_bam_chunked(bam, codes, args.reads, n_cells)
-    print("wrote %s: %d reads, %.0f MB in %.1fs" % (bam, args.reads, nbytes / 1e6, time.time() - t0), file=sys.stderr)
+    if reuse:
+        nbytes = os.path.getsize(bam)
+    else:
+        nbytes = write_bam_chunked(bam, codes, args.reads, n_cells)
+        with open(bam + ".json", "w") as f:
+            json.dump(made, f)
+    print("%s %s: %d reads, %.0f MB in %.1fs" % ("reused" if reuse else "wrote", bam, args.reads, nbytes / 1e6, time.time() - t0), file=sys.stderr)
     from nimble_b200.engine import Engine
     eng = Engine(0, args.cores)
     tsv = os.path.join(args.out_dir, "out.tsv")
     kw = {"engine": eng} if args.gpus <= 1 else {"gpus": args.gpus}
+    if args.counts:
+        counts_bench(args, eng, kw, lib_path, bam, tsv, nbytes)
+        return
     frontend.align(lib_path, tsv, [bam], args.cores, "unstranded", "", None, **kw)          # warm-up (CUDA context, page cache)
     os.remove(tsv)                          # the timed run writes a fresh file (replacing a GB-sized one costs 0.2-0.4 s of unlink alone)
     t0 = time.perf_counter()
