@@ -324,6 +324,28 @@ int32_t nb200_align_10x_fastq(nb200_ctx *ctx, const char *r1_fastq, const char *
                               int32_t cb_len, int32_t umi_len, const int32_t *lib_ids, const char *const *outputs,
                               int32_t n_libs, nb200_cb_stats *stats);
 
+/* fastq-to-bam followed by align --counts (nb200_align_files_counts) on its BAM, in one streaming pass and without the
+ * BAM: raw 10x R1 / R2 FASTQ(.gz) + whitelist in, one counts TSV per library out, byte-identical to the two steps.  Pairs
+ * are zipped in file order and stop at the shorter file; process_pair's rules pick the pairs that reach the correction;
+ * each slab's barcodes are corrected on the device, and the first read (in file order) with a raw barcode that has
+ * several candidates decides for every later read with it, across slabs and devices.  Memory is bounded by the slab pool.
+ * --trim (nb200_library_set_trim) sees the qualities the BAM would hold.  out3 as nb200_align_files_counts; stats (may be
+ * NULL): nb200_fastq_to_bam's counters, summed per slab; cache_size is not computed by this route and is 0.  It fails
+ * where the two steps fail: a pair whose barcode is corrected (so fastq-to-bam writes it) with a read over 500 bases after
+ * the barcode and UMI are cut off, or with a name over 254 bytes. */
+int32_t nb200_fastq_to_counts(nb200_ctx *ctx, const char *r1_fastq, const char *r2_fastq, const char *whitelist_path,
+                              int32_t cb_len, int32_t umi_len, const int32_t *lib_ids, const char *const *counts_outputs,
+                              int32_t n_libs, double umi_threshold, int32_t disable_thresholding, uint64_t *out3,
+                              nb200_cb_stats *stats);
+/* The same over several GPUs, as nb200_align_files_counts_multi (devices may repeat an index); byte-identical to a
+ * one-GPU run. */
+int32_t nb200_fastq_to_counts_multi(const int32_t *devices, int32_t n_devices, int32_t host_threads, const char *r1_fastq,
+                                    const char *r2_fastq, const char *whitelist_path, int32_t cb_len, int32_t umi_len,
+                                    const char *const *library_json, int32_t n_libs, const char *strand_filter, int32_t k,
+                                    const char *trim, const char *const *counts_outputs, double umi_threshold,
+                                    int32_t disable_thresholding, uint64_t *out3, nb200_cb_stats *stats, char *err, size_t err_cap,
+                                    double *stats4);
+
 int32_t nb200_last_timing(const nb200_ctx *ctx, nb200_timing *out);
 /* Batch pipelining (default on): batch k's fingerprint / Smith-Waterman / deferred-call kernels run on a
  * high-priority stream beside batch k+1's probe kernel.  Off = one stream, kernels back to back: the stage

@@ -1,12 +1,12 @@
 """`python -m nimble_b200 <subcommand>` — same sub-commands and flags as `python -m nimble`
 (nimble/__main__.py:373-468) for the hot path: generate, align, report.  `download` reports that
 the aligner is built in; `fastq-to-bam` (nimble/__main__.py:424-431) runs its barcode correction on
-the GPU; `plot` is outside the hot path (DESIGN.md §7)."""
+the GPU; `fastq-to-counts` (an extension) runs fastq-to-bam and align --counts in one pass; `plot` is outside the hot path (DESIGN.md §7)."""
 import argparse
 import sys
 
 from . import __version__
-from .frontend import align, align_10x, fastq_to_bam_with_barcodes, generate, report
+from .frontend import align, align_10x, fastq_to_bam_with_barcodes, fastq_to_counts, generate, report
 
 
 def main(argv=None):
@@ -61,6 +61,24 @@ def main(argv=None):
     f.add_argument("--cb-length", help="Length of cell barcode (default: 16).", type=int, default=16)
     f.add_argument("--umi-length", help="Length of UMI (default: 12).", type=int, default=12)
 
+    fc = sub.add_parser("fastq-to-counts", help="(extension) fastq-to-bam, then align --counts on its BAM, in one pass without the BAM")
+    fc.add_argument("--reference", help="The reference library (comma-separated for several).", type=str, required=True)
+    fc.add_argument("--r1-fastq", help="Path to R1 FASTQ file.", type=str, required=True)
+    fc.add_argument("--r2-fastq", help="Path to R2 FASTQ file.", type=str, required=True)
+    fc.add_argument("--map", required=True, help="Cell barcode whitelist file (one CB per line, .gz or plain text)")
+    fc.add_argument("--counts", help="Path of the counts TSV (one per library, named as align names its outputs).", type=str, required=True)
+    fc.add_argument("-c", "--num_cores", help="The number of host threads to use.", type=int, default=1)
+    fc.add_argument("--strand_filter", help="Filter reads based on strand information.", type=str, default="unstranded")
+    fc.add_argument("--trim", help="<TARGET_LENGTH>:<STRICTNESS>, comma-separated, one entry per library", type=str, default="")
+    fc.add_argument("-k", "--kmer", help="k-mer length of the index (4..32)", type=int, default=20)
+    fc.add_argument("--gpus", help="GPUs of this node to spread the reads over (default 1; also $NB200_GPUS)", type=int, default=None)
+    fc.add_argument("--cb-length", help="Length of cell barcode (default: 16).", type=int, default=16)
+    fc.add_argument("--umi-length", help="Length of UMI (default: 12).", type=int, default=12)
+    fc.add_argument("--threshold", help="Proportional count threshold for filtering features (default: 0.05), as for report",
+                    type=float, default=0.05)
+    fc.add_argument("--disable_thresholding", help="Disable the per-UMI proportional count thresholding algorithm.",
+                    action="store_true", default=False)
+
     pl = sub.add_parser("plot")          # visualisation: outside the hot path (DESIGN.md §7); flags accepted so scripts fail clearly
     pl.add_argument("--input_file", "-i", type=str, required=False)
     pl.add_argument("--output_file", "-o", type=str, required=False)
@@ -96,6 +114,10 @@ def main(argv=None):
     elif args.subcommand == "fastq-to-bam":
         fastq_to_bam_with_barcodes(args.r1_fastq, args.r2_fastq, args.map, args.output, args.num_cores,
                                    args.cb_length, args.umi_length)
+    elif args.subcommand == "fastq-to-counts":
+        sys.exit(fastq_to_counts(args.reference, args.r1_fastq, args.r2_fastq, args.map, args.counts, args.num_cores, args.strand_filter,
+                                 args.trim, k=args.kmer, gpus=args.gpus, cb_length=args.cb_length, umi_length=args.umi_length,
+                                 threshold=args.threshold, disable_thresholding=args.disable_thresholding))
     else:
         parser.print_help()
 

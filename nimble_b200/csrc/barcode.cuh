@@ -258,6 +258,65 @@ __global__ void cb_propagate_kernel(const uint32_t *__restrict__ sorted_idx, con
     const uint32_t h = head[t];
     if (h != t) out_idx[sorted_idx[t]] = out_idx[sorted_idx[h]];      // heads are never written: no race
 }
+
+// ---- fastq-to-counts (nb200_fastq_to_counts): one slab at a time, the cache rule over the whole call ----------------
+// Per read of a slab: key = cell << 32 | umi.  On entry key holds the host's flags << 32 | umi (umi 0xFFFFFFFF for a
+// pandas NA UMI; flags: slab_api.hpp kTenx*, a pair the two-step route refuses once it is written).  The flags of a read
+// whose barcode is corrected (= written by fastq-to-bam) are or-ed into ctr->pad, which makes the host fail the call.
+// cell = whitelist line for exact matches and single-candidate corrections (every read with that raw barcode gets the
+// same answer).  A read with several candidates gets a provisional cell, bit 31 | its entry in the context's log, and is
+// logged with its raw barcode, its file order and its own choice: lane_cb_resolve lets the first logged read of a raw
+// barcode in file order decide for all of them.  Logged whatever its UMI: an uncounted read can still be the first.
+__global__ void __launch_bounds__(256)
+cb_key_kernel(uint32_t n, const uint8_t *__restrict__ status, const int32_t *__restrict__ idx, const uint8_t *__restrict__ multi,
+              const uint64_t *__restrict__ raw, uint64_t order0, uint64_t *__restrict__ key, unsigned long long *__restrict__ log_n,
+              uint64_t *__restrict__ log_key, uint64_t *__restrict__ log_order, int32_t *__restrict__ log_choice,
+              CbCounters *__restrict__ ctr) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint8_t st = status[i];
+    uint64_t k = NB200_NO_BARCODE;
+    if (st == NB200_CB_PERFECT || st == NB200_CB_CORRECTED) {
+        uint32_t cell = (uint32_t)idx[i];
+        if (multi[i]) {
+            const unsigned long long e = atomicAdd(log_n, 1ull);      // (rare: a few per cent of the reads at most)
+            log_key[e] = raw[i];
+            log_order[e] = order0 + i;
+            log_choice[e] = idx[i];
+            cell = 0x80000000u | (uint32_t)e;                         // (lane_cb_resolve refuses logs of 2^31 entries)
+        }
+        const uint64_t u = key[i];
+        if ((uint32_t)u != 0xFFFFFFFFu) k = ((uint64_t)cell << 32) | (u & 0xFFFFFFFFull);
+        if (u >> 32) atomicOr(&ctr->pad, (unsigned long long)(u >> 32));     // (rare)
+    }
+    key[i] = k;
+}
+
+// Gathered rows -> cell = rank of its whitelist line in byte order.  A provisional cell goes through decision[] first:
+// rows [run_row[r], run_row[r + 1]) came from the log whose entries start at run_base[r] there.  A line that is a pandas
+// NA token has rank ~0u: the row becomes NB200_NO_BARCODE (the UMI stage skips it) and is counted in *dropped.
+__global__ void __launch_bounds__(256)
+cb_remap_kernel(uint64_t n, uint64_t *__restrict__ key, const uint32_t *__restrict__ rank, const int32_t *__restrict__ decision,
+                const uint64_t *__restrict__ run_row, const uint64_t *__restrict__ run_base, uint32_t n_runs,
+                unsigned long long *__restrict__ dropped) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    bool drop = false;
+    if (i < n) {
+        const uint64_t k = key[i];
+        uint32_t cell = (uint32_t)(k >> 32);
+        if (cell & 0x80000000u) {
+            uint32_t lo = 0, hi = n_runs;                              // last run with run_row[r] <= i
+            while (hi - lo > 1) { const uint32_t m = (lo + hi) >> 1; if (run_row[m] <= i) lo = m; else hi = m; }
+            cell = (uint32_t)decision[run_base[lo] + (cell & 0x7FFFFFFFu)];
+        }
+        const uint32_t r = rank[cell];
+        drop = r == 0xFFFFFFFFu;
+        key[i] = drop ? NB200_NO_BARCODE : (((uint64_t)r << 32) | (k & 0xFFFFFFFFull));
+    }
+    const unsigned b = __ballot_sync(0xFFFFFFFFu, drop);
+    if ((threadIdx.x & 31) == 0 && b) atomicAdd(dropped, (unsigned long long)__popc(b));
+}
+
 __global__ void cb_count_flags_kernel(const uint8_t *__restrict__ flag, uint64_t n, unsigned long long *__restrict__ out) {
     const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const unsigned b = __ballot_sync(0xFFFFFFFFu, t < n && flag[t]);

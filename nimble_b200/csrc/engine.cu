@@ -118,7 +118,20 @@ struct nb200_ctx {
         size_t h_seg_cap = 0;
         const uint64_t *hkey = nullptr;           // what was submitted (an overflow re-runs it)
         uint64_t n_rows_max = 0;                  // reads of the slab in flight: bound on the rows it appends
+        // fastq-to-counts: the slab's barcodes and their correction (cb_*: device; h_cb: pinned CbCounters + log end)
+        DevBuf cb, cbq, cb_raw, cb_idx, cb_st, cb_miss, cb_multi, cb_ctr;
+        const uint8_t *hcb = nullptr, *hcbq = nullptr;   // what was submitted (an overflow re-runs it)
+        uint64_t seq = 0;
+        unsigned long long *h_cb = nullptr;
     } lane[kFileLanes];
+    // fastq-to-counts (lane_cb_*): the whitelist table, and the log of reads with several candidates (raw barcode, file
+    // order, own choice; tx_n = entries, device-side).  The log grows like the row stores: tx_hi = its end as of the
+    // last slab the host has seen.  tx_dec (first context, lane_cb_resolve): the decision per entry of every log.
+    DevBuf tx_table, tx_key, tx_ord, tx_choice, tx_n, tx_dec;
+    WlDev tx_wl{};
+    uint64_t tx_cap = 0, tx_hi = 0;
+    std::vector<DevBuf> tx_old;
+    std::vector<uint64_t> tx_base;                // first context: where each context's log starts in tx_dec
     // counts mode (slab_api.hpp): per library of the call, the rows that count, appended slab by slab on s_copy[1]
     struct RowStore {
         DevBuf key, nf, ids, hdr, na;             // hdr: rows / ids used (device); na: per feature, name is a pandas NA token
@@ -946,12 +959,90 @@ static void append_rows(nb200_ctx *c, nb200_ctx::FileLane &F, int li, uint64_t n
     c->launches += 4;
 }
 
+// ---- cell-barcode correction shared by the whole-batch path (cb_run) and the slabs of fastq-to-counts ---------------
+struct MaxU32 {
+    __host__ __device__ __forceinline__ uint32_t operator()(uint32_t a, uint32_t b) const { return a > b ? a : b; }
+};
+
+// Phases 1 and 2 (barcode.cuh) over n barcodes on stream s: counters and multi-candidate flags are zeroed first; the
+// miss count stays on the device.  inval may be null (inval_cap 0), hit and elig too.
+static void cb_launch(nb200_ctx *c, const WlDev &W, cudaStream_t s, const uint8_t *chars, const uint8_t *qual, const uint8_t *elig,
+                      uint64_t n, uint64_t *keys, int32_t *idx, uint8_t *status, uint32_t *miss, uint32_t *inval, uint32_t inval_cap,
+                      uint8_t *hit, uint8_t *multi, CbCounters *ctr) {
+    CK(cudaMemsetAsync(ctr, 0, sizeof(CbCounters), s));
+    CK(cudaMemsetAsync(multi, 0, n + 16, s));
+    if (!n) return;
+    cb_exact_kernel<<<nblk(n, 256), 256, 0, s>>>(W, chars, elig, n, keys, idx, status, miss, inval, inval_cap, hit, ctr);
+    cb_hamming_kernel<<<c->sm_count * 8, 128, 0, s>>>(W, qual, keys, miss, idx, status, multi, ctr);
+    CK(cudaGetLastError());
+    c->launches += 2;
+}
+
+// Phase 3, the reference's correction_cache: list = m reads with several candidates in file order (indices into keys /
+// out_idx); afterwards each of them carries the choice of the first one with its raw barcode.  On s_compute.
+static void cb_first_decides(nb200_ctx *c, const uint32_t *list, const uint64_t *keys, uint32_t m, int32_t *out_idx) {
+    cudaStream_t s = c->s_compute;
+    c->k64A.ensure((size_t)m * 8 + 16); c->k64B.ensure((size_t)m * 8 + 16);
+    c->k32A.ensure((size_t)m * 4 + 16); c->k32B.ensure((size_t)m * 4 + 16); c->head.ensure((size_t)m * 4 + 16);
+    cb_gather_keys_kernel<<<nblk(m, 256), 256, 0, s>>>(list, keys, m, c->k64A.as<uint64_t>());
+    cub_sort64(c, c->k64A.as<uint64_t>(), c->k64B.as<uint64_t>(), list, c->k32A.as<uint32_t>(), m, 64);   // stable
+    cb_run_heads_kernel<<<nblk(m, 256), 256, 0, s>>>(c->k64B.as<uint64_t>(), m, c->k32B.as<uint32_t>());
+    size_t bytes = 0;
+    CK(cub::DeviceScan::InclusiveScan(nullptr, bytes, c->k32B.as<uint32_t>(), c->head.as<uint32_t>(), MaxU32(), (int)m, s));
+    c->cub_tmp.ensure(bytes);
+    CK(cub::DeviceScan::InclusiveScan(c->cub_tmp.p, bytes, c->k32B.as<uint32_t>(), c->head.as<uint32_t>(), MaxU32(), (int)m, s));
+    cb_propagate_kernel<<<nblk(m, 256), 256, 0, s>>>(c->k32A.as<uint32_t>(), c->head.as<uint32_t>(), m, out_idx);
+    CK(cudaGetLastError());
+    c->launches += 8;
+}
+
+// fastq-to-counts, per slab (inside lane_submit, on s_compute behind the slab's uploads): correct the barcodes, turn the
+// host's UMI keys into cell << 32 | umi, log the reads with several candidates.  No host synchronise: the log's capacity
+// is bounded on the host (its end as of the last slab seen plus the reads of the slabs in flight).
+static void lane_cb_slab(nb200_ctx *c, nb200_ctx::FileLane &F, uint64_t n) {
+    cudaStream_t s = c->s_compute;
+    uint64_t other = 0;
+    for (auto &G : c->lane) if (&G != &F && G.busy && G.hcb) other += G.n_rows_max;
+    const uint64_t need = c->tx_hi + other + n;
+    if (need > c->tx_cap) {                          // grow: copy on s_compute (every log write is on it), free at the end
+        const uint64_t cap = std::max(need, 2 * c->tx_cap);
+        DevBuf k, o, ch;
+        k.ensure(cap * 8); o.ensure(cap * 8); ch.ensure(cap * 4);
+        const uint64_t keep = std::min(c->tx_hi + other, c->tx_cap);
+        if (keep) {
+            CK(cudaMemcpyAsync(k.p, c->tx_key.p, keep * 8, cudaMemcpyDeviceToDevice, s));
+            CK(cudaMemcpyAsync(o.p, c->tx_ord.p, keep * 8, cudaMemcpyDeviceToDevice, s));
+            CK(cudaMemcpyAsync(ch.p, c->tx_choice.p, keep * 4, cudaMemcpyDeviceToDevice, s));
+        }
+        for (DevBuf *b : {&c->tx_key, &c->tx_ord, &c->tx_choice}) if (b->p) c->tx_old.push_back(*b);
+        c->tx_key = k; c->tx_ord = o; c->tx_choice = ch;
+        c->tx_cap = cap;
+    }
+    const uint64_t nb = std::max<uint64_t>(n, 1);
+    F.cb_raw.ensure(nb * 8); F.cb_idx.ensure(nb * 4); F.cb_st.ensure(nb); F.cb_miss.ensure(nb * 4); F.cb_multi.ensure(nb + 16);
+    F.cb_ctr.ensure(sizeof(CbCounters));
+    CbCounters *ctr = F.cb_ctr.as<CbCounters>();
+    cb_launch(c, c->tx_wl, s, F.cb.as<uint8_t>(), F.cbq.as<uint8_t>(), nullptr, n, F.cb_raw.as<uint64_t>(), F.cb_idx.as<int32_t>(),
+              F.cb_st.as<uint8_t>(), F.cb_miss.as<uint32_t>(), nullptr, 0, nullptr, F.cb_multi.as<uint8_t>(), ctr);
+    if (n) {
+        cb_key_kernel<<<nblk(n, 256), 256, 0, s>>>((uint32_t)n, F.cb_st.as<uint8_t>(), F.cb_idx.as<int32_t>(), F.cb_multi.as<uint8_t>(),
+                                                   F.cb_raw.as<uint64_t>(), F.seq << 21, F.key.as<uint64_t>(), c->tx_n.as<unsigned long long>(),
+                                                   c->tx_key.as<uint64_t>(), c->tx_ord.as<uint64_t>(), c->tx_choice.as<int32_t>(), ctr);
+        CK(cudaGetLastError());
+        c->launches++;
+    }
+    // (read after lane_wait: the lane's done event follows these copies through s_compute's tail)
+    CK(cudaMemcpyAsync(F.h_cb, ctr, sizeof(CbCounters), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(F.h_cb + 8, c->tx_n.p, 8, cudaMemcpyDeviceToHost, s));
+}
+
 void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_reads *r2, const int32_t *lib_ids, int n_libs,
                  nb200_read_result *const *out_res, int32_t *const *out_feats, uint16_t *const *len1, uint16_t *const *len2,
-                 const uint64_t *key) {
+                 const uint64_t *key, const uint8_t *cb, const uint8_t *cb_qual, uint64_t seq) {
     nb200_ctx::FileLane &F = c->lane[lane];
     if (F.busy) throw std::runtime_error("lane is busy");
     if (key && c->rs.size() < (size_t)n_libs) throw std::runtime_error("counts mode without lane_rows_begin");
+    if (cb && (!key || !cb_qual || !c->tx_table.p)) throw std::runtime_error("barcodes without lane_cb_begin");
     validate_reads(r1, "r1");
     if (r2) { validate_reads(r2, "r2"); if (r2->n != r1->n) throw std::runtime_error("r1 and r2 differ in read count"); }
     const uint64_t n = r1->n;
@@ -969,6 +1060,8 @@ void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_read
     if (out_res) F.out_res.assign(out_res, out_res + n_libs);
     if (out_feats) F.out_feats.assign(out_feats, out_feats + n_libs);
     F.hkey = key; F.n_rows_max = key ? n : 0;
+    F.hcb = cb; F.hcbq = cb_qual; F.seq = seq;
+    if (cb && !F.h_cb) CK(cudaMallocHost(&F.h_cb, 9 * 8));
     if (key && (size_t)n_libs > F.h_seg_cap) {
         if (F.h_seg) cudaFreeHost(F.h_seg);
         F.h_seg = nullptr; F.h_seg_cap = 0;
@@ -1002,6 +1095,14 @@ void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_read
         F.key.ensure(n * 8 + 16); F.seg.ensure(5 * 8 * (size_t)n_libs);
         if (n) CK(cudaMemcpyAsync(F.key.p, key, n * 8, cudaMemcpyHostToDevice, sh));
     }
+    if (cb) {
+        const size_t L = (size_t)c->tx_wl.cb_len;
+        F.cb.ensure(n * L + 16); F.cbq.ensure(n * L + 16);
+        if (n) {
+            CK(cudaMemcpyAsync(F.cb.p, cb, n * L, cudaMemcpyHostToDevice, sh));
+            CK(cudaMemcpyAsync(F.cbq.p, cb_qual, n * L, cudaMemcpyHostToDevice, sh));
+        }
+    }
     if (len1 && n) {      // per-library lengths: all up before the first kernel
         F.l1v.resize(std::max<size_t>(F.l1v.size(), (size_t)n_libs)); F.l2v.resize(F.l1v.size());
         for (int li = 0; li < n_libs; li++) {
@@ -1012,6 +1113,7 @@ void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_read
     }
     CK(cudaEventRecord(F.h2d_done, sh));
     CK(cudaStreamWaitEvent(c->s_compute, F.h2d_done, 0));
+    if (cb) lane_cb_slab(c, F, n);                  // the keys are final before any library's rows are appended
     nb200_ctx::BatchBuf &B = c->bb[lane];
     const uint64_t nbmax = std::max<uint64_t>(n, 1);
     B.ro.ensure(nbmax * n_ro * sizeof(RoRec));
@@ -1077,6 +1179,13 @@ void lane_wait(nb200_ctx *c, int lane) {
                 S.hi_rows = std::max<uint64_t>(S.hi_rows, s[0] + s[1]);
                 S.hi_ids = std::max<uint64_t>(S.hi_ids, s[2] + s[3]);
             }
+        if (F.hcb) {
+            c->tx_hi = std::max<uint64_t>(c->tx_hi, F.h_cb[8]);
+            // a pair fastq-to-bam writes (barcode corrected) that it or align on its BAM refuses: CbCounters::pad
+            const unsigned long long bad = F.h_cb[7];
+            if (bad & kTenxLongName) throw std::runtime_error("read name longer than 254 bytes");
+            if (bad & kTenxLongRead) throw std::runtime_error("read longer than 500 bases");
+        }
         unsigned long long need = 0;
         for (size_t li = 0; li < F.libs.size(); li++)
             if (F.h_ctr[li].overflow) need = std::max(need, F.h_ctr[li].items_max);
@@ -1090,7 +1199,8 @@ void lane_wait(nb200_ctx *c, int lane) {
         const std::vector<int32_t *> of = F.out_feats;
         const std::vector<uint16_t *> h1 = F.hlen1, h2 = F.hlen2;
         lane_submit(c, lane, &r1, F.paired ? &r2 : nullptr, libs.data(), (int)libs.size(), orr.empty() ? nullptr : orr.data(),
-                    of.empty() ? nullptr : of.data(), h1.empty() ? nullptr : h1.data(), h2.empty() ? nullptr : h2.data(), F.hkey);
+                    of.empty() ? nullptr : of.data(), h1.empty() ? nullptr : h1.data(), h2.empty() ? nullptr : h2.data(), F.hkey,
+                    F.hcb, F.hcbq, F.seq);
     }
 }
 
@@ -1132,8 +1242,24 @@ void lane_rows_segments(nb200_ctx *c, int lane, RowSeg *out) {
     }
 }
 
+// peer access where the devices allow it (cudaMemcpyPeerAsync stages through the host otherwise); current device = ctxs[0]'s
+static void enable_peers(const std::vector<nb200_ctx *> &ctxs) {
+    const nb200_ctx *c = ctxs[0];
+    for (nb200_ctx *x : ctxs)
+        if (x->device != c->device) {
+            int can = 0;
+            CK(cudaDeviceCanAccessPeer(&can, c->device, x->device));
+            if (can) {
+                const cudaError_t e = cudaDeviceEnablePeerAccess(x->device, 0);
+                if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) CK(e);
+                cudaGetLastError();
+            }
+        }
+}
+
 void lane_rows_count(const std::vector<nb200_ctx *> &ctxs, int li, int32_t lib_id, const std::vector<RowSeg> &segs,
-                     const std::vector<uint32_t> &cell_rank, double threshold, int disable, nb200_counts *counts, uint64_t *rows) {
+                     const std::vector<uint32_t> &cell_rank, double threshold, int disable, nb200_counts *counts, uint64_t *rows,
+                     bool tenx) {
     nb200_ctx *c = ctxs[0];
     for (nb200_ctx *x : ctxs) { CK(cudaSetDevice(x->device)); CK(cudaStreamSynchronize(x->s_copy[1])); }
     CK(cudaSetDevice(c->device));
@@ -1146,20 +1272,11 @@ void lane_rows_count(const std::vector<nb200_ctx *> &ctxs, int li, int32_t lib_i
     c->timing = nb200_timing{};
     c->launches = 0;
     c->gen_key.ensure(R * 8 + 16); c->gen_nf.ensure((R + 1) * 4 + 16); c->gen_off.ensure((R + 1) * 4 + 16); c->gen_feats.ensure(I * 4 + 16);
-    // peer access where the devices allow it (cudaMemcpyPeerAsync stages through the host otherwise)
-    for (nb200_ctx *x : ctxs)
-        if (x->device != c->device) {
-            int can = 0;
-            CK(cudaDeviceCanAccessPeer(&can, c->device, x->device));
-            if (can) {
-                const cudaError_t e = cudaDeviceEnablePeerAccess(x->device, 0);
-                if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) CK(e);
-                cudaGetLastError();
-            }
-        }
+    enable_peers(ctxs);
     // gather in slab order (= per-read TSV order); runs of segments that lie back to back in one store go as one copy
     cudaStream_t s = c->s_compute;
     uint64_t at_r = 0, at_i = 0;
+    std::vector<uint64_t> run_row, run_base;       // fastq-to-counts: where each run's rows start, and its context's log
     for (size_t a = 0; a < segs.size();) {
         size_t b = a + 1;
         while (b < segs.size() && segs[b].ctx == segs[a].ctx && segs[b].row0 == segs[b - 1].row0 + segs[b - 1].rows &&
@@ -1176,15 +1293,30 @@ void lane_rows_count(const std::vector<nb200_ctx *> &ctxs, int li, int32_t lib_i
         copy(c->gen_key.as<uint64_t>() + at_r, S.key.as<uint64_t>() + segs[a].row0, nr * 8);
         copy(c->gen_nf.as<uint32_t>() + at_r, S.nf.as<uint32_t>() + segs[a].row0, nr * 4);
         copy(c->gen_feats.as<int32_t>() + at_i, S.ids.as<int32_t>() + segs[a].id0, ni * 4);
+        if (tenx && nr) { run_row.push_back(at_r); run_base.push_back(c->tx_base.at((size_t)segs[a].ctx)); }
         at_r += nr; at_i += ni;
         a = b;
     }
     CK(cudaMemsetAsync(c->gen_nf.as<uint32_t>() + R, 0, 4, s));
     excl_scan_u32(c, c->gen_nf.as<uint32_t>(), c->gen_off.as<uint32_t>(), (uint32_t)(R + 1));
+    DevBuf runs, dropped;
     if (R) {
         c->rs_rank.ensure(cell_rank.size() * 4 + 16);
         CK(cudaMemcpyAsync(c->rs_rank.p, cell_rank.data(), cell_rank.size() * 4, cudaMemcpyHostToDevice, s));
-        cell_rank_kernel<<<nblk(R, 256), 256, 0, s>>>(R, c->gen_key.as<uint64_t>(), c->rs_rank.as<uint32_t>());
+        if (tenx) {
+            const uint32_t n_runs = (uint32_t)run_row.size();
+            run_row.push_back(R);
+            runs.ensure((run_row.size() + run_base.size()) * 8);
+            dropped.ensure(8);
+            CK(cudaMemcpyAsync(runs.p, run_row.data(), run_row.size() * 8, cudaMemcpyHostToDevice, s));
+            CK(cudaMemcpyAsync(runs.as<uint64_t>() + run_row.size(), run_base.data(), run_base.size() * 8, cudaMemcpyHostToDevice, s));
+            CK(cudaMemsetAsync(dropped.p, 0, 8, s));
+            cb_remap_kernel<<<nblk(R, 256), 256, 0, s>>>(R, c->gen_key.as<uint64_t>(), c->rs_rank.as<uint32_t>(), c->tx_dec.as<int32_t>(),
+                                                          runs.as<uint64_t>(), runs.as<uint64_t>() + run_row.size(), n_runs,
+                                                          dropped.as<unsigned long long>());
+        } else {
+            cell_rank_kernel<<<nblk(R, 256), 256, 0, s>>>(R, c->gen_key.as<uint64_t>(), c->rs_rank.as<uint32_t>());
+        }
         c->launches++;
     }
     CK(cudaMemsetAsync(c->d_ctr, 0, sizeof(Counters), s));
@@ -1195,6 +1327,12 @@ void lane_rows_count(const std::vector<nb200_ctx *> &ctxs, int li, int32_t lib_i
     Counters h2;
     CK(cudaMemcpy(&h2, c->d_ctr, sizeof(h2), cudaMemcpyDeviceToHost));
     counts->dropped_empty = h2.dropped_empty;
+    if (dropped.p) {                                // rows whose cell is a pandas NA token: report never reads them
+        unsigned long long d = 0;
+        CK(cudaMemcpy(&d, dropped.p, 8, cudaMemcpyDeviceToHost));
+        *rows = R - d;
+    }
+    runs.release(); dropped.release();
     // the stores of this library are done with
     for (nb200_ctx *x : ctxs) {
         CK(cudaSetDevice(x->device));
@@ -1210,44 +1348,151 @@ void lane_rows_count(const std::vector<nb200_ctx *> &ctxs, int li, int32_t lib_i
 // ---------------------------------------------------------------------------------------------
 // fastq-to-bam: whitelist table + barcode correction pipeline (barcode.cuh)
 // ---------------------------------------------------------------------------------------------
-static std::unique_ptr<DevWhitelist> build_whitelist(nb200_ctx *c, std::vector<std::string> &&entries, int cb_len) {
+// key of a whitelist line of length cb_len (3-bit codes: integer order == byte order); throws for a byte outside ACGTN
+static uint64_t wl_key(const std::string &e, size_t line) {
+    uint64_t key = 0;
+    for (char ch : e) {
+        const uint32_t code = cb_code((uint8_t)ch);
+        if (code == 7u) throw std::runtime_error("whitelist line " + std::to_string(line + 1) + " has a base outside ACGTN: " + e);
+        key = (key << 3) | code;
+    }
+    return key;
+}
+
+// the open-addressing table of the lines of length cb_len (first line wins for duplicates, as set() keeps one)
+static std::vector<WlSlot> wl_slots(const std::vector<std::string> &entries, int cb_len, uint64_t *n_unique) {
     if (cb_len < 1 || cb_len > kCbMaxLen) throw std::runtime_error("cb_len must be 1..21");
-    auto W = std::make_unique<DevWhitelist>();
-    W->entries = std::move(entries);
-    W->cb_len = cb_len;
-    if (W->entries.size() >= 0x7FFFFFFFull) throw LimitError("whitelist has 2^31 or more lines");
+    if (entries.size() >= 0x7FFFFFFFull) throw LimitError("whitelist has 2^31 or more lines");
     uint64_t same = 0;
-    for (const auto &e : W->entries) same += (int)e.size() == cb_len;
+    for (const auto &e : entries) same += (int)e.size() == cb_len;
     uint64_t slots = 1024;
     while (slots < same * 2 + 2) slots <<= 1;
     std::vector<WlSlot> tab(slots, WlSlot{kCbEmpty, 0, 0});
     const uint64_t mask = slots - 1;
-    for (size_t i = 0; i < W->entries.size(); i++) {
-        const std::string &e = W->entries[i];
+    *n_unique = 0;
+    for (size_t i = 0; i < entries.size(); i++) {
+        const std::string &e = entries[i];
         if ((int)e.size() != cb_len) continue;                  // can never equal a raw barcode or a variant of one
-        uint64_t key = 0;
-        for (int j = 0; j < cb_len; j++) {
-            const uint32_t code = cb_code((uint8_t)e[j]);
-            if (code == 7u) throw std::runtime_error("whitelist line " + std::to_string(i + 1) + " has a base outside ACGTN: " + e);
-            key = (key << 3) | code;
-        }
+        const uint64_t key = wl_key(e, i);
         uint64_t s = cb_hash(key) & mask;
         while (tab[s].key != kCbEmpty && tab[s].key != key) s = (s + 1) & mask;
-        if (tab[s].key == kCbEmpty) { tab[s].key = key; tab[s].idx = (uint32_t)i; W->n_unique++; }   // set(): first line wins
+        if (tab[s].key == kCbEmpty) { tab[s].key = key; tab[s].idx = (uint32_t)i; ++*n_unique; }   // set(): first line wins
     }
+    return tab;
+}
+
+static std::unique_ptr<DevWhitelist> build_whitelist(nb200_ctx *c, std::vector<std::string> &&entries, int cb_len) {
+    auto W = std::make_unique<DevWhitelist>();
+    const std::vector<WlSlot> tab = wl_slots(entries, cb_len, &W->n_unique);
+    W->entries = std::move(entries);
+    W->cb_len = cb_len;
+    const uint64_t slots = tab.size();
     W->n_slots = slots;
     W->table.ensure(slots * sizeof(WlSlot));
     CK(cudaMemcpyAsync(W->table.p, tab.data(), slots * sizeof(WlSlot), cudaMemcpyHostToDevice, c->s_compute));
     CK(cudaStreamSynchronize(c->s_compute));
     W->dev.table = W->table.as<WlSlot>();
-    W->dev.mask = mask;
+    W->dev.mask = slots - 1;
     W->dev.cb_len = cb_len;
     return W;
 }
 
-struct MaxU32 {
-    __host__ __device__ __forceinline__ uint32_t operator()(uint32_t a, uint32_t b) const { return a > b ? a : b; }
-};
+// ---- fastq-to-counts: the whitelist on every context, the cache rule over every context's log (slab_api.hpp) ----------
+void lane_cb_begin(const std::vector<nb200_ctx *> &ctxs, const std::vector<std::string> &whitelist, int cb_len,
+                   std::vector<uint32_t> *rank, std::vector<std::string> *cells) {
+    uint64_t n_unique = 0;
+    const std::vector<WlSlot> tab = wl_slots(whitelist, cb_len, &n_unique);
+    for (nb200_ctx *c : ctxs) {
+        CK(cudaSetDevice(c->device));
+        c->tx_table.ensure(tab.size() * sizeof(WlSlot));
+        CK(cudaMemcpy(c->tx_table.p, tab.data(), tab.size() * sizeof(WlSlot), cudaMemcpyHostToDevice));
+        c->tx_wl = WlDev{c->tx_table.as<WlSlot>(), tab.size() - 1, cb_len};
+        c->tx_n.ensure(8);
+        CK(cudaMemset(c->tx_n.p, 0, 8));
+        c->tx_hi = 0;
+        for (auto &b : c->tx_old) b.release();
+        c->tx_old.clear();
+        c->tx_base.clear();
+    }
+    CK(cudaSetDevice(ctxs[0]->device));
+    // cells: the distinct lines in byte order (= key order), pandas-NA tokens left out (report drops such a cell)
+    std::vector<std::pair<uint64_t, uint32_t>> by_key;
+    by_key.reserve(n_unique);
+    for (size_t i = 0; i < whitelist.size(); i++)
+        if ((int)whitelist[i].size() == cb_len) by_key.emplace_back(wl_key(whitelist[i], i), (uint32_t)i);
+    std::sort(by_key.begin(), by_key.end());
+    rank->assign(whitelist.size(), 0xFFFFFFFFu);
+    cells->clear();
+    for (size_t j = 0; j < by_key.size(); j++) {
+        const uint32_t i = by_key[j].second;
+        if (j && by_key[j].first == by_key[j - 1].first) { (*rank)[i] = (*rank)[by_key[j - 1].second]; continue; }
+        if (pandas_na(whitelist[i])) continue;
+        (*rank)[i] = (uint32_t)cells->size();
+        cells->push_back(whitelist[i]);
+    }
+}
+
+void lane_cb_counters(nb200_ctx *c, int lane, uint64_t *out6) {
+    const unsigned long long *h = c->lane[lane].h_cb;                 // CbCounters: n_miss n_inval perfect corrected none n_multi probes
+    out6[0] = h[2]; out6[1] = h[3]; out6[2] = h[4]; out6[3] = h[0]; out6[4] = h[5]; out6[5] = h[6];
+}
+
+__global__ void iota_u32_kernel(uint32_t n, uint32_t *__restrict__ out) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) out[i] = i;
+}
+
+void lane_cb_resolve(const std::vector<nb200_ctx *> &ctxs) {
+    nb200_ctx *c = ctxs[0];
+    std::vector<uint64_t> cnt(ctxs.size());
+    for (size_t d = 0; d < ctxs.size(); d++) {
+        CK(cudaSetDevice(ctxs[d]->device));
+        CK(cudaStreamSynchronize(ctxs[d]->s_compute));
+        CK(cudaMemcpy(&cnt[d], ctxs[d]->tx_n.p, 8, cudaMemcpyDeviceToHost));
+    }
+    CK(cudaSetDevice(c->device));
+    c->tx_base.assign(ctxs.size(), 0);
+    uint64_t E = 0;
+    for (size_t d = 0; d < ctxs.size(); d++) { c->tx_base[d] = E; E += cnt[d]; }
+    if (E > 0x7FFFFFF0ull) throw LimitError("more than 2^31 reads whose cell barcode has several candidates");
+    c->tx_dec.ensure(E * 4 + 16);
+    if (!E) return;
+    // every log on the first context, in context order (entry j of context d is decision tx_base[d] + j)
+    DevBuf key, ord, sorted, perm;
+    key.ensure(E * 8); ord.ensure(E * 8); sorted.ensure(E * 8); perm.ensure(E * 8);
+    enable_peers(ctxs);
+    cudaStream_t s = c->s_compute;
+    for (size_t d = 0; d < ctxs.size(); d++) {
+        const nb200_ctx *x = ctxs[d];
+        const uint64_t at = c->tx_base[d], n = cnt[d];
+        auto copy = [&](void *dst, const void *src, size_t bytes) {
+            if (!bytes) return;
+            if (x->device == c->device) CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, s));
+            else CK(cudaMemcpyPeerAsync(dst, c->device, src, x->device, bytes, s));
+        };
+        copy(key.as<uint64_t>() + at, x->tx_key.p, n * 8);
+        copy(ord.as<uint64_t>() + at, x->tx_ord.p, n * 8);
+        copy(c->tx_dec.as<int32_t>() + at, x->tx_choice.p, n * 4);
+    }
+    // entries in file order, then the first of each raw barcode decides (a re-run slab's duplicates agree with the original)
+    iota_u32_kernel<<<nblk(E, 256), 256, 0, s>>>((uint32_t)E, perm.as<uint32_t>() + E);
+    cub_sort64(c, ord.as<uint64_t>(), sorted.as<uint64_t>(), perm.as<uint32_t>() + E, perm.as<uint32_t>(), (uint32_t)E, 64);
+    cb_first_decides(c, perm.as<uint32_t>(), key.as<uint64_t>(), (uint32_t)E, c->tx_dec.as<int32_t>());
+    CK(cudaStreamSynchronize(s));
+    for (DevBuf *b : {&key, &ord, &sorted, &perm}) b->release();
+}
+
+void lane_cb_end(const std::vector<nb200_ctx *> &ctxs) {
+    for (nb200_ctx *c : ctxs) {
+        CK(cudaSetDevice(c->device));
+        for (DevBuf *b : {&c->tx_table, &c->tx_key, &c->tx_ord, &c->tx_choice, &c->tx_dec}) b->release();
+        for (auto &b : c->tx_old) b.release();
+        c->tx_old.clear();
+        c->tx_cap = c->tx_hi = 0;
+        c->tx_base.clear();
+    }
+    CK(cudaSetDevice(ctxs[0]->device));
+}
 
 static DevWhitelist &get_wl(const nb200_ctx *c, int32_t id) {
     if (id < 0 || id >= (int32_t)c->wls.size() || !c->wls[id]) throw std::runtime_error("unknown whitelist id");
@@ -1289,43 +1534,27 @@ static void cb_run(nb200_ctx *c, DevWhitelist &W, nb200_cb_stats *st) {
     uint64_t launches = 0;
     cudaEvent_t e0 = new_event(c), e1 = new_event(c);
     CK(cudaEventRecord(e0, s));
-    CK(cudaMemsetAsync(c->d_cbctr, 0, sizeof(CbCounters), s));
-    CK(cudaMemsetAsync(c->flag.p, 0, n + 16, s));
     const size_t n_ent = W.entries.size();
     if (st) {                                           // hit flags per whitelist entry (for the cache-size statistic)
         c->cb_hit.ensure(n_ent + 16);
         CK(cudaMemsetAsync(c->cb_hit.p, 0, n_ent + 16, s));
     }
+    const uint64_t launches0 = c->launches;
+    cb_launch(c, W.dev, s, c->cb_chars.as<uint8_t>(), c->cb_qual.as<uint8_t>(), c->cb_has_elig ? c->cb_elig.as<uint8_t>() : nullptr, n,
+              c->cb_keys.as<uint64_t>(), c->cb_idx.as<int32_t>(), c->cb_status.as<uint8_t>(), c->permA.as<uint32_t>(),
+              c->cb_inval.as<uint32_t>(), (uint32_t)n, st ? c->cb_hit.as<uint8_t>() : nullptr, c->flag.as<uint8_t>(), c->d_cbctr);
     CbCounters h{};
     if (n) {
-        cb_exact_kernel<<<nblk(n, 256), 256, 0, s>>>(W.dev, c->cb_chars.as<uint8_t>(), c->cb_has_elig ? c->cb_elig.as<uint8_t>() : nullptr, n,
-                                                     c->cb_keys.as<uint64_t>(), c->cb_idx.as<int32_t>(), c->cb_status.as<uint8_t>(),
-                                                     c->permA.as<uint32_t>(), c->cb_inval.as<uint32_t>(), (uint32_t)n,
-                                                     st ? c->cb_hit.as<uint8_t>() : nullptr, c->d_cbctr);
-        cb_hamming_kernel<<<c->sm_count * 8, 128, 0, s>>>(W.dev, c->cb_qual.as<uint8_t>(), c->cb_keys.as<uint64_t>(), c->permA.as<uint32_t>(),
-                                                          c->cb_idx.as<int32_t>(), c->cb_status.as<uint8_t>(), c->flag.as<uint8_t>(), c->d_cbctr);
-        CK(cudaGetLastError());
-        launches += 2;
         CK(cudaMemcpyAsync(&h, c->d_cbctr, sizeof h, cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));
         if (h.n_multi) {
             // the reference's correction_cache: first read in file order decides per raw barcode
             c->permB.ensure(n * 4 + 16);
             const uint32_t m = cub_select(c, c->flag.as<uint8_t>(), c->permB.as<uint32_t>(), (uint32_t)n);   // ascending read index
-            c->k64A.ensure((size_t)m * 8 + 16); c->k64B.ensure((size_t)m * 8 + 16);
-            c->k32A.ensure((size_t)m * 4 + 16); c->k32B.ensure((size_t)m * 4 + 16); c->head.ensure((size_t)m * 4 + 16);
-            cb_gather_keys_kernel<<<nblk(m, 256), 256, 0, s>>>(c->permB.as<uint32_t>(), c->cb_keys.as<uint64_t>(), m, c->k64A.as<uint64_t>());
-            cub_sort64(c, c->k64A.as<uint64_t>(), c->k64B.as<uint64_t>(), c->permB.as<uint32_t>(), c->k32A.as<uint32_t>(), m, 64);   // stable
-            cb_run_heads_kernel<<<nblk(m, 256), 256, 0, s>>>(c->k64B.as<uint64_t>(), m, c->k32B.as<uint32_t>());
-            size_t bytes = 0;
-            CK(cub::DeviceScan::InclusiveScan(nullptr, bytes, c->k32B.as<uint32_t>(), c->head.as<uint32_t>(), MaxU32(), (int)m, s));
-            c->cub_tmp.ensure(bytes);
-            CK(cub::DeviceScan::InclusiveScan(c->cub_tmp.p, bytes, c->k32B.as<uint32_t>(), c->head.as<uint32_t>(), MaxU32(), (int)m, s));
-            cb_propagate_kernel<<<nblk(m, 256), 256, 0, s>>>(c->k32A.as<uint32_t>(), c->head.as<uint32_t>(), m, c->cb_idx.as<int32_t>());
-            CK(cudaGetLastError());
-            launches += 8;
+            cb_first_decides(c, c->permB.as<uint32_t>(), c->cb_keys.as<uint64_t>(), m, c->cb_idx.as<int32_t>());
         }
     }
+    launches += c->launches - launches0;
     uint64_t distinct = 0;
     if (st && n) {
         // "Correction cache size": distinct raw barcodes among the eligible reads = whitelist entries hit
@@ -1496,7 +1725,11 @@ void nb200_destroy(nb200_ctx *c) {
         if (F.h_ctr) cudaFreeHost(F.h_ctr);
         F.key.release(); F.seg.release();
         if (F.h_seg) cudaFreeHost(F.h_seg);
+        for (DevBuf *b : {&F.cb, &F.cbq, &F.cb_raw, &F.cb_idx, &F.cb_st, &F.cb_miss, &F.cb_multi, &F.cb_ctr}) b->release();
+        if (F.h_cb) cudaFreeHost(F.h_cb);
     }
+    for (DevBuf *b : {&c->tx_table, &c->tx_key, &c->tx_ord, &c->tx_choice, &c->tx_n, &c->tx_dec}) b->release();
+    for (auto &b : c->tx_old) b.release();
     for (auto &S : c->rs) {
         for (DevBuf *b : {&S.key, &S.nf, &S.ids, &S.hdr, &S.na}) b->release();
         for (auto &b : S.old) b.release();
@@ -1939,7 +2172,8 @@ int32_t nb200_align_files(nb200_ctx *c, const char *const *inputs, int32_t n_inp
 static int32_t files_multi(const int32_t *devices, int32_t n_devices, int32_t host_threads, const char *const *inputs, int32_t n_inputs,
                            const char *const *library_json, int32_t n_libs, const char *strand_filter, int32_t k, const char *trim,
                            const char *const *outputs, const char *const *counts_outputs, double umi_threshold, int32_t disable_thresholding,
-                           uint64_t *out3, char *err, size_t err_cap, double *stats4);
+                           uint64_t *out3, char *err, size_t err_cap, double *stats4, const char *whitelist = nullptr, int32_t cb_len = 16,
+                           int32_t umi_len = 12, nb200_cb_stats *cb_stats = nullptr);
 
 int32_t nb200_align_files_multi(const int32_t *devices, int32_t n_devices, int32_t host_threads, const char *const *inputs, int32_t n_inputs,
                                 const char *const *library_json, int32_t n_libs, const char *strand_filter, int32_t k,
@@ -1992,7 +2226,8 @@ int32_t nb200_align_files_counts(nb200_ctx *c, const char *const *inputs, int32_
 static int32_t files_multi(const int32_t *devices, int32_t n_devices, int32_t host_threads, const char *const *inputs, int32_t n_inputs,
                            const char *const *library_json, int32_t n_libs, const char *strand_filter, int32_t k, const char *trim,
                            const char *const *outputs, const char *const *counts_outputs, double umi_threshold, int32_t disable_thresholding,
-                           uint64_t *out3, char *err, size_t err_cap, double *stats4) {
+                           uint64_t *out3, char *err, size_t err_cap, double *stats4, const char *whitelist, int32_t cb_len,
+                           int32_t umi_len, nb200_cb_stats *cb_stats) {
     auto fail = [&](int32_t rc, const std::string &w) { if (err && err_cap) { snprintf(err, err_cap, "%s", w.c_str()); } return rc; };
     if (!devices || n_devices < 1 || !inputs || n_inputs < 1 || n_inputs > 2 || !library_json || n_libs < 1 || (!outputs && !counts_outputs))
         return fail(NB200_EINVAL, "bad arguments");
@@ -2038,10 +2273,13 @@ static int32_t files_multi(const int32_t *devices, int32_t n_devices, int32_t ho
             job.host_threads = ctxs[0]->host_threads;
             job.umi_threshold = umi_threshold;
             job.disable_thresholding = disable_thresholding;
+            std::vector<std::string> wl;
+            if (whitelist) { read_whitelist_lines(whitelist, wl); job.whitelist = &wl; job.cb_len = cb_len; job.umi_len = umi_len; }
             FileStats st;
             run_file_pipeline(job, &st);
             if (stats4) { stats4[0] = (double)st.n_reads; stats4[1] = st.seconds; stats4[2] = (double)st.called; stats4[3] = (double)st.n_slabs; }
             if (out3) for (size_t i = 0; i < st.counts3.size(); i++) out3[i] = st.counts3[i];
+            if (cb_stats) *cb_stats = st.cb;
         } catch (const IoError &e) { rc = NB200_EIO; what = e.what(); }
         catch (const nb200::CudaError &e) { rc = NB200_ECUDA; what = e.what(); }
         catch (const nb200::LimitError &e) { rc = NB200_ELIMIT; what = e.what(); }
@@ -2049,6 +2287,55 @@ static int32_t files_multi(const int32_t *devices, int32_t n_devices, int32_t ho
     }
     for (nb200_ctx *c : ctxs) nb200_destroy(c);
     return rc == NB200_OK ? NB200_OK : fail(rc, what);
+}
+
+// fastq-to-bam + align --counts without the intermediate BAM, streaming (stream.cpp, 10x mode): one pass from raw R1 / R2
+// to the counts TSVs, the cell barcodes corrected slab by slab on the device, the correction cache over the whole call.
+int32_t nb200_fastq_to_counts(nb200_ctx *c, const char *r1_fastq, const char *r2_fastq, const char *whitelist_path, int32_t cb_len,
+                              int32_t umi_len, const int32_t *lib_ids, const char *const *counts_outputs, int32_t n_libs,
+                              double umi_threshold, int32_t disable_thresholding, uint64_t *out3, nb200_cb_stats *stats) {
+    API_BEGIN(c)
+    if (!r1_fastq || !r2_fastq || !whitelist_path || !lib_ids || !counts_outputs || n_libs < 1 || cb_len < 1 || cb_len > kCbMaxLen || umi_len < 0)
+        throw std::runtime_error("bad arguments");
+    if (out3) for (int i = 0; i < 3 * n_libs; i++) out3[i] = 0;
+    if (stats) *stats = nb200_cb_stats{};
+    try {
+        std::vector<std::string> wl;
+        read_whitelist_lines(whitelist_path, wl);
+        FileJob job;
+        job.inputs = {r1_fastq, r2_fastq};
+        job.ctxs.push_back(c);
+        job.lib_ids.assign(lib_ids, lib_ids + n_libs);
+        for (int i = 0; i < n_libs; i++) { get_lib(c, lib_ids[i]); job.counts_outputs.emplace_back(counts_outputs[i]); }
+        job.host_threads = c->host_threads;
+        job.umi_threshold = umi_threshold;
+        job.disable_thresholding = disable_thresholding;
+        job.whitelist = &wl; job.cb_len = cb_len; job.umi_len = umi_len;
+        FileStats st;
+        run_file_pipeline(job, &st);
+        if (out3) for (size_t i = 0; i < st.counts3.size(); i++) out3[i] = st.counts3[i];
+        if (stats) *stats = st.cb;
+        if (getenv("NB200_TRACE"))
+            fprintf(stderr, "[nb200 trace] file pipeline (fastq-to-counts): %llu pairs in %llu slabs, %.3f s, %d host threads\n",
+                    (unsigned long long)st.cb.total_pairs, (unsigned long long)st.n_slabs, st.seconds, c->host_threads);
+    } catch (const IoError &e) { c->err = e.what(); return NB200_EIO; }
+    API_END(c)
+}
+
+int32_t nb200_fastq_to_counts_multi(const int32_t *devices, int32_t n_devices, int32_t host_threads, const char *r1_fastq,
+                                    const char *r2_fastq, const char *whitelist_path, int32_t cb_len, int32_t umi_len,
+                                    const char *const *library_json, int32_t n_libs, const char *strand_filter, int32_t k,
+                                    const char *trim, const char *const *counts_outputs, double umi_threshold,
+                                    int32_t disable_thresholding, uint64_t *out3, nb200_cb_stats *stats, char *err, size_t err_cap,
+                                    double *stats4) {
+    if (stats) *stats = nb200_cb_stats{};
+    if (!r1_fastq || !r2_fastq || !whitelist_path || !counts_outputs || cb_len < 1 || cb_len > kCbMaxLen || umi_len < 0) {
+        if (err && err_cap) snprintf(err, err_cap, "bad arguments");
+        return NB200_EINVAL;
+    }
+    const char *inputs[2] = {r1_fastq, r2_fastq};
+    return files_multi(devices, n_devices, host_threads, inputs, 2, library_json, n_libs, strand_filter, k, trim, nullptr, counts_outputs,
+                       umi_threshold, disable_thresholding, out3, err, err_cap, stats4, whitelist_path, cb_len, umi_len, stats);
 }
 
 // fastq-to-bam + align without the intermediate BAM: the pairs fastq_to_bam_with_barcodes would write

@@ -52,13 +52,6 @@ void load_fastq_qual(const std::string &path, FastqQ &F) {
     }
 }
 
-static inline bool name_eq_stripped(const char *a, uint32_t la, const char *b, uint32_t lb) {
-    // r1.id.removesuffix('/1') == r2.id.removesuffix('/2')  (:152-156)
-    if (la >= 2 && a[la - 2] == '/' && a[la - 1] == '1') la -= 2;
-    if (lb >= 2 && b[lb - 2] == '/' && b[lb - 1] == '2') lb -= 2;
-    return la == lb && memcmp(a, b, la) == 0;
-}
-
 // process_pair up to the correction call: eligibility + the three skip counters; cb/qual are n x cb_len
 // (zero-filled for ineligible pairs), qual holds phred values (ASCII - 33)
 void slice_barcodes(const FastqQ &A, const FastqQ &B, int cb_len, int umi_len, int threads, uint8_t *cb, uint8_t *qual,

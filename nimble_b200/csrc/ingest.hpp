@@ -50,6 +50,12 @@ void write_bulk_tsv(const std::string &out_path, const nb200_counts &c, const st
 struct FqRec { uint64_t name, seq, qual; uint32_t name_len, len; };   // offsets into FastqQ::text
 struct FastqQ { std::string text; std::vector<FqRec> recs; };
 void load_fastq_qual(const std::string &path, FastqQ &F);
+// process_pair's name check: r1.id.removesuffix('/1') == r2.id.removesuffix('/2')  (:152-156)
+inline bool name_eq_stripped(const char *a, uint32_t la, const char *b, uint32_t lb) {
+    if (la >= 2 && a[la - 2] == '/' && a[la - 1] == '1') la -= 2;
+    if (lb >= 2 && b[lb - 2] == '/' && b[lb - 1] == '2') lb -= 2;
+    return la == lb && std::char_traits<char>::compare(a, b, la) == 0;
+}
 void slice_barcodes(const FastqQ &A, const FastqQ &B, int cb_len, int umi_len, int threads, uint8_t *cb, uint8_t *qual,
                     uint8_t *eligible, nb200_cb_stats &st);
 void write_10x_bam(const std::string &out_path, const FastqQ &A, const FastqQ &B, int cb_len, int umi_len, const int32_t *idx,

@@ -13,6 +13,8 @@
 //   committer thread      writes the formatted slabs in input order, merges bulk tables, recycles slabs
 //
 // Memory is bounded by the slab pool and by the number of inflated chunks in flight, not by the file size.
+// 10x mode (nb200_fastq_to_counts): raw R1 / R2 FASTQ; the parse task keeps the pairs fastq-to-bam would correct
+// (tenx_select) and the GPU threads correct their barcodes slab by slab (slab_api.hpp: lane_cb_*).
 #include "stream.hpp"
 
 #include <zlib.h>
@@ -477,6 +479,10 @@ struct Slab {
     uint64_t bases1 = 0, bases2 = 0, called = 0;
     uint64_t *key = nullptr;                                             // counts mode: cell << 32 | umi per read
     uint64_t tagged = 0;                                                 // counts mode: reads with a CB or UB value
+    // 10x mode: raw cell barcodes and their phred values (n x cb_len) of the pairs in the slab; fastq-to-bam's counters
+    uint8_t *cbc = nullptr, *cbq = nullptr;
+    uint64_t pairs = 0, name_mismatch = 0, too_short = 0, no_remaining_seq = 0;
+    uint64_t cbn[6] = {0, 0, 0, 0, 0, 0};                                // lane_cb_counters
 };
 
 // ---- counts mode: CB / UB strings -> key = cell << 32 | umi -------------------------------------------------------
@@ -537,6 +543,15 @@ static inline bool umi_code(std::string_view s, uint32_t &x) {
     return true;
 }
 
+// the key's low half for a UMI that is not a pandas NA token (seen: the slab's interned UMIs, saves the shared lock)
+static inline uint32_t umi_id(std::string_view ub, BarcodeDict &bc, std::unordered_map<std::string_view, uint32_t> &seen) {
+    uint32_t u;
+    if (umi_code(ub, u)) return u;
+    auto v = seen.find(ub);
+    if (v == seen.end()) v = seen.emplace(ub, bc.umi(ub)).first;
+    return v->second;
+}
+
 // keys of a parsed slab (runs on the pool, inside the parse task): invalid barcodes (absent, empty, a pandas NA token:
 // `report` drops those rows, nimble/__main__.py:244-245) -> NB200_NO_BARCODE
 static void slab_keys(Slab &S, BarcodeDict &bc) {
@@ -557,13 +572,7 @@ static void slab_keys(Slab &S, BarcodeDict &bc) {
             cid = bc.cell(cb);
             if (c == cc.ids.end() && cc.ids.size() < CellCache::kMax) cc.ids.emplace(h, std::make_pair(cid, std::string(cb)));
         }
-        uint32_t u;
-        if (!umi_code(ub, u)) {
-            auto v = umis.find(ub);
-            if (v == umis.end()) v = umis.emplace(ub, bc.umi(ub)).first;
-            u = v->second;
-        }
-        S.key[i] = ((uint64_t)cid << 32) | u;
+        S.key[i] = ((uint64_t)cid << 32) | umi_id(ub, bc, umis);
     }
     g_ns_intern += (uint64_t)((now_s() - t_in) * 1e9);
 }
@@ -574,6 +583,8 @@ struct Entry {                                   // one read (pair) as the walke
     const char *name = nullptr;                  // FASTQ only
     uint32_t ln = 0;
     const char *qa = nullptr, *qb = nullptr;     // FASTQ only: quality lines (phred + 33) of the two mates, when --trim wants them
+    const char *name2 = nullptr;                 // 10x mode: R2's name (process_pair compares the two)
+    uint32_t ln2 = 0;
 };
 
 struct Task {
@@ -589,6 +600,8 @@ struct Task {
     Slab *slab = nullptr;
     const std::vector<TrimTable> *trims = nullptr;   // per library (--trim), or nullptr
     BarcodeDict *bc = nullptr;                   // counts mode
+    int cb_len = 0, umi_len = 0;                 // 10x mode when cb_len > 0 (tenx_select)
+    std::string qconv;                           // 10x mode with --trim: the qualities as fastq-to-bam's BAM stores them
 };
 
 static inline uint32_t le32(const unsigned char *p) { return p[0] | (p[1] << 8) | (p[2] << 16) | ((uint32_t)p[3] << 24); }
@@ -719,8 +732,54 @@ static void pack_ascii(const char *s, uint32_t L, uint8_t *rec, uint32_t words, 
     pack_codes(codes, L, rec, words, stride);
 }
 
+// 10x mode, first step of the parse task: keep the pairs fastq-to-bam would hand to the barcode correction
+// (process_pair's rules, slice_barcodes) and turn each into what that BAM's records hold: raw CB + phred values into the
+// slab, the UMI into the key's low half, read 1 = R1 after barcode and UMI, read 2 = R2.  The rest is counted.
+static void tenx_select(Task &t) {
+    Slab &S = *t.slab;
+    const uint32_t L = (uint32_t)t.cb_len, U = (uint32_t)t.umi_len, bl = L + U;
+    const bool want_q = t.trims && !S.lt1.empty();
+    std::unordered_map<std::string_view, uint32_t> umis;
+    if (want_q) {
+        size_t bytes = 0;
+        for (const Entry &e : t.e) bytes += e.la + e.lb;
+        t.qconv.clear();
+        t.qconv.reserve(bytes);                       // (no reallocation below: the entries point into it)
+    }
+    // the BAM stores phred values (quality byte - 33); align reads 0xFF in the first one as "no qualities"
+    auto bam_qual = [&](const char *q, uint32_t n) -> const char * {
+        const size_t at = t.qconv.size();
+        for (uint32_t j = 0; j < n; j++) t.qconv.push_back((char)(uint8_t)(q[j] - 33));
+        return (n && (uint8_t)t.qconv[at] == 0xFF) ? nullptr : t.qconv.data() + at;
+    };
+    S.pairs = t.e.size(); S.name_mismatch = S.too_short = S.no_remaining_seq = 0;
+    size_t o = 0;
+    for (size_t i = 0; i < t.e.size(); i++) {
+        Entry e = t.e[i];
+        if (!name_eq_stripped(e.name, e.ln, e.name2, e.ln2)) { S.name_mismatch++; continue; }
+        if (e.la < bl) { S.too_short++; continue; }
+        if (e.la == bl) { S.no_remaining_seq++; continue; }
+        // what writing the BAM (a name over 254 bytes) or aligning it (a read over 500 bases) refuses: the two steps fail
+        // only when the pair is written, i.e. its barcode gets a correction, so the device decides (cb_key_kernel).  The
+        // pair still takes part in the correction and its cache rule; an over-long read goes to the kernels empty.
+        uint32_t nl = e.ln;
+        if (nl >= 2 && e.name[nl - 2] == '/' && e.name[nl - 1] == '1') nl -= 2;
+        const uint64_t flags = (nl > 254 ? kTenxLongName : 0) | ((e.la - bl > NB200_MAX_READ_LEN || e.lb > NB200_MAX_READ_LEN) ? kTenxLongRead : 0);
+        memcpy(S.cbc + o * L, e.a, L);
+        for (uint32_t j = 0; j < L; j++) S.cbq[o * L + j] = (uint8_t)(e.qa[j] - 33);
+        const std::string_view umi(e.a + L, U);
+        S.key[o] = (flags << 32) | (pandas_na(umi) ? kTenxNaUmi : umi_id(umi, *t.bc, umis));
+        if (want_q) { e.qa = bam_qual(e.qa + bl, e.la - bl); e.qb = bam_qual(e.qb, e.lb); }
+        e.a += bl; e.la -= bl;
+        if (flags & kTenxLongRead) { e.la = 0; e.lb = 0; }
+        t.e[o++] = e;
+    }
+    t.e.resize(o);
+}
+
 // task -> slab (runs on the pool)
 static void parse_task(Task &t) {
+    if (t.cb_len) tenx_select(t);
     Slab &S = *t.slab;
     const size_t n = t.segs.empty() ? t.e.size() : t.n_seg_records;
     S.n = n; S.paired = t.paired; S.has_tags = t.bam;
@@ -750,8 +809,9 @@ static void parse_task(Task &t) {
         }
         const Entry &e = t.segs.empty() ? t.e[i] : seg_e;
         if (trimming && !t.bam) {
-            trimmed(S.lt1, i, e.la, (const uint8_t *)e.qa, 33, false);
-            if (t.paired) trimmed(S.lt2, i, e.lb, (const uint8_t *)e.qb, 33, false);
+            const int off = t.cb_len ? 0 : 33;         // 10x mode: phred values already (tenx_select)
+            trimmed(S.lt1, i, e.la, (const uint8_t *)e.qa, off, false);
+            if (t.paired) trimmed(S.lt2, i, e.lb, (const uint8_t *)e.qb, off, false);
         }
         if (t.bam) {
             BamView a, b;
@@ -785,7 +845,7 @@ static void parse_task(Task &t) {
             if (t.paired) { pack_ascii(e.b, e.lb, S.p2 + i * (size_t)s2, w2, s2); S.l2[i] = (uint16_t)e.lb; S.bases2 += e.lb; }
         }
     }
-    if (t.bc) slab_keys(S, *t.bc);
+    if (t.bc && !t.cb_len) slab_keys(S, *t.bc);
 }
 
 // ---- output ----------------------------------------------------------------------------------------------
@@ -886,6 +946,7 @@ struct Pipeline {
     bool dry = false;
     bool per_read = true;                          // per-read TSVs are written
     bool counts = false;                           // counts TSVs: keys per read, rows kept on the devices
+    bool tenx = false;                             // raw 10x R1 / R2 in, cell barcodes corrected on the devices (FileJob)
     BarcodeDict bc;
     std::mutex seg_m;
     std::vector<std::vector<RowSeg>> segs;         // counts mode, per library: the segments of every slab on every context
@@ -906,6 +967,7 @@ struct Pipeline {
             S->feats.push_back((int32_t *)S->grab(kSlabReads * (size_t)libs[li].max_hits * 4 + 64));
         }
         if (counts) S->key = (uint64_t *)S->grab(kSlabReads * 8 + 64);
+        if (tenx) { S->cbc = (uint8_t *)S->grab(kSlabReads * (size_t)job.cb_len + 64); S->cbq = (uint8_t *)S->grab(kSlabReads * (size_t)job.cb_len + 64); }
         if (!trims.empty())
             for (size_t li = 0; li < n_libs; li++) S->lt1.push_back((uint16_t *)S->grab(kSlabReads * 2 + 64));
         S->out.resize(n_libs); S->bulk.resize(n_libs);
@@ -926,6 +988,7 @@ struct Pipeline {
         if (!dry) for (const LibOut &lo : libs) g.push_back(lo.max_hits);
         g.push_back(trims.empty() ? 0 : 1);
         g.push_back((per_read ? 1 : 0) | (counts ? 2 : 0));
+        g.push_back(tenx ? job.cb_len : 0);
         return g;
     }
     void start_pool(size_t count, nb200_ctx *bind) {
@@ -994,6 +1057,7 @@ struct Pipeline {
                     for (size_t li = 0; li < sg.size(); li++) { sg[li].seq = S->seq; sg[li].ctx = ctx_index; segs[li].push_back(sg[li]); }
                     if (!per_read) S->called = sg[0].called;
                 }
+                if (tenx) lane_cb_counters(c, l, S->cbn);
                 after_gpu(S);
             };
             for (;;) {
@@ -1008,7 +1072,7 @@ struct Pipeline {
                 lane_submit(c, lane, &S->r1, S->paired ? &S->r2 : nullptr, job.lib_ids.data(), (int)job.lib_ids.size(),
                             S->res.empty() ? nullptr : S->res.data(), S->feats.empty() ? nullptr : S->feats.data(),
                             S->lt1.empty() ? nullptr : S->lt1.data(), (S->paired && !S->lt2.empty()) ? S->lt2.data() : nullptr,
-                            counts ? S->key : nullptr);
+                            counts ? S->key : nullptr, tenx ? S->cbc : nullptr, tenx ? S->cbq : nullptr, S->seq);
                 g_ns_gpu_submit += (uint64_t)((now_s() - t_in) * 1e9);
                 lane ^= 1;
             }
@@ -1058,6 +1122,14 @@ struct Pipeline {
                         stats.n_reads += T->n; stats.bases1 += T->bases1; stats.bases2 += T->bases2; stats.called += T->called;
                         stats.paired |= T->paired; stats.has_tags |= T->has_tags; stats.n_slabs++;
                         tagged += T->tagged;
+                        if (tenx) {
+                            nb200_cb_stats &c = stats.cb;
+                            c.total_pairs += T->pairs; c.name_mismatch += T->name_mismatch; c.too_short += T->too_short;
+                            c.no_remaining_seq += T->no_remaining_seq;
+                            c.cb_perfect_match += T->cbn[0]; c.cb_corrected += T->cbn[1]; c.cb_no_correction += T->cbn[2];
+                            c.n_exact_miss += T->cbn[3]; c.n_multi += T->cbn[4]; c.probes += T->cbn[5];
+                            c.written_pairs += T->cbn[0] + T->cbn[1];
+                        }
                         if (dry && !getenv("NB200_INGEST_NOSUM"))      // reader statistics (nb200_host_ingest_stats): same checksum as readset_checksum
                             for (size_t i = 0; i < T->n; i++) {
                                 mix(T->names.ptr(i), T->names.len(i));
@@ -1089,6 +1161,7 @@ struct Pipeline {
         t->slab = S;
         t->trims = trims.empty() ? nullptr : &trims;
         t->bc = counts ? &bc : nullptr;
+        if (tenx) { t->cb_len = job.cb_len; t->umi_len = job.umi_len; }
         pool->push(Pool::PARSE, [this, t] {
             const double t_in = now_s();
             try { parse_task(*t); } catch (...) { to_commit.push(t->slab); throw; }
@@ -1281,24 +1354,39 @@ static void walk_fastq(Pipeline &P, ByteSource &s1, ByteSource *s2) {
     task->paired = s2 != nullptr;
     auto attach = [&] { c1.attach(&task->keep); if (c2) c2->attach(&task->keep); };
     attach();
-    const bool want_q = !P.trims.empty();
+    const bool want_q = !P.trims.empty() || P.tenx;
+    // 10x mode reads FASTQ as fastq-to-bam does (load_fastq_qual): blank lines between records, a '+' line, qualities as
+    // long as the sequence; read lengths are checked after the barcode and UMI are cut off (tenx_select)
+    const bool tenx = P.tenx;
     auto record = [&](Cursor &c, const std::string &path, const char *&name, uint32_t &nl, const char *&seq, uint32_t &sl, const char *&qual) -> bool {
         qual = nullptr;
         const char *p; size_t n;
         if (!c.line(p, n)) return false;
         if (n == 0 && !c.line(p, n)) return false;          // tolerate one blank line at the end
+        while (tenx && n == 0) if (!c.line(p, n)) return false;
         if (n == 0 || p[0] != '@') throw std::runtime_error("malformed FASTQ record in " + path);
         size_t e = 1;
         while (e < n && p[e] != ' ' && p[e] != '\t') e++;
         name = p + 1; nl = (uint32_t)(e - 1);
         if (!c.line(p, n)) throw std::runtime_error("truncated FASTQ record in " + path);
-        if (n > NB200_MAX_READ_LEN) throw std::runtime_error("read longer than 500 bases");
+        if (n > NB200_MAX_READ_LEN && !tenx) throw std::runtime_error("read longer than 500 bases");
         seq = p; sl = (uint32_t)n;
         const char *q; size_t qn;
+        if (tenx) {
+            if (!c.line(q, qn)) throw std::runtime_error("truncated FASTQ record in " + path);
+            if (qn == 0 || q[0] != '+') throw std::runtime_error("malformed FASTQ record (no '+' line) in " + path);
+            if (!c.line(q, qn)) { q = p; qn = 0; }          // empty quality line at the end of the file
+            if (qn != sl) throw std::runtime_error("FASTQ sequence and quality lengths differ in " + path);
+            qual = q;
+            return true;
+        }
         if (!c.line(q, qn)) return true;                    // '+' line and qualities may be missing at the very end
         if (c.line(q, qn) && want_q && qn == sl) qual = q;  // (a quality line of another length is ignored: no trimming)
         return true;
     };
+    // 10x mode: the longest read the slab will hold of this pair (over-long reads fail in the parse task)
+    const uint32_t bl = tenx ? (uint32_t)(P.job.cb_len + P.job.umi_len) : 0;
+    auto held = [&](uint32_t len, uint32_t cut) { return tenx ? std::min<uint32_t>(len > cut ? len - cut : 0, NB200_MAX_READ_LEN) : len; };
     for (;;) {
         Entry e;
         const char *nm; uint32_t nl;
@@ -1306,9 +1394,18 @@ static void walk_fastq(Pipeline &P, ByteSource &s1, ByteSource *s2) {
         e.name = nm; e.ln = nl;
         if (c2) {
             const char *n2; uint32_t l2;
-            if (!record(*c2, P.job.inputs[1], n2, l2, e.b, e.lb, e.qb)) throw std::runtime_error("R1 and R2 FASTQ files hold different numbers of reads");
+            if (!record(*c2, P.job.inputs[1], n2, l2, e.b, e.lb, e.qb)) {
+                if (!tenx) throw std::runtime_error("R1 and R2 FASTQ files hold different numbers of reads");
+                // fastq-to-bam zips the two files: pairs stop at the shorter one, the rest of R1 is only checked
+                Keep rest;
+                c1.attach(&rest);
+                while (record(c1, P.job.inputs[0], nm, nl, e.a, e.la, e.qa)) { rest.blocks.clear(); rest.side.clear(); }
+                c2.reset();
+                break;
+            }
+            e.name2 = n2; e.ln2 = l2;
         }
-        const uint32_t m1 = std::max(task->max1, e.la), m2 = std::max(task->max2, e.lb);
+        const uint32_t m1 = std::max(task->max1, held(e.la, bl)), m2 = std::max(task->max2, held(e.lb, 0));
         if (task->e.size() + 1 > slab_room(std::max(m1, m2))) {
             auto nt = std::make_shared<Task>();
             nt->paired = task->paired;
@@ -1319,12 +1416,17 @@ static void walk_fastq(Pipeline &P, ByteSource &s1, ByteSource *s2) {
             task = nt;
             attach();
         }
-        task->max1 = std::max(task->max1, e.la); task->max2 = std::max(task->max2, e.lb);
+        task->max1 = std::max(task->max1, held(e.la, bl)); task->max2 = std::max(task->max2, held(e.lb, 0));
         task->e.push_back(e);
     }
     if (c2) {
         const char *n2; uint32_t l2; const char *sq; uint32_t sl; const char *qq;
-        if (record(*c2, P.job.inputs[1], n2, l2, sq, sl, qq)) throw std::runtime_error("R1 and R2 FASTQ files hold different numbers of reads");
+        Keep rest;
+        if (tenx) c2->attach(&rest);
+        while (record(*c2, P.job.inputs[1], n2, l2, sq, sl, qq)) {
+            if (!tenx) throw std::runtime_error("R1 and R2 FASTQ files hold different numbers of reads");
+            rest.blocks.clear(); rest.side.clear();        // 10x mode: the rest of R2 is only checked (zip)
+        }
     }
     P.dispatch(task);
 }
@@ -1351,18 +1453,26 @@ void run_file_pipeline(const FileJob &job, FileStats *stats_out) {
     P.dry = job.ctxs.empty();
     P.counts = counts && !P.dry;
     P.per_read = !job.outputs.empty();
+    P.tenx = job.whitelist != nullptr;
+    if (P.tenx && (!P.counts || P.per_read || job.inputs.size() != 2 || job.umi_len < 0))
+        throw std::runtime_error("bad arguments");
     g_wait_block = g_wait_slab = 0.0;
     g_ns_inflate = 0; g_ns_parse = 0; g_ns_format = 0; g_ns_gpu_wait = 0; g_ns_gpu_submit = 0; g_ns_write = 0; g_ns_intern = 0;
     double t_alloc = 0.0, t_walk = 0.0, t_drain = 0.0, t_finish = 0.0, t_free = 0.0, t_counts = 0.0;
     const int T = std::max(1, job.host_threads);
     const bool bam = ends_with_ci(job.inputs[0], ".bam");
     if (bam && job.inputs.size() != 1) throw std::runtime_error("one BAM file expected");
-    if (P.counts && !bam)
+    if (P.counts && !bam && !P.tenx)
         throw std::runtime_error("counts need cell barcodes and UMIs (CB / UB tags of a BAM file); " + job.inputs[0] + " is FASTQ: write the per-read TSV instead");
+    if (P.tenx && bam) throw std::runtime_error("fastq-to-counts reads raw R1 / R2 FASTQ files; " + job.inputs[0] + " is a BAM file");
     if (P.counts) {                                    // (feature names the per-read TSV cannot carry fail here, before any work)
         for (nb200_ctx *c : job.ctxs) lane_rows_begin(c, job.lib_ids.data(), (int)job.lib_ids.size());
         P.segs.resize(job.lib_ids.size());
     }
+    std::vector<uint32_t> wl_rank;                     // 10x mode: whitelist line -> cell rank (lane_cb_begin)
+    std::vector<std::string> wl_cells;
+    struct CbEnd { const FileJob &j; bool on; ~CbEnd() { if (on) try { lane_cb_end(j.ctxs); } catch (...) {} } } cb_end{job, P.tenx};
+    if (P.tenx) lane_cb_begin(job.ctxs, *job.whitelist, job.cb_len, &wl_rank, &wl_cells);
     // outputs
     for (size_t li = 0; li < (P.dry ? 0 : job.lib_ids.size()); li++) {
         LibOut lo;
@@ -1442,7 +1552,7 @@ void run_file_pipeline(const FileJob &job, FileStats *stats_out) {
             if (P.ab.io) throw IoError(P.ab.what);
             throw std::runtime_error(P.ab.what);
         }
-        if (P.counts && P.stats.n_reads && !P.tagged)
+        if (P.counts && !P.tenx && P.stats.n_reads && !P.tagged)
             throw std::runtime_error("no read of " + job.inputs[0] + " carries a CB or UB tag: counts need cell barcodes and UMIs");
         // finish the files: per-read outputs are complete, bulk tables are written now
         for (LibOut &lo : P.libs) {
@@ -1474,18 +1584,25 @@ void run_file_pipeline(const FileJob &job, FileStats *stats_out) {
             // counts TSVs (nimble/__main__.py:254-293): every library's rows gathered in slab order on the first context,
             // cells ranked by CB bytes, the UMI stage on the device
             const double tc = now_s();
-            std::vector<std::string> cell_names = P.bc.cell_names();
-            std::vector<uint32_t> order(cell_names.size()), rank(cell_names.size());
-            for (uint32_t i = 0; i < order.size(); i++) order[i] = i;
-            std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return cell_names[a] < cell_names[b]; });
-            std::vector<std::string> cells(cell_names.size());
-            for (uint32_t r = 0; r < order.size(); r++) { rank[order[r]] = r; cells[r] = std::move(cell_names[order[r]]); }
+            std::vector<uint32_t> rank;
+            std::vector<std::string> cells;
+            if (P.tenx) {                                   // cells are whitelist lines; the cache rule decides the open ones
+                lane_cb_resolve(job.ctxs);
+                rank.swap(wl_rank); cells.swap(wl_cells);
+            } else {
+                std::vector<std::string> cell_names = P.bc.cell_names();
+                std::vector<uint32_t> order(cell_names.size());
+                rank.resize(cell_names.size()); cells.resize(cell_names.size());
+                for (uint32_t i = 0; i < order.size(); i++) order[i] = i;
+                std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return cell_names[a] < cell_names[b]; });
+                for (uint32_t r = 0; r < order.size(); r++) { rank[order[r]] = r; cells[r] = std::move(cell_names[order[r]]); }
+            }
             for (size_t li = 0; li < P.libs.size(); li++) {
                 std::vector<RowSeg> &sg = P.segs[li];
                 std::sort(sg.begin(), sg.end(), [](const RowSeg &a, const RowSeg &b) { return a.seq < b.seq; });
                 nb200_counts table{};
                 uint64_t rows = 0;
-                lane_rows_count(job.ctxs, (int)li, job.lib_ids[li], sg, rank, job.umi_threshold, job.disable_thresholding, &table, &rows);
+                lane_rows_count(job.ctxs, (int)li, job.lib_ids[li], sg, rank, job.umi_threshold, job.disable_thresholding, &table, &rows, P.tenx);
                 std::vector<std::string> names(P.libs[li].names.size());
                 for (size_t f = 0; f < names.size(); f++) names[f].assign(P.libs[li].names[f].first, P.libs[li].names[f].second);
                 write_counts_tsv(job.counts_outputs[li], table.n_rows ? &table : nullptr, names, cells);

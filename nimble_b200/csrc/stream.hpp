@@ -22,12 +22,18 @@ struct FileJob {
     std::vector<std::string> counts_outputs;
     double umi_threshold = 0.05;
     int disable_thresholding = 0;
+    // 10x mode (nb200_fastq_to_counts, counts only): inputs = raw R1 and R2 FASTQ.  The pairs fastq-to-bam would write
+    // go to the device as its BAM would: CB = R1[0, cb_len) corrected against the whitelist there, UB = R1[cb_len,
+    // cb_len + umi_len), read 1 = the rest of R1, read 2 = R2.
+    const std::vector<std::string> *whitelist = nullptr;   // the non-empty lines of the whitelist file; null = off
+    int cb_len = 16, umi_len = 12;
 };
 
 struct FileStats {
     uint64_t n_reads = 0, paired = 0, has_tags = 0, bases1 = 0, bases2 = 0, checksum = 0, n_slabs = 0, called = 0;
     double seconds = 0.0;
     std::vector<uint64_t> counts3;        // counts mode: per library rows used, count rows written, UMIs dropped
+    nb200_cb_stats cb{};                  // 10x mode: fastq-to-bam's counters (cache_size 0: not computed by this route)
 };
 
 // throws IoError / std::exception

@@ -340,6 +340,21 @@ class Engine:
                                               len(libs), ct.byref(st)))
         return {f: getattr(st, f) for f, _ in CbStats._fields_}
 
+    def fastq_to_counts(self, r1_fastq, r2_fastq, whitelist_path, libs, counts_outputs, cb_length=16, umi_length=12, threshold=0.05,
+                        disable_thresholding=False):
+        """fastq-to-bam + align --counts in one streaming pass, no intermediate BAM (nb200_fastq_to_counts): raw 10x R1 / R2
+        in, one counts TSV per library out.  Returns (barcode statistics as fastq_to_bam's, with cache_size 0; per library
+        (rows used, count rows, dropped UMIs))."""
+        ids = (ct.c_int32 * len(libs))(*[l.id for l in libs])
+        cnt = (ct.c_char_p * len(counts_outputs))(*[os.fspath(p).encode() for p in counts_outputs])
+        out3 = (ct.c_uint64 * (3 * len(libs)))()
+        st = CbStats()
+        self._ck(self.L.nb200_fastq_to_counts(self.ctx, os.fspath(r1_fastq).encode(), os.fspath(r2_fastq).encode(),
+                                              os.fspath(whitelist_path).encode(), int(cb_length), int(umi_length), ids, cnt, len(libs),
+                                              float(threshold), int(bool(disable_thresholding)), out3, ct.byref(st)))
+        return ({f: getattr(st, f) for f, _ in CbStats._fields_},
+                [(int(out3[3 * i]), int(out3[3 * i + 1]), int(out3[3 * i + 2])) for i in range(len(libs))])
+
     def set_overlap(self, on):
         """Batch pipelining on (default) / off (kernels back to back on one stream: per-stage times add up)."""
         self._ck(self.L.nb200_set_overlap(self.ctx, int(bool(on))))

@@ -660,6 +660,14 @@ def fastq_to_bam_with_barcodes(r1_fastq, r2_fastq, cb_whitelist_file, output_bam
     finally:
         if own:
             eng.close()
+    _print_pair_stats(st)
+    print(f"\nCorrection cache size: {st['cache_size']} unique raw CBs")
+    print(f"\nOutput BAM written to: {output_bam}")
+    return st
+
+
+def _print_pair_stats(st):
+    """fastq_to_bam_with_barcodes' statistics (nimble/fastq_barcode_processor.py:284-309) up to the cache size."""
     print("\n=== Processing Statistics ===")
     print(f"Total read pairs: {st['total_pairs']}")
     print(f"Written pairs: {st['written_pairs']}")
@@ -676,6 +684,65 @@ def fastq_to_bam_with_barcodes(r1_fastq, r2_fastq, cb_whitelist_file, output_bam
     print(f"  Name mismatch: {st['name_mismatch']}")
     print(f"  Too short: {st['too_short']}")
     print(f"  No remaining sequence: {st['no_remaining_seq']}")
-    print(f"\nCorrection cache size: {st['cache_size']} unique raw CBs")
-    print(f"\nOutput BAM written to: {output_bam}")
-    return st
+
+
+def fastq_to_counts(reference, r1_fastq, r2_fastq, cb_whitelist_file, counts, num_cores=1, strand_filter="unstranded", trim="",
+                    k=20, gpus=None, cb_length=16, umi_length=12, threshold=0.05, disable_thresholding=False, engine=None):
+    """`fastq-to-bam`, then `align --counts` on its BAM, in one streaming pass without the BAM (an extension: the reference
+    needs fastq-to-bam, align and report).  Raw 10x R1 / R2 FASTQ(.gz) + whitelist in, the counts TSV `report` would
+    write out, one per library (named like align's outputs).  gpus (also $NB200_GPUS): a count or a list of devices.
+    Returns 0 on success, 1 on an error (with a message on stderr), 2 without a CUDA device."""
+    import ctypes as ct
+    from . import _lib
+    from .engine import Engine
+    from ._lib import NimbleB200Error
+    library_list = reference.split(",")
+    cnts = _per_library_paths(counts, library_list)
+    if gpus is None and os.environ.get("NB200_GPUS"):
+        gpus = int(os.environ["NB200_GPUS"])
+    own = engine is None
+    try:
+        trims = parse_trim(trim, len(library_list))
+        if gpus and engine is None and (not isinstance(gpus, int) or gpus > 1):
+            L = _lib.load()
+            devs = list(range(int(gpus))) if isinstance(gpus, int) else [int(g) for g in gpus]
+            d = (ct.c_int32 * len(devs))(*devs)
+            libs = (ct.c_char_p * len(library_list))(*[os.fspath(p).encode() for p in library_list])
+            cnt_c = (ct.c_char_p * len(cnts))(*[os.fspath(p).encode() for p in cnts])
+            out3 = (ct.c_uint64 * (3 * len(cnts)))()
+            cst = _lib.CbStats()
+            err = ct.create_string_buffer(1024)
+            st4 = (ct.c_double * 4)()
+            rc = L.nb200_fastq_to_counts_multi(d, len(devs), int(num_cores or 0), os.fspath(r1_fastq).encode(), os.fspath(r2_fastq).encode(),
+                                               os.fspath(cb_whitelist_file).encode(), int(cb_length), int(umi_length), libs, len(library_list),
+                                               strand_filter.encode(), int(k), (trim or "").encode(), cnt_c, float(threshold),
+                                               int(bool(disable_thresholding)), out3, ct.byref(cst), err, len(err), st4)
+            if rc != 0:
+                print("nimble_b200 aligner error: %s" % err.value.decode(errors="replace"), file=sys.stderr)
+                return 2 if rc == -2 else 1
+            st = {f: getattr(cst, f) for f, _ in _lib.CbStats._fields_}
+            o3 = [tuple(out3[3 * i:3 * i + 3]) for i in range(len(cnts))]
+        else:
+            eng = engine or Engine(int(os.environ.get("LOCAL_RANK", 0)), int(num_cores or 0))
+            try:
+                libs = [eng.load_library(l, strand_filter=strand_filter, k=k) for l in library_list]
+                for lg, (t_len, t_strict) in zip(libs, trims):
+                    lg.set_trim(t_len, t_strict)
+                st, o3 = eng.fastq_to_counts(r1_fastq, r2_fastq, cb_whitelist_file, libs, cnts, cb_length, umi_length, threshold,
+                                             disable_thresholding)
+            finally:
+                if own:
+                    eng.close()
+    except NimbleB200Error as e:
+        print("nimble_b200 aligner error: %s" % e, file=sys.stderr)
+        return 1 if e.code != -2 else 2
+    except (OSError, ValueError) as e:
+        print("nimble_b200 aligner error: %s" % e, file=sys.stderr)
+        return 1
+    _print_pair_stats(st)
+    if st["no_remaining_seq"] and st["cb_perfect_match"] + st["cb_corrected"] + st["cb_no_correction"] == 0:
+        print("nimble_b200: no pair written: every R1 that passed the name and length checks is exactly --cb-length + --umi-length "
+              "(%d) bases long, so no read 1 is left after the barcode and UMI (fastq-to-bam drops such pairs)"
+              % (int(cb_length) + int(umi_length)), file=sys.stderr)
+    _print_counts_summary(cnts, o3)
+    return 0

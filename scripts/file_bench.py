@@ -4,6 +4,7 @@
 metric (bench.py times the hot path); this is what a user of `python -m nimble_b200` waits for.
 
     python scripts/file_bench.py [--reads 2000000] [--out-dir /tmp/nb200_file_bench]
+    python scripts/file_bench.py --tenx [--reads 20000000] [--gpus N]    # raw 10x FASTQ: fastq-to-bam + align --counts vs fastq-to-counts
 """
 import argparse
 import json
@@ -141,6 +142,116 @@ def counts_bench(args, eng, kw, lib_path, bam, tsv, nbytes):
     if not out["counts_identical"] or any(out["rc"]):
         sys.exit(4)
 
+def write_tenx_fastqs(out_dir, codes, n_pairs, chunk=2_000_000, seed=5, level=1):
+    """Seeded raw 10x input: R1 = CB (synth.barcode_workload: 737 k-entry whitelist, errors, N, off-whitelist barcodes, 30 %
+    clustered entries so that the correction cache decides) + UMI (12) + 62 bases, R2 = 90 bases, written as plain gzip
+    (one member per chunk, not BGZF).  Returns (R1, R2, whitelist) paths."""
+    from concurrent.futures import ThreadPoolExecutor
+    r1p, r2p, wlp = (os.path.join(out_dir, f) for f in ("R1.fastq.gz", "R2.fastq.gz", "whitelist.txt"))
+    wl_a = None
+    acgt = np.frombuffer(b"ACGT", np.uint8)
+
+    def fastq(ids, seq, qual, mate):                 # fixed-width names (p<9 digits>/<mate>): one numpy array per chunk
+        n, L = seq.shape
+        rec = np.zeros((n, 14 + 2 * L + 4), np.uint8)
+        rec[:, 0] = ord("@"); rec[:, 1] = ord("p")
+        rec[:, 2:11] = np.stack([(ids // 10 ** k) % 10 for k in range(8, -1, -1)], axis=1).astype(np.uint8) + ord("0")
+        rec[:, 11] = ord("/"); rec[:, 12] = ord("0") + mate; rec[:, 13] = 10
+        rec[:, 14:14 + L] = seq; rec[:, 14 + L] = 10; rec[:, 15 + L] = ord("+"); rec[:, 16 + L] = 10
+        rec[:, 17 + L:17 + 2 * L] = qual; rec[:, -1] = 10
+        return rec.tobytes()
+
+    def gz(b):
+        z = zlib.compressobj(level, zlib.DEFLATED, 31)
+        return z.compress(b) + z.flush()
+
+    with open(r1p, "wb") as f1, open(r2p, "wb") as f2, ThreadPoolExecutor(os.cpu_count() or 4) as ex:
+        for c0 in range(0, n_pairs, chunk):
+            n = min(chunk, n_pairs - c0)
+            s = seed + 7919 * (c0 // chunk)
+            rng = np.random.default_rng(s)
+            if wl_a is None:                         # one whitelist and cell set; each chunk reads them in another order
+                wl_a, cb0, q0 = synth.barcode_workload(chunk, n_whitelist=737_280, n_cells=10000, seed=seed, clustered=0.3)
+            perm = rng.permutation(len(cb0))[:n]
+            cb, q = cb0[perm], q0[perm]
+            r2, _ = synth.sample_reads(codes, n, read_len=90, seed=s + 1)
+            tail, _ = synth.sample_reads(codes, n, read_len=62, seed=s + 2)
+            umi = acgt[rng.integers(0, 4, size=(n, 12))]
+            s1 = np.concatenate([cb, umi, tail], axis=1)
+            q1 = np.concatenate([q + 33, rng.integers(35, 75, size=(n, 74))], axis=1).astype(np.uint8)
+            q2 = rng.integers(35, 75, size=(n, 90)).astype(np.uint8)
+            ids = np.arange(c0, c0 + n)
+            parts = list(ex.map(lambda a: gz(fastq(*a)), [(ids, s1, q1, 1), (ids, r2, q2, 2)]))
+            f1.write(parts[0]); f2.write(parts[1])
+    with open(wlp, "w") as f:
+        f.write("\n".join(bytes(r).decode() for r in wl_a) + "\n")
+    return r1p, r2p, wlp
+
+
+def _write_tenx_child(out_dir, n_pairs):
+    _, codes = synth.allele_family_library(n_founders=40, alleles_per_founder=50, length=1098, snps_mean=15.0, seed=1)
+    write_tenx_fastqs(out_dir, codes, n_pairs)
+
+
+def run_child(argv, env=None):
+    """One `python -m nimble_b200 ...` process: (wall seconds, peak RSS MB, rc)."""
+    import subprocess
+    t0 = time.perf_counter()
+    p = subprocess.Popen([sys.executable, "-m", "nimble_b200"] + argv, cwd=ROOT, stdout=subprocess.DEVNULL, env=env)
+    _, status, ru = os.wait4(p.pid, 0)
+    return time.perf_counter() - t0, ru.ru_maxrss / 1024.0, os.waitstatus_to_exitcode(status)
+
+
+def tenx_bench(args, lib_path):
+    """Raw 10x FASTQ to counts: `fastq-to-bam` then `align --counts` on its BAM (two processes, a BAM between them) against
+    `fastq-to-counts` (one process, no BAM), alternating, two repetitions each.  Wall clock and peak RSS per process; the
+    counts files must be byte-identical."""
+    import filecmp
+    t0 = time.time()
+    made = {"tenx": args.reads}
+    stamp = os.path.join(args.out_dir, "tenx.json")
+    try:
+        reuse = json.load(open(stamp)) == made
+    except (OSError, ValueError):
+        reuse = False
+    r1p, r2p, wlp = (os.path.join(args.out_dir, f) for f in ("R1.fastq.gz", "R2.fastq.gz", "whitelist.txt"))
+    if not reuse:
+        # written by a child process: Linux keeps a process's peak RSS across fork + exec, so the routes timed below must
+        # not be forked from a process that once held the generated data
+        import multiprocessing
+        p = multiprocessing.get_context("spawn").Process(target=_write_tenx_child, args=(args.out_dir, args.reads))
+        p.start(); p.join()
+        if p.exitcode != 0:
+            sys.exit("writing the 10x FASTQs failed")
+        with open(stamp, "w") as f:
+            json.dump(made, f)
+    print("%s 10x FASTQs: %d pairs, %.0f + %.0f MB in %.1fs" % ("reused" if reuse else "wrote", args.reads, os.path.getsize(r1p) / 1e6,
+                                                              os.path.getsize(r2p) / 1e6, time.time() - t0), file=sys.stderr)
+    cores = str(args.cores or os.cpu_count())
+    bam, two, one = (os.path.join(args.out_dir, f) for f in ("tenx.bam", "tenx_counts_two_step.tsv", "tenx_counts_one_pass.tsv"))
+    gp = ["--gpus", str(args.gpus)] if args.gpus > 1 else []
+    step1 = ["fastq-to-bam", "--r1-fastq", r1p, "--r2-fastq", r2p, "--map", wlp, "--output", bam, "-c", cores]
+    step2 = ["align", "--reference", lib_path, "--input", bam, "--counts", two, "-c", cores] + gp
+    fused = ["fastq-to-counts", "--reference", lib_path, "--r1-fastq", r1p, "--r2-fastq", r2p, "--map", wlp, "--counts", one, "-c", cores] + gp
+    out = {"pairs": args.reads, "gpus": args.gpus, "host_threads": int(cores), "r1_mb": os.path.getsize(r1p) / 1e6,
+           "r2_mb": os.path.getsize(r2p) / 1e6, "whitelist": 737_280, "input": "plain gzip (one zlib stream per file)",
+           "fastq_to_bam_s": [], "fastq_to_bam_rss_mb": [], "align_counts_s": [], "align_counts_rss_mb": [], "two_step_s": [],
+           "one_pass_s": [], "one_pass_rss_mb": [], "rc": []}
+    out.update(gpu_info())
+    for _rep in range(2):
+        a = run_child(step1)
+        b = run_child(step2)
+        c = run_child(fused, dict(os.environ, NB200_TRACE="1"))      # (stage times of the pipeline on stderr)
+        out["fastq_to_bam_s"].append(a[0]); out["fastq_to_bam_rss_mb"].append(a[1])
+        out["align_counts_s"].append(b[0]); out["align_counts_rss_mb"].append(b[1]); out["two_step_s"].append(a[0] + b[0])
+        out["one_pass_s"].append(c[0]); out["one_pass_rss_mb"].append(c[1]); out["rc"] += [a[2], b[2], c[2]]
+    out["counts_identical"] = filecmp.cmp(two, one, shallow=False)
+    out["count_rows"] = sum(1 for _ in open(one))
+    out["one_pass_pairs_per_s"] = args.reads / min(out["one_pass_s"])
+    print(json.dumps(out))
+    if not out["counts_identical"] or any(out["rc"]):
+        sys.exit(4)
+
 
 def main():
     ap = argparse.ArgumentParser()
@@ -155,6 +266,8 @@ def main():
                                                        "(the streaming pipeline holds a fixed pool of slabs, not the file)")
     ap.add_argument("--counts", action="store_true", help="time the two-step route (align + report) against the fused `align --counts`, "
                                                           "alternating, two repetitions each, and compare the counts files")
+    ap.add_argument("--tenx", action="store_true", help="raw 10x R1 / R2 FASTQ (plain gzip) + whitelist: fastq-to-bam then align --counts "
+                                                        "on its BAM against fastq-to-counts, alternating; wall clock, peak RSS, identical counts")
     args = ap.parse_args()
     os.makedirs(args.out_dir, exist_ok=True)
     if args.workload == "cfg4":
@@ -166,6 +279,9 @@ def main():
     lib_path = os.path.join(args.out_dir, "lib.json")
     with open(lib_path, "w") as f:
         json.dump(lib, f)
+    if args.tenx:
+        tenx_bench(args, lib_path)
+        return
     bam = os.path.join(args.out_dir, "in.bam")
     made = {"workload": args.workload, "reads": args.reads}
     try:                                    # the same input as an earlier run into this directory: not written again
