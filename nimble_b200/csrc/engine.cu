@@ -10,6 +10,7 @@
 #include <stdexcept>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <unordered_set>
 #include <vector>
 
@@ -39,9 +40,18 @@ struct CudaError : std::runtime_error { using std::runtime_error::runtime_error;
             throw CudaError(std::string(#call) + ": " + cudaGetErrorString(e_));                   \
     } while (0)
 
+// Device memory with one owner: freed by its destructor, handed on only by moving.  A buffer is freed with whatever device
+// is current, so code that frees another device's buffers sets that device first.
 struct DevBuf {
     void *p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(DevBuf &&o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    DevBuf &operator=(DevBuf &&o) noexcept {
+        if (this != &o) { release(); p = o.p; cap = o.cap; o.p = nullptr; o.cap = 0; }
+        return *this;
+    }
+    ~DevBuf() { release(); }
     void ensure(size_t bytes) {
         if (bytes <= cap) return;
         if (p) CK(cudaFree(p));
@@ -53,6 +63,44 @@ struct DevBuf {
     void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
     template <class T> T *as() const { return reinterpret_cast<T *>(p); }
 };
+static_assert(!std::is_copy_constructible<DevBuf>::value && !std::is_copy_assignable<DevBuf>::value &&
+                  std::is_nothrow_move_constructible<DevBuf>::value,
+              "a DevBuf has one owner; std::vector<DevBuf> moves its elements");
+
+// Pinned host memory for `cap` elements of T, owned like a DevBuf.  ensure() allocates exactly what it is asked for.
+template <class T> struct PinnedBuf {
+    T *p = nullptr;
+    size_t cap = 0;
+    PinnedBuf() = default;
+    PinnedBuf(PinnedBuf &&o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    PinnedBuf &operator=(PinnedBuf &&o) noexcept {
+        if (this != &o) { release(); p = o.p; cap = o.cap; o.p = nullptr; o.cap = 0; }
+        return *this;
+    }
+    ~PinnedBuf() { release(); }
+    void ensure(size_t count) {
+        if (count <= cap) return;
+        release();
+        CK(cudaMallocHost(&p, count * sizeof(T)));
+        cap = count;
+    }
+    void release() { if (p) cudaFreeHost(p); p = nullptr; cap = 0; }
+};
+
+// A CUDA stream or event with one owner; converts to the raw handle, so it is passed to the runtime as one.
+template <class H, cudaError_t (*Destroy)(H)> struct CudaHandle {
+    H h = nullptr;
+    CudaHandle() = default;
+    CudaHandle(CudaHandle &&o) noexcept : h(o.h) { o.h = nullptr; }
+    CudaHandle &operator=(CudaHandle &&o) noexcept {
+        if (this != &o) { if (h) Destroy(h); h = o.h; o.h = nullptr; }
+        return *this;
+    }
+    ~CudaHandle() { if (h) Destroy(h); }
+    operator H() const { return h; }
+};
+using Stream = CudaHandle<cudaStream_t, cudaStreamDestroy>;
+using Event = CudaHandle<cudaEvent_t, cudaEventDestroy>;
 
 struct DevLibrary {
     HostLibrary host;
@@ -63,7 +111,6 @@ struct DevLibrary {
     double min_score_for = 0.0;
     bool min_score_ok = false;
     size_t table_bytes = 0, slab_bytes = 0;
-    ~DevLibrary() { slab.release(); tok_end.release(); tok_comma.release(); min_score.release(); }
 };
 
 struct DevWhitelist {
@@ -72,7 +119,6 @@ struct DevWhitelist {
     WlDev dev{};
     uint64_t n_slots = 0, n_unique = 0;
     int cb_len = 16;
-    ~DevWhitelist() { table.release(); }
 };
 
 }  // namespace nb200
@@ -84,8 +130,8 @@ struct nb200_ctx {
     size_t l2_persist_max = 0, l2_window_max = 0;
     const DevLibrary *l2_window_lib = nullptr;
     std::string err;
-    cudaStream_t s_compute = nullptr, s_copy[2] = {nullptr, nullptr};
-    std::vector<cudaEvent_t> ev_pool;
+    Stream s_compute, s_copy[2];
+    std::vector<Event> ev_pool;
     std::vector<std::unique_ptr<DevLibrary>> libs;
     // resident reads
     DevBuf d_r1, d_r1len, d_r2, d_r2len, d_key;
@@ -95,7 +141,7 @@ struct nb200_ctx {
     bool paired = false, has_key = false, resident = false;
     // per batch
     // per-batch state, double-buffered: batch k's alignment/calling kernels (s_tail) overlap batch k+1's probe (s_compute)
-    struct BatchBuf { DevBuf ro, roB, items, sw_pairs, sw_rep, deferred, wide_list, sums, slow_list, setup_list; Counters *ctr = nullptr; cudaEvent_t tail_done = nullptr, probe_done = nullptr; bool busy = false; } bb[2];
+    struct BatchBuf { DevBuf ro, roB, items, sw_pairs, sw_rep, deferred, wide_list, sums, slow_list, setup_list; Counters *ctr = nullptr; Event tail_done, probe_done; bool busy = false; } bb[2];
     DevBuf wide_scratch, wide_v;
     // streaming file path: two slabs in flight, each with its own device buffers (slab_api.hpp)
     struct FileLane {
@@ -103,9 +149,8 @@ struct nb200_ctx {
         std::vector<DevBuf> res, feats, nf;       // per library of the call
         std::vector<DevBuf> l1v, l2v;             // per library: trimmed read lengths (--trim), else unused
         std::vector<uint16_t *> hlen1, hlen2;     // what was submitted (host pointers; empty = no trimming)
-        cudaEvent_t h2d_done = nullptr, done = nullptr;
-        Counters *h_ctr = nullptr;                // pinned: one Counters per library (overflow of the SW work list)
-        size_t h_ctr_cap = 0;
+        Event h2d_done, done;
+        PinnedBuf<Counters> h_ctr;                // one Counters per library (overflow of the SW work list)
         bool busy = false;
         nb200_reads hr1{}, hr2{};                 // what was submitted (an overflow re-runs it)
         bool paired = false;
@@ -114,15 +159,14 @@ struct nb200_ctx {
         std::vector<int32_t *> out_feats;
         // counts mode: the slab's keys, the segment record per library (device / pinned: row0, rows, id0, ids, called)
         DevBuf key, seg;
-        unsigned long long *h_seg = nullptr;
-        size_t h_seg_cap = 0;
+        PinnedBuf<unsigned long long> h_seg;
         const uint64_t *hkey = nullptr;           // what was submitted (an overflow re-runs it)
         uint64_t n_rows_max = 0;                  // reads of the slab in flight: bound on the rows it appends
         // fastq-to-counts: the slab's barcodes and their correction (cb_*: device; h_cb: pinned CbCounters + log end)
         DevBuf cb, cbq, cb_raw, cb_idx, cb_st, cb_miss, cb_multi, cb_ctr;
         const uint8_t *hcb = nullptr, *hcbq = nullptr;   // what was submitted (an overflow re-runs it)
         uint64_t seq = 0;
-        unsigned long long *h_cb = nullptr;
+        PinnedBuf<unsigned long long> h_cb;
     } lane[kFileLanes];
     // fastq-to-counts (lane_cb_*): the whitelist table, and the log of reads with several candidates (raw barcode, file
     // order, own choice; tx_n = entries, device-side).  The log grows like the row stores: tx_hi = its end as of the
@@ -139,25 +183,29 @@ struct nb200_ctx {
         uint64_t hi_rows = 0, hi_ids = 0;         // store end as of the last segment the host has seen
         std::vector<DevBuf> old;                  // outgrown buffers: freed when the call is done with the store
         uint32_t mh = 1;
+        void reset() {                            // empty, its rows and outgrown buffers freed (hdr and na stay)
+            key.release(); nf.release(); ids.release();
+            old.clear();
+            cap_rows = cap_ids = hi_rows = hi_ids = 0;
+        }
     };
     std::vector<RowStore> rs;
     DevBuf rs_val, rs_pos, rs_tmp, rs_rank;
-    cudaStream_t s_tail = nullptr;
+    Stream s_tail;
     int overlap = 1, stats = 0, defer_fetch = 0;
     bool fetch_pending = false, fetch_started = false;   // a count table waits on the device for nb200_fetch_counts / its copies are in flight
     uint32_t items_cap = 0;
     // per read
     DevBuf results, feats, row_nf;
     int32_t feats_stride = 0;
-    Counters *d_ctr = nullptr;
+    DevBuf d_ctr, d_ctr_odd;                      // Counters: bb[0].ctr is d_ctr, bb[1].ctr is d_ctr_odd
     // aggregation
     DevBuf flag, permA, permB, k32A, k32B, k64A, k64B, num, cub_tmp, gstart, head;
     DevBuf u_cell, u_n, u_list, s_rep, s_S, s_U, s_fs, s_fc, s_flags;
     DevBuf row_n, row_off, slow, htable, rep_of, is_rep, cell_ord, rank_of, gstart2;
     DevBuf o_cell_d, o_count_d, o_n_d, o_list_d, gen_feats, gen_nf, gen_off, gen_score, gen_key;
     // count table lives in pinned host memory owned by the context
-    uint32_t *h_cell = nullptr, *h_count = nullptr, *h_off = nullptr, *h_ids = nullptr;
-    size_t h_rows_cap = 0, h_ids_cap = 0;
+    PinnedBuf<uint32_t> h_cell, h_count, h_off, h_ids;
     DevBuf o_off_d, o_ids_d;
     nb200_timing timing{};
     uint64_t launches = 0;
@@ -165,7 +213,7 @@ struct nb200_ctx {
     // fastq-to-bam: whitelists + one resident barcode batch
     std::vector<std::unique_ptr<DevWhitelist>> wls;
     DevBuf cb_chars, cb_qual, cb_elig, cb_keys, cb_idx, cb_status, cb_inval, cb_inval_chars, cb_hit;
-    CbCounters *d_cbctr = nullptr;
+    DevBuf d_cbctr;                               // CbCounters
     uint64_t cb_n = 0;
     int cb_len = 0;
     bool cb_has_elig = false, cb_resident = false;
@@ -177,10 +225,10 @@ constexpr int kWideBlocks = 64;   // persistent grid of the wide-read kernel (4 
 namespace nb200 {
 
 static cudaEvent_t new_event(nb200_ctx *c) {
-    cudaEvent_t e;
-    CK(cudaEventCreate(&e));
-    c->ev_pool.push_back(e);
-    return e;
+    Event e;
+    CK(cudaEventCreate(&e.h));
+    c->ev_pool.push_back(std::move(e));
+    return c->ev_pool.back();
 }
 
 __global__ void end_batch_kernel(Counters *ctr) {
@@ -525,19 +573,9 @@ static void sort_by_feature_string(nb200_ctx *c, const DevLibrary &L, uint32_t m
 
 // the count table lives in pinned host memory owned by the context
 static void ensure_host_table(nb200_ctx *c, size_t nrows, size_t ids) {
-    if (nrows + 1 > c->h_rows_cap) {
-        for (uint32_t **p : {&c->h_cell, &c->h_count, &c->h_off}) { if (*p) cudaFreeHost(*p); *p = nullptr; }
-        c->h_rows_cap = nrows + nrows / 4 + 1024;
-        CK(cudaMallocHost(&c->h_cell, c->h_rows_cap * 4));
-        CK(cudaMallocHost(&c->h_count, c->h_rows_cap * 4));
-        CK(cudaMallocHost(&c->h_off, c->h_rows_cap * 4));
-    }
-    if (ids + 1 > c->h_ids_cap) {
-        if (c->h_ids) cudaFreeHost(c->h_ids);
-        c->h_ids = nullptr;
-        c->h_ids_cap = ids + ids / 4 + 1024;
-        CK(cudaMallocHost(&c->h_ids, c->h_ids_cap * 4));
-    }
+    auto grow = [](PinnedBuf<uint32_t> &b, size_t n) { if (n + 1 > b.cap) b.ensure(n + n / 4 + 1024); };
+    grow(c->h_cell, nrows); grow(c->h_count, nrows); grow(c->h_off, nrows);
+    grow(c->h_ids, ids);
 }
 
 static int bits_for(uint64_t n) { int b = 1; while ((1ull << b) < n) b++; return b; }
@@ -553,10 +591,10 @@ static void aggregate(nb200_ctx *c, const DevLibrary &L, uint64_t n, const uint6
     if (c->fetch_started) { CK(cudaStreamSynchronize(c->s_copy[1])); c->fetch_started = false; }      // (a fetch nobody waited for)
     c->fetch_pending = false;
     host_rows(0, 0);
-    c->h_off[0] = 0;
+    c->h_off.p[0] = 0;
     auto finish = [&]() {
-        counts->cell = c->h_cell; counts->count = c->h_count;
-        counts->feat_off = c->h_off; counts->feat_ids = c->h_ids;
+        counts->cell = c->h_cell.p; counts->count = c->h_count.p;
+        counts->feat_off = c->h_off.p; counts->feat_ids = c->h_ids.p;
     };
     if (n == 0 || n > 0x7FFFFFF0ull) { if (n) throw LimitError("more than 2^31 rows in one call (CUB item counts are int)"); finish(); return; }
     const bool bulk = d_key == nullptr;
@@ -625,7 +663,7 @@ static void aggregate(nb200_ctx *c, const DevLibrary &L, uint64_t n, const uint6
                                                                    c->row_off.as<uint32_t>(), uo, c->slow.as<uint32_t>(), dv);
         umi_general_kernel<<<c->sm_count * 16, 128, 0, c->s_compute>>>(c->slow.as<uint32_t>(), dv, G, c->gstart.as<uint32_t>(), m,
                                                                        c->permA.as<uint32_t>(), c->k64B.as<uint64_t>(), rows, d_score,
-                                                                       threshold, disable, sc, uo, c->d_ctr);
+                                                                       threshold, disable, sc, uo, c->d_ctr.as<Counters>());
         c->launches += 2;
         d_gstart = c->gstart.as<uint32_t>();
     } else {
@@ -685,11 +723,11 @@ static void aggregate(nb200_ctx *c, const DevLibrary &L, uint64_t n, const uint6
                                                                         c->o_count_d.as<uint32_t>(), c->o_n_d.as<uint32_t>());
     const bool defer = c->defer_fetch != 0;       // the table stays on the device until nb200_fetch_counts (nb200_set_defer_fetch)
     if (!defer) {
-        CK(cudaMemcpyAsync(c->h_cell, c->o_cell_d.p, (size_t)n_out * 4, cudaMemcpyDeviceToHost, c->s_compute));
-        CK(cudaMemcpyAsync(c->h_count, c->o_count_d.p, (size_t)n_out * 4, cudaMemcpyDeviceToHost, c->s_compute));
+        CK(cudaMemcpyAsync(c->h_cell.p, c->o_cell_d.p, (size_t)n_out * 4, cudaMemcpyDeviceToHost, c->s_compute));
+        CK(cudaMemcpyAsync(c->h_count.p, c->o_count_d.p, (size_t)n_out * 4, cudaMemcpyDeviceToHost, c->s_compute));
     }
     excl_scan_u32(c, c->o_n_d.as<uint32_t>(), c->o_off_d.as<uint32_t>(), n_out + 1);
-    if (!defer) CK(cudaMemcpyAsync(c->h_off, c->o_off_d.p, (size_t)(n_out + 1) * 4, cudaMemcpyDeviceToHost, c->s_compute));
+    if (!defer) CK(cudaMemcpyAsync(c->h_off.p, c->o_off_d.p, (size_t)(n_out + 1) * 4, cudaMemcpyDeviceToHost, c->s_compute));
     emit_ids_kernel<<<nblk(n_out, 128), 128, 0, c->s_compute>>>(n_out, c->gstart2.as<uint32_t>(), c->permA.as<uint32_t>(), lists,
                                                                  c->o_off_d.as<uint32_t>(), c->o_ids_d.as<uint32_t>());
     c->launches += 4;
@@ -700,9 +738,9 @@ static void aggregate(nb200_ctx *c, const DevLibrary &L, uint64_t n, const uint6
         c->fetch_pending = true;
         return;                                   // host pointers of `counts` stay null: nb200_fetch_counts fills them
     }
-    CK(cudaMemcpyAsync(c->h_ids, c->o_ids_d.p, (size_t)n_ids * 4, cudaMemcpyDeviceToHost, c->s_compute));
+    CK(cudaMemcpyAsync(c->h_ids.p, c->o_ids_d.p, (size_t)n_ids * 4, cudaMemcpyDeviceToHost, c->s_compute));
     CK(cudaStreamSynchronize(c->s_compute));
-    if (c->h_off[n_out] != n_ids) throw std::runtime_error("internal: id count of the table disagrees with its offsets");
+    if (c->h_off.p[n_out] != n_ids) throw std::runtime_error("internal: id count of the table disagrees with its offsets");
     c->timing.d2h_bytes += (uint64_t)n_out * 12 + 4 + (uint64_t)n_ids * 4;
     counts->n_rows = n_out;
     c->dev_rows = n_out; c->dev_ids = n_ids;
@@ -789,7 +827,7 @@ static void run_align(nb200_ctx *c, DevLibrary &L, const HostInput *in, double t
         CK(cudaMemsetAsync(c->bb[1].ctr, 0, sizeof(Counters), c->s_compute));
         c->timing = nb200_timing{};
         c->launches = 0;
-        CK(cudaMemsetAsync(c->d_ctr, 0, sizeof(Counters), c->s_compute));
+        CK(cudaMemsetAsync(c->d_ctr.p, 0, sizeof(Counters), c->s_compute));
         cudaEvent_t e0 = new_event(c), e1 = new_event(c), e_h2d = new_event(c);
         std::vector<cudaEvent_t> ev, ev_pk;
         if (in) {
@@ -834,12 +872,12 @@ static void run_align(nb200_ctx *c, DevLibrary &L, const HostInput *in, double t
         }
         // every batch's tail done, odd-batch counters folded into the main ones
         for (auto &bbuf : c->bb) if (bbuf.busy && c->overlap) CK(cudaStreamWaitEvent(c->s_compute, bbuf.tail_done, 0));
-        merge_counters_kernel<<<1, kCtrSpread, 0, c->s_compute>>>(c->d_ctr, c->bb[1].ctr);
+        merge_counters_kernel<<<1, kCtrSpread, 0, c->s_compute>>>(c->d_ctr.as<Counters>(), c->bb[1].ctr);
         cudaEvent_t e_agg = new_event(c);
         CK(cudaEventRecord(e_agg, c->s_compute));
         // counters (overflow check + max_nf) before the aggregation sizes its sorts
         struct { Counters c; } hc;
-        CK(cudaMemcpyAsync(&hc, c->d_ctr, sizeof(hc), cudaMemcpyDeviceToHost, c->s_compute));
+        CK(cudaMemcpyAsync(&hc, c->d_ctr.p, sizeof(hc), cudaMemcpyDeviceToHost, c->s_compute));
         CK(cudaStreamSynchronize(c->s_compute));
         c->timing.d2h_bytes += sizeof(hc);
         if (hc.c.overflow) {   // SW work list did not fit: grow to the measured demand and redo
@@ -851,7 +889,7 @@ static void run_align(nb200_ctx *c, DevLibrary &L, const HostInput *in, double t
         CK(cudaEventRecord(e1, c->s_compute));
         CK(cudaStreamSynchronize(c->s_compute));
         Counters h2;
-        CK(cudaMemcpy(&h2, c->d_ctr, sizeof(h2), cudaMemcpyDeviceToHost));
+        CK(cudaMemcpy(&h2, c->d_ctr.p, sizeof(h2), cudaMemcpyDeviceToHost));
         counts->dropped_empty = h2.dropped_empty;
         float ms = 0;
         CK(cudaEventElapsedTime(&ms, e0, e1)); c->timing.total_ms = ms;
@@ -879,7 +917,6 @@ static void run_align(nb200_ctx *c, DevLibrary &L, const HostInput *in, double t
         for (int i = 0; i < kCtrSpread; i++) { c->timing.probes += h2.probes[i]; c->timing.probe_slots += h2.probe_slots[i]; }
         c->timing.sw_pairs = h2.sw_pairs; c->timing.sw_cells = h2.sw_cells; c->timing.sw_items = h2.sw_pairs + h2.sw_dups;
         c->timing.launches = c->launches;
-        for (cudaEvent_t x : c->ev_pool) cudaEventDestroy(x);
         c->ev_pool.clear();
         return;
     }
@@ -917,6 +954,19 @@ bool lane_trim(nb200_ctx *c, int32_t lib_id, int *target, double *strictness) {
     return h.trim_on;
 }
 
+// Grow three arrays that work queued on stream s may still read or write: each gets a new buffer of `bytes`, its first
+// `keep` bytes copied over on s; the old buffer goes to `retired`, which the caller frees only when the store is reset.
+struct Regrow { DevBuf &buf; size_t bytes, keep; };
+static void grow_keep_retire(const Regrow (&a)[3], cudaStream_t s, std::vector<DevBuf> &retired) {
+    DevBuf fresh[3];
+    for (int i = 0; i < 3; i++) fresh[i].ensure(a[i].bytes);
+    for (int i = 0; i < 3; i++) {
+        if (a[i].keep) CK(cudaMemcpyAsync(fresh[i].p, a[i].buf.p, a[i].keep, cudaMemcpyDeviceToDevice, s));
+        if (a[i].buf.p) retired.push_back(std::move(a[i].buf));
+        a[i].buf = std::move(fresh[i]);
+    }
+}
+
 // Counts mode: append the slab's rows of store li behind its calling kernels, on s_copy[1] (the stream every lane's
 // result copies use, so that the appends of the two lanes follow one another).  The store grows geometrically; what it
 // must hold is known on the host without a synchronise: its end as of the last segment seen (lane_wait) plus, at most,
@@ -930,17 +980,8 @@ static void append_rows(nb200_ctx *c, nb200_ctx::FileLane &F, int li, uint64_t n
     const uint64_t need_r = live_r + n, need_i = live_i + n * mh;
     if (need_r > S.cap_rows || need_i > S.cap_ids) {
         const uint64_t cr = std::max(need_r, 2 * S.cap_rows), ci = std::max(need_i, 2 * S.cap_ids);
-        DevBuf k, f, d;
-        k.ensure(cr * 8); f.ensure(cr * 4); d.ensure(ci * 4);
         const uint64_t keep_r = std::min(live_r, S.cap_rows), keep_i = std::min(live_i, S.cap_ids);
-        if (keep_r) {
-            CK(cudaMemcpyAsync(k.p, S.key.p, keep_r * 8, cudaMemcpyDeviceToDevice, sd));
-            CK(cudaMemcpyAsync(f.p, S.nf.p, keep_r * 4, cudaMemcpyDeviceToDevice, sd));
-        }
-        if (keep_i) CK(cudaMemcpyAsync(d.p, S.ids.p, keep_i * 4, cudaMemcpyDeviceToDevice, sd));
-        // the old buffers may still be read by work queued on sd: freed only when the call is done with the store
-        for (DevBuf *b : {&S.key, &S.nf, &S.ids}) if (b->p) S.old.push_back(*b);
-        S.key = k; S.nf = f; S.ids = d;
+        grow_keep_retire({{S.key, cr * 8, keep_r * 8}, {S.nf, cr * 4, keep_r * 4}, {S.ids, ci * 4, keep_i * 4}}, sd, S.old);
         S.cap_rows = cr; S.cap_ids = ci;
     }
     c->rs_val.ensure((n + 1) * 8); c->rs_pos.ensure((n + 1) * 8);
@@ -955,7 +996,7 @@ static void append_rows(nb200_ctx *c, nb200_ctx::FileLane &F, int li, uint64_t n
     if (n) row_scatter_kernel<<<nblk(n, 256), 256, 0, sd>>>((uint32_t)n, F.key.as<uint64_t>(), feats, mh, c->rs_pos.as<uint64_t>(),
                                                      S.hdr.as<unsigned long long>(), S.key.as<uint64_t>(), S.nf.as<uint32_t>(), S.ids.as<int32_t>());
     row_advance_kernel<<<1, 1, 0, sd>>>(c->rs_pos.as<uint64_t>() + n, S.hdr.as<unsigned long long>(), seg);
-    CK(cudaMemcpyAsync(F.h_seg + 5 * (size_t)li, seg, 5 * 8, cudaMemcpyDeviceToHost, sd));
+    CK(cudaMemcpyAsync(F.h_seg.p + 5 * (size_t)li, seg, 5 * 8, cudaMemcpyDeviceToHost, sd));
     c->launches += 4;
 }
 
@@ -1006,16 +1047,8 @@ static void lane_cb_slab(nb200_ctx *c, nb200_ctx::FileLane &F, uint64_t n) {
     const uint64_t need = c->tx_hi + other + n;
     if (need > c->tx_cap) {                          // grow: copy on s_compute (every log write is on it), free at the end
         const uint64_t cap = std::max(need, 2 * c->tx_cap);
-        DevBuf k, o, ch;
-        k.ensure(cap * 8); o.ensure(cap * 8); ch.ensure(cap * 4);
         const uint64_t keep = std::min(c->tx_hi + other, c->tx_cap);
-        if (keep) {
-            CK(cudaMemcpyAsync(k.p, c->tx_key.p, keep * 8, cudaMemcpyDeviceToDevice, s));
-            CK(cudaMemcpyAsync(o.p, c->tx_ord.p, keep * 8, cudaMemcpyDeviceToDevice, s));
-            CK(cudaMemcpyAsync(ch.p, c->tx_choice.p, keep * 4, cudaMemcpyDeviceToDevice, s));
-        }
-        for (DevBuf *b : {&c->tx_key, &c->tx_ord, &c->tx_choice}) if (b->p) c->tx_old.push_back(*b);
-        c->tx_key = k; c->tx_ord = o; c->tx_choice = ch;
+        grow_keep_retire({{c->tx_key, cap * 8, keep * 8}, {c->tx_ord, cap * 8, keep * 8}, {c->tx_choice, cap * 4, keep * 4}}, s, c->tx_old);
         c->tx_cap = cap;
     }
     const uint64_t nb = std::max<uint64_t>(n, 1);
@@ -1032,8 +1065,8 @@ static void lane_cb_slab(nb200_ctx *c, nb200_ctx::FileLane &F, uint64_t n) {
         c->launches++;
     }
     // (read after lane_wait: the lane's done event follows these copies through s_compute's tail)
-    CK(cudaMemcpyAsync(F.h_cb, ctr, sizeof(CbCounters), cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(F.h_cb + 8, c->tx_n.p, 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(F.h_cb.p, ctr, sizeof(CbCounters), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(F.h_cb.p + 8, c->tx_n.p, 8, cudaMemcpyDeviceToHost, s));
 }
 
 void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_reads *r2, const int32_t *lib_ids, int n_libs,
@@ -1048,12 +1081,8 @@ void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_read
     const uint64_t n = r1->n;
     if (is_compact(r1) || (r2 && is_compact(r2))) throw std::runtime_error("file lanes take full records");
     if (n > (1ull << 21) || (r2 && n > (1ull << 20))) throw std::runtime_error("slab larger than a batch");
-    if (!F.h2d_done) { CK(cudaEventCreateWithFlags(&F.h2d_done, cudaEventDisableTiming)); CK(cudaEventCreateWithFlags(&F.done, cudaEventDisableTiming)); }
-    if ((size_t)n_libs > F.h_ctr_cap) {
-        if (F.h_ctr) cudaFreeHost(F.h_ctr);
-        CK(cudaMallocHost(&F.h_ctr, sizeof(Counters) * (size_t)n_libs));
-        F.h_ctr_cap = (size_t)n_libs;
-    }
+    if (!F.h2d_done) { CK(cudaEventCreateWithFlags(&F.h2d_done.h, cudaEventDisableTiming)); CK(cudaEventCreateWithFlags(&F.done.h, cudaEventDisableTiming)); }
+    F.h_ctr.ensure((size_t)n_libs);
     F.hr1 = *r1; F.paired = r2 != nullptr; if (r2) F.hr2 = *r2;
     F.libs.assign(lib_ids, lib_ids + n_libs);
     F.out_res.clear(); F.out_feats.clear();
@@ -1061,13 +1090,8 @@ void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_read
     if (out_feats) F.out_feats.assign(out_feats, out_feats + n_libs);
     F.hkey = key; F.n_rows_max = key ? n : 0;
     F.hcb = cb; F.hcbq = cb_qual; F.seq = seq;
-    if (cb && !F.h_cb) CK(cudaMallocHost(&F.h_cb, 9 * 8));
-    if (key && (size_t)n_libs > F.h_seg_cap) {
-        if (F.h_seg) cudaFreeHost(F.h_seg);
-        F.h_seg = nullptr; F.h_seg_cap = 0;
-        CK(cudaMallocHost(&F.h_seg, 5 * 8 * (size_t)n_libs));
-        F.h_seg_cap = (size_t)n_libs;
-    }
+    if (cb) F.h_cb.ensure(9);
+    if (key) F.h_seg.ensure(5 * (size_t)n_libs);
     F.hlen1.clear(); F.hlen2.clear();
     if (len1) F.hlen1.assign(len1, len1 + n_libs);
     if (len2 && r2) F.hlen2.assign(len2, len2 + n_libs);
@@ -1157,7 +1181,7 @@ void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_read
             if (out_feats && out_feats[li]) CK(cudaMemcpyAsync(out_feats[li], io.feats, n * (size_t)mh * 4, cudaMemcpyDeviceToHost, sd));
         }
         if (key) append_rows(c, F, li, n, io.res, io.feats, mh);
-        CK(cudaMemcpyAsync(&F.h_ctr[li], B.ctr, sizeof(Counters), cudaMemcpyDeviceToHost, sd));
+        CK(cudaMemcpyAsync(&F.h_ctr.p[li], B.ctr, sizeof(Counters), cudaMemcpyDeviceToHost, sd));
         // the next library (or the next slab on this lane) resets B.ctr: not before this copy has read it
         CK(cudaEventRecord(F.done, sd));
         CK(cudaStreamWaitEvent(c->s_compute, F.done, 0));
@@ -1174,21 +1198,21 @@ void lane_wait(nb200_ctx *c, int lane) {
         F.busy = false;
         if (F.hkey)                                     // counts mode: where the stores end now (a re-run appends anew)
             for (size_t li = 0; li < F.libs.size(); li++) {
-                const unsigned long long *s = F.h_seg + 5 * li;
+                const unsigned long long *s = F.h_seg.p + 5 * li;
                 nb200_ctx::RowStore &S = c->rs[li];
                 S.hi_rows = std::max<uint64_t>(S.hi_rows, s[0] + s[1]);
                 S.hi_ids = std::max<uint64_t>(S.hi_ids, s[2] + s[3]);
             }
         if (F.hcb) {
-            c->tx_hi = std::max<uint64_t>(c->tx_hi, F.h_cb[8]);
+            c->tx_hi = std::max<uint64_t>(c->tx_hi, F.h_cb.p[8]);
             // a pair fastq-to-bam writes (barcode corrected) that it or align on its BAM refuses: CbCounters::pad
-            const unsigned long long bad = F.h_cb[7];
+            const unsigned long long bad = F.h_cb.p[7];
             if (bad & kTenxLongName) throw std::runtime_error("read name longer than 254 bytes");
             if (bad & kTenxLongRead) throw std::runtime_error("read longer than 500 bases");
         }
         unsigned long long need = 0;
         for (size_t li = 0; li < F.libs.size(); li++)
-            if (F.h_ctr[li].overflow) need = std::max(need, F.h_ctr[li].items_max);
+            if (F.h_ctr.p[li].overflow) need = std::max(need, F.h_ctr.p[li].items_max);
         if (!need) return;
         if (attempt >= 3) throw std::runtime_error("Smith-Waterman work list kept overflowing");
         // the work list did not fit: grow it to the measured demand (cudaFree waits for the other lane) and redo the slab
@@ -1206,16 +1230,11 @@ void lane_wait(nb200_ctx *c, int lane) {
 
 void lane_rows_begin(nb200_ctx *c, const int32_t *lib_ids, int n_libs) {
     CK(cudaSetDevice(c->device));
-    for (auto &S : c->rs) {                         // (a previous call's stores)
-        for (DevBuf *b : {&S.key, &S.nf, &S.ids}) b->release();
-        for (auto &b : S.old) b.release();
-        S.old.clear();
-    }
+    for (auto &S : c->rs) S.reset();                // (a previous call's stores)
     c->rs.resize((size_t)n_libs);
     for (int li = 0; li < n_libs; li++) {
         const HostLibrary &h = lane_lib(c, lib_ids[li]).host;
         nb200_ctx::RowStore &S = c->rs[(size_t)li];
-        S.cap_rows = S.cap_ids = S.hi_rows = S.hi_ids = 0;
         S.mh = (uint32_t)std::max(1, h.cfg.max_hits_to_report);
         std::vector<uint8_t> na(h.feature_names.size() + 1, 0);
         for (size_t f = 0; f < h.feature_names.size(); f++) {
@@ -1237,7 +1256,7 @@ void lane_rows_begin(nb200_ctx *c, const int32_t *lib_ids, int n_libs) {
 void lane_rows_segments(nb200_ctx *c, int lane, RowSeg *out) {
     const nb200_ctx::FileLane &F = c->lane[lane];
     for (size_t li = 0; li < F.libs.size(); li++) {
-        const unsigned long long *s = F.h_seg + 5 * li;
+        const unsigned long long *s = F.h_seg.p + 5 * li;
         out[li].row0 = s[0]; out[li].rows = s[1]; out[li].id0 = s[2]; out[li].ids = s[3]; out[li].called = s[4];
     }
 }
@@ -1319,28 +1338,23 @@ void lane_rows_count(const std::vector<nb200_ctx *> &ctxs, int li, int32_t lib_i
         }
         c->launches++;
     }
-    CK(cudaMemsetAsync(c->d_ctr, 0, sizeof(Counters), s));
+    CK(cudaMemsetAsync(c->d_ctr.p, 0, sizeof(Counters), s));
     // the aligner writes nimble_score = 1 for every row: score NULL
     aggregate(c, L, R, c->gen_key.as<uint64_t>(), Rows{c->gen_feats.as<int32_t>(), c->gen_off.as<uint32_t>(), nullptr, nullptr, 0}, nullptr,
               0, threshold, disable, counts);
     CK(cudaStreamSynchronize(s));
     Counters h2;
-    CK(cudaMemcpy(&h2, c->d_ctr, sizeof(h2), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(&h2, c->d_ctr.p, sizeof(h2), cudaMemcpyDeviceToHost));
     counts->dropped_empty = h2.dropped_empty;
     if (dropped.p) {                                // rows whose cell is a pandas NA token: report never reads them
         unsigned long long d = 0;
         CK(cudaMemcpy(&d, dropped.p, 8, cudaMemcpyDeviceToHost));
         *rows = R - d;
     }
-    runs.release(); dropped.release();
     // the stores of this library are done with
     for (nb200_ctx *x : ctxs) {
         CK(cudaSetDevice(x->device));
-        nb200_ctx::RowStore &S = x->rs[(size_t)li];
-        for (DevBuf *b : {&S.key, &S.nf, &S.ids}) b->release();
-        for (auto &b : S.old) b.release();
-        S.old.clear();
-        S.cap_rows = S.cap_ids = 0;
+        x->rs[(size_t)li].reset();
     }
     CK(cudaSetDevice(c->device));
 }
@@ -1398,21 +1412,26 @@ static std::unique_ptr<DevWhitelist> build_whitelist(nb200_ctx *c, std::vector<s
 }
 
 // ---- fastq-to-counts: the whitelist on every context, the cache rule over every context's log (slab_api.hpp) ----------
+// the multi-candidate log back to empty, its buffers, outgrown buffers and decisions freed (current device: c's)
+static void reset_cb_log(nb200_ctx *c) {
+    for (DevBuf *b : {&c->tx_key, &c->tx_ord, &c->tx_choice, &c->tx_dec}) b->release();
+    c->tx_old.clear();
+    c->tx_cap = c->tx_hi = 0;
+    c->tx_base.clear();
+}
+
 void lane_cb_begin(const std::vector<nb200_ctx *> &ctxs, const std::vector<std::string> &whitelist, int cb_len,
                    std::vector<uint32_t> *rank, std::vector<std::string> *cells) {
     uint64_t n_unique = 0;
     const std::vector<WlSlot> tab = wl_slots(whitelist, cb_len, &n_unique);
     for (nb200_ctx *c : ctxs) {
         CK(cudaSetDevice(c->device));
+        reset_cb_log(c);
         c->tx_table.ensure(tab.size() * sizeof(WlSlot));
         CK(cudaMemcpy(c->tx_table.p, tab.data(), tab.size() * sizeof(WlSlot), cudaMemcpyHostToDevice));
         c->tx_wl = WlDev{c->tx_table.as<WlSlot>(), tab.size() - 1, cb_len};
         c->tx_n.ensure(8);
         CK(cudaMemset(c->tx_n.p, 0, 8));
-        c->tx_hi = 0;
-        for (auto &b : c->tx_old) b.release();
-        c->tx_old.clear();
-        c->tx_base.clear();
     }
     CK(cudaSetDevice(ctxs[0]->device));
     // cells: the distinct lines in byte order (= key order), pandas-NA tokens left out (report drops such a cell)
@@ -1433,7 +1452,7 @@ void lane_cb_begin(const std::vector<nb200_ctx *> &ctxs, const std::vector<std::
 }
 
 void lane_cb_counters(nb200_ctx *c, int lane, uint64_t *out6) {
-    const unsigned long long *h = c->lane[lane].h_cb;                 // CbCounters: n_miss n_inval perfect corrected none n_multi probes
+    const unsigned long long *h = c->lane[lane].h_cb.p;               // CbCounters: n_miss n_inval perfect corrected none n_multi probes
     out6[0] = h[2]; out6[1] = h[3]; out6[2] = h[4]; out6[3] = h[0]; out6[4] = h[5]; out6[5] = h[6];
 }
 
@@ -1479,17 +1498,13 @@ void lane_cb_resolve(const std::vector<nb200_ctx *> &ctxs) {
     cub_sort64(c, ord.as<uint64_t>(), sorted.as<uint64_t>(), perm.as<uint32_t>() + E, perm.as<uint32_t>(), (uint32_t)E, 64);
     cb_first_decides(c, perm.as<uint32_t>(), key.as<uint64_t>(), (uint32_t)E, c->tx_dec.as<int32_t>());
     CK(cudaStreamSynchronize(s));
-    for (DevBuf *b : {&key, &ord, &sorted, &perm}) b->release();
 }
 
 void lane_cb_end(const std::vector<nb200_ctx *> &ctxs) {
     for (nb200_ctx *c : ctxs) {
         CK(cudaSetDevice(c->device));
-        for (DevBuf *b : {&c->tx_table, &c->tx_key, &c->tx_ord, &c->tx_choice, &c->tx_dec}) b->release();
-        for (auto &b : c->tx_old) b.release();
-        c->tx_old.clear();
-        c->tx_cap = c->tx_hi = 0;
-        c->tx_base.clear();
+        c->tx_table.release();
+        reset_cb_log(c);
     }
     CK(cudaSetDevice(ctxs[0]->device));
 }
@@ -1542,10 +1557,10 @@ static void cb_run(nb200_ctx *c, DevWhitelist &W, nb200_cb_stats *st) {
     const uint64_t launches0 = c->launches;
     cb_launch(c, W.dev, s, c->cb_chars.as<uint8_t>(), c->cb_qual.as<uint8_t>(), c->cb_has_elig ? c->cb_elig.as<uint8_t>() : nullptr, n,
               c->cb_keys.as<uint64_t>(), c->cb_idx.as<int32_t>(), c->cb_status.as<uint8_t>(), c->permA.as<uint32_t>(),
-              c->cb_inval.as<uint32_t>(), (uint32_t)n, st ? c->cb_hit.as<uint8_t>() : nullptr, c->flag.as<uint8_t>(), c->d_cbctr);
+              c->cb_inval.as<uint32_t>(), (uint32_t)n, st ? c->cb_hit.as<uint8_t>() : nullptr, c->flag.as<uint8_t>(), c->d_cbctr.as<CbCounters>());
     CbCounters h{};
     if (n) {
-        CK(cudaMemcpyAsync(&h, c->d_cbctr, sizeof h, cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(&h, c->d_cbctr.p, sizeof h, cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));
         if (h.n_multi) {
             // the reference's correction_cache: first read in file order decides per raw barcode
@@ -1615,11 +1630,6 @@ static void cb_run(nb200_ctx *c, DevWhitelist &W, nb200_cb_stats *st) {
     }
 }
 
-static void drop_events(nb200_ctx *c) {
-    for (cudaEvent_t x : c->ev_pool) cudaEventDestroy(x);
-    c->ev_pool.clear();
-}
-
 static void cb_fetch(nb200_ctx *c, int32_t *out_idx, uint8_t *out_status, nb200_cb_stats *st) {
     const uint64_t n = c->cb_n;
     if (n && out_idx) CK(cudaMemcpyAsync(out_idx, c->cb_idx.p, n * 4, cudaMemcpyDeviceToHost, c->s_compute));
@@ -1668,28 +1678,21 @@ int32_t nb200_create(int32_t device, int32_t host_threads, nb200_ctx **out) {
         cudaDeviceProp p;
         CK(cudaGetDeviceProperties(&p, device));
         c->sm_count = p.multiProcessorCount;
-        CK(cudaStreamCreateWithFlags(&c->s_compute, cudaStreamNonBlocking));
-        {   // the copy streams also run the tiny record-expansion kernels of the compact wire form: highest priority, so
-            // that they get an SM slot as soon as a block of the running probe kernel retires and never hold up the DMA queue
-            int least = 0, greatest = 0;
-            CK(cudaDeviceGetStreamPriorityRange(&least, &greatest));
-            CK(cudaStreamCreateWithPriority(&c->s_copy[0], cudaStreamNonBlocking, greatest));
-            CK(cudaStreamCreateWithPriority(&c->s_copy[1], cudaStreamNonBlocking, greatest));
-        }
-        CK(cudaMalloc(&c->d_ctr, sizeof(Counters) + 64));
-        CK(cudaMemset(c->d_ctr, 0, sizeof(Counters) + 64));
-        CK(cudaMalloc(&c->bb[1].ctr, sizeof(Counters) + 64));
-        CK(cudaMemset(c->bb[1].ctr, 0, sizeof(Counters) + 64));
-        c->bb[0].ctr = c->d_ctr;
-        {
-            int least = 0, greatest = 0;
-            CK(cudaDeviceGetStreamPriorityRange(&least, &greatest));
-            CK(cudaStreamCreateWithPriority(&c->s_tail, cudaStreamNonBlocking, greatest));
-        }
-        for (auto &b : c->bb) { CK(cudaEventCreateWithFlags(&b.tail_done, cudaEventDisableTiming)); CK(cudaEventCreateWithFlags(&b.probe_done, cudaEventDisableTiming)); }
+        CK(cudaStreamCreateWithFlags(&c->s_compute.h, cudaStreamNonBlocking));
+        // highest priority: the copy streams also run the tiny record-expansion kernels of the compact wire form, so that
+        // they get an SM slot as soon as a block of the running probe kernel retires and never hold up the DMA queue; s_tail
+        // runs each batch's latency-bound tail beside the next batch's probe
+        int least = 0, greatest = 0;
+        CK(cudaDeviceGetStreamPriorityRange(&least, &greatest));
+        for (Stream *s : {&c->s_copy[0], &c->s_copy[1], &c->s_tail}) CK(cudaStreamCreateWithPriority(&s->h, cudaStreamNonBlocking, greatest));
+        auto counters = [](DevBuf &b, size_t bytes) { CK(cudaMalloc(&b.p, bytes)); b.cap = bytes; CK(cudaMemset(b.p, 0, bytes)); };
+        counters(c->d_ctr, sizeof(Counters) + 64);
+        counters(c->d_ctr_odd, sizeof(Counters) + 64);
+        counters(c->d_cbctr, sizeof(CbCounters) + 64);
+        c->bb[0].ctr = c->d_ctr.as<Counters>();
+        c->bb[1].ctr = c->d_ctr_odd.as<Counters>();
+        for (auto &b : c->bb) { CK(cudaEventCreateWithFlags(&b.tail_done.h, cudaEventDisableTiming)); CK(cudaEventCreateWithFlags(&b.probe_done.h, cudaEventDisableTiming)); }
         if (const char *e = getenv("NB200_OVERLAP")) c->overlap = atoi(e) != 0;
-        CK(cudaMalloc(&c->d_cbctr, sizeof(CbCounters) + 64));
-        CK(cudaMemset(c->d_cbctr, 0, sizeof(CbCounters) + 64));
         c->l2_persist_max = (size_t)std::max(0, p.persistingL2CacheMaxSize);
         c->l2_window_max = (size_t)std::max(0, p.accessPolicyMaxWindowSize);
         if (c->l2_persist_max && cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, c->l2_persist_max) != cudaSuccess) {
@@ -1708,45 +1711,7 @@ void nb200_destroy(nb200_ctx *c) {
     if (!c) return;
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
-    c->libs.clear();
-    for (DevBuf *b : {&c->d_r1, &c->d_r1len, &c->d_r2, &c->d_r2len, &c->d_key, &c->stage1, &c->stage2, &c->d_nidx, &c->d_nmask, &c->bb[0].ro, &c->bb[0].roB, &c->bb[0].items, &c->bb[0].sw_pairs, &c->bb[0].sw_rep, &c->bb[0].deferred, &c->bb[0].wide_list, &c->bb[0].sums, &c->bb[0].slow_list, &c->bb[1].sums, &c->bb[1].slow_list, &c->bb[0].setup_list, &c->bb[1].setup_list,
-                      &c->bb[1].ro, &c->bb[1].roB, &c->bb[1].items, &c->bb[1].sw_pairs, &c->bb[1].sw_rep, &c->bb[1].deferred, &c->bb[1].wide_list, &c->wide_scratch, &c->wide_v, &c->results,
-                      &c->feats, &c->row_nf, &c->flag, &c->permA, &c->permB, &c->k32A, &c->k32B, &c->k64A, &c->k64B,
-                      &c->num, &c->cub_tmp, &c->gstart, &c->head, &c->u_cell, &c->u_n, &c->u_list, &c->s_rep, &c->s_S,
-                      &c->s_U, &c->s_fs, &c->s_fc, &c->s_flags, &c->o_cell_d, &c->o_count_d, &c->o_n_d, &c->o_list_d, &c->o_off_d, &c->o_ids_d,
-                      &c->gen_feats, &c->gen_nf, &c->gen_off, &c->gen_score, &c->gen_key, &c->row_n, &c->row_off, &c->slow, &c->htable, &c->rep_of, &c->is_rep, &c->cell_ord, &c->rank_of, &c->gstart2,
-                      &c->cb_chars, &c->cb_qual, &c->cb_elig, &c->cb_keys, &c->cb_idx, &c->cb_status, &c->cb_inval, &c->cb_inval_chars, &c->cb_hit})
-        b->release();
-    for (auto &F : c->lane) {
-        for (DevBuf *b : {&F.r1, &F.l1, &F.r2, &F.l2}) b->release();
-        for (auto *v : {&F.res, &F.feats, &F.nf, &F.l1v, &F.l2v}) for (auto &b : *v) b.release();
-        if (F.h2d_done) cudaEventDestroy(F.h2d_done);
-        if (F.done) cudaEventDestroy(F.done);
-        if (F.h_ctr) cudaFreeHost(F.h_ctr);
-        F.key.release(); F.seg.release();
-        if (F.h_seg) cudaFreeHost(F.h_seg);
-        for (DevBuf *b : {&F.cb, &F.cbq, &F.cb_raw, &F.cb_idx, &F.cb_st, &F.cb_miss, &F.cb_multi, &F.cb_ctr}) b->release();
-        if (F.h_cb) cudaFreeHost(F.h_cb);
-    }
-    for (DevBuf *b : {&c->tx_table, &c->tx_key, &c->tx_ord, &c->tx_choice, &c->tx_n, &c->tx_dec}) b->release();
-    for (auto &b : c->tx_old) b.release();
-    for (auto &S : c->rs) {
-        for (DevBuf *b : {&S.key, &S.nf, &S.ids, &S.hdr, &S.na}) b->release();
-        for (auto &b : S.old) b.release();
-    }
-    for (DevBuf *b : {&c->rs_val, &c->rs_pos, &c->rs_tmp, &c->rs_rank}) b->release();
-    c->wls.clear();
-    if (c->d_cbctr) cudaFree(c->d_cbctr);
-    if (c->d_ctr) cudaFree(c->d_ctr);
-    if (c->bb[1].ctr) cudaFree(c->bb[1].ctr);
-    for (auto &b : c->bb) { if (b.tail_done) cudaEventDestroy(b.tail_done); if (b.probe_done) cudaEventDestroy(b.probe_done); }
-    if (c->s_tail) cudaStreamDestroy(c->s_tail);
-    for (uint32_t *p : {c->h_cell, c->h_count, c->h_off, c->h_ids}) if (p) cudaFreeHost(p);
-    for (cudaEvent_t e : c->ev_pool) cudaEventDestroy(e);
-    if (c->s_compute) cudaStreamDestroy(c->s_compute);
-    if (c->s_copy[0]) cudaStreamDestroy(c->s_copy[0]);
-    if (c->s_copy[1]) cudaStreamDestroy(c->s_copy[1]);
-    delete c;
+    delete c;                      // every buffer, pinned buffer, event and stream frees itself, with c's device current
 }
 
 const char *nb200_last_error(const nb200_ctx *c) { return c ? c->err.c_str() : g_create_err.c_str(); }
@@ -2370,7 +2335,7 @@ int32_t nb200_align_10x_fastq(nb200_ctx *c, const char *r1_fastq, const char *r2
         cb_upload(c, cb_len, (const char *)cb.data(), qual.data(), elig.data(), n, &dev);
         cb_run(c, *W, &dev);
         cb_fetch(c, idx.data(), status.data(), &dev);
-        drop_events(c);
+        c->ev_pool.clear();
         c->cb_resident = false;
         dev.total_pairs = st.total_pairs; dev.name_mismatch = st.name_mismatch; dev.too_short = st.too_short;
         dev.no_remaining_seq = st.no_remaining_seq;
@@ -2424,7 +2389,7 @@ int32_t nb200_umi_counts(nb200_ctx *c, int32_t lib_id, uint64_t n_rows, const ui
     c->gen_off.ensure((n_rows + 1) * 4 + 16); c->gen_feats.ensure(n_ids * 4 + 16); c->gen_key.ensure(n_rows * 8 + 16);
     cudaEvent_t e0 = new_event(c), e1 = new_event(c);
     CK(cudaEventRecord(e0, c->s_compute));
-    CK(cudaMemsetAsync(c->d_ctr, 0, sizeof(Counters), c->s_compute));
+    CK(cudaMemsetAsync(c->d_ctr.p, 0, sizeof(Counters), c->s_compute));
     if (n_rows) {
         CK(cudaMemcpyAsync(c->gen_off.p, off, (n_rows + 1) * 4, cudaMemcpyHostToDevice, c->s_compute));
         if (n_ids) CK(cudaMemcpyAsync(c->gen_feats.p, feat_ids, n_ids * 4, cudaMemcpyHostToDevice, c->s_compute));
@@ -2454,14 +2419,13 @@ int32_t nb200_umi_counts(nb200_ctx *c, int32_t lib_id, uint64_t n_rows, const ui
     CK(cudaEventRecord(e1, c->s_compute));
     CK(cudaStreamSynchronize(c->s_compute));
     Counters h2;
-    CK(cudaMemcpy(&h2, c->d_ctr, sizeof(h2), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(&h2, c->d_ctr.p, sizeof(h2), cudaMemcpyDeviceToHost));
     counts->dropped_empty = h2.dropped_empty;
     float ms = 0;
     CK(cudaEventElapsedTime(&ms, e0, e1)); c->timing.total_ms = ms;
     CK(cudaEventElapsedTime(&ms, e_in, e1)); c->timing.agg_ms = ms;
     CK(cudaEventElapsedTime(&ms, e0, e_in)); c->timing.h2d_ms = ms;
     c->timing.launches = c->launches;
-    for (cudaEvent_t x : c->ev_pool) cudaEventDestroy(x);
     c->ev_pool.clear();
     API_END(c)
 }
@@ -2564,8 +2528,8 @@ int32_t nb200_bench_dpx_peak(nb200_ctx *c, uint32_t iters, double *dpx_ginst_per
     if (!dpx_ginst_per_s || !row_gcups || iters < 16) throw std::runtime_error("bad arguments");
     DevBuf sink;
     sink.ensure(64);
-    cudaEvent_t e0, e1;
-    CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
+    Event e0, e1;
+    CK(cudaEventCreate(&e0.h)); CK(cudaEventCreate(&e1.h));
     const unsigned b_dpx = (unsigned)c->sm_count * 8, b_row = (unsigned)c->sm_count * 16;
     auto time_best = [&](auto launch) {
         launch(16u);                                            // warm-up
@@ -2584,10 +2548,8 @@ int32_t nb200_bench_dpx_peak(nb200_ctx *c, uint32_t iters, double *dpx_ginst_per
     const double s_dpx = time_best([&](uint32_t it) { dpx_peak_kernel<<<b_dpx, 256, 0, c->s_compute>>>(it, 12345u + it, sink.as<uint32_t>()); });
     const double s_row = time_best([&](uint32_t it) { sw_row_peak_kernel<<<b_row, 128, 0, c->s_compute>>>(it, 999u + it, sink.as<uint32_t>()); });
     CK(cudaGetLastError());
-    cudaEventDestroy(e0); cudaEventDestroy(e1);
     *dpx_ginst_per_s = (double)b_dpx * 256.0 * iters * 12.0 / s_dpx / 1e9;         // thread-level DPX instructions (s16x2 each)
     *row_gcups = (double)b_row * 128.0 * iters * (2.0 * kNB) / s_row / 1e9;         // two alignments per thread
-    sink.release();
     API_END(c)
 }
 
@@ -2646,7 +2608,7 @@ int32_t nb200_correct_barcodes_resident(nb200_ctx *c, int32_t wl_id, int32_t *ou
     cb_run(c, get_wl(c, wl_id), stats);
     cb_fetch(c, out_idx, out_status, stats);
     if (stats) stats->total_ms = stats->kernel_ms;
-    drop_events(c);
+    c->ev_pool.clear();
     API_END(c)
 }
 
@@ -2664,7 +2626,7 @@ int32_t nb200_correct_barcodes(nb200_ctx *c, int32_t wl_id, const char *cb, cons
     CK(cudaEventRecord(e1, c->s_compute));
     CK(cudaEventSynchronize(e1));
     if (stats) CK(cudaEventElapsedTime(&stats->total_ms, e0, e1));
-    drop_events(c);
+    c->ev_pool.clear();
     API_END(c)
 }
 
@@ -2699,7 +2661,7 @@ int32_t nb200_fastq_to_bam(nb200_ctx *c, const char *r1_fastq, const char *r2_fa
         CK(cudaEventRecord(e1, c->s_compute));
         CK(cudaEventSynchronize(e1));
         CK(cudaEventElapsedTime(&dev.total_ms, e0, e1));
-        drop_events(c);
+        c->ev_pool.clear();
         dev.total_pairs = st.total_pairs; dev.name_mismatch = st.name_mismatch; dev.too_short = st.too_short;
         dev.no_remaining_seq = st.no_remaining_seq;
         write_10x_bam(output_bam, A, B, cb_len, umi_len, idx.data(), status.data(), W->entries, c->host_threads, dev);
@@ -2718,8 +2680,8 @@ int32_t nb200_bench_random_access(nb200_ctx *c, uint64_t bytes, uint32_t iters, 
     const uint64_t n_sectors = bytes / 32;
     const unsigned blocks = (unsigned)c->sm_count * 16;
     iters = (iters + 3) & ~3u;
-    cudaEvent_t e0, e1;
-    CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
+    Event e0, e1;
+    CK(cudaEventCreate(&e0.h)); CK(cudaEventCreate(&e1.h));
     random_gather_kernel<<<blocks, 256, 0, c->s_compute>>>(buf.as<uint4>(), n_sectors, 64, 1, sink.as<uint32_t>());   // warm-up
     float best = 1e30f;
     for (int rep = 0; rep < 3; rep++) {
@@ -2731,11 +2693,9 @@ int32_t nb200_bench_random_access(nb200_ctx *c, uint64_t bytes, uint32_t iters, 
         CK(cudaEventElapsedTime(&ms, e0, e1));
         best = std::min(best, ms);
     }
-    cudaEventDestroy(e0); cudaEventDestroy(e1);
     const double loads = (double)blocks * 256.0 * iters;
     *gbytes_per_s = loads * 32.0 / (best * 1e-3) / 1e9;
     if (gloads_per_s) *gloads_per_s = loads / (best * 1e-3) / 1e9;
-    buf.release(); sink.release();
     API_END(c)
 }
 
@@ -2755,13 +2715,13 @@ int32_t nb200_set_defer_fetch(nb200_ctx *c, int32_t on) {
 static void start_table_fetch(nb200_ctx *c) {
     const uint64_t n_out = c->dev_rows, n_ids = c->dev_ids;
     ensure_host_table(c, n_out, n_ids);
-    c->h_off[0] = 0;
+    c->h_off.p[0] = 0;
     if (!c->fetch_pending || !n_out || c->fetch_started) return;
     cudaStream_t s = c->s_copy[1];
-    CK(cudaMemcpyAsync(c->h_cell, c->o_cell_d.p, (size_t)n_out * 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(c->h_count, c->o_count_d.p, (size_t)n_out * 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(c->h_off, c->o_off_d.p, (size_t)(n_out + 1) * 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(c->h_ids, c->o_ids_d.p, (size_t)n_ids * 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(c->h_cell.p, c->o_cell_d.p, (size_t)n_out * 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(c->h_count.p, c->o_count_d.p, (size_t)n_out * 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(c->h_off.p, c->o_off_d.p, (size_t)(n_out + 1) * 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(c->h_ids.p, c->o_ids_d.p, (size_t)n_ids * 4, cudaMemcpyDeviceToHost, s));
     c->fetch_started = true;
 }
 
@@ -2779,12 +2739,12 @@ int32_t nb200_fetch_counts(nb200_ctx *c, nb200_counts *counts) {
     if (c->fetch_pending && n_out) {
         CK(cudaStreamSynchronize(c->s_copy[1]));
         c->fetch_started = false;
-        if (c->h_off[n_out] != n_ids) throw std::runtime_error("internal: id count of the table disagrees with its offsets");
+        if (c->h_off.p[n_out] != n_ids) throw std::runtime_error("internal: id count of the table disagrees with its offsets");
         c->timing.d2h_bytes += n_out * 12 + 4 + n_ids * 4;
         c->fetch_pending = false;
     }
     counts->n_rows = n_out;
-    counts->cell = c->h_cell; counts->count = c->h_count; counts->feat_off = c->h_off; counts->feat_ids = c->h_ids;
+    counts->cell = c->h_cell.p; counts->count = c->h_count.p; counts->feat_off = c->h_off.p; counts->feat_ids = c->h_ids.p;
     API_END(c)
 }
 
