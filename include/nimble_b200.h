@@ -118,8 +118,9 @@ typedef struct nb200_timing {
     uint64_t launches;  /* kernels launched inside the call (ours + CUB)               */
     uint64_t h2d_bytes, d2h_bytes;
     uint64_t sw_items;  /* candidate pairs before identical band windows were merged   */
-    float probe_kernel_ms; /* probe_kernel alone (part of probe_ms, which also covers the calling kernels that follow it) */
+    float probe_kernel_ms; /* the probe kernels alone (part of probe_ms, which also covers the calling kernels that follow it) */
     float pad_;
+    uint64_t probe_warp_reads; /* single-end reads the thread-per-read probe left to the warp-per-read probe */
 } nb200_timing;
 
 typedef struct nb200_ctx nb200_ctx;

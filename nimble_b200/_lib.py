@@ -58,7 +58,8 @@ class Timing(ct.Structure):
                 ("agg_ms", ct.c_float), ("h2d_ms", ct.c_float), ("probes", ct.c_uint64), ("probe_slots", ct.c_uint64),
                 ("sw_pairs", ct.c_uint64), ("sw_cells", ct.c_uint64), ("launches", ct.c_uint64),
                 ("h2d_bytes", ct.c_uint64), ("d2h_bytes", ct.c_uint64), ("sw_items", ct.c_uint64),
-                ("probe_kernel_ms", ct.c_float), ("pad_", ct.c_float)]
+                ("probe_kernel_ms", ct.c_float), ("pad_", ct.c_float),
+                ("probe_warp_reads", ct.c_uint64)]
 
 
 class CbStats(ct.Structure):

@@ -110,6 +110,7 @@ struct DevLibrary {
     DevBuf min_score;        // score_percent as a per-length table (call_params), rebuilt when score_percent changes
     double min_score_for = 0.0;
     bool min_score_ok = false;
+    bool probe_warp = false;     // NB200_PROBE_WARP=1: every read through the warp-per-read probe (the in-tree reference)
     size_t table_bytes = 0, slab_bytes = 0;
 };
 
@@ -141,7 +142,7 @@ struct nb200_ctx {
     bool paired = false, has_key = false, resident = false;
     // per batch
     // per-batch state, double-buffered: batch k's alignment/calling kernels (s_tail) overlap batch k+1's probe (s_compute)
-    struct BatchBuf { DevBuf ro, roB, items, sw_pairs, sw_rep, deferred, wide_list, sums, slow_list, setup_list; Counters *ctr = nullptr; Event tail_done, probe_done; bool busy = false; } bb[2];
+    struct BatchBuf { DevBuf ro, roB, items, sw_pairs, sw_rep, deferred, wide_list, warp_list, sums, slow_list, setup_list; Counters *ctr = nullptr; Event tail_done, probe_done; bool busy = false; } bb[2];
     DevBuf wide_scratch, wide_v;
     // streaming file path: two slabs in flight, each with its own device buffers (slab_api.hpp)
     struct FileLane {
@@ -238,6 +239,8 @@ __global__ void end_batch_kernel(Counters *ctr) {
     ctr->alloc = 0;
     ctr->wide_total += ctr->n_wide;
     ctr->n_wide = 0;
+    ctr->probe_warp_total += ctr->n_probe_warp;
+    ctr->n_probe_warp = 0;
     ctr->sw_items += items;
     ctr->n_swpairs = 0;
     ctr->n_slow = 0;
@@ -252,6 +255,7 @@ __global__ void merge_counters_kernel(Counters *a, Counters *b) {
     if (t == 0) {
         a->overflow += b->overflow; a->sw_pairs += b->sw_pairs; a->sw_cells += b->sw_cells; a->sw_dups += b->sw_dups;
         a->sw_items += b->sw_items; a->deferred_total += b->deferred_total; a->wide_total += b->wide_total;
+        a->probe_warp_total += b->probe_warp_total; b->probe_warp_total = 0;
         if (b->max_nf > a->max_nf) a->max_nf = b->max_nf;
         if (b->items_max > a->items_max) a->items_max = b->items_max;
         b->overflow = 0; b->sw_pairs = 0; b->sw_cells = 0; b->sw_dups = 0; b->sw_items = 0; b->deferred_total = 0; b->wide_total = 0;
@@ -351,6 +355,7 @@ static void upload_library(nb200_ctx *c, DevLibrary &L) {
         L.dev.n_refs = h.n_refs; L.dev.n_features = h.n_features; L.dev.n_words = h.n_words;
         L.dev.narrow_cap = kCap;
         if (const char *e = getenv("NB200_NARROW_CAP")) L.dev.narrow_cap = (uint32_t)std::min<long>(kCap, std::max<long>(0, atol(e)));   // tests: force the wide path
+        if (const char *e = getenv("NB200_PROBE_WARP")) L.probe_warp = atol(e) != 0;
         L.dev.k = h.cfg.k; L.dev.identity = h.identity_features ? 1 : 0;
         L.dev.kmask = h.cfg.k == 32 ? ~0ull : ((1ull << (2 * h.cfg.k)) - 1);
         L.dev.kbits = h.cfg.k == 32 ? 0xFFFFFFFFull : ((1ull << h.cfg.k) - 1);
@@ -443,14 +448,21 @@ static void launch_batch(nb200_ctx *c, const DevLibrary &L, const CallParams &cp
     const ReadsDev &r1 = io.r1, &r2 = io.r2;
     RoRec *ro = B.ro.as<RoRec>();
     uint32_t *roB = B.roB.as<uint32_t>(), *deferred = B.deferred.as<uint32_t>(), *wide_list = B.wide_list.as<uint32_t>();
+    uint32_t *warp_list = B.warp_list.as<uint32_t>();
     SwItem *items = B.items.as<SwItem>();
     OriSum *sums = B.sums.as<OriSum>();
     uint32_t *slow_list = B.slow_list.as<uint32_t>(), *setup_list = B.setup_list.as<uint32_t>();
 #define NB200_PROBE(NM, ST) probe_kernel<NM, ST><<<blocks, pthreads, 0, sp>>>(L.dev, r1, r2, read0, nb, sums, roB, wide_list, B.ctr)
+    // single-end: one thread per read, then the warp form on the reads it could not keep in registers
+#define NB200_PROBE_THREAD(ST)                                                                                                \
+    probe_thread_kernel<ST><<<nblk(nb, kProbeThreads), kProbeThreads, 0, sp>>>(L.dev, r1, read0, nb, sums, warp_list, B.ctr); \
+    probe_list_kernel<ST><<<c->sm_count * kProbeListBlocks, pthreads, 0, sp>>>(L.dev, r1, read0, warp_list, sums, roB, wide_list, B.ctr)
     if (n_mates == 2) { if (c->stats) NB200_PROBE(2, true); else NB200_PROBE(2, false); }
-    else { if (c->stats) NB200_PROBE(1, true); else NB200_PROBE(1, false); }
+    else if (L.probe_warp) { if (c->stats) NB200_PROBE(1, true); else NB200_PROBE(1, false); }
+    else { if (c->stats) { NB200_PROBE_THREAD(true); } else { NB200_PROBE_THREAD(false); } }
+#undef NB200_PROBE_THREAD
 #undef NB200_PROBE
-    if (e_pk) CK(cudaEventRecord(e_pk, sp));          // probe_kernel alone (the roofline's kernel), before the calling kernels
+    if (e_pk) CK(cudaEventRecord(e_pk, sp));          // the probe kernels alone (the roofline's kernel), before the calling kernels
     // reads whose narrowest class is wider than the shared-memory lists (rare): generic path on global scratch
     wide_kernel<<<kWideBlocks, 128, 0, sp>>>(L.dev, cp, r1, r2, read0, n_mates, wide_list, c->wide_scratch.as<uint32_t>(),
                                              c->wide_v.as<uint32_t>(), res, feats, nf, B.ctr);
@@ -495,7 +507,7 @@ static void launch_batch(nb200_ctx *c, const DevLibrary &L, const CallParams &cp
     if (e_call) CK(cudaEventRecord(e_call, st));
     CK(cudaEventRecord(B.tail_done, st));
     B.busy = true;
-    c->launches += 11;
+    c->launches += (n_mates == 1 && !L.probe_warp) ? 12 : 11;
 }
 
 static void cub_sort32(nb200_ctx *c, const uint32_t *kin, uint32_t *kout, const uint32_t *vin, uint32_t *vout, uint32_t m, int bits) {
@@ -799,6 +811,7 @@ static void run_align(nb200_ctx *c, DevLibrary &L, const HostInput *in, double t
         b.roB.ensure(nbmax * n_ro * (size_t)2 * kCap * 4);
         b.deferred.ensure(nbmax * 4);
         b.wide_list.ensure(nbmax * 4);
+        b.warp_list.ensure(nbmax * 4);
         b.sums.ensure(nbmax * n_ro * sizeof(OriSum));
         b.slow_list.ensure(nbmax * 4);
         b.setup_list.ensure(nbmax * 4);
@@ -916,6 +929,7 @@ static void run_align(nb200_ctx *c, DevLibrary &L, const HostInput *in, double t
         }
         for (int i = 0; i < kCtrSpread; i++) { c->timing.probes += h2.probes[i]; c->timing.probe_slots += h2.probe_slots[i]; }
         c->timing.sw_pairs = h2.sw_pairs; c->timing.sw_cells = h2.sw_cells; c->timing.sw_items = h2.sw_pairs + h2.sw_dups;
+        c->timing.probe_warp_reads = h2.probe_warp_total;
         c->timing.launches = c->launches;
         c->ev_pool.clear();
         return;
@@ -1144,6 +1158,7 @@ void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_read
     B.roB.ensure(nbmax * n_ro * (size_t)2 * kCap * 4);
     B.deferred.ensure(nbmax * 4);
     B.wide_list.ensure(nbmax * 4);
+    B.warp_list.ensure(nbmax * 4);
     B.sums.ensure(nbmax * n_ro * sizeof(OriSum));
     B.slow_list.ensure(nbmax * 4);
     B.setup_list.ensure(nbmax * 4);

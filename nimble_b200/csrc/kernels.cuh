@@ -81,6 +81,7 @@ struct Counters {
     unsigned long long alloc, overflow, dropped_empty, max_nf, sw_pairs, sw_cells, items_max, deferred_total;
     unsigned long long n_wide, wide_total, n_swpairs, sw_dups, sw_items, n_slow, n_setup, n_warpdef;
     unsigned long long probes[kCtrSpread], probe_slots[kCtrSpread];
+    unsigned long long n_probe_warp, probe_warp_total;   // reads probe_thread_kernel left to the warp form (batch / call)
 };
 constexpr unsigned long long kItemMask = (1ull << 40) - 1;
 constexpr int kRoIdxBits = 22;               // a batch holds at most 2^22 read orientations (engine.cu: 2^21 reads x 2, 2^20 pairs x 4)
@@ -789,21 +790,15 @@ __device__ __forceinline__ void carve_scratch(uint32_t *s, uint32_t cap, List *L
 // read, so it runs one THREAD per read in call_fast_kernel (a warp per read would idle 31 lanes on it), and only the
 // reads that need Smith-Waterman or carry wide candidate sets take the warp-per-read call_slow_kernel.
 // Wide reads (narrowest class wider than the shared-memory lists) go to wide_kernel.
+// Single-end batches run probe_thread_kernel first; this warp form then takes only the reads it listed
+// (probe_list_kernel).  Paired-end batches and NB200_PROBE_WARP=1 run probe_kernel on every read.
 // ---------------------------------------------------------------------------------------------
 template <int NM, bool kStats>       // mates per read; kStats: count lookups / sectors (nb200_set_stats)
-__global__ void __launch_bounds__(kProbeWarps * 32, (NM == 2 ? 24 : 36) / kProbeWarps)
-probe_kernel(LibDev lib, ReadsDev r1, ReadsDev r2, uint64_t read0, uint64_t n_reads, OriSum *__restrict__ sums,
-             uint32_t *__restrict__ roB, uint32_t *__restrict__ wide_list, Counters *__restrict__ ctr) {
-    __shared__ uint32_t smem[kProbeWarps * 4 * 2 * kCap];          // per warp: four lists (generic path only)
-    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-    const uint32_t gw = blockIdx.x * kProbeWarps + wib;            // a batch is at most 2^21 reads
-    if (gw >= n_reads) return;
+__device__ __forceinline__ void probe_read(const LibDev &lib, const ReadsDev &r1, const ReadsDev &r2, uint64_t read0, uint32_t gw,
+                                           OriSum *__restrict__ sums, uint32_t *__restrict__ roB, uint32_t *__restrict__ wide_list,
+                                           Counters *__restrict__ ctr, List *L4, int lane, uint32_t &n_probe, uint32_t &slots_read) {
     const uint64_t read = read0 + gw;
     constexpr int n_ro = NM * 2;
-    List L4[4];
-#pragma unroll
-    for (int q = 0; q < 4; q++) { L4[q].w = smem + ((size_t)wib * 4 + q) * 2 * kCap; L4[q].b = L4[q].w + kCap; L4[q].n = 0; }
-    uint32_t n_probe = 0, slots_read = 0;
     bool wide = false;
 #pragma unroll
     for (int m = 0; m < NM; m++) {
@@ -837,19 +832,273 @@ probe_kernel(LibDev lib, ReadsDev r1, ReadsDev r2, uint64_t read0, uint64_t n_re
             }
         }
     }
-    if (kStats) {
-        n_probe = warp_sum(n_probe);
-        slots_read = warp_sum(slots_read);
-        if (lane == 0 && n_probe) {
-            atomicAdd(&ctr->probes[blockIdx.x & (kCtrSpread - 1)], (unsigned long long)n_probe);
-            atomicAdd(&ctr->probe_slots[blockIdx.x & (kCtrSpread - 1)], (unsigned long long)slots_read);
-        }
-    }
     if (wide && lane == 0) {
         wide_list[atomicAdd(&ctr->n_wide, 1ull)] = gw;
         reinterpret_cast<uint4 *>(sums + (size_t)gw * n_ro)[0] = make_uint4(0u, (uint32_t)kSumWide << 8, 0xFFFFFFFFu, 0xFFFFFFFFu);
     }
 }
+
+template <bool kStats>
+__device__ __forceinline__ void add_probe_stats(Counters *ctr, int lane, uint32_t n_probe, uint32_t slots_read) {
+    if (!kStats) return;
+    n_probe = warp_sum(n_probe);
+    slots_read = warp_sum(slots_read);
+    if (lane == 0 && n_probe) {
+        atomicAdd(&ctr->probes[blockIdx.x & (kCtrSpread - 1)], (unsigned long long)n_probe);
+        atomicAdd(&ctr->probe_slots[blockIdx.x & (kCtrSpread - 1)], (unsigned long long)slots_read);
+    }
+}
+
+__device__ __forceinline__ void carve_probe_lists(uint32_t *smem, int wib, List *L4) {
+#pragma unroll
+    for (int q = 0; q < 4; q++) { L4[q].w = smem + ((size_t)wib * 4 + q) * 2 * kCap; L4[q].b = L4[q].w + kCap; L4[q].n = 0; }
+}
+
+template <int NM, bool kStats>
+__global__ void __launch_bounds__(kProbeWarps * 32, (NM == 2 ? 24 : 36) / kProbeWarps)
+probe_kernel(LibDev lib, ReadsDev r1, ReadsDev r2, uint64_t read0, uint64_t n_reads, OriSum *__restrict__ sums,
+             uint32_t *__restrict__ roB, uint32_t *__restrict__ wide_list, Counters *__restrict__ ctr) {
+    __shared__ uint32_t smem[kProbeWarps * 4 * 2 * kCap];          // per warp: four lists (generic path only)
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    const uint32_t gw = blockIdx.x * kProbeWarps + wib;            // a batch is at most 2^21 reads
+    if (gw >= n_reads) return;
+    List L4[4];
+    carve_probe_lists(smem, wib, L4);
+    uint32_t n_probe = 0, slots_read = 0;
+    probe_read<NM, kStats>(lib, r1, r2, read0, gw, sums, roB, wide_list, ctr, L4, lane, n_probe, slots_read);
+    add_probe_stats<kStats>(ctr, lane, n_probe, slots_read);
+}
+
+// The reads probe_thread_kernel listed (ctr->n_probe_warp of them): the warp form above, one warp per read over a
+// grid-stride loop, with its anchor rule, wide-path decision and wide_list unchanged.  Single-end only.
+constexpr int kProbeListBlocks = 24 / kProbeWarps;   // per SM: 85 registers for the grid-stride loop, no spills
+template <bool kStats>
+__global__ void __launch_bounds__(kProbeWarps * 32, kProbeListBlocks)
+probe_list_kernel(LibDev lib, ReadsDev r1, uint64_t read0, const uint32_t *__restrict__ warp_list, OriSum *__restrict__ sums,
+                  uint32_t *__restrict__ roB, uint32_t *__restrict__ wide_list, Counters *__restrict__ ctr) {
+    __shared__ uint32_t smem[kProbeWarps * 4 * 2 * kCap];
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    const uint32_t n = (uint32_t)ctr->n_probe_warp;
+    List L4[4];
+    carve_probe_lists(smem, wib, L4);
+    uint32_t n_probe = 0, slots_read = 0;
+    for (uint32_t t = blockIdx.x * kProbeWarps + wib; t < n; t += gridDim.x * kProbeWarps) {
+        __syncwarp();                                              // the previous read's lists are no longer read
+        probe_read<1, kStats>(lib, r1, r1, read0, warp_list[t], sums, roB, wide_list, ctr, L4, lane, n_probe, slots_read);
+    }
+    add_probe_stats<kStats>(ctr, lane, n_probe, slots_read);
+}
+
+// ---------------------------------------------------------------------------------------------
+// X3a + X3b, one THREAD per single-end read: the thread walks its read's k-mer positions in order.
+//
+// The k-mer and its reverse complement roll along the read one base at a time (64-bit words, 2 bits per base); a
+// k-mer is valid when the last N base lies before it.  The lookup is that of probe_mate and host_lookup (canonical
+// form, kmer_mix, one 256-bit load of the first bucket; second bucket and dual records on a cold branch).  Positions
+// go in groups of kProbeGroup: the group's bucket loads, then its class-record loads, are issued before the first is
+// used.  On a B200 a larger group bought nothing: its registers cost occupancy, and the kernel's speed follows the
+// number of resident warps (cfg2 probe time, 10 M reads: 8.0 / 8.4 / 9.7 / 12.8 / 22.5 ms for groups of 1 / 2 / 3 / 4 / 8,
+// before the candidate sets moved to shared memory).  So the group is 1 and the register budget is what is tuned.
+//
+// Candidate set per orientation (hit count, previous class and seed in registers, B in shared memory): B is anchored
+// on the orientation's FIRST hit class and every later hit class is ANDed in.  A hit whose class id equals the previous hit's in that orientation skips the record load and the
+// AND (AND is idempotent; runs of one class are the normal case for allele families).  B only shrinks, so its members
+// do not depend on the anchor: OriSum differs from probe_kernel's only in which (empty) words B keeps.
+//
+// A read whose anchor is an overflow-form record or has more than min(4, narrow_cap) words is appended to warp_list
+// (one atomic per warp) and nothing else is written for it: probe_list_kernel probes it as probe_kernel would, and
+// counts its lookups, so the kStats counters equal probe_kernel's.
+// ---------------------------------------------------------------------------------------------
+constexpr int kProbeThreads = 128;
+constexpr int kProbeGroup = 1;
+constexpr int kProbeThreadBlocks = 10;   // blocks per SM: 47 registers, no spills (12 blocks: 40 registers, spills, slower)
+
+struct ThreadB {                 // one orientation, in registers: hits, previous hit class, seed
+    uint32_t nh, prev;
+    int seed;                    // orientation 0: first hit position; orientation 1: last
+};
+// The rest of an orientation's state lives in shared memory, one column per thread (conflict-free), because it is only
+// touched when the class changes: registers decide the kernel's occupancy, and occupancy its speed.
+enum { SB_NA = 0, SB_W01, SB_W23, SB_B0, SB_B1, SB_B2, SB_B3, SB_N };
+#define NB200_SB(f) sb[(f) * kProbeThreads]
+
+// one hit of class `cl` at position i in orientation o; (c_b, c_w) is its record when `cl` differs from the previous hit
+// class (loaded by the caller).  Returns false when the read must take the warp form.
+__device__ __forceinline__ bool thread_hit(const LibDev &lib, ThreadB &T, uint32_t *sb, uint32_t cl, int i, int o, uint32_t cap,
+                                           const uint4 c_b, const uint4 c_w) {
+    T.nh++;
+    if (o == 0) T.seed = T.seed < 0 ? i : T.seed; else T.seed = i;
+    if (cl == T.prev) return true;
+    const bool inl = (int32_t)c_w.z >= 0;
+    if (T.prev == kInvalid) {                                      // anchor
+        T.prev = cl;
+        const uint32_t na = c_w.z & 0xFFu;
+        NB200_SB(SB_NA) = na;
+        if (!inl || na > cap) return false;
+        NB200_SB(SB_W01) = c_w.x; NB200_SB(SB_W23) = c_w.y;
+        NB200_SB(SB_B0) = c_b.x; NB200_SB(SB_B1) = c_b.y; NB200_SB(SB_B2) = c_b.z; NB200_SB(SB_B3) = c_b.w;
+        return true;
+    }
+    T.prev = cl;
+    const uint32_t w01 = NB200_SB(SB_W01), w23 = NB200_SB(SB_W23);
+    uint4 m = c_b;                                                 // same reference words: word by word
+    if (!(inl && c_w.x == w01 && c_w.y == w23)) {                  // unused words of B (0xFFFF) are zeroed at the end
+        m.x = rec_bits(lib, c_b, c_w, w01 & 0xFFFFu);
+        m.y = rec_bits(lib, c_b, c_w, w01 >> 16);
+        m.z = rec_bits(lib, c_b, c_w, w23 & 0xFFFFu);
+        m.w = rec_bits(lib, c_b, c_w, w23 >> 16);
+    }
+    NB200_SB(SB_B0) &= m.x; NB200_SB(SB_B1) &= m.y; NB200_SB(SB_B2) &= m.z; NB200_SB(SB_B3) &= m.w;
+    return true;
+}
+
+template <bool kStats>
+__global__ void __launch_bounds__(kProbeThreads, kProbeThreadBlocks)
+probe_thread_kernel(LibDev lib, ReadsDev R, uint64_t read0, uint64_t n_reads, OriSum *__restrict__ sums,
+                    uint32_t *__restrict__ warp_list, Counters *__restrict__ ctr) {
+    const uint32_t gr = blockIdx.x * kProbeThreads + threadIdx.x;   // a batch is at most 2^21 reads
+    const bool active = gr < n_reads;
+    const uint64_t read = read0 + (active ? gr : 0u);
+    const uint8_t *rec = R.packed + read * R.stride;
+    const uint64_t *seq = reinterpret_cast<const uint64_t *>(rec);
+    const int W = (int)R.words, k = lib.k;
+    const int P = (active ? read_length(R, read) : 0) - k + 1;
+    const uint64_t kmask = lib.kmask;
+    const int top = 2 * k - 2;                                     // bit of the newest base in the forward k-mer
+    const uint32_t nb = lib.n_buckets, cap = min(4u, lib.narrow_cap);
+    __shared__ uint32_t s_b[2 * SB_N * kProbeThreads];
+    uint32_t *const sb0 = s_b + threadIdx.x, *const sb1 = sb0 + SB_N * kProbeThreads;
+    ThreadB T[2];
+#pragma unroll
+    for (int o = 0; o < 2; o++) {
+        uint32_t *sb = o ? sb1 : sb0;
+        T[o].nh = 0; T[o].prev = kInvalid; T[o].seed = -1;
+        NB200_SB(SB_NA) = 0; NB200_SB(SB_W01) = NB200_SB(SB_W23) = 0xFFFFFFFFu;
+        NB200_SB(SB_B0) = NB200_SB(SB_B1) = NB200_SB(SB_B2) = NB200_SB(SB_B3) = 0;
+    }
+    uint32_t n_probe = 0, slots_read = 0;
+    bool fallback = false;
+    // base stream: `cur` holds the packed word of base p onwards, `ncur` its N bits
+    uint64_t cur = 0, x = 0, y = 0;
+    uint32_t ncur = 0;
+    int p = 0, last_n = -1;
+    auto push_base = [&]() {
+        if ((p & 31) == 0) {
+            const int w = p >> 5;
+            cur = w < W ? seq[w] : 0ull;
+            ncur = w < W ? reinterpret_cast<const uint32_t *>(seq + W)[w] : 0u;   // N masks follow the sequence words
+        }
+        const uint32_t b = (uint32_t)cur & 3u;
+        last_n = (ncur & 1u) ? p : last_n;
+        cur >>= 2; ncur >>= 1;
+        x = (x >> 2) | ((uint64_t)b << top);
+        y = ((y << 2) | (b ^ 3u)) & kmask;
+        p++;
+    };
+    if (P > 0)
+        for (int t = 0; t < k - 1; t++) push_base();
+#pragma unroll 1
+    for (int i0 = 0; i0 < P; i0 += kProbeGroup) {
+        uint32_t c_lo[kProbeGroup], c_hi[kProbeGroup];
+        bool valid[kProbeGroup], xs[kProbeGroup], ys[kProbeGroup];
+        uint4 e_lo[kProbeGroup], e_hi[kProbeGroup];
+#pragma unroll
+        for (int g = 0; g < kProbeGroup; g++) {
+            push_base();
+            const int i = i0 + g;
+            valid[g] = i < P && last_n < i;
+            const bool x_lt = x < y;
+            xs[g] = x <= y; ys[g] = !x_lt;
+            const uint64_t c = x_lt ? x : y;
+            c_lo[g] = (uint32_t)c; c_hi[g] = (uint32_t)(c >> 32);
+            e_lo[g] = make_uint4(kInvalid, kInvalid, 0u, 0u); e_hi[g] = e_lo[g];
+            if (valid[g]) ldg256(lib.table + 2 * (size_t)kmer_bucket1(kmer_mix(c_lo[g], c_hi[g]), nb), e_lo[g], e_hi[g]);
+        }
+        uint32_t cl0[kProbeGroup], cl1[kProbeGroup];
+#pragma unroll
+        for (int g = 0; g < kProbeGroup; g++) {
+            const uint32_t clo = c_lo[g], chi = c_hi[g];
+            bool m0 = e_lo[g].x == clo && e_lo[g].y == chi, m1 = e_hi[g].x == clo && e_hi[g].y == chi;
+            uint32_t ecls = m0 ? e_lo[g].z : e_hi[g].z;
+            bool found = valid[g] && (m0 || m1);
+            const bool need2 = valid[g] && !(m0 || m1) && (e_lo[g].z & kDevSpill);
+            if (kStats) { n_probe += valid[g] ? 1u : 0u; slots_read += (valid[g] ? 1u : 0u) + (need2 ? 1u : 0u); }
+            if (need2 || (found && (ecls & kDevDual))) {           // cold: the key's second bucket, or a dual record
+                if (need2) {
+                    const uint32_t mix = kmer_mix(clo, chi);
+                    uint4 f_lo, f_hi;
+                    ldg256(lib.table + 2 * (size_t)kmer_bucket2(mix, clo, kmer_bucket1(mix, nb), nb), f_lo, f_hi);
+                    m0 = f_lo.x == clo && f_lo.y == chi; m1 = f_hi.x == clo && f_hi.y == chi;
+                    found = m0 || m1;
+                    ecls = m0 ? f_lo.z : f_hi.z;
+                }
+                cl0[g] = (found && xs[g] != ((ecls & kDevRc) != 0)) ? (ecls & kDevIdMask) : kInvalid;
+                cl1[g] = (found && ys[g] != ((ecls & kDevRc) != 0)) ? (ecls & kDevIdMask) : kInvalid;
+                if (found && (ecls & kDevDual)) {
+                    const uint4 d = __ldg(lib.dual + (ecls & kDevIdMask));
+                    cl0[g] = xs[g] ? d.x : d.z;
+                    cl1[g] = ys[g] ? d.x : d.z;
+                }
+            } else {
+                cl0[g] = (found && xs[g] != ((ecls & kDevRc) != 0)) ? (ecls & kDevIdMask) : kInvalid;
+                cl1[g] = (found && ys[g] != ((ecls & kDevRc) != 0)) ? (ecls & kDevIdMask) : kInvalid;
+            }
+        }
+        // the class records the group needs (a class that differs from the previous hit class of its orientation), all
+        // loads issued before the first is used: one per position, orientation 0 first.  Both orientations hit with
+        // different classes only through dual records; orientation 1's record is then loaded on its own.
+        uint4 r_b[kProbeGroup], r_w[kProbeGroup];
+        uint32_t r_cl[kProbeGroup];
+        {
+            uint32_t p0 = T[0].prev, p1 = T[1].prev;
+#pragma unroll
+            for (int g = 0; g < kProbeGroup; g++) {
+                const bool n0 = cl0[g] != kInvalid && cl0[g] != p0, n1 = cl1[g] != kInvalid && cl1[g] != p1;
+                r_cl[g] = n0 ? cl0[g] : (n1 ? cl1[g] : kInvalid);
+                if (cl0[g] != kInvalid) p0 = cl0[g];
+                if (cl1[g] != kInvalid) p1 = cl1[g];
+                r_b[g] = make_uint4(0u, 0u, 0u, 0u); r_w[g] = r_b[g];
+                if (r_cl[g] != kInvalid) ldg256_cached(lib.class_rec + 2 * (size_t)r_cl[g], r_b[g], r_w[g]);
+            }
+        }
+#pragma unroll
+        for (int g = 0; g < kProbeGroup; g++) {
+            if (cl0[g] != kInvalid && !thread_hit(lib, T[0], sb0, cl0[g], i0 + g, 0, cap, r_b[g], r_w[g])) fallback = true;
+            if (cl1[g] != kInvalid) {
+                uint4 c_b = r_b[g], c_w = r_w[g];
+                if (cl1[g] != T[1].prev && cl1[g] != r_cl[g]) ldg256_cached(lib.class_rec + 2 * (size_t)cl1[g], c_b, c_w);
+                if (!thread_hit(lib, T[1], sb1, cl1[g], i0 + g, 1, cap, c_b, c_w)) fallback = true;
+            }
+        }
+        if (fallback) break;
+    }
+    // the reads left to the warp form: one atomic per warp
+    const unsigned fb = __ballot_sync(kFull, active && fallback);
+    if (fb) {
+        const int lane = threadIdx.x & 31, leader = __ffs(fb) - 1;
+        uint32_t base = 0;
+        if (lane == leader) base = (uint32_t)atomicAdd(&ctr->n_probe_warp, (unsigned long long)__popc(fb));
+        base = __shfl_sync(kFull, base, leader);
+        if (active && fallback) warp_list[base + __popc(fb & ((1u << lane) - 1))] = gr;
+    }
+    if (fallback) n_probe = slots_read = 0;                        // probe_list_kernel counts the read
+    add_probe_stats<kStats>(ctr, threadIdx.x & 31, n_probe, slots_read);
+    if (!active || fallback) return;
+    uint4 *dst = reinterpret_cast<uint4 *>(sums + (size_t)gr * 2);
+#pragma unroll
+    for (int o = 0; o < 2; o++) {
+        const ThreadB &B = T[o];
+        const uint32_t *sb = o ? sb1 : sb0;
+        const uint32_t na = B.prev == kInvalid ? 0u : NB200_SB(SB_NA);
+        const int seed = B.nh == 0 ? -1 : (o == 0 ? B.seed : P - 1 - B.seed);
+        const uint32_t flags = (B.nh && (int)B.nh == P) ? kSumFull : 0u;
+        dst[2 * o] = make_uint4((B.nh & 0xFFFFu) | ((uint32_t)(seed & 0xFFFF) << 16), na | (flags << 8) | ((uint32_t)(P + k - 1) << 16),
+                                NB200_SB(SB_W01), NB200_SB(SB_W23));
+        dst[2 * o + 1] = make_uint4(NB200_SB(SB_B0), na > 1 ? NB200_SB(SB_B1) : 0u, na > 2 ? NB200_SB(SB_B2) : 0u,
+                                    na > 3 ? NB200_SB(SB_B3) : 0u);
+    }
+}
+#undef NB200_SB
 
 // ---------------------------------------------------------------------------------------------
 // X4, one THREAD per read: every read whose orientations all resolved without alignment (no hit / empty class / every
