@@ -786,6 +786,35 @@ static void validate_reads(const nb200_reads *r, const char *what) {
 
 struct HostInput { const nb200_reads *r1, *r2; const uint64_t *key; };
 
+// Device state of one batch of up to nbmax reads with n_ro mate-orientations, and the wide-read scratch of library L.
+// The Smith-Waterman work list starts at 8 items a read (NB200_ITEMS_CAP overrides it: tests force the overflow-and-retry
+// path with it) and only grows after an overflow (grown_items_cap).
+static void size_batch(nb200_ctx *c, nb200_ctx::BatchBuf &b, uint64_t nbmax, int n_ro, const DevLibrary &L) {
+    if (c->items_cap == 0) {
+        c->items_cap = (uint32_t)std::max<uint64_t>(1u << 20, std::min<uint64_t>(nbmax * 8, 1ull << 28));
+        if (const char *e = getenv("NB200_ITEMS_CAP")) c->items_cap = (uint32_t)std::max(2l, atol(e));
+    }
+    b.ro.ensure(nbmax * n_ro * sizeof(RoRec));
+    b.roB.ensure(nbmax * n_ro * (size_t)2 * kCap * 4);
+    b.deferred.ensure(nbmax * 4);
+    b.wide_list.ensure(nbmax * 4);
+    b.warp_list.ensure(nbmax * 4);
+    b.sums.ensure(nbmax * n_ro * sizeof(OriSum));
+    b.slow_list.ensure(nbmax * 4);
+    b.setup_list.ensure(nbmax * 4);
+    b.items.ensure((size_t)c->items_cap * sizeof(SwItem));
+    b.sw_pairs.ensure(((size_t)c->items_cap + 64) * 4);      // distinct-window work list
+    b.sw_rep.ensure(((size_t)c->items_cap + 64) * 4);        // representative of every candidate
+    const size_t warps = (size_t)kWideBlocks * 4;
+    c->wide_scratch.ensure(warps * 16 * (size_t)L.dev.n_words * 4);
+    c->wide_v.ensure(warps * ((size_t)L.dev.n_words * 32 + 32) * 4);
+}
+
+// the work list after an overflow: the measured demand of the batch and some room
+static uint32_t grown_items_cap(unsigned long long need) {
+    return (uint32_t)std::min<unsigned long long>(need + need / 4 + 1024, 0xFFFFFFF0ull);
+}
+
 // The whole hot path for one library.  `in` == nullptr: reads already resident.
 static void run_align(nb200_ctx *c, DevLibrary &L, const HostInput *in, double threshold, int disable,
                       nb200_counts *counts) {
@@ -806,35 +835,14 @@ static void run_align(nb200_ctx *c, DevLibrary &L, const HostInput *in, double t
     c->feats_stride = (int32_t)mh;
     const uint64_t B = c->paired ? (1ull << 20) : (1ull << 21);
     const uint64_t nbmax = std::min<uint64_t>(B, std::max<uint64_t>(n, 1));
-    for (auto &b : c->bb) {
-        b.ro.ensure(nbmax * n_ro * sizeof(RoRec));
-        b.roB.ensure(nbmax * n_ro * (size_t)2 * kCap * 4);
-        b.deferred.ensure(nbmax * 4);
-        b.wide_list.ensure(nbmax * 4);
-        b.warp_list.ensure(nbmax * 4);
-        b.sums.ensure(nbmax * n_ro * sizeof(OriSum));
-        b.slow_list.ensure(nbmax * 4);
-        b.setup_list.ensure(nbmax * 4);
-    }
-    {
-        const size_t warps = (size_t)kWideBlocks * 4;
-        c->wide_scratch.ensure(warps * 16 * (size_t)L.dev.n_words * 4);
-        c->wide_v.ensure(warps * ((size_t)L.dev.n_words * 32 + 32) * 4);
-    }
     if (in) {   // compact wire form: staging sized once for the largest batch (a reallocation inside the loop would sync)
         if (is_compact(in->r1)) c->stage1.ensure(nbmax * (size_t)in->r1->stride + 64);
         if (in->r2 && is_compact(in->r2)) c->stage2.ensure(nbmax * (size_t)in->r2->stride + 64);
     }
     pin_index_in_l2(c, L);
-    if (c->items_cap == 0) {
-        c->items_cap = (uint32_t)std::max<uint64_t>(1u << 20, std::min<uint64_t>(nbmax * 8, 1ull << 28));
-        if (const char *e = getenv("NB200_ITEMS_CAP")) c->items_cap = (uint32_t)std::max(2l, atol(e));   // tests: force the retry path
-    }
     for (int attempt = 0; attempt < 3; attempt++) {
         for (auto &b : c->bb) {
-            b.items.ensure((size_t)c->items_cap * sizeof(SwItem));
-            b.sw_pairs.ensure(((size_t)c->items_cap + 64) * 4);      // distinct-window work list
-            b.sw_rep.ensure(((size_t)c->items_cap + 64) * 4);        // representative of every candidate
+            size_batch(c, b, nbmax, n_ro, L);
             b.busy = false;
         }
         CK(cudaMemsetAsync(c->bb[1].ctr, 0, sizeof(Counters), c->s_compute));
@@ -894,7 +902,7 @@ static void run_align(nb200_ctx *c, DevLibrary &L, const HostInput *in, double t
         CK(cudaStreamSynchronize(c->s_compute));
         c->timing.d2h_bytes += sizeof(hc);
         if (hc.c.overflow) {   // SW work list did not fit: grow to the measured demand and redo
-            c->items_cap = (uint32_t)std::min<unsigned long long>(hc.c.items_max + hc.c.items_max / 4 + 1024, 0xFFFFFFF0ull);
+            c->items_cap = grown_items_cap(hc.c.items_max);
             continue;
         }
         aggregate(c, L, n, c->has_key ? c->d_key.as<uint64_t>() : nullptr, Rows{c->feats.as<int32_t>(), nullptr, nullptr, c->row_nf.as<uint16_t>(), mh},
@@ -1154,18 +1162,6 @@ void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_read
     if (cb) lane_cb_slab(c, F, n);                  // the keys are final before any library's rows are appended
     nb200_ctx::BatchBuf &B = c->bb[lane];
     const uint64_t nbmax = std::max<uint64_t>(n, 1);
-    B.ro.ensure(nbmax * n_ro * sizeof(RoRec));
-    B.roB.ensure(nbmax * n_ro * (size_t)2 * kCap * 4);
-    B.deferred.ensure(nbmax * 4);
-    B.wide_list.ensure(nbmax * 4);
-    B.warp_list.ensure(nbmax * 4);
-    B.sums.ensure(nbmax * n_ro * sizeof(OriSum));
-    B.slow_list.ensure(nbmax * 4);
-    B.setup_list.ensure(nbmax * 4);
-    if (c->items_cap == 0) c->items_cap = (uint32_t)std::max<uint64_t>(1u << 20, std::min<uint64_t>((c->paired ? (1ull << 20) : (1ull << 21)) * 8, 1ull << 28));
-    B.items.ensure((size_t)c->items_cap * sizeof(SwItem));
-    B.sw_pairs.ensure(((size_t)c->items_cap + 64) * 4);
-    B.sw_rep.ensure(((size_t)c->items_cap + 64) * 4);
     for (int li = 0; li < n_libs; li++) {
         DevLibrary &L = lane_lib(c, lib_ids[li]);
         if (!L.host.has_index) throw std::runtime_error("library has no k-mer index (feature dictionary only)");
@@ -1174,11 +1170,7 @@ void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_read
         F.res[li].ensure(nbmax * sizeof(nb200_read_result) + 64);
         F.feats[li].ensure(nbmax * (size_t)mh * 4 + 64);
         F.nf[li].ensure(nbmax * 2 + 64);
-        {
-            const size_t warps = (size_t)kWideBlocks * 4;
-            c->wide_scratch.ensure(warps * 16 * (size_t)L.dev.n_words * 4);
-            c->wide_v.ensure(warps * ((size_t)L.dev.n_words * 32 + 32) * 4);
-        }
+        size_batch(c, B, nbmax, n_ro, L);
         pin_index_in_l2(c, L);
         if (B.busy && c->overlap) CK(cudaStreamWaitEvent(c->s_compute, B.tail_done, 0));
         CK(cudaMemsetAsync(B.ctr, 0, sizeof(Counters), c->s_compute));
@@ -1231,7 +1223,7 @@ void lane_wait(nb200_ctx *c, int lane) {
         if (!need) return;
         if (attempt >= 3) throw std::runtime_error("Smith-Waterman work list kept overflowing");
         // the work list did not fit: grow it to the measured demand (cudaFree waits for the other lane) and redo the slab
-        c->items_cap = (uint32_t)std::min<unsigned long long>(need + need / 4 + 1024, 0xFFFFFFF0ull);
+        c->items_cap = grown_items_cap(need);
         const nb200_reads r1 = F.hr1, r2 = F.hr2;
         const std::vector<int32_t> libs = F.libs;
         const std::vector<nb200_read_result *> orr = F.out_res;
@@ -1653,6 +1645,16 @@ static void cb_fetch(nb200_ctx *c, int32_t *out_idx, uint8_t *out_status, nb200_
     if (st) st->d2h_bytes += (out_idx ? n * 4 : 0) + (out_status ? n : 0);
 }
 
+// Inside a catch block: the status code of the exception being handled, its message in `what`.
+static int32_t status_of_exception(std::string &what) {
+    try { throw; }
+    catch (const IoError &e) { what = e.what(); return NB200_EIO; }
+    catch (const CudaError &e) { what = e.what(); cudaGetLastError(); return NB200_ECUDA; }
+    catch (const LimitError &e) { what = e.what(); return NB200_ELIMIT; }
+    catch (const std::bad_alloc &) { what = "out of host memory"; return NB200_EINVAL; }
+    catch (const std::exception &e) { what = e.what(); return NB200_EINVAL; }
+}
+
 }  // namespace nb200
 
 // =============================================================================================
@@ -1664,10 +1666,7 @@ static void cb_fetch(nb200_ctx *c, int32_t *out_idx, uint8_t *out_status, nb200_
         if (cudaSetDevice((ctx)->device) != cudaSuccess) { (ctx)->err = "cudaSetDevice failed"; return NB200_ECUDA; }
 #define API_END(ctx)                                                                               \
     }                                                                                              \
-    catch (const nb200::CudaError &e) { (ctx)->err = e.what(); cudaGetLastError(); return NB200_ECUDA; } \
-    catch (const nb200::LimitError &e) { (ctx)->err = e.what(); return NB200_ELIMIT; }             \
-    catch (const std::bad_alloc &) { (ctx)->err = "out of host memory"; return NB200_EINVAL; }     \
-    catch (const std::exception &e) { (ctx)->err = e.what(); return NB200_EINVAL; }                \
+    catch (const std::exception &) { return nb200::status_of_exception((ctx)->err); }              \
     return NB200_OK;
 
 extern "C" {
@@ -2079,10 +2078,7 @@ int32_t nb200_align(nb200_ctx *c, int32_t lib_id, const nb200_reads *r1, const n
     API_END(c)
 }
 
-// File-level entry: what the aligner process does between its argv and its exit code
-// (nimble/__main__.py:177-196).  One ingest, one pass per library, per-read TSV per library
-// (bulk `features<TAB>count` when the input carries no CB/UB tags, i.e. FASTQ).
-// reads in memory -> per library: GPU path -> per-read TSV (tagged reads) or bulk table
+// reads in memory (the 10x one-pass route) -> per library: GPU path -> per-read TSV
 static void align_readset(nb200_ctx *c, const ReadSet &R, const int32_t *lib_ids, const char *const *outputs, int32_t n_libs,
                           PhaseTimer &pt) {
     const uint64_t n = R.r1.size();
@@ -2101,7 +2097,7 @@ static void align_readset(nb200_ctx *c, const ReadSet &R, const int32_t *lib_ids
     std::vector<uint16_t> l1, l2;
     nb200_reads p1{}, p2{};
     pack(R.r1, b1, l1, p1);
-    if (R.paired) pack(R.r2, b2, l2, p2);
+    pack(R.r2, b2, l2, p2);
     pt.lap("2-bit pack");
     for (int li = 0; li < n_libs; li++) {
         DevLibrary &L = get_lib(c, lib_ids[li]);
@@ -2109,8 +2105,8 @@ static void align_readset(nb200_ctx *c, const ReadSet &R, const int32_t *lib_ids
         std::vector<nb200_read_result> res(n + 1);
         std::vector<int32_t> feats((n + 1) * (size_t)mh);
         nb200_counts counts{};
-        ensure_read_buffers(c, &p1, R.paired ? &p2 : nullptr, false);
-        HostInput hin{&p1, R.paired ? &p2 : nullptr, nullptr};
+        ensure_read_buffers(c, &p1, &p2, false);
+        HostInput hin{&p1, &p2, nullptr};
         run_align(c, L, &hin, 0.05, 0, &counts);
         c->resident = true;
         pt.lap("GPU align");
@@ -2119,29 +2115,46 @@ static void align_readset(nb200_ctx *c, const ReadSet &R, const int32_t *lib_ids
             CK(cudaMemcpy(feats.data(), c->feats.p, n * (size_t)mh * 4, cudaMemcpyDeviceToHost));
         }
         pt.lap("fetch per-read results");
-        if (R.has_tags) write_per_read_tsv(outputs[li], R, res.data(), feats.data(), mh, L.host.feature_names, c->host_threads);
-        else write_bulk_tsv(outputs[li], counts, L.host.feature_names);
+        write_per_read_tsv(outputs[li], R, res.data(), feats.data(), mh, L.host.feature_names, c->host_threads);
         pt.lap("write TSV");
     }
+}
+
+// File-level entries: what the aligner process does between its argv and its exit code (nimble/__main__.py:177-196),
+// streaming (stream.cpp).  One pass over `inputs` on the contexts `ctxs`, whose libraries carry the same ids in the same
+// order; per library a per-read TSV (outputs) and/or a counts TSV (counts_outputs).  whitelist: the 10x mode of
+// fastq-to-counts (inputs = raw R1 and R2), null otherwise.
+static FileStats run_job(const std::vector<nb200_ctx *> &ctxs, const int32_t *lib_ids, int32_t n_libs, const char *const *inputs,
+                         int32_t n_inputs, const char *const *outputs, const char *const *counts_outputs, double umi_threshold,
+                         int32_t disable_thresholding, const char *whitelist, int32_t cb_len, int32_t umi_len) {
+    FileJob job;
+    std::vector<std::string> wl;
+    if (whitelist) { read_whitelist_lines(whitelist, wl); job.whitelist = &wl; job.cb_len = cb_len; job.umi_len = umi_len; }
+    job.inputs.assign(inputs, inputs + n_inputs);
+    job.ctxs = ctxs;
+    job.lib_ids.assign(lib_ids, lib_ids + n_libs);
+    for (int i = 0; i < n_libs; i++) {
+        get_lib(ctxs[0], lib_ids[i]);
+        if (outputs) job.outputs.emplace_back(outputs[i]);
+        if (counts_outputs) job.counts_outputs.emplace_back(counts_outputs[i]);
+    }
+    job.host_threads = ctxs[0]->host_threads;
+    job.umi_threshold = umi_threshold;
+    job.disable_thresholding = disable_thresholding;
+    FileStats st;
+    run_file_pipeline(job, &st);
+    if (getenv("NB200_TRACE"))
+        fprintf(stderr, "[nb200 trace] file pipeline: %llu reads in %llu slabs on %zu GPUs, %.3f s (%.2f M reads/s), %d host threads\n",
+                (unsigned long long)st.n_reads, (unsigned long long)st.n_slabs, ctxs.size(), st.seconds,
+                st.n_reads / std::max(st.seconds, 1e-9) / 1e6, job.host_threads);
+    return st;
 }
 
 int32_t nb200_align_files(nb200_ctx *c, const char *const *inputs, int32_t n_inputs, const int32_t *lib_ids,
                           const char *const *outputs, int32_t n_libs) {
     API_BEGIN(c)
     if (!inputs || n_inputs < 1 || n_inputs > 2 || !lib_ids || !outputs || n_libs < 1) throw std::runtime_error("bad arguments");
-    try {
-        FileJob job;
-        for (int i = 0; i < n_inputs; i++) job.inputs.emplace_back(inputs[i]);
-        job.ctxs.push_back(c);
-        job.lib_ids.assign(lib_ids, lib_ids + n_libs);
-        for (int i = 0; i < n_libs; i++) { get_lib(c, lib_ids[i]); job.outputs.emplace_back(outputs[i]); }
-        job.host_threads = c->host_threads;
-        FileStats st;
-        run_file_pipeline(job, &st);
-        if (getenv("NB200_TRACE"))
-            fprintf(stderr, "[nb200 trace] file pipeline: %llu reads in %llu slabs, %.3f s (%.2f M reads/s), %d host threads\n",
-                    (unsigned long long)st.n_reads, (unsigned long long)st.n_slabs, st.seconds, st.n_reads / std::max(st.seconds, 1e-9) / 1e6, c->host_threads);
-    } catch (const IoError &e) { c->err = e.what(); return NB200_EIO; }
+    run_job({c}, lib_ids, n_libs, inputs, n_inputs, outputs, nullptr, 0.05, 0, nullptr, 0, 0);
     API_END(c)
 }
 
@@ -2180,26 +2193,9 @@ int32_t nb200_align_files_counts(nb200_ctx *c, const char *const *inputs, int32_
     API_BEGIN(c)
     if (!inputs || n_inputs < 1 || n_inputs > 2 || !lib_ids || !counts_outputs || n_libs < 1) throw std::runtime_error("bad arguments");
     if (out3) for (int i = 0; i < 3 * n_libs; i++) out3[i] = 0;
-    try {
-        FileJob job;
-        for (int i = 0; i < n_inputs; i++) job.inputs.emplace_back(inputs[i]);
-        job.ctxs.push_back(c);
-        job.lib_ids.assign(lib_ids, lib_ids + n_libs);
-        for (int i = 0; i < n_libs; i++) {
-            get_lib(c, lib_ids[i]);
-            if (per_read_outputs) job.outputs.emplace_back(per_read_outputs[i]);
-            job.counts_outputs.emplace_back(counts_outputs[i]);
-        }
-        job.host_threads = c->host_threads;
-        job.umi_threshold = umi_threshold;
-        job.disable_thresholding = disable_thresholding;
-        FileStats st;
-        run_file_pipeline(job, &st);
-        if (out3) for (size_t i = 0; i < st.counts3.size(); i++) out3[i] = st.counts3[i];
-        if (getenv("NB200_TRACE"))
-            fprintf(stderr, "[nb200 trace] file pipeline (counts): %llu reads in %llu slabs, %.3f s (%.2f M reads/s), %d host threads\n",
-                    (unsigned long long)st.n_reads, (unsigned long long)st.n_slabs, st.seconds, st.n_reads / std::max(st.seconds, 1e-9) / 1e6, c->host_threads);
-    } catch (const IoError &e) { c->err = e.what(); return NB200_EIO; }
+    const FileStats st = run_job({c}, lib_ids, n_libs, inputs, n_inputs, per_read_outputs, counts_outputs, umi_threshold,
+                                 disable_thresholding, nullptr, 0, 0);
+    if (out3) for (size_t i = 0; i < st.counts3.size(); i++) out3[i] = st.counts3[i];
     API_END(c)
 }
 
@@ -2242,28 +2238,12 @@ static int32_t files_multi(const int32_t *devices, int32_t n_devices, int32_t ho
     }
     if (rc == NB200_OK) {
         try {
-            FileJob job;
-            for (int i = 0; i < n_inputs; i++) job.inputs.emplace_back(inputs[i]);
-            job.ctxs = ctxs;
-            job.lib_ids = ids;
-            for (int i = 0; i < n_libs; i++) {
-                if (outputs) job.outputs.emplace_back(outputs[i]);
-                if (counts_outputs) job.counts_outputs.emplace_back(counts_outputs[i]);
-            }
-            job.host_threads = ctxs[0]->host_threads;
-            job.umi_threshold = umi_threshold;
-            job.disable_thresholding = disable_thresholding;
-            std::vector<std::string> wl;
-            if (whitelist) { read_whitelist_lines(whitelist, wl); job.whitelist = &wl; job.cb_len = cb_len; job.umi_len = umi_len; }
-            FileStats st;
-            run_file_pipeline(job, &st);
+            const FileStats st = run_job(ctxs, ids.data(), n_libs, inputs, n_inputs, outputs, counts_outputs, umi_threshold,
+                                         disable_thresholding, whitelist, cb_len, umi_len);
             if (stats4) { stats4[0] = (double)st.n_reads; stats4[1] = st.seconds; stats4[2] = (double)st.called; stats4[3] = (double)st.n_slabs; }
             if (out3) for (size_t i = 0; i < st.counts3.size(); i++) out3[i] = st.counts3[i];
             if (cb_stats) *cb_stats = st.cb;
-        } catch (const IoError &e) { rc = NB200_EIO; what = e.what(); }
-        catch (const nb200::CudaError &e) { rc = NB200_ECUDA; what = e.what(); }
-        catch (const nb200::LimitError &e) { rc = NB200_ELIMIT; what = e.what(); }
-        catch (const std::exception &e) { rc = NB200_EINVAL; what = e.what(); }
+        } catch (const std::exception &) { rc = status_of_exception(what); }
     }
     for (nb200_ctx *c : ctxs) nb200_destroy(c);
     return rc == NB200_OK ? NB200_OK : fail(rc, what);
@@ -2279,26 +2259,11 @@ int32_t nb200_fastq_to_counts(nb200_ctx *c, const char *r1_fastq, const char *r2
         throw std::runtime_error("bad arguments");
     if (out3) for (int i = 0; i < 3 * n_libs; i++) out3[i] = 0;
     if (stats) *stats = nb200_cb_stats{};
-    try {
-        std::vector<std::string> wl;
-        read_whitelist_lines(whitelist_path, wl);
-        FileJob job;
-        job.inputs = {r1_fastq, r2_fastq};
-        job.ctxs.push_back(c);
-        job.lib_ids.assign(lib_ids, lib_ids + n_libs);
-        for (int i = 0; i < n_libs; i++) { get_lib(c, lib_ids[i]); job.counts_outputs.emplace_back(counts_outputs[i]); }
-        job.host_threads = c->host_threads;
-        job.umi_threshold = umi_threshold;
-        job.disable_thresholding = disable_thresholding;
-        job.whitelist = &wl; job.cb_len = cb_len; job.umi_len = umi_len;
-        FileStats st;
-        run_file_pipeline(job, &st);
-        if (out3) for (size_t i = 0; i < st.counts3.size(); i++) out3[i] = st.counts3[i];
-        if (stats) *stats = st.cb;
-        if (getenv("NB200_TRACE"))
-            fprintf(stderr, "[nb200 trace] file pipeline (fastq-to-counts): %llu pairs in %llu slabs, %.3f s, %d host threads\n",
-                    (unsigned long long)st.cb.total_pairs, (unsigned long long)st.n_slabs, st.seconds, c->host_threads);
-    } catch (const IoError &e) { c->err = e.what(); return NB200_EIO; }
+    const char *inputs[2] = {r1_fastq, r2_fastq};
+    const FileStats st = run_job({c}, lib_ids, n_libs, inputs, 2, nullptr, counts_outputs, umi_threshold, disable_thresholding,
+                                 whitelist_path, cb_len, umi_len);
+    if (out3) for (size_t i = 0; i < st.counts3.size(); i++) out3[i] = st.counts3[i];
+    if (stats) *stats = st.cb;
     API_END(c)
 }
 
@@ -2326,60 +2291,55 @@ int32_t nb200_align_10x_fastq(nb200_ctx *c, const char *r1_fastq, const char *r2
     API_BEGIN(c)
     if (!r1_fastq || !r2_fastq || !whitelist_path || !lib_ids || !outputs || n_libs < 1 || cb_len < 1 || umi_len < 0)
         throw std::runtime_error("bad arguments");
-    try {
-        PhaseTimer pt;
-        nb200_cb_stats st{};
-        std::vector<std::string> lines;
-        read_whitelist_lines(whitelist_path, lines);
-        std::unique_ptr<DevWhitelist> W = build_whitelist(c, std::move(lines), cb_len);
-        FastqQ A, B;
-        {
-            std::string err;
-            std::thread t([&] { try { load_fastq_qual(r2_fastq, B); } catch (const std::exception &e) { err = e.what(); } });
-            try { load_fastq_qual(r1_fastq, A); } catch (...) { t.join(); throw; }
-            t.join();
-            if (!err.empty()) throw IoError(err);
-        }
-        pt.lap("whitelist + FASTQ parse");
-        const size_t n = std::min(A.recs.size(), B.recs.size());
-        std::vector<uint8_t> cb(n * (size_t)cb_len + 16), qual(n * (size_t)cb_len + 16), elig(n + 16);
-        slice_barcodes(A, B, cb_len, umi_len, c->host_threads, cb.data(), qual.data(), elig.data(), st);
-        std::vector<int32_t> idx(n + 1);
-        std::vector<uint8_t> status(n + 1);
-        nb200_cb_stats dev{};
-        cb_upload(c, cb_len, (const char *)cb.data(), qual.data(), elig.data(), n, &dev);
-        cb_run(c, *W, &dev);
-        cb_fetch(c, idx.data(), status.data(), &dev);
-        c->ev_pool.clear();
-        c->cb_resident = false;
-        dev.total_pairs = st.total_pairs; dev.name_mismatch = st.name_mismatch; dev.too_short = st.too_short;
-        dev.no_remaining_seq = st.no_remaining_seq;
-        pt.lap("barcode correction");
-        ReadSet R;
-        R.paired = true; R.has_tags = true;
-        const uint32_t bl = (uint32_t)(cb_len + umi_len);
-        uint64_t written = 0;
-        for (size_t i = 0; i < n; i++) {
-            if (status[i] != NB200_CB_PERFECT && status[i] != NB200_CB_CORRECTED) continue;
-            const FqRec &x = A.recs[i], &y = B.recs[i];
-            const char *t1 = A.text.data(), *t2 = B.text.data();
-            uint32_t nl = x.name_len;
-            if (nl >= 2 && t1[x.name + nl - 2] == '/' && t1[x.name + nl - 1] == '1') nl -= 2;
-            const std::string &cbs = W->entries[(size_t)idx[i]];
-            R.names.add(t1 + x.name, nl);
-            R.r1.add(t1 + x.seq + bl, x.len - bl);
-            R.r2.add(t2 + y.seq, y.len);
-            R.cb.add(cbs.data(), cbs.size());
-            R.ub.add(t1 + x.seq + cb_len, (size_t)umi_len);
-            R.ur.add("", 0); R.gn.add("", 0);
-            R.pos1.push_back(0); R.pos2.push_back(0);            // unaligned records carry no position
-            written++;
-        }
-        dev.written_pairs = written;
-        pt.lap("build read set");
-        align_readset(c, R, lib_ids, outputs, n_libs, pt);
-        if (stats) *stats = dev;
-    } catch (const IoError &e) { c->err = e.what(); return NB200_EIO; }
+    PhaseTimer pt;
+    nb200_cb_stats st{};
+    std::vector<std::string> lines;
+    read_whitelist_lines(whitelist_path, lines);
+    std::unique_ptr<DevWhitelist> W = build_whitelist(c, std::move(lines), cb_len);
+    FastqQ A, B;
+    {
+        std::string err;
+        std::thread t([&] { try { load_fastq_qual(r2_fastq, B); } catch (const std::exception &e) { err = e.what(); } });
+        try { load_fastq_qual(r1_fastq, A); } catch (...) { t.join(); throw; }
+        t.join();
+        if (!err.empty()) throw IoError(err);
+    }
+    pt.lap("whitelist + FASTQ parse");
+    const size_t n = std::min(A.recs.size(), B.recs.size());
+    std::vector<uint8_t> cb(n * (size_t)cb_len + 16), qual(n * (size_t)cb_len + 16), elig(n + 16);
+    slice_barcodes(A, B, cb_len, umi_len, c->host_threads, cb.data(), qual.data(), elig.data(), st);
+    std::vector<int32_t> idx(n + 1);
+    std::vector<uint8_t> status(n + 1);
+    nb200_cb_stats dev{};
+    cb_upload(c, cb_len, (const char *)cb.data(), qual.data(), elig.data(), n, &dev);
+    cb_run(c, *W, &dev);
+    cb_fetch(c, idx.data(), status.data(), &dev);
+    c->ev_pool.clear();
+    c->cb_resident = false;
+    dev.total_pairs = st.total_pairs; dev.name_mismatch = st.name_mismatch; dev.too_short = st.too_short;
+    dev.no_remaining_seq = st.no_remaining_seq;
+    pt.lap("barcode correction");
+    ReadSet R;
+    const uint32_t bl = (uint32_t)(cb_len + umi_len);
+    uint64_t written = 0;
+    for (size_t i = 0; i < n; i++) {
+        if (status[i] != NB200_CB_PERFECT && status[i] != NB200_CB_CORRECTED) continue;
+        const FqRec &x = A.recs[i], &y = B.recs[i];
+        const char *t1 = A.text.data(), *t2 = B.text.data();
+        uint32_t nl = x.name_len;
+        if (nl >= 2 && t1[x.name + nl - 2] == '/' && t1[x.name + nl - 1] == '1') nl -= 2;
+        const std::string &cbs = W->entries[(size_t)idx[i]];
+        R.names.add(t1 + x.name, nl);
+        R.r1.add(t1 + x.seq + bl, x.len - bl);
+        R.r2.add(t2 + y.seq, y.len);
+        R.cb.add(cbs.data(), cbs.size());
+        R.ub.add(t1 + x.seq + cb_len, (size_t)umi_len);
+        written++;
+    }
+    dev.written_pairs = written;
+    pt.lap("build read set");
+    align_readset(c, R, lib_ids, outputs, n_libs, pt);
+    if (stats) *stats = dev;
     API_END(c)
 }
 
@@ -2450,26 +2410,24 @@ int32_t nb200_report_file(nb200_ctx *c, const char *in_tsv, const char *out_tsv,
     API_BEGIN(c)
     if (!in_tsv || !out_tsv) throw std::runtime_error("bad arguments");
     if (out3) out3[0] = out3[1] = out3[2] = 0;
-    try {
-        ReportRows R;
-        if (!parse_per_read_tsv(in_tsv, R, c->host_threads)) {
-            write_counts_tsv(out_tsv, nullptr, R.feature_names, R.cells);       // write_empty_df
-            return NB200_OK;
-        }
-        int32_t lib_id = -1;
-        {
-            auto L = std::make_unique<DevLibrary>();
-            build_feature_dictionary(R.feature_names, L->host);
-            finish_library(c, std::move(L), &lib_id);
-        }
-        nb200_counts counts{};
-        const int32_t rc = nb200_umi_counts(c, lib_id, R.key.size(), R.key.data(), R.off.data(), R.ids.data(), R.score.data(),
-                                            umi_threshold, disable_thresholding, &counts);
-        c->libs.pop_back();                                                     // the dictionary was only for this call
-        if (rc != NB200_OK) return rc;
-        write_counts_tsv(out_tsv, &counts, R.feature_names, R.cells);
-        if (out3) { out3[0] = R.key.size(); out3[1] = counts.n_rows; out3[2] = counts.dropped_empty; }
-    } catch (const IoError &e) { c->err = e.what(); return NB200_EIO; }
+    ReportRows R;
+    if (!parse_per_read_tsv(in_tsv, R, c->host_threads)) {
+        write_counts_tsv(out_tsv, nullptr, R.feature_names, R.cells);       // write_empty_df
+        return NB200_OK;
+    }
+    int32_t lib_id = -1;
+    {
+        auto L = std::make_unique<DevLibrary>();
+        build_feature_dictionary(R.feature_names, L->host);
+        finish_library(c, std::move(L), &lib_id);
+    }
+    nb200_counts counts{};
+    const int32_t rc = nb200_umi_counts(c, lib_id, R.key.size(), R.key.data(), R.off.data(), R.ids.data(), R.score.data(),
+                                        umi_threshold, disable_thresholding, &counts);
+    c->libs.pop_back();                                                     // the dictionary was only for this call
+    if (rc != NB200_OK) return rc;
+    write_counts_tsv(out_tsv, &counts, R.feature_names, R.cells);
+    if (out3) { out3[0] = R.key.size(); out3[1] = counts.n_rows; out3[2] = counts.dropped_empty; }
     API_END(c)
 }
 
@@ -2583,12 +2541,10 @@ int32_t nb200_load_whitelist_mem(nb200_ctx *c, const char *entries, uint64_t n, 
 int32_t nb200_load_whitelist(nb200_ctx *c, const char *path, int32_t cb_len, int32_t *wl_id) {
     API_BEGIN(c)
     if (!path || !wl_id) throw std::runtime_error("bad arguments");
-    try {
-        std::vector<std::string> e;
-        read_whitelist_lines(path, e);
-        c->wls.push_back(build_whitelist(c, std::move(e), cb_len));
-        *wl_id = (int32_t)c->wls.size() - 1;
-    } catch (const IoError &ex) { c->err = ex.what(); return NB200_EIO; }
+    std::vector<std::string> e;
+    read_whitelist_lines(path, e);
+    c->wls.push_back(build_whitelist(c, std::move(e), cb_len));
+    *wl_id = (int32_t)c->wls.size() - 1;
     API_END(c)
 }
 
@@ -2649,40 +2605,38 @@ int32_t nb200_fastq_to_bam(nb200_ctx *c, const char *r1_fastq, const char *r2_fa
                            const char *output_bam, int32_t cb_len, int32_t umi_len, nb200_cb_stats *stats) {
     API_BEGIN(c)
     if (!r1_fastq || !r2_fastq || !whitelist_path || !output_bam || cb_len < 1 || umi_len < 0) throw std::runtime_error("bad arguments");
-    try {
-        nb200_cb_stats st{};
-        std::vector<std::string> lines;
-        read_whitelist_lines(whitelist_path, lines);
-        std::unique_ptr<DevWhitelist> W = build_whitelist(c, std::move(lines), cb_len);
-        FastqQ A, B;
-        {
-            std::string err;
-            std::thread t([&] { try { load_fastq_qual(r2_fastq, B); } catch (const std::exception &e) { err = e.what(); } });
-            try { load_fastq_qual(r1_fastq, A); } catch (...) { t.join(); throw; }
-            t.join();
-            if (!err.empty()) throw IoError(err);
-        }
-        const size_t n = std::min(A.recs.size(), B.recs.size());
-        std::vector<uint8_t> cb(n * (size_t)cb_len + 16), qual(n * (size_t)cb_len + 16), elig(n + 16);
-        slice_barcodes(A, B, cb_len, umi_len, c->host_threads, cb.data(), qual.data(), elig.data(), st);
-        std::vector<int32_t> idx(n + 1);
-        std::vector<uint8_t> status(n + 1);
-        nb200_cb_stats dev{};
-        cudaEvent_t e0 = new_event(c), e1 = new_event(c);
-        CK(cudaEventRecord(e0, c->s_compute));
-        cb_upload(c, cb_len, (const char *)cb.data(), qual.data(), elig.data(), n, &dev);
-        cb_run(c, *W, &dev);
-        cb_fetch(c, idx.data(), status.data(), &dev);
-        CK(cudaEventRecord(e1, c->s_compute));
-        CK(cudaEventSynchronize(e1));
-        CK(cudaEventElapsedTime(&dev.total_ms, e0, e1));
-        c->ev_pool.clear();
-        dev.total_pairs = st.total_pairs; dev.name_mismatch = st.name_mismatch; dev.too_short = st.too_short;
-        dev.no_remaining_seq = st.no_remaining_seq;
-        write_10x_bam(output_bam, A, B, cb_len, umi_len, idx.data(), status.data(), W->entries, c->host_threads, dev);
-        c->cb_resident = false;
-        if (stats) *stats = dev;
-    } catch (const IoError &e) { c->err = e.what(); return NB200_EIO; }
+    nb200_cb_stats st{};
+    std::vector<std::string> lines;
+    read_whitelist_lines(whitelist_path, lines);
+    std::unique_ptr<DevWhitelist> W = build_whitelist(c, std::move(lines), cb_len);
+    FastqQ A, B;
+    {
+        std::string err;
+        std::thread t([&] { try { load_fastq_qual(r2_fastq, B); } catch (const std::exception &e) { err = e.what(); } });
+        try { load_fastq_qual(r1_fastq, A); } catch (...) { t.join(); throw; }
+        t.join();
+        if (!err.empty()) throw IoError(err);
+    }
+    const size_t n = std::min(A.recs.size(), B.recs.size());
+    std::vector<uint8_t> cb(n * (size_t)cb_len + 16), qual(n * (size_t)cb_len + 16), elig(n + 16);
+    slice_barcodes(A, B, cb_len, umi_len, c->host_threads, cb.data(), qual.data(), elig.data(), st);
+    std::vector<int32_t> idx(n + 1);
+    std::vector<uint8_t> status(n + 1);
+    nb200_cb_stats dev{};
+    cudaEvent_t e0 = new_event(c), e1 = new_event(c);
+    CK(cudaEventRecord(e0, c->s_compute));
+    cb_upload(c, cb_len, (const char *)cb.data(), qual.data(), elig.data(), n, &dev);
+    cb_run(c, *W, &dev);
+    cb_fetch(c, idx.data(), status.data(), &dev);
+    CK(cudaEventRecord(e1, c->s_compute));
+    CK(cudaEventSynchronize(e1));
+    CK(cudaEventElapsedTime(&dev.total_ms, e0, e1));
+    c->ev_pool.clear();
+    dev.total_pairs = st.total_pairs; dev.name_mismatch = st.name_mismatch; dev.too_short = st.too_short;
+    dev.no_remaining_seq = st.no_remaining_seq;
+    write_10x_bam(output_bam, A, B, cb_len, umi_len, idx.data(), status.data(), W->entries, c->host_threads, dev);
+    c->cb_resident = false;
+    if (stats) *stats = dev;
     API_END(c)
 }
 

@@ -1,7 +1,5 @@
-// Native read ingest and per-read TSV output (SURVEY.md §8a X2/X5, §8f rank 1): FASTQ(.gz) and
-// BAM (BGZF, inflated block-parallel, no htslib) -> names / sequences / CB,UB,UR,GN tags ->
-// nb200_pack_reads -> nb200_align -> the TSV nimble's `report` consumes
-// (nimble/__main__.py:219,237-241).  Used by nb200_align_files and the `aligner` executable.
+// Whole-file reads (slurp_maybe_gz: fastq-to-bam, the 10x one-pass route, report) and the per-read TSV of the 10x one-pass
+// route (nb200_align_10x_fastq, `align --map`).  The aligner's file entries stream their input instead (stream.cpp).
 #include "ingest.hpp"
 
 #include <zlib.h>
@@ -10,11 +8,7 @@
 #include <atomic>
 #include <cstdio>
 #include <cstring>
-#include <memory>
-#include <stdexcept>
-#include <chrono>
 #include <thread>
-#include <unordered_map>
 
 namespace nb200 {
 
@@ -74,334 +68,6 @@ void Arena::add(const char *p, size_t n) {
     off.push_back((int64_t)data.size());
 }
 
-static void read_fastq(const std::string &path, Arena &names, Arena &seqs) {
-    std::string text;
-    slurp_gz(path, text);
-    const char *p = text.data(), *end = p + text.size();
-    while (p < end) {
-        const char *l1 = (const char *)memchr(p, '\n', end - p);
-        if (!l1) break;
-        const char *l2 = (const char *)memchr(l1 + 1, '\n', end - (l1 + 1));
-        if (!l2) l2 = end;
-        if (*p != '@') throw std::runtime_error("malformed FASTQ record in " + path);
-        const char *ne = p + 1;
-        while (ne < l1 && *ne != ' ' && *ne != '\t' && *ne != '\r') ne++;
-        names.add(p + 1, ne - (p + 1));
-        const char *se = l2;
-        while (se > l1 + 1 && (se[-1] == '\r' || se[-1] == '\n')) se--;
-        seqs.add(l1 + 1, se - (l1 + 1));
-        // skip '+' line and quality line
-        const char *q = l2 < end ? l2 + 1 : end;
-        for (int k = 0; k < 2 && q < end; k++) {
-            const char *nl = (const char *)memchr(q, '\n', end - q);
-            q = nl ? nl + 1 : end;
-        }
-        p = q;
-    }
-}
-
-// ---- BAM -----------------------------------------------------------------------------------------
-// out: uninitialised buffer of n bytes (a std::string would zero-fill half a gigabyte first)
-static void inflate_bgzf(const std::string &path, int threads, std::unique_ptr<char[]> &out, size_t &n_out) {
-    FILE *f = fopen(path.c_str(), "rb");
-    if (!f) throw IoError("cannot open " + path);
-    std::string raw;
-    {
-        std::vector<char> buf(1 << 22);
-        size_t n;
-        while ((n = fread(buf.data(), 1, buf.size(), f)) > 0) raw.append(buf.data(), n);
-        fclose(f);
-    }
-    struct Blk { size_t off, clen, uoff, ulen; };
-    std::vector<Blk> blks;
-    size_t p = 0, utotal = 0;
-    bool bgzf = true;
-    while (p + 18 <= raw.size()) {
-        const unsigned char *h = (const unsigned char *)raw.data() + p;
-        if (h[0] != 31 || h[1] != 139 || !(h[3] & 4)) { bgzf = false; break; }
-        const size_t xlen = h[10] | (h[11] << 8);
-        size_t bsize = 0, q = 12;
-        while (q + 4 <= 12 + xlen) {
-            const size_t slen = h[q + 2] | (h[q + 3] << 8);
-            if (h[q] == 'B' && h[q + 1] == 'C' && slen == 2) bsize = (size_t)(h[q + 4] | (h[q + 5] << 8)) + 1;
-            q += 4 + slen;
-        }
-        if (!bsize || p + bsize > raw.size()) { bgzf = false; break; }
-        const unsigned char *t = h + bsize - 4;
-        const size_t isize = t[0] | (t[1] << 8) | (t[2] << 16) | ((size_t)t[3] << 24);
-        blks.push_back({p + 12 + xlen, bsize - 12 - xlen - 8, utotal, isize});
-        utotal += isize;
-        p += bsize;
-    }
-    if (!bgzf || blks.empty()) {       // plain gzip (e.g. written by python's gzip module): one stream
-        std::string tmp;
-        slurp_gz(path, tmp);
-        n_out = tmp.size();
-        out.reset(new char[n_out + 1]);
-        memcpy(out.get(), tmp.data(), n_out);
-        return;
-    }
-    n_out = utotal;
-    out.reset(new char[utotal + 1]);
-    std::atomic<size_t> next{0};
-    std::atomic<int> bad{0};
-    auto work = [&] {
-        z_stream zs;
-        for (size_t i; (i = next.fetch_add(1)) < blks.size();) {
-            if (!blks[i].ulen) continue;
-            memset(&zs, 0, sizeof(zs));
-            if (inflateInit2(&zs, -15) != Z_OK) { bad = 1; return; }
-            zs.next_in = (Bytef *)raw.data() + blks[i].off; zs.avail_in = (uInt)blks[i].clen;
-            zs.next_out = (Bytef *)(out.get() + blks[i].uoff); zs.avail_out = (uInt)blks[i].ulen;
-            if (inflate(&zs, Z_FINISH) != Z_STREAM_END) bad = 1;
-            inflateEnd(&zs);
-        }
-    };
-    std::vector<std::thread> th;
-    for (int t = 0; t < std::max(1, threads); t++) th.emplace_back(work);
-    for (auto &x : th) x.join();
-    if (bad) throw IoError("corrupt BGZF block in " + path);
-}
-
-static inline uint32_t le32(const unsigned char *p) { return p[0] | (p[1] << 8) | (p[2] << 16) | ((uint32_t)p[3] << 24); }
-
-// BAM records -> ReadSet.  Three steps so that the heavy parts run on all host threads: (1) one
-// sequential walk over the record sizes, (2) block-parallel field/tag location, (3) a sequential
-// mate-pairing pass on names (records of a pair are adjacent in unaligned / name-sorted BAMs; a small
-// look-back window tolerates interleaving), (4) block-parallel decoding into the arenas.
-struct BamRec {
-    const unsigned char *name, *seq;     // seq: 4-bit packed
-    const char *tag[4];                  // CB UB UR GN (Z)
-    uint32_t name_len, l_seq, tag_len[4], flag;
-    int64_t pos;
-};
-
-template <class F>
-static void parallel_ranges(size_t n, int threads, F f) {
-    const int T = (int)std::max<size_t>(1, std::min<size_t>((size_t)std::max(1, threads), (n + 4095) / 4096));
-    if (T == 1) { f(0, (size_t)0, n); return; }
-    std::vector<std::thread> th;
-    std::vector<std::string> errs(T);
-    const size_t per = (n + T - 1) / T;
-    for (int t = 0; t < T; t++)
-        th.emplace_back([&, t] {
-            try { f(t, std::min(n, t * per), std::min(n, (t + 1) * per)); } catch (const std::exception &e) { errs[t] = e.what(); }
-        });
-    for (auto &x : th) x.join();
-    for (auto &e : errs) if (!e.empty()) throw std::runtime_error(e);
-}
-
-static void arena_layout(Arena &a, const std::vector<uint32_t> &lens) {      // offsets from lengths, data sized
-    a.off.resize(lens.size() + 1);
-    a.off[0] = 0;
-    for (size_t i = 0; i < lens.size(); i++) a.off[i + 1] = a.off[i] + lens[i];
-    a.data.resize((size_t)a.off[lens.size()]);
-}
-
-static void read_bam(const std::string &path, int threads, ReadSet &R) {
-    PhaseTimer pt;
-    std::unique_ptr<char[]> buf;
-    size_t n = 0;
-    inflate_bgzf(path, threads, buf, n);
-    pt.lap("read + inflate");
-    const unsigned char *b = (const unsigned char *)buf.get();
-    if (n < 12 || memcmp(b, "BAM\1", 4) != 0) throw std::runtime_error(path + " is not a BAM file");
-    size_t p = 4;
-    p += 4 + le32(b + p);
-    if (p + 4 > n) throw std::runtime_error("truncated BAM header in " + path);
-    const uint32_t n_ref = le32(b + p); p += 4;
-    for (uint32_t i = 0; i < n_ref && p + 4 <= n; i++) p += 4 + le32(b + p) + 4;
-    // (1) record starts
-    std::vector<size_t> starts;
-    starts.reserve(n / 128 + 16);
-    while (p + 4 <= n) {
-        const uint32_t bs = le32(b + p);
-        if (p + 4 + bs > n || bs < 32) throw std::runtime_error("truncated BAM record in " + path);
-        starts.push_back(p + 4);
-        p += 4 + bs;
-    }
-    const size_t nr = starts.size();
-    pt.lap("record walk");
-    // (2) locate fields and tags
-    std::vector<BamRec> recs(nr);
-    parallel_ranges(nr, threads, [&](int, size_t lo, size_t hi) {
-        for (size_t i = lo; i < hi; i++) {
-            const unsigned char *r = b + starts[i];
-            const unsigned char *end = r + le32(r - 4);
-            BamRec &x = recs[i];
-            x.pos = (int64_t)(int32_t)le32(r + 4) + 1;
-            const uint32_t l_name = r[8];
-            const uint32_t n_cigar = r[12] | (r[13] << 8);
-            x.flag = r[14] | (r[15] << 8);
-            x.l_seq = le32(r + 16);
-            const unsigned char *q = r + 32;
-            x.name = q; x.name_len = l_name ? l_name - 1 : 0;
-            q += l_name + 4 * (size_t)n_cigar;
-            x.seq = q;
-            q += (x.l_seq + 1) / 2 + (size_t)x.l_seq;
-            if (q > end) throw std::runtime_error("corrupt BAM record in " + path);
-            for (int t = 0; t < 4; t++) { x.tag[t] = nullptr; x.tag_len[t] = 0; }
-            while (q + 3 <= end) {
-                const char t0 = (char)q[0], t1 = (char)q[1], ty = (char)q[2]; q += 3;
-                size_t adv = 0;
-                const char *zs = nullptr;
-                switch (ty) {
-                case 'Z': case 'H': { zs = (const char *)q; adv = strnlen(zs, end - q) + 1; break; }
-                case 'A': case 'c': case 'C': adv = 1; break;
-                case 's': case 'S': adv = 2; break;
-                case 'i': case 'I': case 'f': adv = 4; break;
-                case 'B': { if (q + 5 > end) throw std::runtime_error("corrupt BAM tag in " + path);
-                            const char sub = (char)q[0]; const uint32_t cnt = le32(q + 1);
-                            const int es = (sub == 'c' || sub == 'C') ? 1 : (sub == 's' || sub == 'S') ? 2 : 4; adv = 5 + (size_t)cnt * es; break; }
-                default: throw std::runtime_error("unknown BAM tag type in " + path);
-                }
-                if (zs) {
-                    int slot = -1;
-                    if (t0 == 'C' && t1 == 'B') slot = 0; else if (t0 == 'U' && t1 == 'B') slot = 1;
-                    else if (t0 == 'U' && t1 == 'R') slot = 2; else if (t0 == 'G' && t1 == 'N') slot = 3;
-                    if (slot >= 0) { x.tag[slot] = zs; x.tag_len[slot] = (uint32_t)(adv - 1); }
-                }
-                q += adv;
-            }
-        }
-    });
-    pt.lap("locate fields");
-    // (3) pair mates by name
-    struct Out { int64_t m[2]; };
-    std::vector<Out> outs;
-    outs.reserve(nr / 2 + 16);
-    bool any_paired = false;
-    auto same_name = [&](const BamRec &x, const BamRec &y) {
-        return x.name_len == y.name_len && memcmp(x.name, y.name, x.name_len) == 0;
-    };
-    // half-open pairs by name hash -> output index, at any distance (coordinate-sorted BAMs keep mates far apart);
-    // the reference name-sorts first (samtools sort -t UR -n, nimble/__main__.py:345), so mates always meet there
-    std::unordered_multimap<uint64_t, size_t> open;
-    auto name_hash = [](const BamRec &x) {
-        uint64_t h = 1469598103934665603ull;
-        for (uint32_t j = 0; j < x.name_len; j++) { h ^= x.name[j]; h *= 1099511628211ull; }
-        return h;
-    };
-    for (size_t i = 0; i < nr; i++) {
-        const BamRec &x = recs[i];
-        if (x.flag & 0x900) continue;                       // secondary / supplementary
-        const int which = (x.flag & 0x80) ? 1 : 0;
-        if (which) any_paired = true;
-        if (!(x.flag & 0x1)) { outs.push_back(Out{{-1, -1}}); outs.back().m[which] = (int64_t)i; continue; }   // unpaired record
-        const uint64_t h = name_hash(x);
-        int64_t at = -1;
-        auto range = open.equal_range(h);
-        for (auto it = range.first; it != range.second; ++it) {
-            const Out &o = outs[it->second];
-            if (o.m[which] >= 0) continue;                  // same mate number again: not its partner
-            const BamRec &y = recs[(size_t)(o.m[0] >= 0 ? o.m[0] : o.m[1])];
-            if (same_name(x, y)) { at = (int64_t)it->second; open.erase(it); break; }
-        }
-        if (at < 0) { outs.push_back(Out{{-1, -1}}); at = (int64_t)outs.size() - 1; open.emplace(h, (size_t)at); }
-        outs[(size_t)at].m[which] = (int64_t)i;
-    }
-    // records still open here are true singletons (their mate is not in the file): kept with an empty partner,
-    // like frontend.load_reads
-    R.paired = any_paired;
-    R.has_tags = true;
-    pt.lap("pair mates");
-    // (4) decode into the arenas
-    const size_t no = outs.size();
-    auto first = [&](const Out &o) -> const BamRec * {     // the record that supplies name / tags / read 1
-        const int64_t i = (o.m[0] >= 0 || any_paired) ? o.m[0] : o.m[1];
-        return i >= 0 ? &recs[(size_t)i] : nullptr;
-    };
-    std::vector<uint32_t> ln(no), l1(no), l2(any_paired ? no : 0), lcb(no), lub(no), lur(no), lgn(no);
-    parallel_ranges(no, threads, [&](int, size_t lo, size_t hi) {
-        for (size_t i = lo; i < hi; i++) {
-            const Out &o = outs[i];
-            const BamRec *a = first(o);
-            const BamRec &nm = recs[(size_t)(o.m[0] >= 0 ? o.m[0] : o.m[1])];
-            ln[i] = nm.name_len;
-            l1[i] = a ? a->l_seq : 0;
-            if (any_paired) l2[i] = o.m[1] >= 0 ? recs[(size_t)o.m[1]].l_seq : 0;
-            lcb[i] = a ? a->tag_len[0] : 0;
-            lub[i] = a ? a->tag_len[1] : 0;      // r1_UB is the UB tag only: report() drops rows without it (nimble/__main__.py:237-245)
-            lur[i] = a ? a->tag_len[2] : 0;
-            lgn[i] = a ? a->tag_len[3] : 0;
-        }
-    });
-    arena_layout(R.names, ln); arena_layout(R.r1, l1); arena_layout(R.cb, lcb); arena_layout(R.ub, lub);
-    arena_layout(R.ur, lur); arena_layout(R.gn, lgn);
-    if (any_paired) arena_layout(R.r2, l2);
-    R.pos1.assign(no, -1); R.pos2.assign(no, -1);
-    static const char code[] = "=ACMGRSVTWYHKDBN";
-    char pair_lut[256][2];                                  // packed byte -> its two bases
-    for (int v = 0; v < 256; v++) { pair_lut[v][0] = code[v >> 4]; pair_lut[v][1] = code[v & 15]; }
-    auto decode = [&](const BamRec &x, char *dst) {
-        const uint32_t full = x.l_seq >> 1;
-        for (uint32_t i = 0; i < full; i++) memcpy(dst + 2 * i, pair_lut[x.seq[i]], 2);
-        if (x.l_seq & 1) dst[x.l_seq - 1] = code[x.seq[full] >> 4];
-        if (x.flag & 0x10) {                                // stored reverse-complemented: restore the read as sequenced
-            std::reverse(dst, dst + x.l_seq);
-            for (uint32_t i = 0; i < x.l_seq; i++) { char &c = dst[i]; c = c == 'A' ? 'T' : c == 'C' ? 'G' : c == 'G' ? 'C' : c == 'T' ? 'A' : c; }
-        }
-    };
-    parallel_ranges(no, threads, [&](int, size_t lo, size_t hi) {
-        for (size_t i = lo; i < hi; i++) {
-            const Out &o = outs[i];
-            const BamRec *a = first(o);
-            const BamRec &nm = recs[(size_t)(o.m[0] >= 0 ? o.m[0] : o.m[1])];
-            memcpy(&R.names.data[(size_t)R.names.off[i]], nm.name, nm.name_len);
-            if (a) {
-                decode(*a, &R.r1.data[(size_t)R.r1.off[i]]);
-                if (a->tag_len[0]) memcpy(&R.cb.data[(size_t)R.cb.off[i]], a->tag[0], a->tag_len[0]);
-                if (a->tag_len[1]) memcpy(&R.ub.data[(size_t)R.ub.off[i]], a->tag[1], a->tag_len[1]);
-                if (a->tag_len[2]) memcpy(&R.ur.data[(size_t)R.ur.off[i]], a->tag[2], a->tag_len[2]);
-                if (a->tag_len[3]) memcpy(&R.gn.data[(size_t)R.gn.off[i]], a->tag[3], a->tag_len[3]);
-                R.pos1[i] = a->pos;
-            }
-            if (any_paired && o.m[1] >= 0) {
-                const BamRec &m2 = recs[(size_t)o.m[1]];
-                decode(m2, &R.r2.data[(size_t)R.r2.off[i]]);
-                R.pos2[i] = m2.pos;
-            }
-        }
-    });
-    pt.lap("decode");
-}
-
-void load_reads(const std::vector<std::string> &inputs, int threads, ReadSet &R) {
-    if (inputs.empty() || inputs.size() > 2) throw std::runtime_error("expected one or two --input files");
-    std::string lower = inputs[0];
-    std::transform(lower.begin(), lower.end(), lower.begin(), ::tolower);
-    if (ends_with(lower, ".bam")) { read_bam(inputs[0], threads, R); return; }
-    if (inputs.size() == 2) {                               // the two files inflate and parse side by side
-        Arena n2;
-        std::string err;
-        std::thread t([&] { try { read_fastq(inputs[1], n2, R.r2); } catch (const std::exception &e) { err = e.what(); } });
-        try { read_fastq(inputs[0], R.names, R.r1); } catch (...) { t.join(); throw; }
-        t.join();
-        if (!err.empty()) throw std::runtime_error(err);
-        if (R.r2.size() != R.r1.size()) throw std::runtime_error("R1 and R2 FASTQ files hold different numbers of reads");
-        R.paired = true;
-    } else {
-        read_fastq(inputs[0], R.names, R.r1);
-    }
-}
-
-// FNV-1a over every field of every read in order: lets a test compare this reader with another one
-uint64_t readset_checksum(const ReadSet &R) {
-    uint64_t h = 1469598103934665603ull;
-    auto mix = [&](const char *p, size_t n) {
-        for (size_t i = 0; i < n; i++) { h ^= (unsigned char)p[i]; h *= 1099511628211ull; }
-        h ^= 0xFF; h *= 1099511628211ull;                   // field separator
-    };
-    const size_t n = R.r1.size();
-    for (size_t i = 0; i < n; i++) {
-        mix(R.names.ptr(i), R.names.len(i));
-        mix(R.r1.ptr(i), R.r1.len(i));
-        if (R.paired) mix(R.r2.ptr(i), R.r2.len(i));
-        if (R.has_tags) { mix(R.cb.ptr(i), R.cb.len(i)); mix(R.ub.ptr(i), R.ub.len(i)); }
-    }
-    return h;
-}
-
 // ---- TSV output ------------------------------------------------------------------------------------
 struct Sink {
     FILE *f = nullptr;
@@ -443,11 +109,7 @@ void write_per_read_tsv(const std::string &out_path, const ReadSet &R, const nb2
             out += '\t'; out.append(R.names.ptr(i), R.names.len(i));
             out += '\t'; out.append(R.cb.ptr(i), R.cb.len(i));
             out += '\t'; out.append(R.ub.ptr(i), R.ub.len(i));
-            out += '\t'; out.append(R.ur.ptr(i), R.ur.len(i));
-            out += '\t'; out.append(R.gn.ptr(i), R.gn.len(i));
-            out += '\t'; if (R.pos1[i] > 0) out.append(num, (size_t)snprintf(num, sizeof num, "%lld", (long long)R.pos1[i]));
-            out += '\t'; if (R.pos2[i] > 0) out.append(num, (size_t)snprintf(num, sizeof num, "%lld", (long long)R.pos2[i]));
-            out += '\n';
+            out += "\t\t\t\t\n";                           // r1_UR, r1_GN, r1_POS, r2_POS: unaligned records carry none
         }
     };
     for (size_t base = 0; base < n; base += kSlab * (size_t)T) {
@@ -458,22 +120,6 @@ void write_per_read_tsv(const std::string &out_path, const ReadSet &R, const nb2
             th.emplace_back([&, k] { format(base + k * kSlab, std::min(n, base + (k + 1) * kSlab), outs[k]); });
         for (auto &x : th) x.join();
         for (auto &o : outs) s.put(o);
-    }
-    s.close();
-    if (rename(tmp.c_str(), out_path.c_str()) != 0) throw IoError("cannot rename " + tmp);
-}
-
-void write_bulk_tsv(const std::string &out_path, const nb200_counts &c, const std::vector<std::string> &feature_names) {
-    const std::string tmp = out_path + ".tmp";
-    Sink s;
-    s.open(tmp, ends_with(out_path, ".gz"));
-    s.put("nimble_features\tnimble_score\n");
-    std::string line;
-    for (uint64_t i = 0; i < c.n_rows; i++) {
-        line.clear();
-        for (uint32_t j = c.feat_off[i]; j < c.feat_off[i + 1]; j++) { if (j > c.feat_off[i]) line += ','; line += feature_names[c.feat_ids[j]]; }
-        line += '\t'; line += std::to_string(c.count[i]); line += '\n';
-        s.put(line);
     }
     s.close();
     if (rename(tmp.c_str(), out_path.c_str()) != 0) throw IoError("cannot rename " + tmp);

@@ -1,4 +1,4 @@
-// Native read ingest / TSV output used by nb200_align_files and the `aligner` executable.
+// Host file code outside the streaming pipeline: whole-file reads, the 10x one-pass route's per-read TSV, fastq-to-bam, report.
 #pragma once
 #include <chrono>
 #include <cstdint>
@@ -34,17 +34,12 @@ struct Arena {                 // strings back to back: data + offsets (n + 1)
     size_t len(size_t i) const { return (size_t)(off[i + 1] - off[i]); }
 };
 
-struct ReadSet {
-    Arena names, r1, r2, cb, ub, ur, gn;
-    std::vector<int64_t> pos1, pos2;
-    bool paired = false, has_tags = false;
+struct ReadSet {                // the pairs of the 10x one-pass route: corrected CB, raw UB, read 1, read 2
+    Arena names, r1, r2, cb, ub;
 };
 
-void load_reads(const std::vector<std::string> &inputs, int threads, ReadSet &out);
-uint64_t readset_checksum(const ReadSet &R);
 void write_per_read_tsv(const std::string &out_path, const ReadSet &R, const nb200_read_result *res, const int32_t *feats,
                         int max_hits, const std::vector<std::string> &feature_names, int threads = 1);
-void write_bulk_tsv(const std::string &out_path, const nb200_counts &c, const std::vector<std::string> &feature_names);
 
 // ---- fastq-to-bam (fastq2bam.cpp) -------------------------------------------------------------------
 struct FqRec { uint64_t name, seq, qual; uint32_t name_len, len; };   // offsets into FastqQ::text

@@ -1130,7 +1130,7 @@ struct Pipeline {
                             c.n_exact_miss += T->cbn[3]; c.n_multi += T->cbn[4]; c.probes += T->cbn[5];
                             c.written_pairs += T->cbn[0] + T->cbn[1];
                         }
-                        if (dry && !getenv("NB200_INGEST_NOSUM"))      // reader statistics (nb200_host_ingest_stats): same checksum as readset_checksum
+                        if (dry && !getenv("NB200_INGEST_NOSUM"))      // reader statistics (nb200_host_ingest_stats): FNV-1a over every field of every read
                             for (size_t i = 0; i < T->n; i++) {
                                 mix(T->names.ptr(i), T->names.len(i));
                                 unpack(T->r1, i); mix(bases.data(), bases.size());

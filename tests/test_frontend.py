@@ -267,7 +267,7 @@ def test_report_with_summarize_writes_both_files(engine, tmp_path, monkeypatch):
 
 
 def _fnv_reads(d):
-    """Same FNV-1a as readset_checksum (csrc/ingest.cpp) over the Python reader's view of the file."""
+    """Same FNV-1a as nb200_host_ingest_stats (csrc/stream.cpp) over the Python reader's view of the file."""
     h = 1469598103934665603
     M = (1 << 64) - 1
 
