@@ -1672,6 +1672,8 @@ __device__ __forceinline__ void row_matches(const RefWin &w, uint32_t qrep, uint
 // One DP row of the band for two alignments at once (s16 halves).  y0/y1/y2: match flags of cells 0-7 / 8-15 / 16
 // (cell b at bit 2(b & 7) of each half).  H = max(0, diag + s, max(up, left) + gap): packed add, packed max,
 // DPX add-max with ReLU (VIADDMNMX.S16x2.RELU); row maxima with the DPX three-way max (VIMNMX3.S16x2).
+// s16 headroom: a read that reaches SW has a k-mer the library lacks, so no window matches all of its bases; at 500
+// bases V <= 64 * 499, and diag + kMatchDelta < 64 * 499 + 193 < 32767 (test_long_reads_gpu.py::test_sw_near_s16_ceiling).
 __device__ __forceinline__ void sw_row(uint32_t (&H)[kNB], uint32_t y0, uint32_t y1, uint32_t y2, uint32_t &best) {
     uint32_t left = 0, rowmax = 0;
 #pragma unroll

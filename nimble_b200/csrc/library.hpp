@@ -13,6 +13,7 @@ namespace nb200 {
 
 constexpr uint32_t kEmptyClass = 0xFFFFFFFFu;
 constexpr uint32_t kRefPad = 640;        // invalid bases before/after every reference (>= 500 + band + 64)
+                                          // (a 500-base read may overhang a reference by 480: test_long_reads_gpu.py::test_reference_overhangs)
 constexpr uint32_t kMaxRefs = 65535u * 32u;        // class words are indexed with 16 bits, 0xFFFF = no word
 
 // k-mer table: bucketed cuckoo hashing keyed by the CANONICAL k-mer.  Entry = 16 B; bucket = 2 entries = 32 B =
