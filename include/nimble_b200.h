@@ -133,7 +133,11 @@ const char *nb200_version(void);
 
 /* `-r LIB.json` (nimble/__main__.py:182-189): parse [config, data] (nimble/__main__.py:64-65,
  * nimble/types.py:10-32), build the k-mer -> equivalence-class index and upload it.
- * strand_filter: "unstranded" | "fiveprime" | "threeprime" | "none". */
+ * strand_filter: "unstranded" | "fiveprime" | "threeprime" | "none".
+ * The path may also name an index file written by nb200_index_write (told apart by its magic bytes, not its
+ * extension): it is loaded without a build and each device checks its copy of the image (a damaged file is
+ * NB200_EINVAL, nothing is registered).  k <= 0: the index's own k (20 for a JSON); any other k that differs from an
+ * index's k is NB200_EINVAL.  So every entry that takes library paths (the *_multi calls too) takes index files. */
 int32_t nb200_load_library(nb200_ctx *ctx, const char *json_path, const char *strand_filter, int32_t k,
                            int32_t *lib_id);
 /* same, from memory: names/sequences/feature names per reference + explicit config */
@@ -155,6 +159,15 @@ const char *nb200_feature_name(const nb200_ctx *ctx, int32_t lib_id, uint32_t fe
 /* host-only dry run of nb200_load_library (no CUDA call): out6 = n_refs, n_features, n_kmers,
  * n_classes, n_slots, identity_features.  Errors via nb200_last_error(NULL). */
 int32_t nb200_host_index_stats(const char *json_path, const char *strand_filter, int32_t k, int64_t *out6);
+/* host-only (no CUDA call, runs on a machine without a GPU): build the index of `json_path` at k (<= 0: 20) and write
+ * it to out_path (via out_path.tmp, then rename) as an index file (DESIGN.md §4) that nb200_load_library reads in
+ * place of the JSON.  host_threads <= 0: all cores.  Errors via nb200_last_error(NULL). */
+int32_t nb200_index_write(const char *json_path, int32_t k, int32_t host_threads, const char *out_path);
+/* host-only: header of an index file.  out9 = format version, k, n_refs, n_features, n_kmers, n_classes, n_slots,
+ * identity_features (as nb200_host_index_stats), device image bytes.  The header and host sections are always checked;
+ * verify = 1 also checks the image's checksum and looks every valid k-mer of every reference up in the image read back
+ * (it must find a class that holds that reference).  A damaged or foreign file: NB200_EINVAL with the reason. */
+int32_t nb200_index_info(const char *path, int32_t verify, int64_t *out9);
 
 /* test hook (host only): the raw-DEFLATE decoder the BGZF reader tries before zlib (csrc/fast_inflate.hpp).
  * 1 = the stream decoded into exactly out_len bytes, 0 = declined (the reader then uses zlib). */

@@ -1,12 +1,14 @@
 """`python -m nimble_b200 <subcommand>` — same sub-commands and flags as `python -m nimble`
 (nimble/__main__.py:373-468) for the hot path: generate, align, report.  `download` reports that
 the aligner is built in; `fastq-to-bam` (nimble/__main__.py:424-431) runs its barcode correction on
-the GPU; `fastq-to-counts` (an extension) runs fastq-to-bam and align --counts in one pass; `plot` is outside the hot path (DESIGN.md §7)."""
+the GPU; `fastq-to-counts` (an extension) runs fastq-to-bam and align --counts in one pass; `index` (an extension) saves a
+library's k-mer index to a file that every command taking --reference loads without a build; `plot` is outside the hot
+path (DESIGN.md §7)."""
 import argparse
 import sys
 
 from . import __version__
-from .frontend import align, align_10x, fastq_to_bam_with_barcodes, fastq_to_counts, generate, report
+from .frontend import align, align_10x, fastq_to_bam_with_barcodes, fastq_to_counts, generate, index, report
 
 
 def main(argv=None):
@@ -30,7 +32,7 @@ def main(argv=None):
     a.add_argument("--strand_filter", help="Filter reads based on strand information.", type=str, default="unstranded")
     a.add_argument("--trim", help="<TARGET_LENGTH>:<STRICTNESS>, comma-separated, one entry per library", type=str, default="")
     a.add_argument("--tmpdir", help="Path to a temporary directory for sorting .bam files", type=str, default=None)
-    a.add_argument("-k", "--kmer", help="k-mer length of the index (4..32)", type=int, default=20)
+    a.add_argument("-k", "--kmer", help="k-mer length of the index (4..32; default: an index file's own, 20 for a JSON)", type=int, default=None)
     a.add_argument("--map", help="(extension) cell barcode whitelist: --input is a raw 10x R1/R2 FASTQ pair, fastq-to-bam runs in "
                                  "the same pass without writing a BAM", type=str, default=None)
     a.add_argument("--gpus", help="(extension) GPUs of this node to spread the reads over (default 1; also $NB200_GPUS)", type=int, default=None)
@@ -70,7 +72,7 @@ def main(argv=None):
     fc.add_argument("-c", "--num_cores", help="The number of host threads to use.", type=int, default=1)
     fc.add_argument("--strand_filter", help="Filter reads based on strand information.", type=str, default="unstranded")
     fc.add_argument("--trim", help="<TARGET_LENGTH>:<STRICTNESS>, comma-separated, one entry per library", type=str, default="")
-    fc.add_argument("-k", "--kmer", help="k-mer length of the index (4..32)", type=int, default=20)
+    fc.add_argument("-k", "--kmer", help="k-mer length of the index (4..32; default: an index file's own, 20 for a JSON)", type=int, default=None)
     fc.add_argument("--gpus", help="GPUs of this node to spread the reads over (default 1; also $NB200_GPUS)", type=int, default=None)
     fc.add_argument("--cb-length", help="Length of cell barcode (default: 16).", type=int, default=16)
     fc.add_argument("--umi-length", help="Length of UMI (default: 12).", type=int, default=12)
@@ -78,6 +80,13 @@ def main(argv=None):
                     type=float, default=0.05)
     fc.add_argument("--disable_thresholding", help="Disable the per-UMI proportional count thresholding algorithm.",
                     action="store_true", default=False)
+
+    ix = sub.add_parser("index", help="(extension) build one library's k-mer index on the host and save it; --reference LIB.nb200idx "
+                                      "then loads it without a build")
+    ix.add_argument("--reference", help="The reference library JSON (one per call).", type=str, required=True)
+    ix.add_argument("--output", help="Path of the index file (e.g. LIB.nb200idx).", type=str, required=True)
+    ix.add_argument("-k", "--kmer", help="k-mer length of the index (4..32, default: 20)", type=int, default=None)
+    ix.add_argument("-c", "--num_cores", help="The number of host threads to use (default: all cores).", type=int, default=0)
 
     pl = sub.add_parser("plot")          # visualisation: outside the hot path (DESIGN.md §7); flags accepted so scripts fail clearly
     pl.add_argument("--input_file", "-i", type=str, required=False)
@@ -118,6 +127,10 @@ def main(argv=None):
         sys.exit(fastq_to_counts(args.reference, args.r1_fastq, args.r2_fastq, args.map, args.counts, args.num_cores, args.strand_filter,
                                  args.trim, k=args.kmer, gpus=args.gpus, cb_length=args.cb_length, umi_length=args.umi_length,
                                  threshold=args.threshold, disable_thresholding=args.disable_thresholding))
+    elif args.subcommand == "index":
+        if "," in args.reference:
+            parser.error("index takes one library per call")
+        sys.exit(index(args.reference, args.output, k=args.kmer, num_cores=args.num_cores))
     else:
         parser.print_help()
 

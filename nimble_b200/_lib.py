@@ -28,6 +28,7 @@ EXPORTS = [
     "nb200_align_10x_fastq", "nb200_set_overlap", "nb200_bench_dpx_peak", "nb200_set_stats", "nb200_align_files_multi",
     "nb200_library_set_trim", "nb200_trim_maxinfo", "nb200_set_defer_fetch", "nb200_fetch_counts", "nb200_fetch_counts_start", "nb200_fast_inflate",
     "nb200_align_files_counts", "nb200_align_files_counts_multi", "nb200_fastq_to_counts", "nb200_fastq_to_counts_multi",
+    "nb200_index_write", "nb200_index_info",
 ]
 
 CB_SKIPPED, CB_PERFECT, CB_CORRECTED, CB_NONE = 0, 1, 2, 3
@@ -128,6 +129,8 @@ def load():
     L.nb200_bench_random_access.argtypes = [vp, u64, u32, ct.POINTER(dbl), ct.POINTER(dbl)]
     L.nb200_bench_dpx_peak.argtypes = [vp, u32, ct.POINTER(dbl), ct.POINTER(dbl)]
     L.nb200_host_index_stats.argtypes = [ct.c_char_p, ct.c_char_p, i32, ct.POINTER(ct.c_int64)]
+    L.nb200_index_write.argtypes = [ct.c_char_p, i32, i32, ct.c_char_p]
+    L.nb200_index_info.argtypes = [ct.c_char_p, i32, ct.POINTER(ct.c_int64)]
     L.nb200_align_10x_fastq.argtypes = [vp, ct.c_char_p, ct.c_char_p, ct.c_char_p, i32, i32, ct.POINTER(i32), ct.POINTER(ct.c_char_p), i32,
                                         ct.POINTER(CbStats)]
     L.nb200_set_overlap.argtypes = [vp, i32]

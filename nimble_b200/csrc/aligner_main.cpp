@@ -1,5 +1,6 @@
 // `aligner` — drop-in for the binary nimble's front end execs (nimble/__main__.py:154,195-196):
 //   aligner --input F [--input F2] -c N --strand_filter S { -r LIB.json -o OUT }... [-t TRIM]   [--gpus N | $NB200_GPUS]
+// -r also takes an index file written by `python -m nimble_b200 index` (LIB.nb200idx): no index build at start-up.
 // (argv built at nimble/__main__.py:177-192).  Copy it to <site-packages>/nimble/aligner next to
 // libnimble_b200.so and the unmodified `python -m nimble align` runs on the B200 backend.
 // Exit code 0 on success, non-zero otherwise (forwarded by nimble, __main__.py:198,211).
@@ -14,7 +15,7 @@
 int main(int argc, char **argv) {
     std::vector<const char *> inputs, libs, outs;
     const char *strand = "unstranded", *trim = "";
-    int cores = 0, k = 20, gpus = getenv("NB200_GPUS") ? atoi(getenv("NB200_GPUS")) : 1;
+    int cores = 0, k = 0, gpus = getenv("NB200_GPUS") ? atoi(getenv("NB200_GPUS")) : 1;
     for (int i = 1; i < argc; i++) {
         const std::string a = argv[i];
         auto need = [&](const char *what) -> const char * {

@@ -5,7 +5,9 @@
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
+#include <chrono>
 #include <cstring>
+#include <functional>
 #include <memory>
 #include <stdexcept>
 #include <string>
@@ -21,6 +23,7 @@
 #include "../../include/nimble_b200.h"
 #include "agg.cuh"
 #include "barcode.cuh"
+#include "checksum.hpp"
 #include "kernels.cuh"
 #include "ingest.hpp"
 #include "library.hpp"
@@ -316,8 +319,10 @@ static uint64_t h2d_reads(nb200_ctx *c, cudaStream_t cs, const nb200_reads *h, D
     return bytes;
 }
 
-static void upload_library(nb200_ctx *c, DevLibrary &L) {
-    HostLibrary &h = L.host;
+// Allocates L's slab for an image of layout `lay` (library.cpp), points L.dev into it and uploads the feature token
+// ranks.  The image itself arrives through copy_image.
+static void place_library(nb200_ctx *c, DevLibrary &L, const ImageLayout &lay) {
+    const HostLibrary &h = L.host;
     auto up = [&](DevBuf &b, const void *src, size_t bytes) {
         b.ensure(bytes ? bytes : 16);
         if (bytes) CK(cudaMemcpyAsync(b.p, src, bytes, cudaMemcpyHostToDevice, c->s_compute));
@@ -325,33 +330,23 @@ static void upload_library(nb200_ctx *c, DevLibrary &L) {
     up(L.tok_end, h.tok_end.data(), h.tok_end.size() * 4);
     up(L.tok_comma, h.tok_comma.data(), h.tok_comma.size() * 4);
     if (h.has_index) {
-        // hottest first: the window may only cover a prefix when the index outgrows the L2 set-aside
-        struct Part { const void *src; size_t bytes; size_t off; };   // table first: hottest
-        Part parts[11] = {{h.table.data(), h.table.size() * sizeof(Entry), 0}, {h.class_rec.data(), h.class_rec.size() * sizeof(ClassRec), 0},
-                          {h.ov_w.data(), h.ov_w.size() * 4, 0}, {h.ov_b.data(), h.ov_b.size() * 4, 0}, {h.ov_pre.data(), h.ov_pre.size() * 4, 0},
-                          {h.positions.data(), h.positions.size() * 4, 0}, {h.ref_gstart.data(), h.ref_gstart.size() * 4, 0},
-                          {h.ref_feature.data(), h.ref_feature.size() * 4, 0}, {h.ref2bit.data(), h.ref2bit.size() * 8, 0},
-                          {h.refN.data(), h.refN.size() * 4, 0}, {h.dual.data(), h.dual.size() * sizeof(DualRec), 0}};
-        size_t tot = 0;
-        for (auto &p : parts) { p.off = tot; tot += ((p.bytes + 255) & ~(size_t)255) + 256; }
-        L.slab.ensure(tot + 256);
-        L.slab_bytes = tot;
-        uint8_t *base = L.slab.as<uint8_t>();
-        for (auto &p : parts)
-            if (p.bytes) CK(cudaMemcpyAsync(base + p.off, p.src, p.bytes, cudaMemcpyHostToDevice, c->s_compute));
-        L.table_bytes = parts[0].bytes;
-        L.dev.table = reinterpret_cast<const uint4 *>(base + parts[0].off);
+        L.slab.ensure(lay.total + 256);
+        L.slab_bytes = lay.total;
+        const uint8_t *base = L.slab.as<uint8_t>();
+        auto at = [&](int part) { return base + lay.off[part]; };
+        L.table_bytes = lay.bytes[kPartTable];
+        L.dev.table = reinterpret_cast<const uint4 *>(at(kPartTable));
         L.dev.n_buckets = (uint32_t)h.n_buckets;
-        L.dev.dual = reinterpret_cast<const uint4 *>(base + parts[10].off);
-        L.dev.class_rec = reinterpret_cast<const uint4 *>(base + parts[1].off);
-        L.dev.ov_w = reinterpret_cast<const uint32_t *>(base + parts[2].off);
-        L.dev.ov_b = reinterpret_cast<const uint32_t *>(base + parts[3].off);
-        L.dev.ov_pre = reinterpret_cast<const uint32_t *>(base + parts[4].off);
-        L.dev.positions = reinterpret_cast<const uint32_t *>(base + parts[5].off);
-        L.dev.ref_gstart = reinterpret_cast<const uint32_t *>(base + parts[6].off);
-        L.dev.ref_feature = reinterpret_cast<const uint32_t *>(base + parts[7].off);
-        L.dev.ref2bit = reinterpret_cast<const uint64_t *>(base + parts[8].off);
-        L.dev.refN = reinterpret_cast<const uint32_t *>(base + parts[9].off);
+        L.dev.dual = reinterpret_cast<const uint4 *>(at(kPartDual));
+        L.dev.class_rec = reinterpret_cast<const uint4 *>(at(kPartClassRec));
+        L.dev.ov_w = reinterpret_cast<const uint32_t *>(at(kPartOvW));
+        L.dev.ov_b = reinterpret_cast<const uint32_t *>(at(kPartOvB));
+        L.dev.ov_pre = reinterpret_cast<const uint32_t *>(at(kPartOvPre));
+        L.dev.positions = reinterpret_cast<const uint32_t *>(at(kPartPositions));
+        L.dev.ref_gstart = reinterpret_cast<const uint32_t *>(at(kPartRefGstart));
+        L.dev.ref_feature = reinterpret_cast<const uint32_t *>(at(kPartRefFeature));
+        L.dev.ref2bit = reinterpret_cast<const uint64_t *>(at(kPartRef2bit));
+        L.dev.refN = reinterpret_cast<const uint32_t *>(at(kPartRefN));
         L.dev.n_refs = h.n_refs; L.dev.n_features = h.n_features; L.dev.n_words = h.n_words;
         L.dev.narrow_cap = kCap;
         if (const char *e = getenv("NB200_NARROW_CAP")) L.dev.narrow_cap = (uint32_t)std::min<long>(kCap, std::max<long>(0, atol(e)));   // tests: force the wide path
@@ -361,16 +356,170 @@ static void upload_library(nb200_ctx *c, DevLibrary &L) {
         L.dev.kbits = h.cfg.k == 32 ? 0xFFFFFFFFull : ((1ull << h.cfg.k) - 1);
     }
     CK(cudaStreamSynchronize(c->s_compute));
-    // the big host images are only needed for the upload
-    std::vector<Entry>().swap(h.table);
-    std::vector<DualRec>().swap(h.dual);
-    std::vector<ClassRec>().swap(h.class_rec);
-    std::vector<uint32_t>().swap(h.ov_w);
-    std::vector<uint32_t>().swap(h.ov_b);
-    std::vector<uint32_t>().swap(h.ov_pre);
-    std::vector<uint32_t>().swap(h.positions);
-    std::vector<uint64_t>().swap(h.ref2bit);
-    std::vector<uint32_t>().swap(h.refN);
+}
+
+// image bytes [offset, offset + len) into dst: from an index file or from a freshly built HostLibrary
+using ImageFill = std::function<void(uint64_t offset, uint64_t len, uint8_t *dst)>;
+
+// Copies one image of `total` bytes into the slab of Ls[d] on context cs[d], for every d: a pool of pinned staging
+// buffers is filled chunk by chunk and each chunk goes to every device on its compute stream; a buffer is filled again
+// once the copies out of it have completed on all devices.  Host memory is bounded by the pool, not by the image.
+static void copy_image(const std::vector<nb200_ctx *> &cs, const std::vector<DevLibrary *> &Ls, uint64_t total, const ImageFill &fill) {
+    constexpr uint64_t kChunk = 64ull << 20;
+    constexpr uint64_t kBuffers = 4;
+    struct Staging {
+        void *p = nullptr;
+        std::vector<Event> copied;              // per device
+        ~Staging() { if (p) cudaFreeHost(p); }
+    };
+    std::vector<Staging> pool((size_t)std::min<uint64_t>(kBuffers, (total + kChunk - 1) / kChunk));
+    auto drain = [&] { for (nb200_ctx *c : cs) { cudaSetDevice(c->device); cudaStreamSynchronize(c->s_compute); } };
+    try {
+        for (Staging &s : pool) {
+            CK(cudaHostAlloc(&s.p, (size_t)std::min(kChunk, total), cudaHostAllocPortable));
+            for (nb200_ctx *c : cs) {
+                CK(cudaSetDevice(c->device));
+                Event e;
+                CK(cudaEventCreateWithFlags(&e.h, cudaEventDisableTiming));
+                s.copied.push_back(std::move(e));
+            }
+        }
+        uint64_t i = 0;
+        for (uint64_t a = 0; a < total; a += kChunk, i++) {
+            Staging &s = pool[i % pool.size()];
+            const uint64_t n = std::min(kChunk, total - a);
+            if (i >= pool.size()) for (Event &e : s.copied) CK(cudaEventSynchronize(e));
+            fill(a, n, static_cast<uint8_t *>(s.p));
+            for (size_t d = 0; d < cs.size(); d++) {
+                CK(cudaSetDevice(cs[d]->device));
+                CK(cudaMemcpyAsync(Ls[d]->slab.as<uint8_t>() + a, s.p, n, cudaMemcpyHostToDevice, cs[d]->s_compute));
+                CK(cudaEventRecord(s.copied[d], cs[d]->s_compute));
+            }
+        }
+        for (nb200_ctx *c : cs) { CK(cudaSetDevice(c->device)); CK(cudaStreamSynchronize(c->s_compute)); }
+    } catch (...) {
+        drain();                               // no copy may still read a staging buffer when the pool is freed
+        throw;
+    }
+}
+
+// Index-file check on the device: the checksum of checksum.hpp over the copy of the image the kernels will read.
+// Grid-stride over 64-bit words, one atomicAdd per block.
+__global__ void __launch_bounds__(256) image_checksum_kernel(const uint64_t *__restrict__ w, uint64_t n, unsigned long long *sum) {
+    __shared__ unsigned long long part[8];
+    unsigned long long s = 0;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x)
+        s += image_word_sum(__ldg(w + i), i);
+    for (int o = 16; o; o >>= 1) s += __shfl_down_sync(0xFFFFFFFFu, s, o);
+    if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = s;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int j = 1; j < 8; j++) s += part[j];
+        atomicAdd(sum, s);
+    }
+}
+
+// Runs image_checksum_kernel on every device side by side; throws when a device's copy differs from `want`.
+static void check_image_sums(const std::vector<nb200_ctx *> &cs, const std::vector<DevLibrary *> &Ls, uint64_t want, const std::string &path,
+                             float *kernel_ms) {
+    std::vector<DevBuf> sum(cs.size());
+    std::vector<Event> t0(cs.size()), t1(cs.size());
+    std::vector<unsigned long long> got(cs.size(), 0);
+    for (size_t d = 0; d < cs.size(); d++) {
+        nb200_ctx *c = cs[d];
+        CK(cudaSetDevice(c->device));
+        CK(cudaEventCreate(&t0[d].h)); CK(cudaEventCreate(&t1[d].h));
+        sum[d].ensure(8);
+        CK(cudaMemsetAsync(sum[d].p, 0, 8, c->s_compute));
+        CK(cudaEventRecord(t0[d], c->s_compute));
+        image_checksum_kernel<<<(unsigned)c->sm_count * 8, 256, 0, c->s_compute>>>(Ls[d]->slab.as<uint64_t>(), Ls[d]->slab_bytes / 8,
+                                                                                  sum[d].as<unsigned long long>());
+        CK(cudaGetLastError());
+        CK(cudaEventRecord(t1[d], c->s_compute));
+        c->launches++;
+        CK(cudaMemcpyAsync(&got[d], sum[d].p, 8, cudaMemcpyDeviceToHost, c->s_compute));
+    }
+    *kernel_ms = 0.0f;
+    for (size_t d = 0; d < cs.size(); d++) {
+        CK(cudaSetDevice(cs[d]->device));
+        CK(cudaStreamSynchronize(cs[d]->s_compute));
+        float ms = 0.0f;
+        CK(cudaEventElapsedTime(&ms, t0[d], t1[d]));
+        *kernel_ms = std::max(*kernel_ms, ms);
+        sum[d].release();
+    }
+    for (size_t d = 0; d < cs.size(); d++)
+        if (got[d] != want)
+            throw std::runtime_error("index file " + path + " is damaged: the device image on GPU " + std::to_string(cs[d]->device) +
+                                     " fails its checksum");
+}
+
+// One library onto every context of `cs`, under the same id on each (they hold the same libraries): `meta` is the library
+// without its images, `fill` produces the image of `lay`, copied once to all devices.  With `want_sum` (an index file)
+// each device checks its copy; a failure leaves every context as it was.
+static void install_library(const std::vector<nb200_ctx *> &cs, const HostLibrary &meta, const ImageLayout &lay, const ImageFill &fill,
+                            const uint64_t *want_sum, const std::string &path, double host_s, int32_t *lib_id) {
+    std::vector<std::unique_ptr<DevLibrary>> Ls;
+    std::vector<DevLibrary *> raw;
+    auto t0 = std::chrono::steady_clock::now();
+    float sum_ms = 0.0f;
+    try {
+        for (nb200_ctx *c : cs) {
+            CK(cudaSetDevice(c->device));
+            Ls.push_back(std::make_unique<DevLibrary>());
+            Ls.back()->host = library_meta(meta);
+            raw.push_back(Ls.back().get());
+            place_library(c, *Ls.back(), lay);
+        }
+        if (meta.has_index) {
+            copy_image(cs, raw, lay.total, fill);
+            if (want_sum) check_image_sums(cs, raw, *want_sum, path, &sum_ms);
+        }
+    } catch (...) {
+        for (size_t d = 0; d < Ls.size(); d++) { cudaSetDevice(cs[d]->device); Ls[d].reset(); }   // frees each slab on its own device
+        throw;
+    }
+    if (getenv("NB200_TRACE") && meta.has_index)
+        fprintf(stderr, "[nb200 trace] library %s: %s %.3f s, image %.1f MB to %zu GPUs %.3f s, device checksum %.3f ms\n", path.c_str(),
+                want_sum ? "index read" : "index built", host_s, lay.total / 1e6, cs.size(),
+                std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count(), sum_ms);
+    for (size_t d = 0; d < cs.size(); d++) {
+        cs[d]->libs.push_back(std::move(Ls[d]));
+        if (d == 0 && lib_id) *lib_id = (int32_t)cs[d]->libs.size() - 1;
+    }
+}
+
+// From a library JSON (built on the host) or an index file (told apart by its magic bytes, not its extension): the
+// library loaded onto every context of `cs`.  k <= 0: the index's own k, or 20 for a JSON.
+static void load_library_path(const std::vector<nb200_ctx *> &cs, const char *path, const char *strand_filter, int32_t k, int host_threads,
+                              int32_t *lib_id) {
+    if (!path) throw std::runtime_error("library path is null");
+    const int sf = parse_strand_filter(strand_filter);
+    if (sf < 0) throw std::runtime_error(std::string("unknown --strand_filter value: ") + strand_filter);
+    const auto t0 = std::chrono::steady_clock::now();
+    auto since = [&] { return std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count(); };
+    if (is_index_file(path)) {
+        IndexFile f;
+        HostLibrary meta;
+        open_index_file(path, f, meta);
+        if (k > 0 && k != meta.cfg.k)
+            throw std::runtime_error(std::string("index file ") + path + " was built with k = " + std::to_string(meta.cfg.k) +
+                                     "; the call asks for k = " + std::to_string(k));
+        meta.cfg.strand_filter = sf;
+        const uint64_t want = f.h.sec[kSecImage].sum;
+        install_library(cs, meta, image_layout(f.h.part_bytes), [&](uint64_t a, uint64_t n, uint8_t *dst) { f.read_image(a, n, dst); },
+                        &want, path, since(), lib_id);
+        return;
+    }
+    std::vector<std::string> names, seqs, feats;
+    nb200_config cfg{};
+    parse_library_json(path, names, seqs, feats, cfg);
+    cfg.k = k > 0 ? k : 20;
+    cfg.strand_filter = sf;
+    HostLibrary h;
+    build_library(names, seqs, feats, cfg, host_threads, h, getenv("NB200_VERIFY_TABLE") != nullptr);
+    const ImageLayout lay = image_layout(h);
+    install_library(cs, h, lay, [&](uint64_t a, uint64_t n, uint8_t *dst) { image_fill(h, lay, a, n, dst); }, nullptr, path, since(), lib_id);
 }
 
 // Keep the index resident in L2 while reads and per-read outputs stream through it: persisting
@@ -1730,26 +1879,15 @@ void nb200_destroy(nb200_ctx *c) {
 
 const char *nb200_last_error(const nb200_ctx *c) { return c ? c->err.c_str() : g_create_err.c_str(); }
 
-static int32_t finish_library(nb200_ctx *c, std::unique_ptr<DevLibrary> L, int32_t *lib_id) {
-    upload_library(c, *L);
-    c->libs.push_back(std::move(L));
-    if (lib_id) *lib_id = (int32_t)c->libs.size() - 1;
-    return NB200_OK;
+// a library built in memory: installed as a freshly built JSON library is
+static void install_built(nb200_ctx *c, const HostLibrary &h, int32_t *lib_id) {
+    const ImageLayout lay = image_layout(h);
+    install_library({c}, h, lay, [&](uint64_t a, uint64_t n, uint8_t *dst) { image_fill(h, lay, a, n, dst); }, nullptr, "(memory)", 0.0, lib_id);
 }
 
 int32_t nb200_load_library(nb200_ctx *c, const char *json_path, const char *strand_filter, int32_t k, int32_t *lib_id) {
     API_BEGIN(c)
-    if (!json_path) throw std::runtime_error("json_path is null");
-    int sf = parse_strand_filter(strand_filter);
-    if (sf < 0) throw std::runtime_error(std::string("unknown --strand_filter value: ") + strand_filter);
-    std::vector<std::string> names, seqs, feats;
-    nb200_config cfg{};
-    parse_library_json(json_path, names, seqs, feats, cfg);
-    cfg.k = k > 0 ? k : 20;
-    cfg.strand_filter = sf;
-    auto L = std::make_unique<DevLibrary>();
-    build_library(names, seqs, feats, cfg, c->host_threads, L->host, getenv("NB200_VERIFY_TABLE") != nullptr);
-    finish_library(c, std::move(L), lib_id);
+    load_library_path({c}, json_path, strand_filter, k, c->host_threads, lib_id);
     API_END(c)
 }
 
@@ -1759,9 +1897,9 @@ int32_t nb200_load_library_mem(nb200_ctx *c, int32_t n_refs, const char *const *
     if (n_refs <= 0 || !names || !seqs || !cfg) throw std::runtime_error("bad arguments");
     std::vector<std::string> n(n_refs), s(n_refs), f(n_refs);
     for (int i = 0; i < n_refs; i++) { n[i] = names[i]; s[i] = seqs[i]; f[i] = features ? features[i] : names[i]; }
-    auto L = std::make_unique<DevLibrary>();
-    build_library(n, s, f, *cfg, c->host_threads, L->host);
-    finish_library(c, std::move(L), lib_id);
+    HostLibrary h;
+    build_library(n, s, f, *cfg, c->host_threads, h);
+    install_built(c, h, lib_id);
     API_END(c)
 }
 
@@ -1770,9 +1908,9 @@ int32_t nb200_load_feature_names(nb200_ctx *c, int32_t n, const char *const *nam
     if (n < 0 || (n && !names)) throw std::runtime_error("bad arguments");
     std::vector<std::string> v(n);
     for (int i = 0; i < n; i++) v[i] = names[i];
-    auto L = std::make_unique<DevLibrary>();
-    build_feature_dictionary(v, L->host);
-    finish_library(c, std::move(L), lib_id);
+    HostLibrary h;
+    build_feature_dictionary(v, h);
+    install_built(c, h, lib_id);
     API_END(c)
 }
 
@@ -1852,6 +1990,37 @@ int32_t nb200_host_index_stats(const char *json_path, const char *strand_filter,
         out6[4] = (int64_t)(2 * L.n_buckets); out6[5] = L.identity_features ? 1 : 0;
     } catch (const LimitError &e) { g_create_err = e.what(); return NB200_ELIMIT; }
     catch (const std::exception &e) { g_create_err = e.what(); return NB200_EINVAL; }
+    return NB200_OK;
+}
+
+int32_t nb200_index_write(const char *json_path, int32_t k, int32_t host_threads, const char *out_path) {
+    // host-only: the index of nb200_load_library, written as an index file (library.hpp) that loads without a build
+    if (!json_path || !out_path) { g_create_err = "bad arguments"; return NB200_EINVAL; }
+    try {
+        if (is_index_file(json_path)) throw std::runtime_error(std::string(json_path) + " is an index file already; index takes a library JSON");
+        std::vector<std::string> names, seqs, feats;
+        nb200_config cfg{};
+        parse_library_json(json_path, names, seqs, feats, cfg);
+        cfg.k = k > 0 ? k : 20;
+        const int T = host_threads > 0 ? host_threads : (int)std::max(1u, std::thread::hardware_concurrency());
+        HostLibrary L;
+        build_library(names, seqs, feats, cfg, T, L, getenv("NB200_VERIFY_TABLE") != nullptr);
+        write_index_file(L, json_path, out_path, T);
+    } catch (const std::exception &) { return status_of_exception(g_create_err); }
+    return NB200_OK;
+}
+
+int32_t nb200_index_info(const char *path, int32_t verify, int64_t *out9) {
+    if (!path || !out9) { g_create_err = "bad arguments"; return NB200_EINVAL; }
+    try {
+        IndexFile f;
+        HostLibrary meta;
+        open_index_file(path, f, meta);
+        if (verify) verify_index_file(f, meta, (int)std::max(1u, std::thread::hardware_concurrency()));
+        out9[0] = f.h.version; out9[1] = meta.cfg.k;
+        out9[2] = meta.n_refs; out9[3] = meta.n_features; out9[4] = (int64_t)meta.n_kmers; out9[5] = (int64_t)meta.n_classes;
+        out9[6] = (int64_t)(2 * meta.n_buckets); out9[7] = meta.identity_features ? 1 : 0; out9[8] = (int64_t)f.h.sec[kSecImage].bytes;
+    } catch (const std::exception &) { return status_of_exception(g_create_err); }
     return NB200_OK;
 }
 
@@ -2221,20 +2390,18 @@ static int32_t files_multi(const int32_t *devices, int32_t n_devices, int32_t ho
     }
     std::vector<int32_t> ids(n_libs, -1);
     if (rc == NB200_OK) {
-        // one index build per device, side by side (the builder is multi-threaded itself: share the host threads)
-        std::vector<std::thread> th;
-        std::vector<int32_t> rcs(ctxs.size(), NB200_OK);
-        for (size_t d = 0; d < ctxs.size(); d++)
-            th.emplace_back([&, d] {
-                for (int li = 0; li < n_libs && rcs[d] == NB200_OK; li++) {
-                    int32_t id = -1;
-                    rcs[d] = nb200_load_library(ctxs[d], library_json[li], strand_filter, k, &id);
-                    if (rcs[d] == NB200_OK && !trims.empty()) rcs[d] = nb200_library_set_trim(ctxs[d], id, trims[(size_t)li].first, trims[(size_t)li].second);
-                    if (d == 0) ids[li] = id;
-                }
-            });
-        for (auto &t : th) t.join();
-        for (size_t d = 0; d < ctxs.size(); d++) if (rcs[d] != NB200_OK && rc == NB200_OK) { rc = rcs[d]; what = nb200_last_error(ctxs[d]); }
+        // each library built (or its index file read) once, its image copied to every device
+        try {
+            for (int li = 0; li < n_libs; li++) {
+                load_library_path(ctxs, library_json[li], strand_filter, k, ctxs[0]->host_threads, &ids[li]);
+                if (!trims.empty())
+                    for (nb200_ctx *c : ctxs) {
+                        rc = nb200_library_set_trim(c, ids[li], trims[(size_t)li].first, trims[(size_t)li].second);
+                        if (rc != NB200_OK) { what = nb200_last_error(c); break; }
+                    }
+                if (rc != NB200_OK) break;
+            }
+        } catch (const std::exception &) { rc = status_of_exception(what); }
     }
     if (rc == NB200_OK) {
         try {
@@ -2417,9 +2584,9 @@ int32_t nb200_report_file(nb200_ctx *c, const char *in_tsv, const char *out_tsv,
     }
     int32_t lib_id = -1;
     {
-        auto L = std::make_unique<DevLibrary>();
-        build_feature_dictionary(R.feature_names, L->host);
-        finish_library(c, std::move(L), &lib_id);
+        HostLibrary h;
+        build_feature_dictionary(R.feature_names, h);
+        install_built(c, h, &lib_id);
     }
     nb200_counts counts{};
     const int32_t rc = nb200_umi_counts(c, lib_id, R.key.size(), R.key.data(), R.off.data(), R.ids.data(), R.score.data(),

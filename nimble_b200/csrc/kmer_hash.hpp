@@ -12,7 +12,8 @@
 namespace nb200 {
 
 // canonical k-mer (lo, hi halves) -> mixed 32-bit value; the first bucket uses its upper bits (multiply-high by
-// the bucket count), the second bucket a second mix of it and the key
+// the bucket count), the second bucket a second mix of it and the key.  Index files store tables built with these:
+// any change to kmer_mix or the bucket functions must bump kIndexVersion (library.hpp).
 NB200_HD uint32_t kmer_mix(uint32_t clo, uint32_t chi) {
     uint32_t a = clo * 0x9E3779B1u + chi * 0x85EBCA77u;
     a ^= a >> 15;

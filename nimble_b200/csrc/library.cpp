@@ -3,6 +3,7 @@
 
 #include <algorithm>
 #include <atomic>
+#include <cerrno>
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -14,6 +15,12 @@
 #include <thread>
 #include <unordered_map>
 
+#include <fcntl.h>
+#include <sys/stat.h>
+#include <unistd.h>
+
+#include "checksum.hpp"
+#include "ingest.hpp"
 #include "json.hpp"
 #include "kmer_hash.hpp"
 
@@ -553,6 +560,321 @@ void build_library(const std::vector<std::string> &names, const std::vector<std:
         if (bad) throw std::runtime_error("k-mer table self-check failed for " + std::to_string((uint64_t)bad) + " k-mers");
         lap("table self-check");
     }
+}
+
+// ---- device image -------------------------------------------------------------------------------------------------
+
+ImageLayout image_layout(const uint64_t bytes[kImageParts]) {
+    ImageLayout lay;
+    for (int p = 0; p < kImageParts; p++) {
+        lay.bytes[p] = bytes[p];
+        lay.off[p] = lay.total;
+        lay.total += ((bytes[p] + 255) & ~(uint64_t)255) + 256;
+    }
+    return lay;
+}
+
+struct PartSrc { const void *p; uint64_t bytes; };
+static void image_parts(const HostLibrary &L, PartSrc out[kImageParts]) {
+    auto v = [](const auto &vec) { return PartSrc{vec.data(), (uint64_t)vec.size() * sizeof(vec[0])}; };
+    out[kPartTable] = v(L.table); out[kPartClassRec] = v(L.class_rec);
+    out[kPartOvW] = v(L.ov_w); out[kPartOvB] = v(L.ov_b); out[kPartOvPre] = v(L.ov_pre);
+    out[kPartPositions] = v(L.positions); out[kPartRefGstart] = v(L.ref_gstart); out[kPartRefFeature] = v(L.ref_feature);
+    out[kPartRef2bit] = v(L.ref2bit); out[kPartRefN] = v(L.refN); out[kPartDual] = v(L.dual);
+}
+
+ImageLayout image_layout(const HostLibrary &L) {
+    PartSrc src[kImageParts];
+    image_parts(L, src);
+    uint64_t bytes[kImageParts];
+    for (int p = 0; p < kImageParts; p++) bytes[p] = src[p].bytes;
+    return image_layout(bytes);
+}
+
+void image_fill(const HostLibrary &L, const ImageLayout &lay, uint64_t offset, uint64_t len, uint8_t *dst) {
+    PartSrc src[kImageParts];
+    image_parts(L, src);
+    memset(dst, 0, len);
+    for (int p = 0; p < kImageParts; p++) {
+        const uint64_t a = std::max(offset, lay.off[p]), b = std::min(offset + len, lay.off[p] + lay.bytes[p]);
+        if (a < b) memcpy(dst + (a - offset), static_cast<const uint8_t *>(src[p].p) + (a - lay.off[p]), b - a);
+    }
+}
+
+HostLibrary library_meta(const HostLibrary &L) {
+    HostLibrary m;
+    m.cfg = L.cfg; m.has_index = L.has_index;
+    m.trim_on = L.trim_on; m.trim_target = L.trim_target; m.trim_strictness = L.trim_strictness;
+    m.feature_names = L.feature_names; m.tok_end = L.tok_end; m.tok_comma = L.tok_comma;
+    m.ref_names = L.ref_names; m.ref_feature = L.ref_feature; m.ref_len = L.ref_len; m.ref_gstart = L.ref_gstart;
+    m.identity_features = L.identity_features;
+    m.n_refs = L.n_refs; m.n_features = L.n_features; m.n_words = L.n_words;
+    m.n_kmers = L.n_kmers; m.n_classes = L.n_classes; m.n_buckets = L.n_buckets; m.n_spilled = L.n_spilled;
+    m.total_gbases = L.total_gbases;
+    return m;
+}
+
+// ---- index file ---------------------------------------------------------------------------------------------------
+
+static const char kIndexMagic[8] = {'N', 'B', '2', '0', '0', 'I', 'D', 'X'};
+static const char *const kSectionName[kIndexSections] = {"feature_names", "tok_end", "tok_comma", "device image"};
+constexpr uint64_t kIndexChunk = 64ull << 20;
+
+uint64_t index_checksum(const void *p, uint64_t bytes, uint64_t word0, int threads) {
+    const uint8_t *b = static_cast<const uint8_t *>(p);
+    const uint64_t nw = bytes / 8;
+    std::atomic<uint64_t> sum{0};
+    parallel_for(threads, (size_t)nw, [&](int, size_t a, size_t e) {
+        uint64_t s = 0;
+        for (size_t i = a; i < e; i++) {
+            uint64_t w;
+            memcpy(&w, b + 8 * i, 8);
+            s += image_word_sum(w, word0 + i);
+        }
+        sum += s;
+    });
+    uint64_t s = sum;
+    if (bytes % 8) {
+        uint64_t w = 0;
+        memcpy(&w, b + 8 * nw, bytes % 8);
+        s += image_word_sum(w, word0 + nw);
+    }
+    return s;
+}
+
+static uint64_t header_checksum(IndexHeader h) {
+    h.header_sum = 0;
+    return index_checksum(&h, sizeof h, 0);
+}
+
+bool is_index_file(const std::string &path) {
+    char m[8];
+    const int fd = open(path.c_str(), O_RDONLY);
+    if (fd < 0) return false;
+    const bool yes = pread(fd, m, 8, 0) == 8 && memcmp(m, kIndexMagic, 8) == 0;
+    close(fd);
+    return yes;
+}
+
+static uint64_t align256(uint64_t x) { return (x + 255) & ~(uint64_t)255; }
+
+void write_index_file(const HostLibrary &L, const std::string &json_path, const std::string &out_path, int threads) {
+    if (!L.has_index) throw std::runtime_error("library has no k-mer index");
+    IndexHeader h{};
+    memcpy(h.magic, kIndexMagic, 8);
+    h.version = kIndexVersion; h.header_bytes = sizeof(IndexHeader);
+    h.sizeof_entry = sizeof(Entry); h.sizeof_classrec = sizeof(ClassRec); h.sizeof_dualrec = sizeof(DualRec);
+    const nb200_config &c = L.cfg;
+    h.k = (uint32_t)c.k;
+    h.score_threshold = c.score_threshold; h.score_filter = c.score_filter; h.num_mismatches = c.num_mismatches;
+    h.discard_multiple_matches = c.discard_multiple_matches; h.intersect_level = c.intersect_level;
+    h.discard_multi_hits = c.discard_multi_hits; h.require_valid_pair = c.require_valid_pair;
+    h.max_hits_to_report = c.max_hits_to_report; h.score_percent = c.score_percent;
+    h.n_refs = L.n_refs; h.n_features = L.n_features; h.n_words = L.n_words; h.identity_features = L.identity_features ? 1 : 0;
+    h.n_kmers = L.n_kmers; h.n_classes = L.n_classes; h.n_buckets = L.n_buckets; h.n_spilled = L.n_spilled;
+    h.total_gbases = L.total_gbases;
+    {
+        std::ifstream jf(json_path, std::ios::binary);
+        if (!jf) throw std::runtime_error("cannot open library file " + json_path);
+        uint64_t fnv = 0xCBF29CE484222325ull, n = 0;
+        std::vector<char> buf(1 << 20);
+        while (jf) {
+            jf.read(buf.data(), (std::streamsize)buf.size());
+            const std::streamsize got = jf.gcount();
+            for (std::streamsize i = 0; i < got; i++) fnv = (fnv ^ (uint8_t)buf[(size_t)i]) * 0x100000001B3ull;
+            n += (uint64_t)got;
+        }
+        h.json_bytes = n; h.json_fnv1a = fnv;
+    }
+    snprintf(h.lib_version, sizeof h.lib_version, "%s", nb200_version());
+    const ImageLayout lay = image_layout(L);
+    for (int p = 0; p < kImageParts; p++) h.part_bytes[p] = lay.bytes[p];
+    std::string names;
+    for (const std::string &s : L.feature_names) { names += s; names.push_back('\0'); }
+    const void *host_src[kSecImage] = {names.data(), L.tok_end.data(), L.tok_comma.data()};
+    const uint64_t host_bytes[kSecImage] = {names.size(), L.tok_end.size() * 4ull, L.tok_comma.size() * 4ull};
+    uint64_t off = align256(sizeof(IndexHeader));
+    for (int s = 0; s < kSecImage; s++) {
+        h.sec[s] = IndexSection{off, host_bytes[s], index_checksum(host_src[s], host_bytes[s], 0)};
+        off = align256(off + host_bytes[s]);
+    }
+    h.sec[kSecImage] = IndexSection{off, lay.total, 0};
+    h.file_bytes = off + lay.total;
+
+    const std::string tmp = out_path + ".tmp";
+    FILE *f = fopen(tmp.c_str(), "wb");
+    if (!f) throw IoError("cannot write " + tmp);
+    try {
+        auto put_at = [&](uint64_t at, const void *p, uint64_t n) {
+            if (fseeko(f, (off_t)at, SEEK_SET) != 0 || (n && fwrite(p, 1, n, f) != n)) throw IoError("write failed: " + tmp);
+        };
+        for (int s = 0; s < kSecImage; s++) put_at(h.sec[s].off, host_src[s], host_bytes[s]);
+        std::vector<uint8_t> buf(std::min<uint64_t>(kIndexChunk, lay.total));
+        uint64_t sum = 0;
+        for (uint64_t a = 0; a < lay.total; a += buf.size()) {
+            const uint64_t n = std::min<uint64_t>(buf.size(), lay.total - a);
+            image_fill(L, lay, a, n, buf.data());
+            sum += index_checksum(buf.data(), n, a / 8, threads);
+            put_at(h.sec[kSecImage].off + a, buf.data(), n);
+        }
+        h.sec[kSecImage].sum = sum;
+        h.header_sum = header_checksum(h);
+        put_at(0, &h, sizeof h);
+        const int rc = fclose(f);
+        f = nullptr;
+        if (rc != 0) throw IoError("write failed: " + tmp);
+        if (rename(tmp.c_str(), out_path.c_str()) != 0) throw IoError("cannot rename " + tmp);
+    } catch (...) {
+        if (f) fclose(f);
+        remove(tmp.c_str());
+        throw;
+    }
+}
+
+IndexFile::~IndexFile() { if (fd >= 0) close(fd); }
+
+static void pread_all(int fd, uint64_t at, uint64_t len, uint8_t *dst, const std::string &path) {
+    while (len) {
+        const ssize_t got = pread(fd, dst, (size_t)std::min<uint64_t>(len, 1ull << 30), (off_t)at);
+        if (got < 0 && errno == EINTR) continue;
+        if (got <= 0) throw IoError("cannot read index file " + path);
+        dst += got; at += (uint64_t)got; len -= (uint64_t)got;
+    }
+}
+
+void IndexFile::read_image(uint64_t offset, uint64_t len, uint8_t *dst) const {
+    pread_all(fd, h.sec[kSecImage].off + offset, len, dst, path);
+}
+
+void open_index_file(const std::string &path, IndexFile &f, HostLibrary &meta) {
+    auto bad = [&](const std::string &why) { return std::runtime_error("index file " + path + " " + why); };
+    f.path = path;
+    f.fd = open(path.c_str(), O_RDONLY);
+    if (f.fd < 0) throw std::runtime_error("cannot open index file " + path);
+    struct stat st;
+    if (fstat(f.fd, &st) != 0) throw IoError("cannot stat index file " + path);
+    const uint64_t size = (uint64_t)st.st_size;
+    if (size < 8) throw bad("is truncated");
+    IndexHeader &h = f.h;
+    pread_all(f.fd, 0, std::min<uint64_t>(size, sizeof h), reinterpret_cast<uint8_t *>(&h), path);
+    if (memcmp(h.magic, kIndexMagic, 8) != 0) throw bad("is not an nb200 index (bad magic)");
+    if (size < sizeof h) throw bad("is truncated");
+    if (h.version != kIndexVersion)
+        throw bad("has format version " + std::to_string(h.version) + "; this build reads version " + std::to_string(kIndexVersion) +
+                  " (write it again with `python -m nimble_b200 index`)");
+    if (h.header_bytes != sizeof h || h.sizeof_entry != sizeof(Entry) || h.sizeof_classrec != sizeof(ClassRec) ||
+        h.sizeof_dualrec != sizeof(DualRec))
+        throw bad("was written with a different record layout");
+    if (header_checksum(h) != h.header_sum) throw bad("is damaged: the header fails its checksum");
+    if (size < h.file_bytes) throw bad("is truncated: " + std::to_string(size) + " of " + std::to_string(h.file_bytes) + " bytes");
+    if (size != h.file_bytes) throw bad("has " + std::to_string(size - h.file_bytes) + " bytes after its end");
+    const ImageLayout lay = image_layout(h.part_bytes);
+    const uint64_t ref_words = (h.total_gbases + 31) / 32 + 2;
+    bool ok = h.k >= 4 && h.k <= 32 && h.max_hits_to_report >= 1 && h.max_hits_to_report <= 64 && h.n_refs >= 1 &&
+              h.n_refs <= kMaxRefs && h.n_features >= 1 && h.n_features <= h.n_refs && h.n_words == (h.n_refs + 31) / 32 &&
+              h.n_buckets >= 1 && h.n_buckets < 0xFFFFFFFFull && h.part_bytes[kPartTable] == h.n_buckets * 2 * sizeof(Entry) &&
+              h.part_bytes[kPartClassRec] == h.n_classes * sizeof(ClassRec) && h.part_bytes[kPartRefGstart] == 4ull * h.n_refs &&
+              h.part_bytes[kPartRefFeature] == 4ull * h.n_refs && h.part_bytes[kPartRef2bit] == 8 * ref_words &&
+              h.part_bytes[kPartRefN] == 4 * ref_words && h.sec[kSecImage].bytes == lay.total &&
+              h.sec[kSecTokEnd].bytes == 4ull * h.n_features && h.sec[kSecTokComma].bytes == 4ull * h.n_features;
+    for (int s = 0; s < kIndexSections && ok; s++)
+        ok = h.sec[s].off % 8 == 0 && h.sec[s].off >= sizeof h && h.sec[s].bytes <= h.file_bytes && h.sec[s].off <= h.file_bytes - h.sec[s].bytes;
+    if (!ok) throw bad("is damaged: inconsistent header");
+    std::vector<uint8_t> sec[kSecImage];
+    for (int s = 0; s < kSecImage; s++) {
+        sec[s].resize(h.sec[s].bytes);
+        pread_all(f.fd, h.sec[s].off, h.sec[s].bytes, sec[s].data(), path);
+        if (index_checksum(sec[s].data(), sec[s].size(), 0) != h.sec[s].sum)
+            throw bad(std::string("is damaged: section ") + kSectionName[s] + " fails its checksum");
+    }
+    meta = HostLibrary{};
+    nb200_config &c = meta.cfg;
+    c.k = (int32_t)h.k;
+    c.score_threshold = h.score_threshold; c.score_filter = h.score_filter; c.num_mismatches = h.num_mismatches;
+    c.discard_multiple_matches = h.discard_multiple_matches; c.intersect_level = h.intersect_level;
+    c.discard_multi_hits = h.discard_multi_hits; c.require_valid_pair = h.require_valid_pair;
+    c.max_hits_to_report = h.max_hits_to_report; c.score_percent = h.score_percent;
+    meta.has_index = true;
+    const std::vector<uint8_t> &nm = sec[kSecFeatureNames];
+    for (size_t a = 0; a < nm.size();) {
+        const uint8_t *z = static_cast<const uint8_t *>(memchr(nm.data() + a, 0, nm.size() - a));
+        if (!z) throw bad("is damaged: unterminated feature name");
+        meta.feature_names.emplace_back(reinterpret_cast<const char *>(nm.data() + a), (size_t)(z - nm.data()) - a);
+        a = (size_t)(z - nm.data()) + 1;
+    }
+    if (meta.feature_names.size() != h.n_features) throw bad("is damaged: feature count differs from the header");
+    meta.tok_end.resize(h.n_features); meta.tok_comma.resize(h.n_features);
+    memcpy(meta.tok_end.data(), sec[kSecTokEnd].data(), 4ull * h.n_features);
+    memcpy(meta.tok_comma.data(), sec[kSecTokComma].data(), 4ull * h.n_features);
+    meta.identity_features = h.identity_features != 0;
+    meta.n_refs = h.n_refs; meta.n_features = h.n_features; meta.n_words = h.n_words;
+    meta.n_kmers = h.n_kmers; meta.n_classes = h.n_classes; meta.n_buckets = h.n_buckets; meta.n_spilled = h.n_spilled;
+    meta.total_gbases = h.total_gbases;
+}
+
+static bool class_has(const HostLibrary &L, uint32_t c, uint32_t r) {
+    if (c >= L.class_rec.size()) return false;
+    const ClassRec &rec = L.class_rec[c];
+    const uint32_t w = r >> 5, bit = 1u << (r & 31);
+    if (rec.meta & kRecOverflow) {
+        for (uint64_t j = rec.b[0]; j < (uint64_t)rec.b[0] + rec.b[1] && j < L.ov_w.size() && j < L.ov_b.size(); j++)
+            if (L.ov_w[j] == w) return (L.ov_b[j] & bit) != 0;
+        return false;
+    }
+    const uint32_t ws[kRecInline] = {rec.w01 & 0xFFFFu, rec.w01 >> 16, rec.w23 & 0xFFFFu, rec.w23 >> 16};
+    for (int i = 0; i < kRecInline; i++)
+        if (ws[i] == w) return (rec.b[i] & bit) != 0;
+    return false;
+}
+
+void verify_index_file(const IndexFile &f, const HostLibrary &meta, int threads) {
+    const IndexHeader &h = f.h;
+    const ImageLayout lay = image_layout(h.part_bytes);
+    uint64_t sum = 0;
+    {
+        std::vector<uint8_t> buf(std::min<uint64_t>(kIndexChunk, lay.total));
+        for (uint64_t a = 0; a < lay.total; a += buf.size()) {
+            const uint64_t n = std::min<uint64_t>(buf.size(), lay.total - a);
+            f.read_image(a, n, buf.data());
+            sum += index_checksum(buf.data(), n, a / 8, threads);
+        }
+    }
+    if (sum != h.sec[kSecImage].sum) throw std::runtime_error("index file " + f.path + " is damaged: the device image fails its checksum");
+    HostLibrary L = library_meta(meta);
+    auto part = [&](auto &vec, int p) {
+        vec.resize(lay.bytes[p] / sizeof(vec[0]));
+        f.read_image(lay.off[p], lay.bytes[p], reinterpret_cast<uint8_t *>(vec.data()));
+    };
+    part(L.table, kPartTable); part(L.class_rec, kPartClassRec); part(L.ov_w, kPartOvW); part(L.ov_b, kPartOvB);
+    part(L.ov_pre, kPartOvPre); part(L.positions, kPartPositions); part(L.ref_gstart, kPartRefGstart);
+    part(L.ref_feature, kPartRefFeature); part(L.ref2bit, kPartRef2bit); part(L.refN, kPartRefN); part(L.dual, kPartDual);
+    // lookup pass: every valid k-mer of every reference, read back from the image, finds a class holding that reference
+    const int k = L.cfg.k;
+    const uint64_t kmask = k == 32 ? ~0ull : ((1ull << (2 * k)) - 1);
+    const uint64_t gend = L.total_gbases >= 128 ? L.total_gbases - 128 : 0;
+    std::atomic<uint64_t> bad{0};
+    parallel_for(threads, L.n_refs, [&](int, size_t ra, size_t rb) {
+        uint64_t nbad = 0;
+        for (size_t r = ra; r < rb; r++) {
+            const uint64_t g0 = L.ref_gstart[r], g1 = (r + 1 < L.n_refs ? (uint64_t)L.ref_gstart[r + 1] : gend);
+            if (g1 < g0 + kRefPad || g1 > gend) { nbad++; continue; }
+            uint64_t x = 0;
+            int valid = 0;
+            for (uint64_t gp = g0; gp < g1 - kRefPad; gp++) {
+                if ((L.refN[gp >> 5] >> (gp & 31)) & 1u) { valid = 0; x = 0; continue; }
+                const uint64_t c = (L.ref2bit[gp >> 5] >> (2 * (gp & 31))) & 3u;
+                x = ((x >> 2) | (c << (2 * (k - 1)))) & kmask;
+                if (++valid < k) continue;
+                uint32_t cl[2], of[2];
+                host_lookup(L, x, cl, of);
+                if (cl[0] == kEmptyClass || !class_has(L, cl[0], (uint32_t)r)) nbad++;
+            }
+        }
+        bad += nbad;
+    });
+    if (bad)
+        throw std::runtime_error("index file " + f.path + " is damaged: " + std::to_string((uint64_t)bad) +
+                                 " reference k-mers do not find their reference through the table");
 }
 
 }  // namespace nb200

@@ -17,7 +17,7 @@ constexpr uint32_t kRefPad = 640;        // invalid bases before/after every ref
 constexpr uint32_t kMaxRefs = 65535u * 32u;        // class words are indexed with 16 bits, 0xFFFF = no word
 
 // k-mer table: bucketed cuckoo hashing keyed by the CANONICAL k-mer.  Entry = 16 B; bucket = 2 entries = 32 B =
-// one L2 sector.  A key lives in its first bucket b1 or in its second bucket b2 (two independent 32-bit halves of
+// one L2 sector (a change to Entry, DualRec or ClassRec must bump kIndexVersion).  A key lives in its first bucket b1 or in its second bucket b2 (two independent 32-bit halves of
 // hash_kmer, range-reduced by multiply-high); the SPILL bit of a bucket says "some key whose b1 is this bucket
 // lives in its b2", so a lookup is one sector load plus, for the few flagged buckets, a second one - straight-line,
 // no probe loop.  One entry answers both read orientations.
@@ -75,7 +75,67 @@ struct HostLibrary {
     uint64_t total_gbases = 0;
 };
 
-uint64_t hash_kmer(uint64_t x);
+// ---- device image: the index as one slab in HBM, and as the image section of an index file ----------------------
+// Parts at 256-byte aligned offsets, hottest first (the L2 persistence window may only cover a prefix).  Any change to
+// this layout, to Entry / ClassRec / DualRec or to hash_kmer / kmer_mix must bump kIndexVersion.
+enum ImagePart { kPartTable, kPartClassRec, kPartOvW, kPartOvB, kPartOvPre, kPartPositions, kPartRefGstart, kPartRefFeature,
+                 kPartRef2bit, kPartRefN, kPartDual, kImageParts };
+struct ImageLayout {
+    uint64_t bytes[kImageParts] = {};     // payload of each part
+    uint64_t off[kImageParts] = {};
+    uint64_t total = 0;                   // image size; a multiple of 256
+};
+ImageLayout image_layout(const uint64_t bytes[kImageParts]);
+ImageLayout image_layout(const HostLibrary &L);      // of L's host images
+// image bytes [offset, offset + len) of L's host images, padding as zeros
+void image_fill(const HostLibrary &L, const ImageLayout &lay, uint64_t offset, uint64_t len, uint8_t *dst);
+// L without its host images (what a device library keeps once its image is uploaded)
+HostLibrary library_meta(const HostLibrary &L);
+
+// ---- index file (.nb200idx, little-endian): header, host sections, the device image byte for byte --------------
+constexpr uint32_t kIndexVersion = 1;
+enum IndexSectionId { kSecFeatureNames, kSecTokEnd, kSecTokComma, kSecImage, kIndexSections };
+struct IndexSection { uint64_t off, bytes, sum; };    // sum: index_checksum over the section's words
+struct IndexHeader {
+    char magic[8];                        // "NB200IDX"
+    uint32_t version, header_bytes;
+    uint32_t sizeof_entry, sizeof_classrec, sizeof_dualrec, k;
+    int32_t score_threshold, score_filter, num_mismatches, discard_multiple_matches, intersect_level, discard_multi_hits,
+        require_valid_pair, max_hits_to_report;   // the library JSON's config (strand_filter is a call parameter)
+    double score_percent;
+    uint32_t n_refs, n_features, n_words, identity_features;
+    uint64_t n_kmers, n_classes, n_buckets, n_spilled, total_gbases;
+    uint64_t json_bytes, json_fnv1a;      // the source JSON (provenance only)
+    char lib_version[64];                 // nb200_version() of the writer
+    uint64_t part_bytes[kImageParts];
+    IndexSection sec[kIndexSections];
+    uint64_t file_bytes;
+    uint64_t header_sum;                  // index_checksum of the header with this field 0
+};
+static_assert(sizeof(IndexHeader) == 408, "index header has no padding");
+
+// sum over the 64-bit words of p[0, bytes) (a partial last word is zero-padded), word i counted as word0 + i
+uint64_t index_checksum(const void *p, uint64_t bytes, uint64_t word0, int threads = 1);
+bool is_index_file(const std::string &path);
+void write_index_file(const HostLibrary &L, const std::string &json_path, const std::string &out_path, int threads);
+// An opened index file: header and host sections read and checked (a damaged or foreign file throws); the image is
+// read on demand.
+struct IndexFile {
+    IndexHeader h{};
+    int fd = -1;
+    std::string path;
+    IndexFile() = default;
+    IndexFile(const IndexFile &) = delete;
+    IndexFile &operator=(const IndexFile &) = delete;
+    ~IndexFile();
+    void read_image(uint64_t offset, uint64_t len, uint8_t *dst) const;
+};
+void open_index_file(const std::string &path, IndexFile &f, HostLibrary &meta);
+// nb200_index_info with verify = 1: the image section's checksum, then every valid k-mer of every reference must look
+// up (host_lookup) to a class that holds that reference.  Throws on a mismatch.
+void verify_index_file(const IndexFile &f, const HostLibrary &meta, int threads);
+
+uint64_t hash_kmer(uint64_t x);        // a change here or in kmer_mix (kmer_hash.hpp) must bump kIndexVersion
 uint64_t revcomp_kmer(uint64_t x, int k);
 
 // throws std::runtime_error (EINVAL-class) / LimitError

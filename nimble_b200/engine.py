@@ -151,19 +151,21 @@ class Engine:
             raise NimbleB200Error(rc, (self.L.nb200_last_error(self.ctx) or b"").decode())
 
     # ---- library ---------------------------------------------------------------------------
-    def load_library(self, library, strand_filter="unstranded", k=20):
-        """library: path to a nimble library JSON, or the parsed [config, data] object."""
+    def load_library(self, library, strand_filter="unstranded", k=None):
+        """library: path to a nimble library JSON or to an index file written by `index` (told apart by its first bytes),
+        or the parsed [config, data] object.  k: None = the index file's own k, 20 for a JSON; a k that differs from an
+        index file's raises NimbleB200Error."""
         if strand_filter not in _lib.STRAND:
             raise NimbleB200Error(_lib.EINVAL, "unknown --strand_filter value: %r" % (strand_filter,))
         lid = ct.c_int32(-1)
         if isinstance(library, (str, os.PathLike)):
-            self._ck(self.L.nb200_load_library(self.ctx, os.fspath(library).encode(), strand_filter.encode(), int(k), ct.byref(lid)))
+            self._ck(self.L.nb200_load_library(self.ctx, os.fspath(library).encode(), strand_filter.encode(), int(k or 0), ct.byref(lid)))
         else:
             with tempfile.NamedTemporaryFile("w", suffix=".json", delete=False) as f:
                 json.dump(library, f)
                 path = f.name
             try:
-                self._ck(self.L.nb200_load_library(self.ctx, path.encode(), strand_filter.encode(), int(k), ct.byref(lid)))
+                self._ck(self.L.nb200_load_library(self.ctx, path.encode(), strand_filter.encode(), int(k or 0), ct.byref(lid)))
             finally:
                 os.unlink(path)
         return LibraryHandle(self, lid.value)

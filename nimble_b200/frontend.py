@@ -286,7 +286,7 @@ PER_READ_COLUMNS = ["nimble_features", "nimble_score", "r1_forward_score", "r1_r
 
 
 def align_10x(reference, output, r1_fastq, r2_fastq, cb_whitelist_file, num_cores=1, strand_filter="unstranded", cb_length=16,
-              umi_length=12, k=20, engine=None):
+              umi_length=12, k=None, engine=None):
     """`fastq-to-bam` + `align` in one pass over raw 10x FASTQs, without the BAM in between (an extension: the
     reference needs both commands).  Output = the per-read TSV(s) `align` would write for that BAM."""
     from .engine import Engine
@@ -369,13 +369,13 @@ def align_multi_gpu(reference, output, input, num_cores, strand_filter, k, gpus,
     err = ct.create_string_buffer(1024)
     st = (ct.c_double * 4)()
     if cnts is None:
-        rc = L.nb200_align_files_multi(d, len(devs), int(num_cores or 0), ins, len(input), libs, len(library_list), strand_filter.encode(), int(k),
+        rc = L.nb200_align_files_multi(d, len(devs), int(num_cores or 0), ins, len(input), libs, len(library_list), strand_filter.encode(), int(k or 0),
                                        out_c, (trim or "").encode(), err, len(err), st)
     else:
         cnt_c = (ct.c_char_p * len(cnts))(*[os.fspath(p).encode() for p in cnts])
         out3 = (ct.c_uint64 * (3 * len(cnts)))()
         rc = L.nb200_align_files_counts_multi(d, len(devs), int(num_cores or 0), ins, len(input), libs, len(library_list), strand_filter.encode(),
-                                              int(k), (trim or "").encode(), out_c, cnt_c, float(threshold), int(bool(disable_thresholding)),
+                                              int(k or 0), (trim or "").encode(), out_c, cnt_c, float(threshold), int(bool(disable_thresholding)),
                                               out3, err, len(err), st)
     if rc != 0:
         print("nimble_b200 aligner error: %s" % err.value.decode(errors="replace"), file=sys.stderr)
@@ -388,7 +388,39 @@ def align_multi_gpu(reference, output, input, num_cores, strand_filter, k, gpus,
     return 0
 
 
-def align(reference, output, input, num_cores, strand_filter, trim, tmpdir, k=20, engine=None, native=True, gpus=None, counts=None,
+def index(reference, output, k=None, num_cores=0):
+    """`index` (extension): build the k-mer index of ONE library JSON on the host (no GPU needed) and save it as an index
+    file.  `align`, `fastq-to-counts`, the `aligner` executable and Engine.load_library take that file wherever they take
+    the JSON and load it without building the index again.  k: None = 20; num_cores: host threads (0 = all cores).
+    Prints k, the reference, feature and k-mer counts and the file size; returns 0, or 1 on an error."""
+    from . import _lib
+    L = _lib.load()
+    rc = L.nb200_index_write(os.fspath(reference).encode(), int(k or 0), int(num_cores or 0), os.fspath(output).encode())
+    if rc != 0:
+        print("nimble_b200 index error: %s" % (L.nb200_last_error(None) or b"").decode(errors="replace"), file=sys.stderr)
+        return 1
+    info = index_info(output)
+    print("nimble_b200: wrote %s: k = %d, %d references, %d features, %d k-mers, %d bytes"
+          % (output, info["k"], info["n_refs"], info["n_features"], info["n_kmers"], os.path.getsize(output)))
+    return 0
+
+
+def index_info(path, verify=False):
+    """Header of an index file written by `index` (nb200_index_info) as a dict.  verify=True also checks the device image's
+    checksum and looks every k-mer of every reference up in the image read back.  A damaged or foreign file raises
+    NimbleB200Error."""
+    import ctypes as ct
+    from . import _lib
+    L = _lib.load()
+    out = (ct.c_int64 * 9)()
+    rc = L.nb200_index_info(os.fspath(path).encode(), int(bool(verify)), out)
+    if rc != 0:
+        raise _lib.NimbleB200Error(rc, (L.nb200_last_error(None) or b"").decode(errors="replace"))
+    keys = ("version", "k", "n_refs", "n_features", "n_kmers", "n_classes", "n_slots", "identity_features", "image_bytes")
+    return dict(zip(keys, (int(v) for v in out)))
+
+
+def align(reference, output, input, num_cores, strand_filter, trim, tmpdir, k=None, engine=None, native=True, gpus=None, counts=None,
           threshold=0.05, disable_thresholding=False):
     """Drop-in for nimble/__main__.py:153-211.  Returns the aligner's return code (0 = success).
     gpus (extension; also $NB200_GPUS): a count or list of devices -> the streaming pipeline over all of them.
@@ -687,7 +719,7 @@ def _print_pair_stats(st):
 
 
 def fastq_to_counts(reference, r1_fastq, r2_fastq, cb_whitelist_file, counts, num_cores=1, strand_filter="unstranded", trim="",
-                    k=20, gpus=None, cb_length=16, umi_length=12, threshold=0.05, disable_thresholding=False, engine=None):
+                    k=None, gpus=None, cb_length=16, umi_length=12, threshold=0.05, disable_thresholding=False, engine=None):
     """`fastq-to-bam`, then `align --counts` on its BAM, in one streaming pass without the BAM (an extension: the reference
     needs fastq-to-bam, align and report).  Raw 10x R1 / R2 FASTQ(.gz) + whitelist in, the counts TSV `report` would
     write out, one per library (named like align's outputs).  gpus (also $NB200_GPUS): a count or a list of devices.
@@ -715,7 +747,7 @@ def fastq_to_counts(reference, r1_fastq, r2_fastq, cb_whitelist_file, counts, nu
             st4 = (ct.c_double * 4)()
             rc = L.nb200_fastq_to_counts_multi(d, len(devs), int(num_cores or 0), os.fspath(r1_fastq).encode(), os.fspath(r2_fastq).encode(),
                                                os.fspath(cb_whitelist_file).encode(), int(cb_length), int(umi_length), libs, len(library_list),
-                                               strand_filter.encode(), int(k), (trim or "").encode(), cnt_c, float(threshold),
+                                               strand_filter.encode(), int(k or 0), (trim or "").encode(), cnt_c, float(threshold),
                                                int(bool(disable_thresholding)), out3, ct.byref(cst), err, len(err), st4)
             if rc != 0:
                 print("nimble_b200 aligner error: %s" % err.value.decode(errors="replace"), file=sys.stderr)
