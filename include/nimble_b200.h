@@ -32,6 +32,15 @@ extern "C" {
 #define NB200_MAX_READ_LEN 500
 #define NB200_NO_BARCODE UINT64_MAX
 
+/* Flags word of the counting entries (the `int32_t disable_thresholding` parameter of nb200_umi_counts,
+ * nb200_report_file, nb200_align_files_counts(_multi), nb200_fastq_to_counts(_multi); 0 and 1 keep their meaning):
+ * NB200_UMI_NO_THRESHOLD skips the per-UMI proportional thresholding; NB200_UMI_CORRECT merges, per cell, each UMI into
+ * its best-supported one-substitution neighbour before the UMI stage (DESIGN.md §2.12).  With NB200_UMI_CORRECT, out3
+ * holds 4 values per library: the 3 documented at each entry, then the number of (cell, UMI) keys corrected.  Other bits:
+ * NB200_EINVAL.  nb200_align and nb200_align_resident refuse NB200_UMI_CORRECT (their keys are caller-assigned ids). */
+#define NB200_UMI_NO_THRESHOLD 1
+#define NB200_UMI_CORRECT 2
+
 /* strand filter: the reference forwards `--strand_filter` verbatim (nimble/__main__.py:180,399) */
 enum { NB200_UNSTRANDED = 0, NB200_FIVEPRIME = 1, NB200_THREEPRIME = 2, NB200_STRAND_NONE = 3 };
 
@@ -169,6 +178,11 @@ int32_t nb200_index_write(const char *json_path, int32_t k, int32_t host_threads
  * (it must find a class that holds that reference).  A damaged or foreign file: NB200_EINVAL with the reason. */
 int32_t nb200_index_info(const char *path, int32_t verify, int64_t *out9);
 
+/* test hook (host only): the one-substitution neighbours of UMI code `code` as the correction kernel visits them
+ * (codes and byte-order values, see nb200_umis_corrected); returns their number (<= 52), -1 for a value that is not a
+ * code.  out_code / out_value hold 52 entries. */
+int32_t nb200_umi_neighbours(uint32_t code, uint32_t *out_code, uint32_t *out_value);
+
 /* test hook (host only): the raw-DEFLATE decoder the BGZF reader tries before zlib (csrc/fast_inflate.hpp).
  * 1 = the stream decoded into exactly out_len bytes, 0 = declined (the reader then uses zlib). */
 int32_t nb200_fast_inflate(const uint8_t *in, uint64_t in_len, uint8_t *out, uint64_t out_len);
@@ -270,6 +284,11 @@ int32_t nb200_counts_device(const nb200_ctx *ctx, uint64_t *n_rows, uint64_t *n_
 int32_t nb200_umi_counts(nb200_ctx *ctx, int32_t lib_id, uint64_t n_rows, const uint64_t *key,
                          const uint32_t *off, const uint32_t *feat_ids, const double *score,
                          double umi_threshold, int32_t disable_thresholding, nb200_counts *counts);
+/* (cell, UMI) keys corrected by the last UMI stage run on the context (0 without NB200_UMI_CORRECT).  With
+ * NB200_UMI_CORRECT, nb200_umi_counts reads the UMI as the low half of the key: 1 ..= 1525878905 is the bijective base-5
+ * code of an ACGTN string of 1..13 bases (A C G T N = digits 1..5, last base least significant); any other value is an
+ * id that is never corrected. */
+int32_t nb200_umis_corrected(const nb200_ctx *ctx, uint64_t *out);
 /* report() file to file (nimble/__main__.py:254-293): per-read TSV (.gz or plain; columns nimble_features,
  * nimble_score, r1_CB, r1_UB) -> `feature<TAB>count<TAB>cell_barcode` without header, rows in the
  * reference's order.  Rows with a missing cell (pandas' NaN markers) are dropped (:244-245); an input

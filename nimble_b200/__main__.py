@@ -44,6 +44,8 @@ def main(argv=None):
                    type=float, default=0.05)
     a.add_argument("--disable_thresholding", help="with --counts: disable the per-UMI proportional count thresholding algorithm",
                    action="store_true", default=False)
+    a.add_argument("--correct-umis", help="(extension) with --counts: merge each UMI into a better-supported UMI of the same cell one "
+                                          "substitution away before counting (DESIGN.md §2.12)", action="store_true", default=False)
 
     r = sub.add_parser("report")
     r.add_argument("-i", "--input", help="The input file.", type=str, required=True)
@@ -53,6 +55,8 @@ def main(argv=None):
                    type=float, default=0.05)
     r.add_argument("--disable_thresholding", help="Disable the per-UMI proportional count thresholding algorithm.",
                    action="store_true", default=False)
+    r.add_argument("--correct-umis", help="(extension) merge each UMI into a better-supported UMI of the same cell one substitution "
+                                          "away before counting (DESIGN.md §2.12)", action="store_true", default=False)
 
     f = sub.add_parser("fastq-to-bam")
     f.add_argument("--r1-fastq", help="Path to R1 FASTQ file.", type=str, required=True)
@@ -80,6 +84,8 @@ def main(argv=None):
                     type=float, default=0.05)
     fc.add_argument("--disable_thresholding", help="Disable the per-UMI proportional count thresholding algorithm.",
                     action="store_true", default=False)
+    fc.add_argument("--correct-umis", help="(extension) merge each UMI into a better-supported UMI of the same cell one substitution "
+                                           "away before counting (DESIGN.md §2.12)", action="store_true", default=False)
 
     ix = sub.add_parser("index", help="(extension) build one library's k-mer index on the host and save it; --reference LIB.nb200idx "
                                       "then loads it without a build")
@@ -99,6 +105,8 @@ def main(argv=None):
         generate(args.file, args.opt_file, args.output_path)
     elif args.subcommand == "align" and args.output is None and args.counts is None:
         parser.error("align needs --output, --counts or both")
+    elif args.subcommand == "align" and args.correct_umis and args.counts is None:
+        parser.error("--correct-umis needs --counts")
     elif args.subcommand == "align" and args.map:
         if args.counts is not None:
             parser.error("--counts does not combine with --map: run align --map, then report on its per-read TSV")
@@ -112,10 +120,10 @@ def main(argv=None):
     elif args.subcommand == "align":
         sys.exit(align(args.reference, args.output, args.input, args.num_cores, args.strand_filter, args.trim,
                        args.tmpdir, k=args.kmer, gpus=args.gpus, counts=args.counts, threshold=args.threshold,
-                       disable_thresholding=args.disable_thresholding))
+                       disable_thresholding=args.disable_thresholding, correct_umis=args.correct_umis))
     elif args.subcommand == "report":
         cols = args.summarize.split(",") if args.summarize else None
-        report(args.input, args.output, cols, args.threshold, args.disable_thresholding)
+        report(args.input, args.output, cols, args.threshold, args.disable_thresholding, correct_umis=args.correct_umis)
     elif args.subcommand == "plot":
         print("nimble_b200: `plot` (HTML report, nimble/report_generation.py) is not part of the B200 backend; the per-read TSV "
               "written by `align` carries every column it reads, so `python -m nimble plot` works on it unchanged.", file=sys.stderr)
@@ -126,7 +134,8 @@ def main(argv=None):
     elif args.subcommand == "fastq-to-counts":
         sys.exit(fastq_to_counts(args.reference, args.r1_fastq, args.r2_fastq, args.map, args.counts, args.num_cores, args.strand_filter,
                                  args.trim, k=args.kmer, gpus=args.gpus, cb_length=args.cb_length, umi_length=args.umi_length,
-                                 threshold=args.threshold, disable_thresholding=args.disable_thresholding))
+                                 threshold=args.threshold, disable_thresholding=args.disable_thresholding,
+                                 correct_umis=args.correct_umis))
     elif args.subcommand == "index":
         if "," in args.reference:
             parser.error("index takes one library per call")

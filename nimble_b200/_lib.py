@@ -28,8 +28,15 @@ EXPORTS = [
     "nb200_align_10x_fastq", "nb200_set_overlap", "nb200_bench_dpx_peak", "nb200_set_stats", "nb200_align_files_multi",
     "nb200_library_set_trim", "nb200_trim_maxinfo", "nb200_set_defer_fetch", "nb200_fetch_counts", "nb200_fetch_counts_start", "nb200_fast_inflate",
     "nb200_align_files_counts", "nb200_align_files_counts_multi", "nb200_fastq_to_counts", "nb200_fastq_to_counts_multi",
-    "nb200_index_write", "nb200_index_info",
+    "nb200_index_write", "nb200_index_info", "nb200_umis_corrected", "nb200_umi_neighbours",
 ]
+
+# flags word of the counting entries (the disable_thresholding parameter)
+UMI_NO_THRESHOLD, UMI_CORRECT = 1, 2
+
+
+def umi_flags(disable_thresholding, correct_umis):
+    return (UMI_NO_THRESHOLD if disable_thresholding else 0) | (UMI_CORRECT if correct_umis else 0)
 
 CB_SKIPPED, CB_PERFECT, CB_CORRECTED, CB_NONE = 0, 1, 2, 3
 
@@ -155,6 +162,8 @@ def load():
     L.nb200_trim_maxinfo.argtypes = [vp, u32, i32, i32, dbl]
     L.nb200_trim_maxinfo.restype = u32
     L.nb200_report_file.argtypes = [vp, ct.c_char_p, ct.c_char_p, dbl, i32, ct.POINTER(u64)]
+    L.nb200_umis_corrected.argtypes = [vp, ct.POINTER(u64)]
+    L.nb200_umi_neighbours.argtypes = [u32, ct.POINTER(u32), ct.POINTER(u32)]
     L.nb200_host_ingest_stats.argtypes = [ct.POINTER(ct.c_char_p), i32, i32, ct.POINTER(u64)]
     L.nb200_counts_device.argtypes = [vp, ct.POINTER(u64), ct.POINTER(u64)] + [ct.POINTER(vp)] * 4
     L.nb200_load_whitelist.argtypes = [vp, ct.c_char_p, i32, ct.POINTER(i32)]

@@ -16,6 +16,7 @@
 #include <cuda_runtime.h>
 
 #include "kernels.cuh"
+#include "umi_code.hpp"
 
 namespace nb200 {
 
@@ -98,6 +99,121 @@ __global__ void gather_tok_kernel(uint32_t m, const uint32_t *__restrict__ perm,
         key = (key << bits) | v;
     }
     out[i] = key;
+}
+
+// ---- UMI correction (DESIGN.md §2.12): a key-rewrite pre-pass over the selected rows, before the key sort -----------
+// Open addressing over 16 B slots, linear probing, load factor <= 0.5.  A slot stores ~key, so that the zeroed table is
+// empty: the one key that maps to 0 is NB200_NO_BARCODE, and mark_rows_kernel never selects it.
+struct UmiSlot {
+    unsigned long long nkey;   // ~key; 0 = empty
+    uint32_t count;            // rows with this key
+    uint32_t target;           // slot of the key this one is rewritten to (umi_correct_kernel)
+};
+static_assert(sizeof(UmiSlot) == 16, "one UMI slot is 16 B");
+
+__host__ __device__ __forceinline__ uint32_t umi_slot_hash(uint64_t k) {
+    k ^= k >> 33; k *= 0xFF51AFD7ED558CCDull; k ^= k >> 33; k *= 0xC4CEB9FE1A85EC53ull; k ^= k >> 33;
+    return (uint32_t)k;
+}
+
+// slot of a key present in the table, or 0xFFFFFFFF
+__device__ __forceinline__ uint32_t umi_find(const UmiSlot *__restrict__ t, uint32_t mask, uint64_t key) {
+    const unsigned long long nk = ~key;
+    for (uint32_t s = umi_slot_hash(key) & mask;; s = (s + 1) & mask) {
+        const unsigned long long v = t[s].nkey;
+        if (v == nk) return s;
+        if (v == 0) return 0xFFFFFFFFu;
+    }
+}
+
+// byte rank of a code digit (A1 C2 G3 T4 N5): the byte order A < C < G < N < T
+__host__ __device__ __forceinline__ int umi_digit_rank(uint32_t d) { return d <= 3 ? (int)d - 1 : (d == 4 ? 4 : 3); }
+
+// The UMI's bytes as a fixed-length base-5 number over the byte ranks: for UMIs of one length, numeric order is byte order.
+__host__ __device__ __forceinline__ uint32_t umi_byte_value(uint32_t u) {
+    uint32_t v = 0, p5 = 1;
+    for (uint32_t x = u; x; p5 *= 5) {
+        const uint32_t q = (x - 1) / 5;
+        v += (uint32_t)umi_digit_rank(x - 5 * q) * p5;
+        x = q;
+    }
+    return v;
+}
+
+// Every one-substitution neighbour of code u (1 <= u <= kUmiCodeMax): each position, each of A C G T other than the base
+// there (N positions included), never N.  f(code, byte value) with byte value as umi_byte_value would give it.  A neighbour
+// is one add to the code, (d' - d) * 5^p, and one to the byte value.  (Host callers pass host lambdas: nb200_umi_neighbours.)
+#pragma nv_exec_check_disable
+template <class F>
+__host__ __device__ __forceinline__ void umi_for_each_neighbour(uint32_t u, uint32_t bv, F &&f) {
+    uint32_t p5 = 1;
+    for (uint32_t x = u; x; p5 *= 5) {
+        const uint32_t q = (x - 1) / 5, d = x - 5 * q;
+        const int rd = umi_digit_rank(d);
+        for (uint32_t e = 1; e <= 4; e++) {
+            if (e == d) continue;
+            f((uint32_t)((int64_t)u + ((int64_t)e - (int64_t)d) * p5), (uint32_t)((int64_t)bv + (int64_t)(umi_digit_rank(e) - rd) * p5));
+        }
+        x = q;
+    }
+}
+
+// one thread per selected row: its key into the table, one more row for it
+__global__ void __launch_bounds__(256)
+umi_count_kernel(uint32_t m, const uint64_t *__restrict__ key, UmiSlot *__restrict__ t, uint32_t mask) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= m) return;
+    const uint64_t k = key[i];
+    const unsigned long long nk = ~k;
+    for (uint32_t s = umi_slot_hash(k) & mask;; s = (s + 1) & mask) {
+        unsigned long long v = *(volatile unsigned long long *)&t[s].nkey;
+        if (v == 0) v = atomicCAS(&t[s].nkey, 0ull, nk);
+        if (v == 0 || v == nk) { atomicAdd(&t[s].count, 1u); return; }
+    }
+}
+
+// one thread per slot: target = the maximum of (rows, bytes) over the key itself and its present one-substitution
+// neighbours in the same cell, from the counts as umi_count_kernel left them (no slot's count changes here, so targets do
+// not depend on thread order).  Keys whose UMI is not a code (interned) keep themselves.  *corrected += keys whose target
+// is another key (one atomic per block).
+__global__ void __launch_bounds__(256)
+umi_correct_kernel(uint32_t tsize, UmiSlot *__restrict__ t, uint32_t mask, uint32_t *__restrict__ corrected) {
+    const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
+    int moved = 0;
+    if (s < tsize) {
+        const unsigned long long nk = t[s].nkey;
+        uint32_t best = s;
+        if (nk) {
+            const uint64_t k = ~nk;
+            const uint32_t u = (uint32_t)k;
+            if (u >= 1 && u <= kUmiCodeMax) {
+                const uint64_t cell = k & 0xFFFFFFFF00000000ull;
+                uint32_t best_n = t[s].count, best_bv = umi_byte_value(u);
+                umi_for_each_neighbour(u, best_bv, [&](uint32_t v, uint32_t bv) {
+                    const uint32_t o = umi_find(t, mask, cell | v);
+                    if (o == 0xFFFFFFFFu) return;
+                    const uint32_t n = t[o].count;
+                    if (n > best_n || (n == best_n && bv > best_bv)) { best = o; best_n = n; best_bv = bv; }
+                });
+            }
+            t[s].target = best;
+            moved = best != s;
+        }
+    }
+    moved = __syncthreads_count(moved);
+    if (threadIdx.x == 0 && moved) atomicAdd(corrected, (uint32_t)moved);
+}
+
+// one thread per selected row (key[i] is row perm[i]'s key): out[perm[i]] = the key of its slot's target.  out is
+// indexed like the caller's key array, so every later reader of a row's key (gather_key64_kernel, also on the second key
+// sort of the large-group path) sees the rewritten key.
+__global__ void __launch_bounds__(256)
+umi_rewrite_kernel(uint32_t m, const uint32_t *__restrict__ perm, const uint64_t *__restrict__ key, const UmiSlot *__restrict__ t,
+                   uint32_t mask, uint64_t *__restrict__ out) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= m) return;
+    const uint32_t s = umi_find(t, mask, key[i]);
+    out[perm[i]] = ~t[t[s].target].nkey;
 }
 
 __global__ void gather_key64_kernel(uint32_t m, const uint32_t *__restrict__ perm, const uint64_t *__restrict__ key,

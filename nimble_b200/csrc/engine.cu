@@ -207,6 +207,8 @@ struct nb200_ctx {
     DevBuf flag, permA, permB, k32A, k32B, k64A, k64B, num, cub_tmp, gstart, head;
     DevBuf u_cell, u_n, u_list, s_rep, s_S, s_U, s_fs, s_fc, s_flags;
     DevBuf row_n, row_off, slow, htable, rep_of, is_rep, cell_ord, rank_of, gstart2;
+    DevBuf umi_table, umi_key;                    // UMI correction (NB200_UMI_CORRECT): the slot table, the rewritten keys
+    uint64_t umis_corrected = 0;                  // of the last UMI stage (nb200_umis_corrected)
     DevBuf o_cell_d, o_count_d, o_n_d, o_list_d, gen_feats, gen_nf, gen_off, gen_score, gen_key;
     // count table lives in pinned host memory owned by the context
     PinnedBuf<uint32_t> h_cell, h_count, h_off, h_ids;
@@ -694,8 +696,8 @@ static void cub_select_async(nb200_ctx *c, const uint8_t *flag, uint32_t *out, u
     CK(cub::DeviceSelect::Flagged(c->cub_tmp.p, bytes, it, flag, out, d_count, (int)n, c->s_compute));
 }
 // the aggregation's device scalars (c->num): 0 groups, 1 largest group, 2 UMIs for the general kernel, 3 distinct lists,
-// 4 ids of the table, 5 UMIs with a result, 6 table rows, 7 selected rows, 8 longest selected row
-enum { DV_GROUPS = 0, DV_MAXGROUP, DV_GENERAL, DV_LISTS, DV_IDS, DV_LIVE, DV_ROWS, DV_SELECTED, DV_MAXLEN, DV_COUNT };
+// 4 ids of the table, 5 UMIs with a result, 6 table rows, 7 selected rows, 8 longest selected row, 9 UMIs corrected
+enum { DV_GROUPS = 0, DV_MAXGROUP, DV_GENERAL, DV_LISTS, DV_IDS, DV_LIVE, DV_ROWS, DV_SELECTED, DV_MAXLEN, DV_CORRECTED, DV_COUNT };
 static void fetch_scalars(nb200_ctx *c, uint32_t *h) {           // ONE host sync for all of them
     CK(cudaMemcpyAsync(h, c->num.p, DV_COUNT * 4, cudaMemcpyDeviceToHost, c->s_compute));
     CK(cudaStreamSynchronize(c->s_compute));
@@ -741,13 +743,35 @@ static void ensure_host_table(nb200_ctx *c, size_t nrows, size_t ids) {
 
 static int bits_for(uint64_t n) { int b = 1; while ((1ull << b) < n) b++; return b; }
 
+// UMI correction (DESIGN.md §2.12) over the m selected rows (permA, input order): rows counted per key in a table sized
+// from m, every key's target found from those counts, each row's key rewritten to its target's.  Returns the rewritten
+// keys, indexed like d_key (only the selected rows' entries are written); the number of keys corrected goes to
+// dv[DV_CORRECTED].
+static const uint64_t *correct_umis(nb200_ctx *c, uint64_t n, const uint64_t *d_key, uint32_t m, uint32_t *dv) {
+    uint32_t tsize = 1024;
+    while (tsize < 2ull * m && tsize < (1u << 31)) tsize <<= 1;      // load factor <= 0.5 (m < 2^31 keeps a slot free)
+    c->k64A.ensure((size_t)m * 8); c->umi_table.ensure((size_t)tsize * sizeof(UmiSlot)); c->umi_key.ensure(n * 8);
+    UmiSlot *t = c->umi_table.as<UmiSlot>();
+    CK(cudaMemsetAsync(t, 0, (size_t)tsize * sizeof(UmiSlot), c->s_compute));
+    gather_key64_kernel<<<nblk(m, 256), 256, 0, c->s_compute>>>(m, c->permA.as<uint32_t>(), d_key, c->k64A.as<uint64_t>());
+    umi_count_kernel<<<nblk(m, 256), 256, 0, c->s_compute>>>(m, c->k64A.as<uint64_t>(), t, tsize - 1);
+    umi_correct_kernel<<<nblk(tsize, 256), 256, 0, c->s_compute>>>(tsize, t, tsize - 1, dv + DV_CORRECTED);
+    umi_rewrite_kernel<<<nblk(m, 256), 256, 0, c->s_compute>>>(m, c->permA.as<uint32_t>(), c->k64A.as<uint64_t>(), t, tsize - 1,
+                                                                c->umi_key.as<uint64_t>());
+    c->launches += 4;
+    return c->umi_key.as<uint64_t>();
+}
+
 // A6 (nimble/__main__.py:234-293).  Inputs resident on device; fills ctx->o_* host vectors.
 // rows: padded or CSR (agg.cuh); max_nf_hint: longest row if known (0: stride); ids_bound: upper bound of the names of
 // all rows together (sizes nothing but a sanity check; the pools are sized from the device-side total).
+// umi_flags: NB200_UMI_NO_THRESHOLD, NB200_UMI_CORRECT (keyed rows only; bulk data has no UMIs).
 static void aggregate(nb200_ctx *c, const DevLibrary &L, uint64_t n, const uint64_t *d_key, const Rows &rows,
-                      const double *d_score, uint32_t max_nf_hint, double threshold, int disable, nb200_counts *counts) {
+                      const double *d_score, uint32_t max_nf_hint, double threshold, int umi_flags, nb200_counts *counts) {
+    const int disable = umi_flags & NB200_UMI_NO_THRESHOLD;
     counts->n_rows = 0; counts->dropped_empty = 0; counts->n_called = 0; counts->n_umis = 0;
     c->dev_rows = 0; c->dev_ids = 0;
+    c->umis_corrected = 0;
     auto host_rows = [&](size_t nrows, size_t ids) { ensure_host_table(c, nrows, ids); };
     if (c->fetch_started) { CK(cudaStreamSynchronize(c->s_copy[1])); c->fetch_started = false; }      // (a fetch nobody waited for)
     c->fetch_pending = false;
@@ -783,6 +807,7 @@ static void aggregate(nb200_ctx *c, const DevLibrary &L, uint64_t n, const uint6
         // insertion sort replaces a global LSD sort over every token column of every row.
         c->k64A.ensure((size_t)m * 8); c->k64B.ensure((size_t)m * 8); c->permB.ensure((size_t)m * 4);
         c->head.ensure(m); c->gstart.ensure((size_t)m * 4);
+        if (umi_flags & NB200_UMI_CORRECT) d_key = correct_umis(c, n, d_key, m, dv);
         auto sort_by_key = [&]() {
             gather_key64_kernel<<<nblk(m, 256), 256, 0, c->s_compute>>>(m, c->permA.as<uint32_t>(), d_key, c->k64A.as<uint64_t>());
             c->launches++;
@@ -802,6 +827,7 @@ static void aggregate(nb200_ctx *c, const DevLibrary &L, uint64_t n, const uint6
         G = hv[DV_GROUPS];
         const uint32_t T = hv[DV_IDS];
         counts->n_umis = G;
+        c->umis_corrected = hv[DV_CORRECTED];
         if (hv[DV_MAXGROUP] <= kLocalSortMax) {
             group_sort_kernel<<<nblk(G, 128), 128, 0, c->s_compute>>>(G, c->gstart.as<uint32_t>(), m, c->permA.as<uint32_t>(), rows,
                                                                        L.tok_end.as<uint32_t>(), L.tok_comma.as<uint32_t>());
@@ -1433,7 +1459,7 @@ static void enable_peers(const std::vector<nb200_ctx *> &ctxs) {
 }
 
 void lane_rows_count(const std::vector<nb200_ctx *> &ctxs, int li, int32_t lib_id, const std::vector<RowSeg> &segs,
-                     const std::vector<uint32_t> &cell_rank, double threshold, int disable, nb200_counts *counts, uint64_t *rows,
+                     const std::vector<uint32_t> &cell_rank, double threshold, int umi_flags, nb200_counts *counts, uint64_t *rows,
                      bool tenx) {
     nb200_ctx *c = ctxs[0];
     for (nb200_ctx *x : ctxs) { CK(cudaSetDevice(x->device)); CK(cudaStreamSynchronize(x->s_copy[1])); }
@@ -1497,7 +1523,7 @@ void lane_rows_count(const std::vector<nb200_ctx *> &ctxs, int li, int32_t lib_i
     CK(cudaMemsetAsync(c->d_ctr.p, 0, sizeof(Counters), s));
     // the aligner writes nimble_score = 1 for every row: score NULL
     aggregate(c, L, R, c->gen_key.as<uint64_t>(), Rows{c->gen_feats.as<int32_t>(), c->gen_off.as<uint32_t>(), nullptr, nullptr, 0}, nullptr,
-              0, threshold, disable, counts);
+              0, threshold, umi_flags, counts);
     CK(cudaStreamSynchronize(s));
     Counters h2;
     CK(cudaMemcpy(&h2, c->d_ctr.p, sizeof(h2), cudaMemcpyDeviceToHost));
@@ -2200,13 +2226,37 @@ int32_t nb200_upload(nb200_ctx *c, const nb200_reads *r1, const nb200_reads *r2,
     API_END(c)
 }
 
+// The flags word of the counting entries (NB200_UMI_*).  may_correct = false where keys are caller-assigned ids rather
+// than UMI codes (nb200_align, nb200_align_resident).
+static int32_t check_umi_flags(int32_t flags, bool may_correct) {
+    if (flags & ~(NB200_UMI_NO_THRESHOLD | NB200_UMI_CORRECT)) throw std::runtime_error("unknown bits in the UMI flags word");
+    if (!may_correct && (flags & NB200_UMI_CORRECT))
+        throw std::runtime_error("NB200_UMI_CORRECT needs UMIs as sequence codes: use the file or report entries");
+    return flags;
+}
+
 int32_t nb200_align_resident(nb200_ctx *c, int32_t lib_id, double umi_threshold, int32_t disable_thresholding,
                              nb200_counts *counts) {
     API_BEGIN(c)
     if (!counts) throw std::runtime_error("counts is null");
+    check_umi_flags(disable_thresholding, false);
     if (!c->resident) throw std::runtime_error("no resident reads: call nb200_upload first");
     run_align(c, get_lib(c, lib_id), nullptr, umi_threshold, disable_thresholding, counts);
     API_END(c)
+}
+
+int32_t nb200_umi_neighbours(uint32_t code, uint32_t *out_code, uint32_t *out_value) {
+    if (!out_code || !out_value) return NB200_EINVAL;
+    if (code < 1 || code > kUmiCodeMax) return -1;
+    int n = 0;
+    umi_for_each_neighbour(code, umi_byte_value(code), [&](uint32_t v, uint32_t bv) { out_code[n] = v; out_value[n] = bv; n++; });
+    return n;
+}
+
+int32_t nb200_umis_corrected(const nb200_ctx *c, uint64_t *out) {
+    if (!c || !out) return NB200_EINVAL;
+    *out = c->umis_corrected;
+    return NB200_OK;
 }
 
 int32_t nb200_counts_device(const nb200_ctx *c, uint64_t *n_rows, uint64_t *n_ids, const uint32_t **cell, const uint32_t **count,
@@ -2230,6 +2280,7 @@ int32_t nb200_align(nb200_ctx *c, int32_t lib_id, const nb200_reads *r1, const n
                     nb200_counts *counts) {
     API_BEGIN(c)
     if (!r1 || !counts) throw std::runtime_error("r1 / counts is null");
+    check_umi_flags(disable_thresholding, false);
     validate_reads(r1, "r1");
     if (r2) { validate_reads(r2, "r2"); if (r2->n != r1->n) throw std::runtime_error("r1 and r2 differ in read count"); }
     ensure_read_buffers(c, r1, r2, key != nullptr);
@@ -2289,6 +2340,9 @@ static void align_readset(nb200_ctx *c, const ReadSet &R, const int32_t *lib_ids
     }
 }
 
+// values per library in the out3 of the counting entries: rows used, count rows written, UMIs dropped (+ UMIs corrected)
+static int out3_per_lib(int32_t umi_flags) { return (umi_flags & NB200_UMI_CORRECT) ? 4 : 3; }
+
 // File-level entries: what the aligner process does between its argv and its exit code (nimble/__main__.py:177-196),
 // streaming (stream.cpp).  One pass over `inputs` on the contexts `ctxs`, whose libraries carry the same ids in the same
 // order; per library a per-read TSV (outputs) and/or a counts TSV (counts_outputs).  whitelist: the 10x mode of
@@ -2309,7 +2363,7 @@ static FileStats run_job(const std::vector<nb200_ctx *> &ctxs, const int32_t *li
     }
     job.host_threads = ctxs[0]->host_threads;
     job.umi_threshold = umi_threshold;
-    job.disable_thresholding = disable_thresholding;
+    job.umi_flags = disable_thresholding;
     FileStats st;
     run_file_pipeline(job, &st);
     if (getenv("NB200_TRACE"))
@@ -2361,7 +2415,8 @@ int32_t nb200_align_files_counts(nb200_ctx *c, const char *const *inputs, int32_
                                  double umi_threshold, int32_t disable_thresholding, uint64_t *out3) {
     API_BEGIN(c)
     if (!inputs || n_inputs < 1 || n_inputs > 2 || !lib_ids || !counts_outputs || n_libs < 1) throw std::runtime_error("bad arguments");
-    if (out3) for (int i = 0; i < 3 * n_libs; i++) out3[i] = 0;
+    check_umi_flags(disable_thresholding, true);
+    if (out3) for (int i = 0; i < out3_per_lib(disable_thresholding) * n_libs; i++) out3[i] = 0;
     const FileStats st = run_job({c}, lib_ids, n_libs, inputs, n_inputs, per_read_outputs, counts_outputs, umi_threshold,
                                  disable_thresholding, nullptr, 0, 0);
     if (out3) for (size_t i = 0; i < st.counts3.size(); i++) out3[i] = st.counts3[i];
@@ -2376,7 +2431,8 @@ static int32_t files_multi(const int32_t *devices, int32_t n_devices, int32_t ho
     auto fail = [&](int32_t rc, const std::string &w) { if (err && err_cap) { snprintf(err, err_cap, "%s", w.c_str()); } return rc; };
     if (!devices || n_devices < 1 || !inputs || n_inputs < 1 || n_inputs > 2 || !library_json || n_libs < 1 || (!outputs && !counts_outputs))
         return fail(NB200_EINVAL, "bad arguments");
-    if (out3 && counts_outputs) for (int i = 0; i < 3 * n_libs; i++) out3[i] = 0;
+    try { check_umi_flags(disable_thresholding, true); } catch (const std::exception &e) { return fail(NB200_EINVAL, e.what()); }
+    if (out3 && counts_outputs) for (int i = 0; i < out3_per_lib(disable_thresholding) * n_libs; i++) out3[i] = 0;
     std::vector<std::pair<int, double>> trims;
     try { trims = parse_trim_arg(trim, (size_t)n_libs); } catch (const std::exception &e) { return fail(NB200_EINVAL, e.what()); }
     std::vector<nb200_ctx *> ctxs;
@@ -2424,7 +2480,8 @@ int32_t nb200_fastq_to_counts(nb200_ctx *c, const char *r1_fastq, const char *r2
     API_BEGIN(c)
     if (!r1_fastq || !r2_fastq || !whitelist_path || !lib_ids || !counts_outputs || n_libs < 1 || cb_len < 1 || cb_len > kCbMaxLen || umi_len < 0)
         throw std::runtime_error("bad arguments");
-    if (out3) for (int i = 0; i < 3 * n_libs; i++) out3[i] = 0;
+    check_umi_flags(disable_thresholding, true);
+    if (out3) for (int i = 0; i < out3_per_lib(disable_thresholding) * n_libs; i++) out3[i] = 0;
     if (stats) *stats = nb200_cb_stats{};
     const char *inputs[2] = {r1_fastq, r2_fastq};
     const FileStats st = run_job({c}, lib_ids, n_libs, inputs, 2, nullptr, counts_outputs, umi_threshold, disable_thresholding,
@@ -2515,6 +2572,7 @@ int32_t nb200_umi_counts(nb200_ctx *c, int32_t lib_id, uint64_t n_rows, const ui
                          nb200_counts *counts) {
     API_BEGIN(c)
     if (!counts || (n_rows && (!off || !key))) throw std::runtime_error("bad arguments");
+    check_umi_flags(disable_thresholding, true);
     DevLibrary &L = get_lib(c, lib_id);
     uint32_t stride = 1;
     for (uint64_t i = 0; i < n_rows; i++) {
@@ -2576,7 +2634,8 @@ int32_t nb200_report_file(nb200_ctx *c, const char *in_tsv, const char *out_tsv,
                           uint64_t *out3) {
     API_BEGIN(c)
     if (!in_tsv || !out_tsv) throw std::runtime_error("bad arguments");
-    if (out3) out3[0] = out3[1] = out3[2] = 0;
+    check_umi_flags(disable_thresholding, true);
+    if (out3) for (int i = 0; i < out3_per_lib(disable_thresholding); i++) out3[i] = 0;
     ReportRows R;
     if (!parse_per_read_tsv(in_tsv, R, c->host_threads)) {
         write_counts_tsv(out_tsv, nullptr, R.feature_names, R.cells);       // write_empty_df
@@ -2594,7 +2653,10 @@ int32_t nb200_report_file(nb200_ctx *c, const char *in_tsv, const char *out_tsv,
     c->libs.pop_back();                                                     // the dictionary was only for this call
     if (rc != NB200_OK) return rc;
     write_counts_tsv(out_tsv, &counts, R.feature_names, R.cells);
-    if (out3) { out3[0] = R.key.size(); out3[1] = counts.n_rows; out3[2] = counts.dropped_empty; }
+    if (out3) {
+        out3[0] = R.key.size(); out3[1] = counts.n_rows; out3[2] = counts.dropped_empty;
+        if (disable_thresholding & NB200_UMI_CORRECT) out3[3] = c->umis_corrected;
+    }
     API_END(c)
 }
 

@@ -2,11 +2,11 @@
 // UMI stage (agg.cuh) -> counts TSV.  The arithmetic (merge, thresholding, intersection, counting)
 // runs on the GPU; this file only parses, interns strings and writes.
 #include "ingest.hpp"
+#include "library.hpp"
 #include "pandas_na.hpp"
+#include "umi_code.hpp"
 
 #include <algorithm>
-#include <array>
-#include <atomic>
 #include <exception>
 #include <mutex>
 #include <thread>
@@ -72,34 +72,25 @@ static void intern_sorted_mt(const std::vector<std::string_view> &vals, std::vec
     });
 }
 
-// UMI strings -> ids.  Only equality matters (the UMI order never reaches the output), so barcodes over ACGTN are
-// encoded arithmetically: base 5 up to 13 bases, 2 bits per base up to 16 bases without N; anything else is interned.
+// UMI strings -> ids (umi_code.hpp): an ACGTN UMI of 1..13 bases is its code, any other is interned with bit 31 set.
+// Only equality matters (the UMI order never reaches the output).
 static void umi_ids(const std::vector<std::string_view> &vals, std::vector<uint32_t> &ids, int T) {
     const size_t n = vals.size();
-    const size_t L = n ? vals[0].size() : 0;
     ids.resize(n);
-    std::atomic<int> mode_ok5{L >= 1 && L <= 13}, mode_ok4{L >= 1 && L <= 16};
-    static const auto code = [] { std::array<uint8_t, 256> c; c.fill(255); c['A'] = 0; c['C'] = 1; c['G'] = 2; c['T'] = 3; c['N'] = 4; return c; }();
-    if (mode_ok5 || mode_ok4) {
-        const bool five = mode_ok5;
-        parallel_for(std::max(1, T), [&](int t) {
-            const size_t a = n * (size_t)t / std::max(1, T), b = n * (size_t)(t + 1) / std::max(1, T);
-            for (size_t i = a; i < b; i++) {
-                const std::string_view v = vals[i];
-                if (v.size() != L) { mode_ok5 = 0; mode_ok4 = 0; return; }
-                uint32_t x = 0;
-                for (size_t j = 0; j < L; j++) {
-                    const uint8_t cd = code[(unsigned char)v[j]];
-                    if (cd > (five ? 4 : 3)) { if (five) mode_ok5 = 0; else mode_ok4 = 0; return; }
-                    x = five ? x * 5u + cd : (x << 2) | cd;
-                }
-                ids[i] = x;
-            }
-        });
-        if (five ? (int)mode_ok5 : (int)mode_ok4) return;
-    }
+    const int P = n < 100000 ? 1 : std::max(1, T);
+    parallel_for(P, [&](int t) {
+        const size_t a = n * (size_t)t / P, b = n * (size_t)(t + 1) / P;
+        for (size_t i = a; i < b; i++) if (!umi_code(vals[i], ids[i])) ids[i] = 0;       // 0: no code (codes start at 1)
+    });
+    std::vector<std::string_view> other;
+    std::vector<size_t> at;
+    for (size_t i = 0; i < n; i++) if (!ids[i]) { other.push_back(vals[i]); at.push_back(i); }
+    if (other.empty()) return;
+    std::vector<uint32_t> oid;
     std::vector<std::string> names;
-    intern_sorted(vals, ids, names);
+    intern_sorted(other, oid, names);
+    if (names.size() >= kUmiInterned) throw LimitError("more than 2^31 distinct UMIs that are not ACGTN of up to 13 bases");
+    for (size_t j = 0; j < at.size(); j++) ids[at[j]] = oid[j] | kUmiInterned;
 }
 
 // returns false when there is nothing to report (empty file / header only / no usable row)

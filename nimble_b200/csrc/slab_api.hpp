@@ -63,9 +63,10 @@ void lane_rows_segments(nb200_ctx *c, int lane, RowSeg *out);
 // (cell_rank[id], so that cell order is byte order), run the UMI stage.  *counts is the context's table as
 // nb200_umi_counts returns it; *rows = rows that reached the UMI stage.  Throws LimitError beyond 2^31 rows.
 // tenx (fastq-to-counts, after lane_cb_resolve): cells are whitelist lines, provisional ones are decided first, and
-// cell_rank is lane_cb_begin's rank (~0u: the row is dropped and not counted in *rows).
+// cell_rank is lane_cb_begin's rank (~0u: the row is dropped and not counted in *rows).  umi_flags: NB200_UMI_* (with
+// NB200_UMI_CORRECT the UMIs are corrected after the cells are final).
 void lane_rows_count(const std::vector<nb200_ctx *> &ctxs, int li, int32_t lib_id, const std::vector<RowSeg> &segs,
-                     const std::vector<uint32_t> &cell_rank, double threshold, int disable, nb200_counts *counts, uint64_t *rows,
+                     const std::vector<uint32_t> &cell_rank, double threshold, int umi_flags, nb200_counts *counts, uint64_t *rows,
                      bool tenx = false);
 
 // ---- fastq-to-counts: cell barcodes corrected slab by slab, the correction cache over the whole call ------------

@@ -42,6 +42,7 @@
 #include "pandas_na.hpp"
 #include "slab_api.hpp"
 #include "trim.hpp"
+#include "umi_code.hpp"
 
 namespace nb200 {
 namespace {
@@ -496,7 +497,7 @@ public:
     BarcodeDict() { static std::atomic<uint64_t> calls{0}; gen_ = ++calls; }
     uint64_t gen() const { return gen_; }        // tells the per-thread caches of one call from those of another
     uint32_t cell(std::string_view s) { return get(cells_, n_cells_, s); }
-    uint32_t umi(std::string_view s) { return get(umis_, n_umis_, s) | 0x80000000u; }
+    uint32_t umi(std::string_view s) { return get(umis_, n_umis_, s) | kUmiInterned; }
     std::vector<std::string> cell_names() const {                        // id -> CB
         std::vector<std::string> v(n_cells_.load());
         for (const Shard &S : cells_) for (const auto &kv : S.map) v[kv.second] = kv.first;
@@ -529,19 +530,6 @@ struct CellCache {
     uint64_t gen = 0;
     std::unordered_map<size_t, std::pair<uint32_t, std::string>> ids;      // hash of the CB -> (id, CB)
 };
-
-// bijective base 5 (A C G T N = 1..5) of an ACGTN string of 1..13 bases; false for anything else
-static inline bool umi_code(std::string_view s, uint32_t &x) {
-    static const auto digit = [] { std::array<uint8_t, 256> d{}; d['A'] = 1; d['C'] = 2; d['G'] = 3; d['T'] = 4; d['N'] = 5; return d; }();
-    if (s.size() > 13) return false;
-    x = 0;
-    for (char ch : s) {
-        const uint32_t d = digit[(unsigned char)ch];
-        if (!d) return false;
-        x = x * 5u + d;
-    }
-    return true;
-}
 
 // the key's low half for a UMI that is not a pandas NA token (seen: the slab's interned UMIs, saves the shared lock)
 static inline uint32_t umi_id(std::string_view ub, BarcodeDict &bc, std::unordered_map<std::string_view, uint32_t> &seen) {
@@ -1602,11 +1590,16 @@ void run_file_pipeline(const FileJob &job, FileStats *stats_out) {
                 std::sort(sg.begin(), sg.end(), [](const RowSeg &a, const RowSeg &b) { return a.seq < b.seq; });
                 nb200_counts table{};
                 uint64_t rows = 0;
-                lane_rows_count(job.ctxs, (int)li, job.lib_ids[li], sg, rank, job.umi_threshold, job.disable_thresholding, &table, &rows, P.tenx);
+                lane_rows_count(job.ctxs, (int)li, job.lib_ids[li], sg, rank, job.umi_threshold, job.umi_flags, &table, &rows, P.tenx);
                 std::vector<std::string> names(P.libs[li].names.size());
                 for (size_t f = 0; f < names.size(); f++) names[f].assign(P.libs[li].names[f].first, P.libs[li].names[f].second);
                 write_counts_tsv(job.counts_outputs[li], table.n_rows ? &table : nullptr, names, cells);
                 P.stats.counts3.push_back(rows); P.stats.counts3.push_back(table.n_rows); P.stats.counts3.push_back(table.dropped_empty);
+                if (job.umi_flags & NB200_UMI_CORRECT) {
+                    uint64_t corrected = 0;
+                    nb200_umis_corrected(job.ctxs[0], &corrected);
+                    P.stats.counts3.push_back(corrected);
+                }
             }
             lane_bind_thread(job.ctxs[0]);
             t_counts = now_s() - tc;

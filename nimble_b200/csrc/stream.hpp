@@ -21,7 +21,7 @@ struct FileJob {
     // counts mode (nb200_align_files_counts): one counts TSV per library, the UMI stage on the device
     std::vector<std::string> counts_outputs;
     double umi_threshold = 0.05;
-    int disable_thresholding = 0;
+    int umi_flags = 0;                    // NB200_UMI_NO_THRESHOLD | NB200_UMI_CORRECT
     // 10x mode (nb200_fastq_to_counts, counts only): inputs = raw R1 and R2 FASTQ.  The pairs fastq-to-bam would write
     // go to the device as its BAM would: CB = R1[0, cb_len) corrected against the whitelist there, UB = R1[cb_len,
     // cb_len + umi_len), read 1 = the rest of R1, read 2 = R2.
@@ -32,7 +32,7 @@ struct FileJob {
 struct FileStats {
     uint64_t n_reads = 0, paired = 0, has_tags = 0, bases1 = 0, bases2 = 0, checksum = 0, n_slabs = 0, called = 0;
     double seconds = 0.0;
-    std::vector<uint64_t> counts3;        // counts mode: per library rows used, count rows written, UMIs dropped
+    std::vector<uint64_t> counts3;        // counts mode: per library rows used, count rows written, UMIs dropped (+ UMIs corrected)
     nb200_cb_stats cb{};                  // 10x mode: fastq-to-bam's counters (cache_size 0: not computed by this route)
 };
 

@@ -56,6 +56,7 @@ class CountTable:
     dropped_empty: int
     n_called: int
     n_umis: int
+    umis_corrected: int = 0   # (cell, UMI) keys corrected (umi_counts with correct_umis=True)
 
     def __len__(self):
         return len(self.cell)
@@ -312,25 +313,29 @@ class Engine:
         outs = (ct.c_char_p * len(outputs))(*[os.fspath(p).encode() for p in outputs])
         self._ck(self.L.nb200_align_files(self.ctx, ins, len(inputs), ids, outs, len(libs)))
 
-    def align_files_counts(self, inputs, libs, counts_outputs, outputs=None, threshold=0.05, disable_thresholding=False):
+    def align_files_counts(self, inputs, libs, counts_outputs, outputs=None, threshold=0.05, disable_thresholding=False,
+                           correct_umis=False):
         """`align` + `report` in one pass (nb200_align_files_counts): BAM with CB/UB tags in, one counts TSV per library
         out (outputs: per-read TSVs written in the same pass, or None).  Returns per library (rows used, count rows,
-        dropped UMIs), as report_file does."""
+        dropped UMIs), as report_file does; correct_umis=True (DESIGN.md §2.12) adds the number of UMIs corrected."""
         ins = (ct.c_char_p * len(inputs))(*[os.fspath(p).encode() for p in inputs])
         ids = (ct.c_int32 * len(libs))(*[l.id for l in libs])
         cnt = (ct.c_char_p * len(counts_outputs))(*[os.fspath(p).encode() for p in counts_outputs])
         outs = (ct.c_char_p * len(outputs))(*[os.fspath(p).encode() for p in outputs]) if outputs else None
-        out3 = (ct.c_uint64 * (3 * len(libs)))()
+        w = 4 if correct_umis else 3
+        out3 = (ct.c_uint64 * (w * len(libs)))()
         self._ck(self.L.nb200_align_files_counts(self.ctx, ins, len(inputs), ids, outs, cnt, len(libs), float(threshold),
-                                                 int(bool(disable_thresholding)), out3))
-        return [(int(out3[3 * i]), int(out3[3 * i + 1]), int(out3[3 * i + 2])) for i in range(len(libs))]
+                                                 _lib.umi_flags(disable_thresholding, correct_umis), out3))
+        return [tuple(int(v) for v in out3[w * i:w * (i + 1)]) for i in range(len(libs))]
 
-    def report_file(self, in_tsv, out_tsv, threshold=0.05, disable_thresholding=False):
-        """report() file to file (nb200_report_file).  Returns (rows used, count rows, dropped UMIs)."""
-        out = (ct.c_uint64 * 3)()
+    def report_file(self, in_tsv, out_tsv, threshold=0.05, disable_thresholding=False, correct_umis=False):
+        """report() file to file (nb200_report_file).  Returns (rows used, count rows, dropped UMIs), and with
+        correct_umis=True (DESIGN.md §2.12) the number of UMIs corrected after them."""
+        w = 4 if correct_umis else 3
+        out = (ct.c_uint64 * w)()
         self._ck(self.L.nb200_report_file(self.ctx, os.fspath(in_tsv).encode(), os.fspath(out_tsv).encode(), float(threshold),
-                                          int(bool(disable_thresholding)), out))
-        return int(out[0]), int(out[1]), int(out[2])
+                                          _lib.umi_flags(disable_thresholding, correct_umis), out))
+        return tuple(int(v) for v in out)
 
     def align_10x_fastq(self, r1_fastq, r2_fastq, whitelist_path, libs, outputs, cb_length=16, umi_length=12):
         """fastq-to-bam + align in one call, no intermediate BAM (nb200_align_10x_fastq).  Returns the barcode statistics."""
@@ -343,19 +348,20 @@ class Engine:
         return {f: getattr(st, f) for f, _ in CbStats._fields_}
 
     def fastq_to_counts(self, r1_fastq, r2_fastq, whitelist_path, libs, counts_outputs, cb_length=16, umi_length=12, threshold=0.05,
-                        disable_thresholding=False):
+                        disable_thresholding=False, correct_umis=False):
         """fastq-to-bam + align --counts in one streaming pass, no intermediate BAM (nb200_fastq_to_counts): raw 10x R1 / R2
         in, one counts TSV per library out.  Returns (barcode statistics as fastq_to_bam's, with cache_size 0; per library
-        (rows used, count rows, dropped UMIs))."""
+        (rows used, count rows, dropped UMIs[, UMIs corrected with correct_umis=True])."""
         ids = (ct.c_int32 * len(libs))(*[l.id for l in libs])
         cnt = (ct.c_char_p * len(counts_outputs))(*[os.fspath(p).encode() for p in counts_outputs])
-        out3 = (ct.c_uint64 * (3 * len(libs)))()
+        w = 4 if correct_umis else 3
+        out3 = (ct.c_uint64 * (w * len(libs)))()
         st = CbStats()
         self._ck(self.L.nb200_fastq_to_counts(self.ctx, os.fspath(r1_fastq).encode(), os.fspath(r2_fastq).encode(),
                                               os.fspath(whitelist_path).encode(), int(cb_length), int(umi_length), ids, cnt, len(libs),
-                                              float(threshold), int(bool(disable_thresholding)), out3, ct.byref(st)))
+                                              float(threshold), _lib.umi_flags(disable_thresholding, correct_umis), out3, ct.byref(st)))
         return ({f: getattr(st, f) for f, _ in CbStats._fields_},
-                [(int(out3[3 * i]), int(out3[3 * i + 1]), int(out3[3 * i + 2])) for i in range(len(libs))])
+                [tuple(int(v) for v in out3[w * i:w * (i + 1)]) for i in range(len(libs))])
 
     def set_overlap(self, on):
         """Batch pipelining on (default) / off (kernels back to back on one stream: per-stage times add up)."""
@@ -397,7 +403,9 @@ class Engine:
         self._ck(self.L.nb200_fetch_results(self.ctx, res.ctypes.data, feats.ctypes.data))
         return res, feats
 
-    def umi_counts(self, lib, key, off, feat_ids, score=None, threshold=0.05, disable_thresholding=False):
+    def umi_counts(self, lib, key, off, feat_ids, score=None, threshold=0.05, disable_thresholding=False, correct_umis=False):
+        """report()'s UMI stage on rows (nb200_umi_counts).  correct_umis=True (DESIGN.md §2.12) reads the low half of each
+        key as a UMI code (frontend.umi_code) and sets the table's umis_corrected."""
         key = np.ascontiguousarray(key, np.uint64)
         off = np.ascontiguousarray(off, np.uint32)
         feat_ids = np.ascontiguousarray(feat_ids, np.uint32)
@@ -408,8 +416,12 @@ class Engine:
         c = Counts()
         self._ck(self.L.nb200_umi_counts(self.ctx, lib.id, len(key), key.ctypes.data if len(key) else None,
                                          off.ctypes.data, feat_ids.ctypes.data if len(feat_ids) else None, sp,
-                                         float(threshold), int(bool(disable_thresholding)), ct.byref(c)))
-        return self._counts(c)
+                                         float(threshold), _lib.umi_flags(disable_thresholding, correct_umis), ct.byref(c)))
+        table = self._counts(c)
+        n = ct.c_uint64()
+        self._ck(self.L.nb200_umis_corrected(self.ctx, ct.byref(n)))
+        table.umis_corrected = int(n.value)
+        return table
 
     # ---- fastq-to-bam: cell-barcode correction (nimble/fastq_barcode_processor.py) --------------
     def load_whitelist(self, whitelist, cb_length=16):

@@ -277,6 +277,32 @@ def _string_ids(values):
     return np.array([idx.get(v, -1) for v in arr], np.int64), uniq
 
 
+_UMI_DIGIT = {"A": 1, "C": 2, "G": 3, "T": 4, "N": 5}
+UMI_CODE_MAX = 1525878905          # NNNNNNNNNNNNN
+UMI_INTERNED = 0x80000000
+
+
+def umi_code(umi):
+    """The UMI stage's code of a UMI (csrc/umi_code.hpp): an ACGTN string of 1..13 bases is its bijective base-5 value
+    (A C G T N = digits 1..5, last base least significant); None for any other string."""
+    if not 1 <= len(umi) <= 13:
+        return None
+    x = 0
+    for ch in umi:
+        d = _UMI_DIGIT.get(ch)
+        if d is None:
+            return None
+        x = x * 5 + d
+    return x
+
+
+def _umi_ids(values):
+    """UMI strings -> the ids nb200_report_file gives them: the code, else the rank among the other UMIs with bit 31 set."""
+    codes = [umi_code(v) for v in values]
+    other = {v: i for i, v in enumerate(sorted({v for v, c in zip(values, codes) if c is None}))}
+    return np.array([c if c is not None else other[v] | UMI_INTERNED for v, c in zip(values, codes)], np.uint64)
+
+
 def _open_out(path, gz):
     return gzip.open(path, "wt", newline="") if gz else open(path, "w", newline="")
 
@@ -339,18 +365,26 @@ def _per_library_paths(path, library_list):
             for l in library_list]
 
 
+def _print_umi_summary(used, dropped, corrected=None):
+    """What `report` prints after writing its counts TSV (nimble/__main__.py:279, write_empty_df); corrected: UMIs merged
+    by --correct-umis, printed only when the flag was given."""
+    if used == 0:
+        print("No data to parse from input file, writing empty output.")
+    else:
+        if corrected is not None:
+            print(f"Corrected {corrected} UMIs (Hamming distance 1)")
+        print(f"Dropped {dropped} UMIs due to empty intersections")
+
+
 def _print_counts_summary(counts_paths, out3):
-    """What `report` prints after writing its counts TSV (nimble/__main__.py:279, write_empty_df)."""
-    for path, (used, _n_rows, dropped) in zip(counts_paths, out3):
-        if used == 0:
-            print("No data to parse from input file, writing empty output.")
-        else:
-            print(f"Dropped {dropped} UMIs due to empty intersections")
+    """_print_umi_summary per counts file; out3 per library: (rows used, count rows, dropped[, corrected])."""
+    for path, o in zip(counts_paths, out3):
+        _print_umi_summary(o[0], o[2], o[3] if len(o) > 3 else None)
         print("nimble_b200: wrote %s" % path)
 
 
 def align_multi_gpu(reference, output, input, num_cores, strand_filter, k, gpus, trim="", counts=None, threshold=0.05,
-                    disable_thresholding=False):
+                    disable_thresholding=False, correct_umis=False):
     """`align` over several GPUs of the node from this one process (nb200_align_files_multi): every library is loaded on
     every GPU, the reader deals slabs of reads to the GPUs, the writer restores input order (outputs byte-identical to a
     one-GPU run).  gpus: a count (devices 0..N-1) or a list of device indices.  counts: the counts TSV path
@@ -373,10 +407,11 @@ def align_multi_gpu(reference, output, input, num_cores, strand_filter, k, gpus,
                                        out_c, (trim or "").encode(), err, len(err), st)
     else:
         cnt_c = (ct.c_char_p * len(cnts))(*[os.fspath(p).encode() for p in cnts])
-        out3 = (ct.c_uint64 * (3 * len(cnts)))()
+        w = 4 if correct_umis else 3
+        out3 = (ct.c_uint64 * (w * len(cnts)))()
         rc = L.nb200_align_files_counts_multi(d, len(devs), int(num_cores or 0), ins, len(input), libs, len(library_list), strand_filter.encode(),
-                                              int(k or 0), (trim or "").encode(), out_c, cnt_c, float(threshold), int(bool(disable_thresholding)),
-                                              out3, err, len(err), st)
+                                              int(k or 0), (trim or "").encode(), out_c, cnt_c, float(threshold),
+                                              _lib.umi_flags(disable_thresholding, correct_umis), out3, err, len(err), st)
     if rc != 0:
         print("nimble_b200 aligner error: %s" % err.value.decode(errors="replace"), file=sys.stderr)
         return 2 if rc == -2 else 1
@@ -384,7 +419,7 @@ def align_multi_gpu(reference, output, input, num_cores, strand_filter, k, gpus,
     for o in outs or []:
         print("nimble_b200: wrote %s" % o)
     if cnts is not None:
-        _print_counts_summary(cnts, [tuple(out3[3 * i:3 * i + 3]) for i in range(len(cnts))])
+        _print_counts_summary(cnts, [tuple(out3[w * i:w * (i + 1)]) for i in range(len(cnts))])
     return 0
 
 
@@ -421,7 +456,7 @@ def index_info(path, verify=False):
 
 
 def align(reference, output, input, num_cores, strand_filter, trim, tmpdir, k=None, engine=None, native=True, gpus=None, counts=None,
-          threshold=0.05, disable_thresholding=False):
+          threshold=0.05, disable_thresholding=False, correct_umis=False):
     """Drop-in for nimble/__main__.py:153-211.  Returns the aligner's return code (0 = success).
     gpus (extension; also $NB200_GPUS): a count or list of devices -> the streaming pipeline over all of them.
     One pass over the reads per library; OUT naming follows __main__.py:184-189.
@@ -430,13 +465,18 @@ def align(reference, output, input, num_cores, strand_filter, trim, tmpdir, k=No
     around the same GPU calls (the tests use it to cross-check the native file code).
     counts (extension): also write the counts TSV `report` would write from the per-read TSV (threshold /
     disable_thresholding as for report), in the same pass, the rows kept on the GPU; output may then be None (no per-read
-    TSV).  Several libraries: one counts file per library, named like the outputs."""
+    TSV).  Several libraries: one counts file per library, named like the outputs.
+    correct_umis (extension, with counts): merge UMIs one substitution away from a better-supported UMI of the same cell
+    before the UMI stage (DESIGN.md §2.12)."""
     from .engine import Engine
     from ._lib import NimbleB200Error
     print("Aligning input data to the reference libraries")
     sys.stdout.flush()
     if output is None and counts is None:
         print("nimble_b200 aligner error: align needs --output, --counts or both", file=sys.stderr)
+        return 1
+    if correct_umis and counts is None:
+        print("nimble_b200 aligner error: --correct-umis needs --counts", file=sys.stderr)
         return 1
     if counts is not None and not native:
         print("nimble_b200 aligner error: counts are written by the native file pipeline only (native=True)", file=sys.stderr)
@@ -446,7 +486,8 @@ def align(reference, output, input, num_cores, strand_filter, trim, tmpdir, k=No
     if gpus is None and os.environ.get("NB200_GPUS"):
         gpus = int(os.environ["NB200_GPUS"])
     if gpus and engine is None and native and (not isinstance(gpus, int) or gpus > 1):
-        return align_multi_gpu(reference, output, list(input), num_cores, strand_filter, k, gpus, trim, counts, threshold, disable_thresholding)
+        return align_multi_gpu(reference, output, list(input), num_cores, strand_filter, k, gpus, trim, counts, threshold, disable_thresholding,
+                               correct_umis)
     own = engine is None
     try:
         eng = engine or Engine(int(os.environ.get("LOCAL_RANK", 0)), int(num_cores or 0))
@@ -461,7 +502,7 @@ def align(reference, output, input, num_cores, strand_filter, trim, tmpdir, k=No
             if cnts is None:
                 eng.align_files(list(input), libs, outs)
             else:
-                out3 = eng.align_files_counts(list(input), libs, cnts, outs, threshold, disable_thresholding)
+                out3 = eng.align_files_counts(list(input), libs, cnts, outs, threshold, disable_thresholding, correct_umis)
             for o in outs or []:
                 print("nimble_b200: wrote %s" % o)
             if cnts is not None:
@@ -522,23 +563,25 @@ def write_empty_df(output):
     open(output, "w").close()
 
 
-def report(input, output, summarize_columns_list=None, threshold=0.05, disable_thresholding=False, engine=None, native=True):
+def report(input, output, summarize_columns_list=None, threshold=0.05, disable_thresholding=False, engine=None, native=True,
+           correct_umis=False):
     """Per-read TSV -> counts TSV `feature\\tcount\\tcell_barcode` (no header), UMI stage on the GPU.
     native=True (default): nb200_report_file parses and writes in native code; native=False keeps the TSV
-    handling in Python around nb200_umi_counts (the tests cross-check the two)."""
+    handling in Python around nb200_umi_counts (the tests cross-check the two).
+    correct_umis (extension): merge UMIs one substitution away from a better-supported UMI of the same cell before the
+    UMI stage (DESIGN.md §2.12)."""
     from .engine import Engine
     if native:
         own = engine is None
         eng = engine or Engine(int(os.environ.get("LOCAL_RANK", 0)))
         try:
-            used, n_out, dropped = eng.report_file(input, output, threshold, disable_thresholding)
+            o = eng.report_file(input, output, threshold, disable_thresholding, correct_umis)
         finally:
             if own:
                 eng.close()
-        if used == 0:
-            print("No data to parse from input file, writing empty output.")
-        else:
-            print(f"Dropped {dropped} UMIs due to empty intersections")
+        used = o[0]
+        _print_umi_summary(used, o[2], o[3] if correct_umis else None)
+        if used:
             if summarize_columns_list:
                 summarize_fields_tsv(input, summarize_columns_list, "summarize." + output)     # nimble/__main__.py:291-293
         return
@@ -578,8 +621,7 @@ def report(input, output, summarize_columns_list=None, threshold=0.05, disable_t
     names = sorted({x for r in rows for x in r[2].split(",")})
     fid = {nm: i for i, nm in enumerate(names)}
     cid, cbs = _string_ids([r[0] for r in rows])
-    uid, _ = _string_ids([r[1] for r in rows])
-    key = (cid.astype(np.uint64) << np.uint64(32)) | uid.astype(np.uint64)
+    key = (cid.astype(np.uint64) << np.uint64(32)) | _umi_ids([r[1] for r in rows])
     off = np.zeros(len(rows) + 1, np.uint32)
     ids = []
     for i, r in enumerate(rows):
@@ -589,8 +631,8 @@ def report(input, output, summarize_columns_list=None, threshold=0.05, disable_t
     eng = engine or Engine(int(os.environ.get("LOCAL_RANK", 0)))
     lib = eng.load_feature_names(names)
     table = eng.umi_counts(lib, key, off, np.array(ids, np.uint32), np.array([r[3] for r in rows], np.float64),
-                           threshold, disable_thresholding)
-    print(f"Dropped {table.dropped_empty} UMIs due to empty intersections")
+                           threshold, disable_thresholding, correct_umis)
+    _print_umi_summary(len(rows), table.dropped_empty, table.umis_corrected if correct_umis else None)
     with open(output, "w", newline="") as f:
         for feat, cnt, cell in table.rows(names):
             f.write("%s\t%d\t%s\n" % (feat, cnt, cbs[cell]))
@@ -719,11 +761,13 @@ def _print_pair_stats(st):
 
 
 def fastq_to_counts(reference, r1_fastq, r2_fastq, cb_whitelist_file, counts, num_cores=1, strand_filter="unstranded", trim="",
-                    k=None, gpus=None, cb_length=16, umi_length=12, threshold=0.05, disable_thresholding=False, engine=None):
+                    k=None, gpus=None, cb_length=16, umi_length=12, threshold=0.05, disable_thresholding=False, engine=None,
+                    correct_umis=False):
     """`fastq-to-bam`, then `align --counts` on its BAM, in one streaming pass without the BAM (an extension: the reference
     needs fastq-to-bam, align and report).  Raw 10x R1 / R2 FASTQ(.gz) + whitelist in, the counts TSV `report` would
     write out, one per library (named like align's outputs).  gpus (also $NB200_GPUS): a count or a list of devices.
-    Returns 0 on success, 1 on an error (with a message on stderr), 2 without a CUDA device."""
+    correct_umis (extension): merge UMIs one substitution away from a better-supported UMI of the same cell before the UMI
+    stage (DESIGN.md §2.12).  Returns 0 on success, 1 on an error (with a message on stderr), 2 without a CUDA device."""
     import ctypes as ct
     from . import _lib
     from .engine import Engine
@@ -741,19 +785,20 @@ def fastq_to_counts(reference, r1_fastq, r2_fastq, cb_whitelist_file, counts, nu
             d = (ct.c_int32 * len(devs))(*devs)
             libs = (ct.c_char_p * len(library_list))(*[os.fspath(p).encode() for p in library_list])
             cnt_c = (ct.c_char_p * len(cnts))(*[os.fspath(p).encode() for p in cnts])
-            out3 = (ct.c_uint64 * (3 * len(cnts)))()
+            w = 4 if correct_umis else 3
+            out3 = (ct.c_uint64 * (w * len(cnts)))()
             cst = _lib.CbStats()
             err = ct.create_string_buffer(1024)
             st4 = (ct.c_double * 4)()
             rc = L.nb200_fastq_to_counts_multi(d, len(devs), int(num_cores or 0), os.fspath(r1_fastq).encode(), os.fspath(r2_fastq).encode(),
                                                os.fspath(cb_whitelist_file).encode(), int(cb_length), int(umi_length), libs, len(library_list),
                                                strand_filter.encode(), int(k or 0), (trim or "").encode(), cnt_c, float(threshold),
-                                               int(bool(disable_thresholding)), out3, ct.byref(cst), err, len(err), st4)
+                                               _lib.umi_flags(disable_thresholding, correct_umis), out3, ct.byref(cst), err, len(err), st4)
             if rc != 0:
                 print("nimble_b200 aligner error: %s" % err.value.decode(errors="replace"), file=sys.stderr)
                 return 2 if rc == -2 else 1
             st = {f: getattr(cst, f) for f, _ in _lib.CbStats._fields_}
-            o3 = [tuple(out3[3 * i:3 * i + 3]) for i in range(len(cnts))]
+            o3 = [tuple(out3[w * i:w * (i + 1)]) for i in range(len(cnts))]
         else:
             eng = engine or Engine(int(os.environ.get("LOCAL_RANK", 0)), int(num_cores or 0))
             try:
@@ -761,7 +806,7 @@ def fastq_to_counts(reference, r1_fastq, r2_fastq, cb_whitelist_file, counts, nu
                 for lg, (t_len, t_strict) in zip(libs, trims):
                     lg.set_trim(t_len, t_strict)
                 st, o3 = eng.fastq_to_counts(r1_fastq, r2_fastq, cb_whitelist_file, libs, cnts, cb_length, umi_length, threshold,
-                                             disable_thresholding)
+                                             disable_thresholding, correct_umis)
             finally:
                 if own:
                     eng.close()
