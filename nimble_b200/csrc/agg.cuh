@@ -21,7 +21,9 @@
 namespace nb200 {
 
 constexpr int kMaxRounds = 64;   // bound on the reference's `while True` (nimble/utils.py:141)
-constexpr int kSmallRows = 8, kSmallNames = 16;   // UMIs up to this size are worked on in thread-local arrays (umi_general_kernel)
+// UMIs up to this size are worked on in thread-local arrays (umi_general_kernel); both sides of both bounds are pinned by
+// tests/test_umi_stage_edges_gpu.py::test_general_working_set
+constexpr int kSmallRows = 8, kSmallNames = 16;
 
 // Per-read rows as the kernels see them: padded [n, stride] with a length array (what the alignment kernels write) or
 // CSR (what nb200_umi_counts receives).
@@ -264,7 +266,8 @@ __global__ void max_group_kernel(const uint32_t *__restrict__ dev, const uint32_
 }
 
 // rows of one (cell, umi) group -> ascending feature-string order, stable (insertion sort on the permutation;
-// groups are a handful of rows, the caller falls back to the global sort when one exceeds kLocalSortMax)
+// groups are a handful of rows, the caller falls back to the global sort when one exceeds kLocalSortMax; groups of 48 and
+// 49 rows with order-sensitive scores: tests/test_umi_stage_edges_gpu.py::test_group_sort)
 constexpr uint32_t kLocalSortMax = 48;
 __global__ void __launch_bounds__(128)
 group_sort_kernel(uint32_t n_groups, const uint32_t *__restrict__ gstart, uint32_t m, uint32_t *__restrict__ perm, Rows rows,

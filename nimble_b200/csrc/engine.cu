@@ -722,7 +722,9 @@ static void sort_by_feature_string(nb200_ctx *c, const DevLibrary &L, uint32_t m
     int bits = 1;
     while ((1ull << bits) < 2ull * L.host.n_features + 2) bits++;
     c->k32A.ensure((size_t)m * 4); c->k32B.ensure((size_t)m * 4); c->permB.ensure((size_t)m * 4);
-    const int per_key = std::max(1, 32 / bits);          // token columns per 32-bit radix key
+    // token columns per 32-bit radix key: 4 up to F = 127, 3 up to 511, 2 up to 32 767, 1 above (each side pinned by
+    // tests/test_umi_stage_edges_gpu.py::test_token_packing)
+    const int per_key = std::max(1, 32 / bits);
     for (int hi = (int)max_nf; hi > 0; hi -= per_key) {   // LSD: last group of columns first
         const int p0 = std::max(0, hi - per_key), cols = hi - p0;
         gather_tok_kernel<<<nblk(m, 256), 256, 0, c->s_compute>>>(m, c->permA.as<uint32_t>(), rows, (uint32_t)p0, (uint32_t)cols,
@@ -750,6 +752,7 @@ static int bits_for(uint64_t n) { int b = 1; while ((1ull << b) < n) b++; return
 static const uint64_t *correct_umis(nb200_ctx *c, uint64_t n, const uint64_t *d_key, uint32_t m, uint32_t *dv) {
     uint32_t tsize = 1024;
     while (tsize < 2ull * m && tsize < (1u << 31)) tsize <<= 1;      // load factor <= 0.5 (m < 2^31 keeps a slot free)
+    // (m = 511, 512, 513 and 2^15 - 1 .. 2^15 + 1 around the doublings: tests/test_umi_stage_edges_gpu.py::test_correction_selected_rows)
     c->k64A.ensure((size_t)m * 8); c->umi_table.ensure((size_t)tsize * sizeof(UmiSlot)); c->umi_key.ensure(n * 8);
     UmiSlot *t = c->umi_table.as<UmiSlot>();
     CK(cudaMemsetAsync(t, 0, (size_t)tsize * sizeof(UmiSlot), c->s_compute));
@@ -892,6 +895,8 @@ static void aggregate(nb200_ctx *c, const DevLibrary &L, uint64_t n, const uint6
     c->k64A.ensure((size_t)G * 8); c->k64B.ensure((size_t)G * 8); c->permA.ensure((size_t)G * 4); c->permB.ensure((size_t)G * 4);
     umi_keys_kernel<<<nblk(G, 256), 256, 0, c->s_compute>>>(G, c->cell_ord.as<uint32_t>(), c->rep_of.as<uint32_t>(), c->rank_of.as<uint32_t>(),
                                                              (uint32_t)rank_bits, sentinel, c->k64A.as<uint64_t>(), c->permA.as<uint32_t>());
+    // rank_bits + cell_bits + 1 passes 32 bits with ~10 k cells and ~100 k distinct lists (32, 33 and 40 bits:
+    // tests/test_umi_stage_edges_gpu.py::test_stage2_key_width)
     cub_sort64(c, c->k64A.as<uint64_t>(), c->k64B.as<uint64_t>(), c->permA.as<uint32_t>(), c->permB.as<uint32_t>(), G, rank_bits + cell_bits + 1);
     std::swap(c->permA, c->permB);
     c->head.ensure(G); c->gstart2.ensure((size_t)G * 4);
