@@ -296,6 +296,20 @@ int32_t nb200_umis_corrected(const nb200_ctx *ctx, uint64_t *out);
  * written, UMIs dropped for an empty intersection (:279).  Native parser and writer, UMI stage on the GPU. */
 int32_t nb200_report_file(nb200_ctx *ctx, const char *in_tsv, const char *out_tsv, double umi_threshold,
                           int32_t disable_thresholding, uint64_t *out3);
+/* report -s (nimble/__main__.py:291-297, summarize_fields) file to file: per-read TSV (.gz or plain) -> summary TSV,
+ * byte-identical to frontend.summarize_fields_tsv.  columns: names as given to -s (r1_CB, r1_UB, nimble_features are
+ * renamed cb, umi, features, as report does).  out2 (may be NULL) = data rows read, UMI rows written.
+ * A column missing from the header: NB200_EINVAL naming it (after renaming), as "missing column: <name>"; an empty
+ * file has no columns.  Typing, equality, order and printing: DESIGN.md §2.13.  Parser and writer on the host, grouping,
+ * counting and ordering on the GPU (csrc/summarize.cuh).  2^32 or more rows: NB200_ELIMIT. */
+int32_t nb200_summarize_file(nb200_ctx *ctx, const char *in_tsv, const char *const *columns, int32_t n_columns,
+                             const char *out_path, uint64_t *out2);
+/* test hooks (host only) for nb200_summarize_file: how one cell is typed, 0 = a pandas NA token, 1 = an int
+ * (ASCII [+-]?[0-9]+; *value = float(int(cell))), 2 = accepted by Python's float() (*value = its value), 3 = a string.
+ * nb200_float_repr writes Python's repr(x) NUL-terminated to out (cap bytes) and returns its length (NB200_EINVAL if
+ * it does not fit). */
+int32_t nb200_summary_cell_type(const char *cell, uint64_t len, double *value);
+int32_t nb200_float_repr(double x, char *out, int32_t cap);
 /* feature dictionary for nb200_umi_counts when rows come from a TSV: names sorted ascending */
 int32_t nb200_load_feature_names(nb200_ctx *ctx, int32_t n, const char *const *names, int32_t *lib_id);
 

@@ -29,6 +29,7 @@ EXPORTS = [
     "nb200_library_set_trim", "nb200_trim_maxinfo", "nb200_set_defer_fetch", "nb200_fetch_counts", "nb200_fetch_counts_start", "nb200_fast_inflate",
     "nb200_align_files_counts", "nb200_align_files_counts_multi", "nb200_fastq_to_counts", "nb200_fastq_to_counts_multi",
     "nb200_index_write", "nb200_index_info", "nb200_umis_corrected", "nb200_umi_neighbours",
+    "nb200_summarize_file", "nb200_summary_cell_type", "nb200_float_repr",
 ]
 
 # flags word of the counting entries (the disable_thresholding parameter)
@@ -162,6 +163,9 @@ def load():
     L.nb200_trim_maxinfo.argtypes = [vp, u32, i32, i32, dbl]
     L.nb200_trim_maxinfo.restype = u32
     L.nb200_report_file.argtypes = [vp, ct.c_char_p, ct.c_char_p, dbl, i32, ct.POINTER(u64)]
+    L.nb200_summarize_file.argtypes = [vp, ct.c_char_p, ct.POINTER(ct.c_char_p), i32, ct.c_char_p, ct.POINTER(u64)]
+    L.nb200_summary_cell_type.argtypes = [ct.c_char_p, u64, ct.POINTER(dbl)]
+    L.nb200_float_repr.argtypes = [dbl, ct.c_char_p, i32]
     L.nb200_umis_corrected.argtypes = [vp, ct.POINTER(u64)]
     L.nb200_umi_neighbours.argtypes = [u32, ct.POINTER(u32), ct.POINTER(u32)]
     L.nb200_host_ingest_stats.argtypes = [ct.POINTER(ct.c_char_p), i32, i32, ct.POINTER(u64)]

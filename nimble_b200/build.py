@@ -9,9 +9,9 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libnimble_b200.so")
-SOURCES = ["engine.cu", "library.cpp", "ingest.cpp", "stream.cpp", "fastq2bam.cpp", "report.cpp"]
+SOURCES = ["engine.cu", "library.cpp", "ingest.cpp", "stream.cpp", "fastq2bam.cpp", "report.cpp", "summarize.cpp"]
 ALIGNER = os.path.join(HERE, "aligner")
-HEADERS = ["kernels.cuh", "agg.cuh", "barcode.cuh", "library.hpp", "json.hpp", "ingest.hpp", "kmer_hash.hpp", "checksum.hpp", "stream.hpp", "slab_api.hpp", "trim.hpp", "fast_inflate.hpp", "pandas_na.hpp", "umi_code.hpp", "aligner_main.cpp", os.path.join("..", "..", "include", "nimble_b200.h")]
+HEADERS = ["kernels.cuh", "agg.cuh", "barcode.cuh", "summarize.cuh", "library.hpp", "json.hpp", "ingest.hpp", "kmer_hash.hpp", "checksum.hpp", "stream.hpp", "slab_api.hpp", "trim.hpp", "fast_inflate.hpp", "pandas_na.hpp", "umi_code.hpp", "aligner_main.cpp", os.path.join("..", "..", "include", "nimble_b200.h")]
 
 
 def nvcc_path():

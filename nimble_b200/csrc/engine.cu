@@ -30,6 +30,7 @@
 #include "pandas_na.hpp"
 #include "slab_api.hpp"
 #include "stream.hpp"
+#include "summarize.cuh"
 #include "trim.hpp"
 
 namespace nb200 {
@@ -213,6 +214,8 @@ struct nb200_ctx {
     // count table lives in pinned host memory owned by the context
     PinnedBuf<uint32_t> h_cell, h_count, h_off, h_ids;
     DevBuf o_off_d, o_ids_d;
+    // report -s (summarize.cuh): UMI rank per row, first row per UMI, per run count and first row, the runs in output order
+    DevBuf sum_urank, sum_ufirst, sum_rcount, sum_rfirst, sum_out;
     nb200_timing timing{};
     uint64_t launches = 0;
     uint64_t dev_rows = 0, dev_ids = 0;     // extent of the device-side count table (nb200_counts_device)
@@ -2662,6 +2665,154 @@ int32_t nb200_report_file(nb200_ctx *c, const char *in_tsv, const char *out_tsv,
         out3[0] = R.key.size(); out3[1] = counts.n_rows; out3[2] = counts.dropped_empty;
         if (disable_thresholding & NB200_UMI_CORRECT) out3[3] = c->umis_corrected;
     }
+    API_END(c)
+}
+
+namespace nb200 {
+
+// rows (ascending) whose UMI and cell of column `col` are both present, and their value keys
+static void summary_rows(const SummaryTable &S, int col, std::vector<uint32_t> &rows, std::vector<uint64_t> &keys, int T) {
+    const auto &U = S.cols[(size_t)S.umi].cell;
+    const SumColumn &C = S.cols[(size_t)col];
+    const size_t n = S.n_rows;
+    const int P = n < 100000 ? 1 : std::max(1, T);
+    std::vector<size_t> base((size_t)P + 1, 0);
+    parallel_for(P, [&](int p) {
+        size_t k = 0;
+        for (size_t i = n * (size_t)p / P, e = n * (size_t)(p + 1) / P; i < e; i++) k += U[i] != kSumAbsent && C.cell[i] != kSumAbsent;
+        base[(size_t)p + 1] = k;
+    });
+    for (int p = 0; p < P; p++) base[(size_t)p + 1] += base[(size_t)p];
+    rows.resize(base[(size_t)P]);
+    keys.resize(base[(size_t)P]);
+    parallel_for(P, [&](int p) {
+        size_t k = base[(size_t)p];
+        for (size_t i = n * (size_t)p / P, e = n * (size_t)(p + 1) / P; i < e; i++)
+            if (U[i] != kSumAbsent && C.cell[i] != kSumAbsent) { rows[k] = (uint32_t)i; keys[k] = C.key[i]; k++; }
+    });
+}
+
+static int bit_width(uint64_t x) { int b = 1; while (b < 64 && (x >> b)) b++; return b; }
+
+// report -s on the device (summarize.cuh): the UMI rank of every row, then per summarized column its (UMI, value) runs in
+// output order.  Host syncs: the number of UMIs, and per column the number of runs and the copy of its runs.
+static void summarize_group(nb200_ctx *c, const SummaryTable &S, std::vector<uint32_t> &umi_first, std::vector<SumRuns> &runs) {
+    const uint64_t n = S.n_rows;
+    const int T = std::max(1, c->host_threads);
+    cudaStream_t st = c->s_compute;
+    c->timing = nb200_timing{};
+    c->launches = 0;
+    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> dev;         // device work between each upload and its download
+    cudaEvent_t e0 = new_event(c), e1 = new_event(c);
+    CK(cudaEventRecord(e0, st));
+    std::vector<uint32_t> rows;
+    std::vector<uint64_t> keys;
+    summary_rows(S, S.umi, rows, keys, T);
+    const uint64_t mu = rows.size();
+    umi_first.clear();
+    if (mu > 0x7FFFFFF0ull) throw LimitError("more than 2^31 rows with a UMI (CUB item counts are int)");
+    if (mu) {
+        c->k64A.ensure(mu * 8); c->k64B.ensure(mu * 8);
+        c->permA.ensure(mu * 4); c->permB.ensure(mu * 4); c->k32A.ensure(mu * 4); c->k32B.ensure(mu * 4);
+        c->sum_urank.ensure(n * 4); c->sum_ufirst.ensure(mu * 4);
+        CK(cudaMemcpyAsync(c->k64A.p, keys.data(), mu * 8, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(c->permA.p, rows.data(), mu * 4, cudaMemcpyHostToDevice, st));
+        c->timing.h2d_bytes += mu * 12;
+        dev.emplace_back(new_event(c), new_event(c));
+        CK(cudaEventRecord(dev.back().first, st));
+        cub_sort64(c, c->k64A.as<uint64_t>(), c->k64B.as<uint64_t>(), c->permA.as<uint32_t>(), c->permB.as<uint32_t>(), (uint32_t)mu,
+                   S.cols[(size_t)S.umi].bits);
+        sum_umi_head_kernel<<<nblk(mu, 256), 256, 0, st>>>((uint32_t)mu, c->k64B.as<uint64_t>(), c->k32A.as<uint32_t>());
+        incl_scan_u32(c, c->k32A.as<uint32_t>(), c->k32B.as<uint32_t>(), (uint32_t)mu);
+        sum_umi_rank_kernel<<<nblk(mu, 256), 256, 0, st>>>((uint32_t)mu, c->k32B.as<uint32_t>(), c->permB.as<uint32_t>(),
+                                                          c->sum_urank.as<uint32_t>(), c->sum_ufirst.as<uint32_t>());
+        c->launches += 4;
+        CK(cudaEventRecord(dev.back().second, st));
+        uint32_t n_umi = 0;
+        CK(cudaMemcpyAsync(&n_umi, c->k32B.as<uint32_t>() + mu - 1, 4, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        umi_first.resize(n_umi);
+        CK(cudaMemcpyAsync(umi_first.data(), c->sum_ufirst.p, (size_t)n_umi * 4, cudaMemcpyDeviceToHost, st));
+        c->timing.d2h_bytes += 4 + (uint64_t)n_umi * 4;
+        const int ubits = bit_width(n_umi - 1), rbits = bit_width(n);
+        std::vector<char> done(S.cols.size(), 0);
+        for (int col : S.out_cols) {
+            if (done[(size_t)col]) continue;
+            done[(size_t)col] = 1;
+            summary_rows(S, col, rows, keys, T);
+            const uint64_t m = rows.size();
+            if (!m) continue;
+            const int cbits = bit_width(m);
+            const uint32_t cmask = (uint32_t)((1ull << cbits) - 1);
+            c->k64A.ensure(m * 8); c->k64B.ensure(m * 8);
+            c->permA.ensure(m * 4); c->permB.ensure(m * 4); c->k32A.ensure(m * 4); c->k32B.ensure(m * 4);
+            c->gstart.ensure(m * 4); c->gstart2.ensure(m * 4); c->head.ensure(m * 4); c->flag.ensure(m);
+            c->sum_rcount.ensure(m * 4); c->sum_rfirst.ensure(m * 4); c->sum_out.ensure(m * 12);
+            CK(cudaMemcpyAsync(c->k64A.p, keys.data(), m * 8, cudaMemcpyHostToDevice, st));
+            CK(cudaMemcpyAsync(c->permA.p, rows.data(), m * 4, cudaMemcpyHostToDevice, st));
+            c->timing.h2d_bytes += m * 12;
+            dev.emplace_back(new_event(c), new_event(c));
+            CK(cudaEventRecord(dev.back().first, st));
+            // (value, row) -> (UMI rank, value, row): two stable sorts over rows in file order
+            cub_sort64(c, c->k64A.as<uint64_t>(), c->k64B.as<uint64_t>(), c->permA.as<uint32_t>(), c->permB.as<uint32_t>(), (uint32_t)m,
+                       S.cols[(size_t)col].bits);
+            sum_gather_rank_kernel<<<nblk(m, 256), 256, 0, st>>>((uint32_t)m, c->permB.as<uint32_t>(), c->sum_urank.as<uint32_t>(),
+                                                                 c->k32A.as<uint32_t>(), c->gstart.as<uint32_t>());
+            cub_sort32(c, c->k32A.as<uint32_t>(), c->k32B.as<uint32_t>(), c->gstart.as<uint32_t>(), c->gstart2.as<uint32_t>(), (uint32_t)m, ubits);
+            sum_run_head_kernel<<<nblk(m, 256), 256, 0, st>>>((uint32_t)m, c->k32B.as<uint32_t>(), c->gstart2.as<uint32_t>(),
+                                                              c->k64B.as<uint64_t>(), c->permB.as<uint32_t>(), c->flag.as<uint8_t>(),
+                                                              c->permA.as<uint32_t>());
+            const uint32_t r = cub_select(c, c->flag.as<uint8_t>(), c->head.as<uint32_t>(), (uint32_t)m);
+            // runs -> (UMI rank, count descending, first row): stable sort on the order key, then on the UMI rank
+            sum_run_kernel<<<nblk(r, 256), 256, 0, st>>>(r, (uint32_t)m, c->head.as<uint32_t>(), c->k32B.as<uint32_t>(), c->permA.as<uint32_t>(),
+                                                         cmask, rbits, c->k32A.as<uint32_t>(), c->sum_rcount.as<uint32_t>(),
+                                                         c->sum_rfirst.as<uint32_t>(), c->k64A.as<uint64_t>(), c->gstart.as<uint32_t>());
+            cub_sort64(c, c->k64A.as<uint64_t>(), c->k64B.as<uint64_t>(), c->gstart.as<uint32_t>(), c->gstart2.as<uint32_t>(), r, cbits + rbits);
+            sum_gather_run_umi_kernel<<<nblk(r, 256), 256, 0, st>>>(r, c->gstart2.as<uint32_t>(), c->k32A.as<uint32_t>(), c->k32B.as<uint32_t>(),
+                                                                    c->permB.as<uint32_t>());
+            cub_sort32(c, c->k32B.as<uint32_t>(), c->k32A.as<uint32_t>(), c->permB.as<uint32_t>(), c->permA.as<uint32_t>(), r, ubits);
+            sum_out_kernel<<<nblk(r, 256), 256, 0, st>>>(r, c->k32A.as<uint32_t>(), c->permA.as<uint32_t>(), c->gstart2.as<uint32_t>(),
+                                                         c->sum_rcount.as<uint32_t>(), c->sum_rfirst.as<uint32_t>(), c->sum_out.as<uint32_t>());
+            c->launches += 12;
+            CK(cudaEventRecord(dev.back().second, st));
+            std::vector<uint32_t> out((size_t)r * 3);
+            CK(cudaMemcpyAsync(out.data(), c->sum_out.p, (size_t)r * 12, cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
+            c->timing.d2h_bytes += 4 + (uint64_t)r * 12;
+            SumRuns &R = runs[(size_t)col];
+            R.urank.assign(out.begin(), out.begin() + r);
+            R.count.assign(out.begin() + r, out.begin() + 2 * (size_t)r);
+            R.first.assign(out.begin() + 2 * (size_t)r, out.end());
+        }
+    }
+    CK(cudaEventRecord(e1, st));
+    CK(cudaStreamSynchronize(st));
+    float ms = 0;
+    CK(cudaEventElapsedTime(&ms, e0, e1)); c->timing.total_ms = ms;
+    for (auto &d : dev) { CK(cudaEventElapsedTime(&ms, d.first, d.second)); c->timing.agg_ms += ms; }
+    c->timing.launches = c->launches;
+    c->ev_pool.clear();
+}
+
+}  // namespace nb200
+
+int32_t nb200_summarize_file(nb200_ctx *c, const char *in_tsv, const char *const *columns, int32_t n_columns, const char *out_path,
+                             uint64_t *out2) {
+    API_BEGIN(c)
+    if (!in_tsv || !out_path || n_columns < 0 || (n_columns && !columns)) throw std::runtime_error("bad arguments");
+    std::vector<std::string> cols;
+    for (int32_t i = 0; i < n_columns; i++) {
+        if (!columns[i]) throw std::runtime_error("bad arguments");
+        cols.emplace_back(columns[i]);
+    }
+    if (out2) out2[0] = out2[1] = 0;
+    SummaryTable S;
+    parse_summary_tsv(in_tsv, cols, S, c->host_threads);
+    std::vector<uint32_t> umi_first;
+    std::vector<SumRuns> runs(S.cols.size());
+    summarize_group(c, S, umi_first, runs);
+    write_summary_tsv(out_path, S, umi_first, runs, c->host_threads);
+    if (out2) { out2[0] = S.n_rows; out2[1] = umi_first.size(); }
     API_END(c)
 }
 

@@ -4,8 +4,11 @@
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
+#include <exception>
+#include <mutex>
 #include <stdexcept>
 #include <string>
+#include <thread>
 #include <vector>
 
 #include "../../include/nimble_b200.h"
@@ -13,6 +16,18 @@
 namespace nb200 {
 
 struct IoError : std::runtime_error { using std::runtime_error::runtime_error; };
+
+template <class F>
+void parallel_for(int T, F &&fn) {                             // fn(t) on T threads
+    if (T <= 1) { fn(0); return; }
+    std::vector<std::thread> th;
+    std::exception_ptr err;
+    std::mutex em;
+    for (int t = 0; t < T; t++)
+        th.emplace_back([&, t] { try { fn(t); } catch (...) { std::lock_guard<std::mutex> g(em); if (!err) err = std::current_exception(); } });
+    for (auto &x : th) x.join();
+    if (err) std::rethrow_exception(err);
+}
 
 struct PhaseTimer {                       // NB200_TRACE=1: phase times of the host file code on stderr
     bool on = getenv("NB200_TRACE") != nullptr;
@@ -67,6 +82,38 @@ struct ReportRows {
     std::vector<double> score;
 };
 bool parse_per_read_tsv(const std::string &path, ReportRows &R, int threads = 1);
+// cuts of text t at line ends ('\n') from `body` on: one piece per thread for a large body, one piece below 4 MB;
+// returns pieces + 1 offsets, the last t.size()
+std::vector<size_t> line_pieces(const std::string &t, size_t body, int threads);
+
+// ---- report -s (summarize.cpp; DESIGN.md §2.13) -----------------------------------------------------------
+enum SumKind : int { SUM_INT = 0, SUM_INT_AS_FLOAT, SUM_FLOAT, SUM_STRING };   // typed values of a column (frontend._infer_column)
+struct SumColumn {
+    int header_index = -1;
+    SumKind kind = SUM_INT;
+    std::vector<uint64_t> cell;        // per row: text offset << 24 | length (kSumAbsent: a pandas NA token)
+    std::vector<uint64_t> key;         // per row with a cell: value identity, ascending in typed order, minus the smallest
+    int bits = 1;                      // significant bits of the keys
+};
+constexpr uint64_t kSumAbsent = ~0ull;
+struct SummaryTable {
+    std::string text;
+    uint64_t n_rows = 0;
+    std::vector<SumColumn> cols;       // distinct header columns the summary reads
+    int umi = 0;                       // index into cols of the `umi` column
+    std::vector<int> out_cols;         // per requested column: index into cols
+    std::vector<std::string> out_names;
+};
+// The column `name` (after renaming) is not in the header.
+struct MissingColumn : std::runtime_error {
+    std::string name;
+    explicit MissingColumn(const std::string &n) : std::runtime_error("missing column: " + n), name(n) {}
+};
+void parse_summary_tsv(const std::string &path, const std::vector<std::string> &columns, SummaryTable &S, int threads);
+// (umi rank, count, first row) per (UMI, value) pair of one column, in output order
+struct SumRuns { std::vector<uint32_t> urank, count, first; };
+void write_summary_tsv(const std::string &out_path, const SummaryTable &S, const std::vector<uint32_t> &umi_first,
+                       const std::vector<SumRuns> &runs, int threads);
 void write_counts_tsv(const std::string &out_path, const nb200_counts *c, const std::vector<std::string> &feature_names,
                       const std::vector<std::string> &cells);
 

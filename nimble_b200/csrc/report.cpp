@@ -7,9 +7,6 @@
 #include "umi_code.hpp"
 
 #include <algorithm>
-#include <exception>
-#include <mutex>
-#include <thread>
 #include <cstdlib>
 #include <cstring>
 #include <string_view>
@@ -31,18 +28,6 @@ static void intern_sorted(const std::vector<std::string_view> &vals, std::vector
     for (uint32_t i = 0; i < keys.size(); i++) { seen[keys[i]] = i; uniq.emplace_back(keys[i]); }
     ids.resize(vals.size());
     for (size_t i = 0; i < vals.size(); i++) ids[i] = seen[vals[i]];
-}
-
-template <class F>
-static void parallel_for(int T, F &&fn) {                      // fn(t) on T threads
-    if (T <= 1) { fn(0); return; }
-    std::vector<std::thread> th;
-    std::exception_ptr err;
-    std::mutex em;
-    for (int t = 0; t < T; t++)
-        th.emplace_back([&, t] { try { fn(t); } catch (...) { std::lock_guard<std::mutex> g(em); if (!err) err = std::current_exception(); } });
-    for (auto &x : th) x.join();
-    if (err) std::rethrow_exception(err);
 }
 
 // strings -> dense ids in ascending byte order with few distinct values (cells, feature names): per-thread distinct sets,
@@ -93,6 +78,19 @@ static void umi_ids(const std::vector<std::string_view> &vals, std::vector<uint3
     for (size_t j = 0; j < at.size(); j++) ids[at[j]] = oid[j] | kUmiInterned;
 }
 
+std::vector<size_t> line_pieces(const std::string &t, size_t body, int threads) {
+    const int T = (t.size() - body < (4u << 20)) ? 1 : std::max(1, threads);
+    std::vector<size_t> cut((size_t)T + 1, t.size());
+    cut[0] = body;
+    for (int k = 1; k < T; k++) {
+        size_t p = body + (t.size() - body) * (size_t)k / T;
+        p = std::max(p, cut[(size_t)k - 1]);
+        const size_t e = t.find('\n', p);
+        cut[(size_t)k] = e == std::string::npos ? t.size() : e + 1;
+    }
+    return cut;
+}
+
 // returns false when there is nothing to report (empty file / header only / no usable row)
 bool parse_per_read_tsv(const std::string &path, ReportRows &R, int threads) {
     slurp_maybe_gz(path, R.text);
@@ -125,16 +123,9 @@ bool parse_per_read_tsv(const std::string &path, ReportRows &R, int threads) {
     if (fi < 0 || ui < 0 || ci < 0 || si < 0) throw std::runtime_error("per-read TSV lacks nimble_features / r1_UB / r1_CB / nimble_score");
     const int need = std::max(std::max(fi, ui), std::max(ci, si));
     const size_t body = std::min(t.size(), hdr_end + 1);
-    // the body is cut at line boundaries into one piece per thread; every thread parses its lines into its own vectors
-    const int T = (t.size() - body < (4u << 20)) ? 1 : std::max(1, threads);
-    std::vector<size_t> cut((size_t)T + 1, t.size());
-    cut[0] = body;
-    for (int k = 1; k < T; k++) {
-        size_t p = body + (t.size() - body) * (size_t)k / T;
-        p = std::max(p, cut[(size_t)k - 1]);
-        const size_t e = t.find('\n', p);
-        cut[(size_t)k] = e == std::string::npos ? t.size() : e + 1;
-    }
+    // every thread parses the lines of its piece into its own vectors
+    const std::vector<size_t> cut = line_pieces(t, body, threads);
+    const int T = (int)cut.size() - 1;
     struct Part { std::vector<std::string_view> cb, umi, feat; std::vector<double> score; };
     std::vector<Part> parts((size_t)T);
     parallel_for(T, [&](int k) {

@@ -337,6 +337,21 @@ class Engine:
                                           _lib.umi_flags(disable_thresholding, correct_umis), out))
         return tuple(int(v) for v in out)
 
+    def summarize_file(self, in_tsv, columns, out_path):
+        """report -s file to file (nb200_summarize_file): the summary TSV frontend.summarize_fields_tsv writes.  Returns
+        (data rows read, UMI rows written).  A column missing from the header raises KeyError(name), the name after
+        renaming, as summarize_fields_tsv does."""
+        cols = [os.fspath(c).encode() for c in columns]
+        arr = (ct.c_char_p * max(1, len(cols)))(*cols)
+        out = (ct.c_uint64 * 2)()
+        rc = self.L.nb200_summarize_file(self.ctx, os.fspath(in_tsv).encode(), arr, len(cols), os.fspath(out_path).encode(), out)
+        if rc == _lib.EINVAL:
+            msg = (self.L.nb200_last_error(self.ctx) or b"").decode()
+            if msg.startswith("missing column: "):
+                raise KeyError(msg[len("missing column: "):])
+        self._ck(rc)
+        return int(out[0]), int(out[1])
+
     def align_10x_fastq(self, r1_fastq, r2_fastq, whitelist_path, libs, outputs, cb_length=16, umi_length=12):
         """fastq-to-bam + align in one call, no intermediate BAM (nb200_align_10x_fastq).  Returns the barcode statistics."""
         ids = (ct.c_int32 * len(libs))(*[l.id for l in libs])

@@ -566,8 +566,9 @@ def write_empty_df(output):
 def report(input, output, summarize_columns_list=None, threshold=0.05, disable_thresholding=False, engine=None, native=True,
            correct_umis=False):
     """Per-read TSV -> counts TSV `feature\\tcount\\tcell_barcode` (no header), UMI stage on the GPU.
-    native=True (default): nb200_report_file parses and writes in native code; native=False keeps the TSV
-    handling in Python around nb200_umi_counts (the tests cross-check the two).
+    native=True (default): nb200_report_file parses and writes in native code, and nb200_summarize_file writes the
+    summary; native=False keeps the TSV handling in Python around nb200_umi_counts and summarize_fields_tsv (the tests
+    cross-check the two).
     correct_umis (extension): merge UMIs one substitution away from a better-supported UMI of the same cell before the
     UMI stage (DESIGN.md §2.12)."""
     from .engine import Engine
@@ -576,14 +577,13 @@ def report(input, output, summarize_columns_list=None, threshold=0.05, disable_t
         eng = engine or Engine(int(os.environ.get("LOCAL_RANK", 0)))
         try:
             o = eng.report_file(input, output, threshold, disable_thresholding, correct_umis)
+            used = o[0]
+            _print_umi_summary(used, o[2], o[3] if correct_umis else None)
+            if used and summarize_columns_list:                                          # nimble/__main__.py:291-293
+                eng.summarize_file(input, summarize_columns_list, "summarize." + output)
         finally:
             if own:
                 eng.close()
-        used = o[0]
-        _print_umi_summary(used, o[2], o[3] if correct_umis else None)
-        if used:
-            if summarize_columns_list:
-                summarize_fields_tsv(input, summarize_columns_list, "summarize." + output)     # nimble/__main__.py:291-293
         return
     if os.path.getsize(input) == 0:
         write_empty_df(output)
