@@ -640,7 +640,6 @@ static void launch_batch(nb200_ctx *c, const DevLibrary &L, const CallParams &cp
     if (st != sp) { CK(cudaEventRecord(B.probe_done, sp)); CK(cudaStreamWaitEvent(st, B.probe_done, 0)); }
     if (e_probe) CK(cudaEventRecord(e_probe, sp));
     if (e_tail0) CK(cudaEventRecord(e_tail0, st));
-    window_hash_kernel<<<c->sm_count * 8, 256, 0, st>>>(L.dev, items, c->items_cap, B.ctr);
     dedupe_kernel<<<c->sm_count * 8, 256, 0, st>>>(L.dev, items, c->items_cap, B.sw_rep.as<uint32_t>(), B.sw_pairs.as<uint32_t>(), B.ctr);
     sw_kernel<<<c->sm_count * 8, 128, 0, st>>>(L.dev, r1, r2, read0, n_mates, deferred, items, c->items_cap,
                                                B.sw_pairs.as<uint32_t>(), B.ctr);
@@ -661,7 +660,7 @@ static void launch_batch(nb200_ctx *c, const DevLibrary &L, const CallParams &cp
     if (e_call) CK(cudaEventRecord(e_call, st));
     CK(cudaEventRecord(B.tail_done, st));
     B.busy = true;
-    c->launches += (n_mates == 1 && !L.probe_warp) ? 12 : 11;
+    c->launches += (n_mates == 1 && !L.probe_warp) ? 11 : 10;
 }
 
 static void cub_sort32(nb200_ctx *c, const uint32_t *kin, uint32_t *kout, const uint32_t *vin, uint32_t *vout, uint32_t m, int bits) {

@@ -1727,14 +1727,16 @@ __device__ __forceinline__ uint32_t sw_pair(const LibDev &lib, const uint64_t *s
 // ---------------------------------------------------------------------------------------------
 // Candidates of one oriented read are alleles that agree on every k-mer the read hit, so most of
 // their band windows (L + 16 reference bases from gwin) are IDENTICAL and so are their V.
-// Two thread-per-item passes: window_hash_kernel fingerprints every candidate's window;
-// dedupe_kernel looks back over the (contiguous) items of the same read orientation for the first
-// one with the same fingerprint, VERIFIES the two windows word by word, and either records it as
-// its representative or appends the item to the flat work list of sw_kernel.  The look-back is
-// bounded (kLookBack items), so a representative may itself have one: readers follow rep[] to
-// the root.  Nothing is modified in place, so the passes need no ordering between threads.
+// dedupe_kernel, one warp per 32 consecutive items: each lane fingerprints its candidate's window, looks back over the
+// (contiguous) items of the same read orientation for the earliest one within kLookBack items with the same
+// fingerprint, VERIFIES the two windows word by word, and either records it as its representative or appends the item
+// to the flat work list of sw_kernel.  Windows of up to kRegWords words stay in registers, so the look-back and the
+// verification are shuffles; the one segment that reaches back into the previous 32 items has those items reloaded
+// and fingerprinted again (the halo), so the representatives are the same as with an unbounded view.  The look-back
+// is bounded, so a representative may itself have one: readers follow rep[] to the root.  items[] is not written.
 // ---------------------------------------------------------------------------------------------
-constexpr int kLookBack = 32;
+constexpr int kLookBack = 32;      // one warp's chunk: the look-back of its last lane ends at the halo's first item
+constexpr int kRegWords = 6;       // windows of up to 192 bases (reads up to 176 bases) are held in registers
 
 __device__ __forceinline__ void window_word(const LibDev &lib, uint32_t g, int w, int rem_last, int n_w, uint64_t &bases, uint32_t &nbits) {
     const uint32_t gg = g + 32u * (uint32_t)w;
@@ -1746,84 +1748,134 @@ __device__ __forceinline__ void window_word(const LibDev &lib, uint32_t g, int w
     if (w == n_w - 1 && rem_last < 32) { bases &= (1ull << (2 * rem_last)) - 1; nbits &= (1u << rem_last) - 1; }
 }
 
-__global__ void __launch_bounds__(256)
-window_hash_kernel(LibDev lib, SwItem *__restrict__ items, uint32_t items_cap, const Counters *__restrict__ ctr) {
-    const unsigned long long total = ctr->alloc & kItemMask;
-    if (total > items_cap) return;
-    for (uint32_t t = blockIdx.x * blockDim.x + threadIdx.x; t < (uint32_t)total; t += gridDim.x * blockDim.x) {
-        const SwItem it = items[t];
-        if (it.ref == kInvalid) continue;                  // padding of an odd segment
-        const int W = (int)((it.ro >> kRoIdxBits) & 0x1FF) + 2 * kBand;
-        const int n_w = (W + 31) >> 5, rem_last = W - 32 * (n_w - 1);
-        uint64_t h = 0x9E3779B97F4A7C15ull;
-        if (n_w <= 6) {                                    // reads <= 176 bases: all loads in flight before the first use
-            uint64_t bs[6]; uint32_t nb[6];
+__device__ __forceinline__ void fp_mix(uint64_t &h, uint64_t bs, uint32_t nb) {
+    h = (h ^ bs) * 0xD6E8FEB86659FD93ull;
+    h = (h ^ (h >> 32) ^ nb) * 0x9FB21C651E98DF25ull;
+}
+
+// A candidate's band window (W = L + 2 kBand bases from g, n_w words): fingerprint, and for n_w <= kRegWords the
+// words themselves (zero beyond n_w; longer windows leave them zero and are verified from memory).  The n_w + 1
+// consecutive words of ref2bit / refN the window spans are all loaded before the first use.
+struct WinRegs { uint64_t bs[kRegWords]; uint32_t nb[kRegWords]; };
+
+__device__ __forceinline__ uint32_t window_fingerprint(const LibDev &lib, uint32_t g, int n_w, int rem_last, WinRegs &R) {
+    uint64_t h = 0x9E3779B97F4A7C15ull;
 #pragma unroll
-            for (int w = 0; w < 6; w++) { bs[w] = 0; nb[w] = 0; if (w < n_w) window_word(lib, it.gwin, w, rem_last, n_w, bs[w], nb[w]); }
+    for (int w = 0; w < kRegWords; w++) { R.bs[w] = 0; R.nb[w] = 0; }
+    if (n_w <= kRegWords) {
+        const uint32_t wi = g >> 5, sh = (g & 31) * 2, nsh = g & 31;
+        uint64_t a[kRegWords + 1]; uint32_t na[kRegWords + 1];
 #pragma unroll
-            for (int w = 0; w < 6; w++)
-                if (w < n_w) {
-                    h = (h ^ bs[w]) * 0xD6E8FEB86659FD93ull;
-                    h = (h ^ (h >> 32) ^ nb[w]) * 0x9FB21C651E98DF25ull;
-                }
-        } else {
-            for (int w = 0; w < n_w; w++) {
-                uint64_t bs; uint32_t nb;
-                window_word(lib, it.gwin, w, rem_last, n_w, bs, nb);
-                h = (h ^ bs) * 0xD6E8FEB86659FD93ull;
-                h = (h ^ (h >> 32) ^ nb) * 0x9FB21C651E98DF25ull;
-            }
+        for (int j = 0; j <= kRegWords; j++) {
+            a[j] = 0; na[j] = 0;
+            if (j <= n_w) { a[j] = __ldg(lib.ref2bit + wi + j); na[j] = __ldg(lib.refN + wi + j); }
         }
-        items[t].v = (uint32_t)(h >> 32) ^ (uint32_t)h;      // overwritten by the score for the items that get aligned
+#pragma unroll
+        for (int w = 0; w < kRegWords; w++) {
+            if (w >= n_w) continue;
+            uint64_t bs = sh ? ((a[w] >> sh) | (a[w + 1] << (64 - sh))) : a[w];
+            uint32_t nb = (uint32_t)((((uint64_t)na[w + 1] << 32) | na[w]) >> nsh);
+            if (w == n_w - 1 && rem_last < 32) { bs &= (1ull << (2 * rem_last)) - 1; nb &= (1u << rem_last) - 1; }
+            R.bs[w] = bs; R.nb[w] = nb;
+            fp_mix(h, bs, nb);
+        }
+    } else {
+        for (int w = 0; w < n_w; w++) {
+            uint64_t bs; uint32_t nb;
+            window_word(lib, g, w, rem_last, n_w, bs, nb);
+            fp_mix(h, bs, nb);
+        }
     }
+    return (uint32_t)(h >> 32) ^ (uint32_t)h;
 }
 
 __global__ void __launch_bounds__(256)
 dedupe_kernel(LibDev lib, const SwItem *__restrict__ items, uint32_t items_cap, uint32_t *__restrict__ rep,
               uint32_t *__restrict__ uniq, Counters *__restrict__ ctr) {
+    static_assert(kLookBack == 32, "the halo is the previous warp-sized chunk");
     const unsigned long long total = ctr->alloc & kItemMask;
-    if (total > items_cap) return;
+    if (total > items_cap) return;                         // overflowed batch: nothing valid, the host retries
     const int lane = threadIdx.x & 31;
     const uint32_t n = (uint32_t)total;
+    const unsigned below = (1u << lane) - 1;
     uint32_t dups = 0;
     for (uint32_t t0 = (blockIdx.x * blockDim.x + threadIdx.x) & ~31u; t0 < n; t0 += gridDim.x * blockDim.x) {
         const uint32_t t = t0 + lane;
-        SwItem it;
+        SwItem it, ht;
         it.ro = 0; it.ref = kInvalid; it.gwin = 0; it.v = 0;
+        ht = it;
         if (t < n) it = items[t];
+        if (t0) ht = items[t0 - 32 + lane];
         const bool live = it.ref != kInvalid;
-        uint32_t r = t;
-        if (live) {
-            const int W = (int)((it.ro >> kRoIdxBits) & 0x1FF) + 2 * kBand;
-            const int n_w = (W + 31) >> 5, rem_last = W - 32 * (n_w - 1);
-            const uint32_t seg = it.ro & kRoIdxMask;
-            // earliest item of the same segment within the look-back with the same fingerprint ...
-            uint32_t e = t;
-            for (int back = 1; back <= kLookBack && back <= (int)t; back++) {
-                const uint32_t oro = items[t - back].ro, ov = items[t - back].v;
-                if ((oro & kRoIdxMask) != seg) break;
-                if (ov == it.v) e = t - back;
+        const uint32_t seg = it.ro & kRoIdxMask;
+        // the halo: items of the previous chunk in the segment of this chunk's first item (segments are contiguous
+        // and each read orientation has one, so only that segment can reach back)
+        const uint32_t seg0 = __shfl_sync(kFull, seg, 0);
+        const bool hlive = ht.ref != kInvalid && (ht.ro & kRoIdxMask) == seg0;
+        const unsigned hmask = __ballot_sync(kFull, hlive);
+        const int W = (int)((it.ro >> kRoIdxBits) & 0x1FF) + 2 * kBand;
+        const int n_w = (W + 31) >> 5, rem_last = W - 32 * (n_w - 1);
+        WinRegs cw, hw;
+        uint32_t fp = 0, hfp = 0;
+        if (live) fp = window_fingerprint(lib, it.gwin, n_w, rem_last, cw);
+        if (hlive) {
+            const int hW = (int)((ht.ro >> kRoIdxBits) & 0x1FF) + 2 * kBand;
+            const int hn_w = (hW + 31) >> 5;
+            hfp = window_fingerprint(lib, ht.gwin, hn_w, hW - 32 * (hn_w - 1), hw);
+        }
+        // earliest item of the same segment within the look-back with the same fingerprint: in the halo (lanes h >= lane
+        // are at most kLookBack items back), else among the earlier lanes of this chunk
+        const unsigned lmask = __ballot_sync(kFull, live);
+        const unsigned m = __match_any_sync(kFull, ((uint64_t)seg << 32) | fp) & lmask & below;
+        uint32_t e = m ? t0 + (uint32_t)(__ffs(m) - 1) : t;
+        const bool in_seg0 = live && seg == seg0;
+        bool from_halo = false;
+        for (unsigned hm = hmask; hm; hm &= hm - 1) {
+            const int h = __ffs(hm) - 1;
+            const uint32_t f = __shfl_sync(kFull, hfp, h);
+            if (!from_halo && in_seg0 && h >= lane && f == fp) { from_halo = true; e = t0 - 32 + (uint32_t)h; }
+        }
+        // ... and a fingerprint is not a proof: compare the windows (the representative's words come from its lane)
+        bool same = false;
+        const bool check = live && e != t;
+        if (__any_sync(kFull, check)) {
+            const int src = (int)((e - t0 + 32u) & 31u);
+            same = true;
+#pragma unroll
+            for (int w = 0; w < kRegWords; w++) {
+                uint64_t ob = __shfl_sync(kFull, cw.bs[w], src);
+                uint32_t on = __shfl_sync(kFull, cw.nb[w], src);
+                if (hmask) {
+                    const uint64_t hb = __shfl_sync(kFull, hw.bs[w], src);
+                    const uint32_t hn = __shfl_sync(kFull, hw.nb[w], src);
+                    if (from_halo) { ob = hb; on = hn; }
+                }
+                same = same && ob == cw.bs[w] && on == cw.nb[w];
             }
-            if (e != t) {                                  // ... and a fingerprint is not a proof: compare the windows
-                const uint32_t og = items[e].gwin;
-                bool same = true;
+            uint32_t og = __shfl_sync(kFull, it.gwin, src);
+            if (hmask) {
+                const uint32_t hg = __shfl_sync(kFull, ht.gwin, src);
+                if (from_halo) og = hg;
+            }
+            if (check && n_w > kRegWords) {                // long windows: word by word from memory
                 for (int w = 0; w < n_w && same; w++) {
                     uint64_t b0, b1; uint32_t n0, n1;
                     window_word(lib, it.gwin, w, rem_last, n_w, b0, n0);
                     window_word(lib, og, w, rem_last, n_w, b1, n1);
                     same = (b0 == b1) && (n0 == n1);
                 }
-                if (same) r = e;
             }
-            rep[t] = r;
+            same = same && check;
         }
+        const uint32_t r = same ? e : t;
+        if (live) rep[t] = r;
         const bool uq = live && r == t;
         const unsigned ub = __ballot_sync(kFull, uq);
         if (ub) {
             uint32_t base = 0;
             if (lane == 0) base = (uint32_t)atomicAdd(&ctr->n_swpairs, (unsigned long long)__popc(ub));
             base = __shfl_sync(kFull, base, 0);
-            if (uq) uniq[base + __popc(ub & ((1u << lane) - 1))] = t;
+            if (uq) uniq[base + __popc(ub & below)] = t;
         }
         dups += (live && !uq) ? 1u : 0u;
     }
@@ -1837,14 +1889,35 @@ struct SwQuery {
     const uint32_t *nm;
     int L, ori;
 };
-__device__ __forceinline__ void query_base(const SwQuery &q, int i, uint32_t &qrep, uint32_t &qmask) {
-    const bool in = i < q.L;
-    const int idx = in ? (q.ori ? (q.L - 1 - i) : i) : 0;
-    uint32_t b = (uint32_t)(q.seq[idx >> 5] >> (2 * (idx & 31))) & 3u;
-    if (q.ori) b = 3u - b;
-    const uint32_t qn = (q.nm[idx >> 5] >> (idx & 31)) & 1u;
-    qrep = b * 0x55555555u;
-    qmask = in ? (qn - 1u) : 0u;                           // read N or past the end of the shorter read: no cell matches
+// The query bases of rows i .. i + 31 in row order (orientation 1: the read backwards and complemented), two bits per
+// row in b, and a flag per row in n that is set for a read N and for rows at or past L: such rows match nothing.
+// Only words that hold bases of these rows are read.
+__device__ __forceinline__ void query_rows32(const SwQuery &q, int i, uint64_t &b, uint32_t &n) {
+    b = 0; n = ~0u;
+    const int left = q.L - i;                              // rows of the 32 inside the read
+    if (left <= 0) return;
+    const int s = q.ori ? left - 32 : i;                   // lowest read index of the 32 (may be below 0 for ori 1)
+    const int w = s >> 5, sh = s & 31;
+    uint64_t lo = 0; uint32_t nlo = 0;
+    if (w >= 0) { lo = __ldg(q.seq + w); nlo = __ldg(q.nm + w); }
+    if (sh) {
+        const uint64_t hi = __ldg(q.seq + w + 1);
+        const uint32_t nhi = __ldg(q.nm + w + 1);
+        lo = (lo >> (2 * sh)) | (hi << (64 - 2 * sh));
+        nlo = __funnelshift_r(nlo, nhi, sh);
+    }
+    if (q.ori) {                                           // reverse the 2-bit groups, complement the bases
+        lo = __brevll(lo);
+        lo = ~(((lo >> 1) & 0x5555555555555555ull) | ((lo & 0x5555555555555555ull) << 1));
+        nlo = __brev(nlo);
+    }
+    b = lo;
+    n = left < 32 ? nlo | (~0u << left) : nlo;
+}
+__device__ __forceinline__ void next_query_row(uint64_t &b, uint32_t &n, uint32_t &qrep, uint32_t &qmask) {
+    qrep = ((uint32_t)b & 3u) * 0x55555555u;               // the base replicated over all 16 two-bit groups
+    qmask = (n & 1u) - 1u;                                 // read N or past the end of the shorter read: no cell matches
+    b >>= 2; n >>= 1;
 }
 __device__ __forceinline__ uint32_t sw_pair2(const LibDev &lib, const SwQuery &qa, const SwQuery &qb, uint32_t gA, uint32_t gB) {
     uint32_t H[kNB];
@@ -1853,15 +1926,21 @@ __device__ __forceinline__ uint32_t sw_pair2(const LibDev &lib, const SwQuery &q
     uint32_t best = 0;
     RefWin wa, wb;
     wa.lo = wa.hi = wa.nlo = wa.nhi = 0; wb = wa;
+    uint64_t sa = 0, sb = 0;
+    uint32_t na = 0, nb = 0;
     const int Lmax = max(qa.L, qb.L);
     for (int i = 0; i < Lmax; i++) {
         if ((i & 15) == 0) {
             load_ref_window32(lib, gA + i, wa);
             load_ref_window32(lib, gB + i, wb);
+            if ((i & 31) == 0) {
+                query_rows32(qa, i, sa, na);
+                query_rows32(qb, i, sb, nb);
+            }
         }
         uint32_t qrepA, qmaskA, qrepB, qmaskB;
-        query_base(qa, i, qrepA, qmaskA);
-        query_base(qb, i, qrepB, qmaskB);
+        next_query_row(sa, na, qrepA, qmaskA);
+        next_query_row(sb, nb, qrepB, qmaskB);
         uint32_t za_lo, za_hi, zb_lo, zb_hi;
         row_matches(wa, qrepA, qmaskA, za_lo, za_hi);
         row_matches(wb, qrepB, qmaskB, zb_lo, zb_hi);
