@@ -361,12 +361,17 @@ int32_t nb200_correct_barcodes_resident(nb200_ctx *ctx, int32_t wl_id, int32_t *
 
 /* `nimble fastq-to-bam` (fastq_to_bam_with_barcodes, :212-316): paired 10x FASTQ(.gz) + whitelist ->
  * unaligned BAM with CB (corrected) / UB (raw) tags, flags 77 / 141, read 1 = R1 minus barcode+UMI.
- * Pairs are written in file order. */
+ * Pairs are written in file order.  Streaming: host memory is bounded by the slab pool, not by the input; each slab's
+ * barcodes are corrected on the device and the first read (in file order) with a raw barcode that has several
+ * candidates decides for every later read with it.  The BAM is written to OUT.tmp and renamed: on an error (a malformed
+ * record in either file, a written pair with a name over 254 bytes) no output is left and a previous one is intact. */
 int32_t nb200_fastq_to_bam(nb200_ctx *ctx, const char *r1_fastq, const char *r2_fastq, const char *whitelist_path,
                            const char *output_bam, int32_t cb_len, int32_t umi_len, nb200_cb_stats *stats);
 /* fastq-to-bam followed by align, without the intermediate BAM (SURVEY.md §8f rank 2): exactly the pairs
  * nb200_fastq_to_bam would write are aligned as nb200_align_files would align that BAM; one per-read TSV
- * per library.  Not a reference entry point: the reference needs both commands and the file between them. */
+ * per library, byte-identical to the two steps, streaming as nb200_fastq_to_bam.  It fails where the two steps fail (a
+ * written pair with a read over 500 bases after the cut, or a name over 254 bytes).  stats: nb200_fastq_to_bam's.
+ * Not a reference entry point: the reference needs both commands and the file between them. */
 int32_t nb200_align_10x_fastq(nb200_ctx *ctx, const char *r1_fastq, const char *r2_fastq, const char *whitelist_path,
                               int32_t cb_len, int32_t umi_len, const int32_t *lib_ids, const char *const *outputs,
                               int32_t n_libs, nb200_cb_stats *stats);
@@ -392,6 +397,16 @@ int32_t nb200_fastq_to_counts_multi(const int32_t *devices, int32_t n_devices, i
                                     const char *trim, const char *const *counts_outputs, double umi_threshold,
                                     int32_t disable_thresholding, uint64_t *out3, nb200_cb_stats *stats, char *err, size_t err_cap,
                                     double *stats4);
+/* nb200_align_10x_fastq over several GPUs of the node, with the arguments of nb200_fastq_to_counts_multi plus
+ * per_read_outputs (one per library): per-read TSVs, counts TSVs or both (at least one of the two), in one pass,
+ * byte-identical to a one-GPU run and to fastq-to-bam followed by align (--counts).  stats: nb200_fastq_to_bam's counters;
+ * cache_size is computed without counts_outputs, and is 0 with them (as nb200_fastq_to_counts_multi keeps it). */
+int32_t nb200_align_10x_fastq_multi(const int32_t *devices, int32_t n_devices, int32_t host_threads, const char *r1_fastq,
+                                    const char *r2_fastq, const char *whitelist_path, int32_t cb_len, int32_t umi_len,
+                                    const char *const *library_json, int32_t n_libs, const char *strand_filter, int32_t k,
+                                    const char *trim, const char *const *per_read_outputs, const char *const *counts_outputs,
+                                    double umi_threshold, int32_t disable_thresholding, uint64_t *out3, nb200_cb_stats *stats,
+                                    char *err, size_t err_cap, double *stats4);
 
 int32_t nb200_last_timing(const nb200_ctx *ctx, nb200_timing *out);
 /* Batch pipelining (default on): batch k's fingerprint / Smith-Waterman / deferred-call kernels run on a

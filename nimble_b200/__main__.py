@@ -73,6 +73,8 @@ def main(argv=None):
     fc.add_argument("--r2-fastq", help="Path to R2 FASTQ file.", type=str, required=True)
     fc.add_argument("--map", required=True, help="Cell barcode whitelist file (one CB per line, .gz or plain text)")
     fc.add_argument("--counts", help="Path of the counts TSV (one per library, named as align names its outputs).", type=str, required=True)
+    fc.add_argument("--output", help="Also write the per-read TSV align --map writes (one per library, named as align names its "
+                                     "outputs), in the same pass", type=str, default=None)
     fc.add_argument("-c", "--num_cores", help="The number of host threads to use.", type=int, default=1)
     fc.add_argument("--strand_filter", help="Filter reads based on strand information.", type=str, default="unstranded")
     fc.add_argument("--trim", help="<TARGET_LENGTH>:<STRICTNESS>, comma-separated, one entry per library", type=str, default="")
@@ -116,7 +118,7 @@ def main(argv=None):
             print("nimble_b200: --trim is applied by the streaming file path only; ignored with --map "
                   "(run fastq-to-bam, then align --trim on its BAM)", file=sys.stderr)
         sys.exit(align_10x(args.reference, args.output, args.input[0], args.input[1], args.map, args.num_cores, args.strand_filter,
-                           args.cb_length, args.umi_length, k=args.kmer))
+                           args.cb_length, args.umi_length, k=args.kmer, gpus=args.gpus))
     elif args.subcommand == "align":
         sys.exit(align(args.reference, args.output, args.input, args.num_cores, args.strand_filter, args.trim,
                        args.tmpdir, k=args.kmer, gpus=args.gpus, counts=args.counts, threshold=args.threshold,
@@ -135,7 +137,7 @@ def main(argv=None):
         sys.exit(fastq_to_counts(args.reference, args.r1_fastq, args.r2_fastq, args.map, args.counts, args.num_cores, args.strand_filter,
                                  args.trim, k=args.kmer, gpus=args.gpus, cb_length=args.cb_length, umi_length=args.umi_length,
                                  threshold=args.threshold, disable_thresholding=args.disable_thresholding,
-                                 correct_umis=args.correct_umis))
+                                 correct_umis=args.correct_umis, output=args.output))
     elif args.subcommand == "index":
         if "," in args.reference:
             parser.error("index takes one library per call")

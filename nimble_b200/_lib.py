@@ -28,6 +28,7 @@ EXPORTS = [
     "nb200_align_10x_fastq", "nb200_set_overlap", "nb200_bench_dpx_peak", "nb200_set_stats", "nb200_align_files_multi",
     "nb200_library_set_trim", "nb200_trim_maxinfo", "nb200_set_defer_fetch", "nb200_fetch_counts", "nb200_fetch_counts_start", "nb200_fast_inflate",
     "nb200_align_files_counts", "nb200_align_files_counts_multi", "nb200_fastq_to_counts", "nb200_fastq_to_counts_multi",
+    "nb200_align_10x_fastq_multi",
     "nb200_index_write", "nb200_index_info", "nb200_umis_corrected", "nb200_umi_neighbours",
     "nb200_summarize_file", "nb200_summary_cell_type", "nb200_float_repr",
 ]
@@ -159,6 +160,10 @@ def load():
     L.nb200_fastq_to_counts_multi.argtypes = [ct.POINTER(i32), i32, i32, ct.c_char_p, ct.c_char_p, ct.c_char_p, i32, i32,
                                               ct.POINTER(ct.c_char_p), i32, ct.c_char_p, i32, ct.c_char_p, ct.POINTER(ct.c_char_p), dbl,
                                               i32, ct.POINTER(u64), ct.POINTER(CbStats), ct.c_char_p, ct.c_size_t, ct.POINTER(dbl)]
+    L.nb200_align_10x_fastq_multi.argtypes = [ct.POINTER(i32), i32, i32, ct.c_char_p, ct.c_char_p, ct.c_char_p, i32, i32,
+                                              ct.POINTER(ct.c_char_p), i32, ct.c_char_p, i32, ct.c_char_p, ct.POINTER(ct.c_char_p),
+                                              ct.POINTER(ct.c_char_p), dbl, i32, ct.POINTER(u64), ct.POINTER(CbStats), ct.c_char_p,
+                                              ct.c_size_t, ct.POINTER(dbl)]
     L.nb200_library_set_trim.argtypes = [vp, i32, i32, dbl]
     L.nb200_trim_maxinfo.argtypes = [vp, u32, i32, i32, dbl]
     L.nb200_trim_maxinfo.restype = u32

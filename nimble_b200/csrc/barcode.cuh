@@ -259,7 +259,7 @@ __global__ void cb_propagate_kernel(const uint32_t *__restrict__ sorted_idx, con
     if (h != t) out_idx[sorted_idx[t]] = out_idx[sorted_idx[h]];      // heads are never written: no race
 }
 
-// ---- fastq-to-counts (nb200_fastq_to_counts): one slab at a time, the cache rule over the whole call ----------------
+// ---- 10x mode of the file pipeline (fastq-to-bam, align --map, fastq-to-counts): one slab at a time ------------------
 // Per read of a slab: key = cell << 32 | umi.  On entry key holds the host's flags << 32 | umi (umi 0xFFFFFFFF for a
 // pandas NA UMI; flags: slab_api.hpp kTenx*, a pair the two-step route refuses once it is written).  The flags of a read
 // whose barcode is corrected (= written by fastq-to-bam) are or-ed into ctr->pad, which makes the host fail the call.
@@ -315,6 +315,23 @@ cb_remap_kernel(uint64_t n, uint64_t *__restrict__ key, const uint32_t *__restri
     }
     const unsigned b = __ballot_sync(0xFFFFFFFFu, drop);
     if ((threadIdx.x & 31) == 0 && b) atomicAdd(dropped, (unsigned long long)__popc(b));
+}
+
+// Cache size over a call (lane_cb_cache_size): the raw keys of a slab's exact misses (miss_list, ctr->n_miss of them)
+// appended to the context's log at *log_n; cb_log_advance_kernel moves the end behind them afterwards.
+__global__ void __launch_bounds__(256)
+cb_log_misses_kernel(uint32_t n, const uint32_t *__restrict__ miss_list, const uint64_t *__restrict__ keys,
+                     const CbCounters *__restrict__ ctr, const unsigned long long *__restrict__ log_n, uint64_t *__restrict__ log) {
+    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t < n && t < ctr->n_miss) log[*log_n + t] = keys[miss_list[t]];
+}
+__global__ void cb_log_advance_kernel(const CbCounters *__restrict__ ctr, unsigned long long *__restrict__ log_n) {
+    *log_n += ctr->n_miss;
+}
+// hit flags of another context or-ed into these
+__global__ void cb_or_flags_kernel(const uint8_t *__restrict__ src, uint64_t n, uint8_t *__restrict__ dst) {
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t < n && src[t]) dst[t] = 1;
 }
 
 __global__ void cb_count_flags_kernel(const uint8_t *__restrict__ flag, uint64_t n, unsigned long long *__restrict__ out) {

@@ -167,19 +167,27 @@ struct nb200_ctx {
         PinnedBuf<unsigned long long> h_seg;
         const uint64_t *hkey = nullptr;           // what was submitted (an overflow re-runs it)
         uint64_t n_rows_max = 0;                  // reads of the slab in flight: bound on the rows it appends
-        // fastq-to-counts: the slab's barcodes and their correction (cb_*: device; h_cb: pinned CbCounters + log end)
+        // 10x mode: the slab's barcodes and their correction (cb_*: device; h_cb: pinned CbCounters + the ends of the logs)
         DevBuf cb, cbq, cb_raw, cb_idx, cb_st, cb_miss, cb_multi, cb_ctr;
-        const uint8_t *hcb = nullptr, *hcbq = nullptr;   // what was submitted (an overflow re-runs it)
+        CbSlab hcb{};                             // what was submitted (an overflow re-runs it)
+        bool has_cb = false;
+        uint64_t n_cb = 0;                        // reads of the slab in flight: bound on what it appends to the logs
         uint64_t seq = 0;
         PinnedBuf<unsigned long long> h_cb;
     } lane[kFileLanes];
-    // fastq-to-counts (lane_cb_*): the whitelist table, and the log of reads with several candidates (raw barcode, file
+    // 10x mode (lane_cb_*): the whitelist table, and the log of reads with several candidates (raw barcode, file
     // order, own choice; tx_n = entries, device-side).  The log grows like the row stores: tx_hi = its end as of the
     // last slab the host has seen.  tx_dec (first context, lane_cb_resolve): the decision per entry of every log.
     DevBuf tx_table, tx_key, tx_ord, tx_choice, tx_n, tx_dec;
     WlDev tx_wl{};
     uint64_t tx_cap = 0, tx_hi = 0;
     std::vector<DevBuf> tx_old;
+    // cache size over the call (lane_cb_cache_size): per whitelist line "hit exactly", and the log of the raw keys of the
+    // exact misses (tx_miss_n entries, device-side), grown as the other log
+    bool tx_cache = false;
+    uint64_t tx_entries = 0, tx_miss_cap = 0, tx_miss_hi = 0;
+    DevBuf tx_hit, tx_miss, tx_miss_n;
+    std::vector<DevBuf> tx_miss_old;
     std::vector<uint64_t> tx_base;                // first context: where each context's log starts in tx_dec
     // counts mode (slab_api.hpp): per library of the call, the rows that count, appended slab by slab on s_copy[1]
     struct RowStore {
@@ -1161,10 +1169,11 @@ bool lane_trim(nb200_ctx *c, int32_t lib_id, int *target, double *strictness) {
 // Grow three arrays that work queued on stream s may still read or write: each gets a new buffer of `bytes`, its first
 // `keep` bytes copied over on s; the old buffer goes to `retired`, which the caller frees only when the store is reset.
 struct Regrow { DevBuf &buf; size_t bytes, keep; };
-static void grow_keep_retire(const Regrow (&a)[3], cudaStream_t s, std::vector<DevBuf> &retired) {
-    DevBuf fresh[3];
-    for (int i = 0; i < 3; i++) fresh[i].ensure(a[i].bytes);
-    for (int i = 0; i < 3; i++) {
+template <size_t N>
+static void grow_keep_retire(const Regrow (&a)[N], cudaStream_t s, std::vector<DevBuf> &retired) {
+    DevBuf fresh[N];
+    for (size_t i = 0; i < N; i++) fresh[i].ensure(a[i].bytes);
+    for (size_t i = 0; i < N; i++) {
         if (a[i].keep) CK(cudaMemcpyAsync(fresh[i].p, a[i].buf.p, a[i].keep, cudaMemcpyDeviceToDevice, s));
         if (a[i].buf.p) retired.push_back(std::move(a[i].buf));
         a[i].buf = std::move(fresh[i]);
@@ -1204,7 +1213,7 @@ static void append_rows(nb200_ctx *c, nb200_ctx::FileLane &F, int li, uint64_t n
     c->launches += 4;
 }
 
-// ---- cell-barcode correction shared by the whole-batch path (cb_run) and the slabs of fastq-to-counts ---------------
+// ---- cell-barcode correction shared by the whole-batch path (cb_run) and the slabs of the 10x mode ----------------
 struct MaxU32 {
     __host__ __device__ __forceinline__ uint32_t operator()(uint32_t a, uint32_t b) const { return a > b ? a : b; }
 };
@@ -1241,45 +1250,67 @@ static void cb_first_decides(nb200_ctx *c, const uint32_t *list, const uint64_t 
     c->launches += 8;
 }
 
-// fastq-to-counts, per slab (inside lane_submit, on s_compute behind the slab's uploads): correct the barcodes, turn the
-// host's UMI keys into cell << 32 | umi, log the reads with several candidates.  No host synchronise: the log's capacity
-// is bounded on the host (its end as of the last slab seen plus the reads of the slabs in flight).
+// 10x mode, per slab (inside lane_submit, on s_compute behind the slab's uploads): correct the barcodes and copy each
+// read's correction back; with keys (counts mode) turn the host's UMI keys into cell << 32 | umi and log the reads with
+// several candidates; with the cache size, mark the lines hit exactly and log the raw keys of the exact misses.  No host
+// synchronise: the logs' capacities are bounded on the host (their ends as of the last slab seen plus the reads of the
+// slabs in flight).
 static void lane_cb_slab(nb200_ctx *c, nb200_ctx::FileLane &F, uint64_t n) {
     cudaStream_t s = c->s_compute;
     uint64_t other = 0;
-    for (auto &G : c->lane) if (&G != &F && G.busy && G.hcb) other += G.n_rows_max;
-    const uint64_t need = c->tx_hi + other + n;
-    if (need > c->tx_cap) {                          // grow: copy on s_compute (every log write is on it), free at the end
-        const uint64_t cap = std::max(need, 2 * c->tx_cap);
+    for (auto &G : c->lane) if (&G != &F && G.busy) other += G.n_cb;
+    const bool keys = F.hkey != nullptr;
+    if (keys && c->tx_hi + other + n > c->tx_cap) {   // grow: copy on s_compute (every log write is on it), free at the end
+        const uint64_t cap = std::max(c->tx_hi + other + n, 2 * c->tx_cap);
         const uint64_t keep = std::min(c->tx_hi + other, c->tx_cap);
         grow_keep_retire({{c->tx_key, cap * 8, keep * 8}, {c->tx_ord, cap * 8, keep * 8}, {c->tx_choice, cap * 4, keep * 4}}, s, c->tx_old);
         c->tx_cap = cap;
+    }
+    if (c->tx_cache && c->tx_miss_hi + other + n > c->tx_miss_cap) {
+        const uint64_t cap = std::max(c->tx_miss_hi + other + n, 2 * c->tx_miss_cap);
+        grow_keep_retire({{c->tx_miss, cap * 8, std::min(c->tx_miss_hi + other, c->tx_miss_cap) * 8}}, s, c->tx_miss_old);
+        c->tx_miss_cap = cap;
     }
     const uint64_t nb = std::max<uint64_t>(n, 1);
     F.cb_raw.ensure(nb * 8); F.cb_idx.ensure(nb * 4); F.cb_st.ensure(nb); F.cb_miss.ensure(nb * 4); F.cb_multi.ensure(nb + 16);
     F.cb_ctr.ensure(sizeof(CbCounters));
     CbCounters *ctr = F.cb_ctr.as<CbCounters>();
     cb_launch(c, c->tx_wl, s, F.cb.as<uint8_t>(), F.cbq.as<uint8_t>(), nullptr, n, F.cb_raw.as<uint64_t>(), F.cb_idx.as<int32_t>(),
-              F.cb_st.as<uint8_t>(), F.cb_miss.as<uint32_t>(), nullptr, 0, nullptr, F.cb_multi.as<uint8_t>(), ctr);
-    if (n) {
+              F.cb_st.as<uint8_t>(), F.cb_miss.as<uint32_t>(), nullptr, 0, c->tx_cache ? c->tx_hit.as<uint8_t>() : nullptr,
+              F.cb_multi.as<uint8_t>(), ctr);
+    if (n && keys) {
         cb_key_kernel<<<nblk(n, 256), 256, 0, s>>>((uint32_t)n, F.cb_st.as<uint8_t>(), F.cb_idx.as<int32_t>(), F.cb_multi.as<uint8_t>(),
                                                    F.cb_raw.as<uint64_t>(), F.seq << 21, F.key.as<uint64_t>(), c->tx_n.as<unsigned long long>(),
                                                    c->tx_key.as<uint64_t>(), c->tx_ord.as<uint64_t>(), c->tx_choice.as<int32_t>(), ctr);
-        CK(cudaGetLastError());
         c->launches++;
     }
+    if (n && c->tx_cache) {
+        cb_log_misses_kernel<<<nblk(n, 256), 256, 0, s>>>((uint32_t)n, F.cb_miss.as<uint32_t>(), F.cb_raw.as<uint64_t>(), ctr,
+                                                          c->tx_miss_n.as<unsigned long long>(), c->tx_miss.as<uint64_t>());
+        cb_log_advance_kernel<<<1, 1, 0, s>>>(ctr, c->tx_miss_n.as<unsigned long long>());
+        c->launches += 2;
+    }
+    CK(cudaGetLastError());
     // (read after lane_wait: the lane's done event follows these copies through s_compute's tail)
     CK(cudaMemcpyAsync(F.h_cb.p, ctr, sizeof(CbCounters), cudaMemcpyDeviceToHost, s));
     CK(cudaMemcpyAsync(F.h_cb.p + 8, c->tx_n.p, 8, cudaMemcpyDeviceToHost, s));
+    if (c->tx_cache) CK(cudaMemcpyAsync(F.h_cb.p + 9, c->tx_miss_n.p, 8, cudaMemcpyDeviceToHost, s));
+    if (n) {
+        CK(cudaMemcpyAsync(F.hcb.idx, F.cb_idx.p, n * 4, cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(F.hcb.status, F.cb_st.p, n, cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(F.hcb.multi, F.cb_multi.p, n, cudaMemcpyDeviceToHost, s));
+    }
 }
 
 void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_reads *r2, const int32_t *lib_ids, int n_libs,
                  nb200_read_result *const *out_res, int32_t *const *out_feats, uint16_t *const *len1, uint16_t *const *len2,
-                 const uint64_t *key, const uint8_t *cb, const uint8_t *cb_qual, uint64_t seq) {
+                 const uint64_t *key, const CbSlab *cb, uint64_t seq) {
     nb200_ctx::FileLane &F = c->lane[lane];
     if (F.busy) throw std::runtime_error("lane is busy");
     if (key && c->rs.size() < (size_t)n_libs) throw std::runtime_error("counts mode without lane_rows_begin");
-    if (cb && (!key || !cb_qual || !c->tx_table.p)) throw std::runtime_error("barcodes without lane_cb_begin");
+    if (cb && (!cb->cb || !cb->qual || !cb->idx || !cb->status || !cb->multi || !c->tx_table.p))
+        throw std::runtime_error("barcodes without lane_cb_begin");
+    if (n_libs < (cb ? 0 : 1)) throw std::runtime_error("no library");
     validate_reads(r1, "r1");
     if (r2) { validate_reads(r2, "r2"); if (r2->n != r1->n) throw std::runtime_error("r1 and r2 differ in read count"); }
     const uint64_t n = r1->n;
@@ -1293,31 +1324,33 @@ void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_read
     if (out_res) F.out_res.assign(out_res, out_res + n_libs);
     if (out_feats) F.out_feats.assign(out_feats, out_feats + n_libs);
     F.hkey = key; F.n_rows_max = key ? n : 0;
-    F.hcb = cb; F.hcbq = cb_qual; F.seq = seq;
-    if (cb) F.h_cb.ensure(9);
+    F.hcb = cb ? *cb : CbSlab{}; F.has_cb = cb != nullptr; F.n_cb = cb ? n : 0; F.seq = seq;
+    if (cb) F.h_cb.ensure(10);
     if (key) F.h_seg.ensure(5 * (size_t)n_libs);
     F.hlen1.clear(); F.hlen2.clear();
     if (len1) F.hlen1.assign(len1, len1 + n_libs);
     if (len2 && r2) F.hlen2.assign(len2, len2 + n_libs);
     F.res.resize(std::max<size_t>(F.res.size(), (size_t)n_libs)); F.feats.resize(F.res.size()); F.nf.resize(F.res.size());
     const int n_mates = r2 ? 2 : 1, n_ro = n_mates * 2;
-    // reads up, once for all libraries
+    // reads up, once for all libraries (without a library: neither uploaded nor given device room)
     cudaStream_t sh = c->s_copy[0], sd = c->s_copy[1];
-    F.r1.ensure(n * (size_t)r1->stride + 64); F.l1.ensure(n * 2 + 16);
-    if (n) {
-        CK(cudaMemcpyAsync(F.r1.p, r1->packed, n * (size_t)r1->stride, cudaMemcpyHostToDevice, sh));
-        CK(cudaMemcpyAsync(F.l1.p, r1->len, n * 2, cudaMemcpyHostToDevice, sh));
-    }
     BatchIO io{};
-    io.r1 = ReadsDev{F.r1.as<uint8_t>(), F.l1.as<uint16_t>(), r1->stride, r1->words};
-    io.r2 = io.r1;
-    if (r2) {
-        F.r2.ensure(n * (size_t)r2->stride + 64); F.l2.ensure(n * 2 + 16);
+    if (n_libs) {
+        F.r1.ensure(n * (size_t)r1->stride + 64); F.l1.ensure(n * 2 + 16);
         if (n) {
-            CK(cudaMemcpyAsync(F.r2.p, r2->packed, n * (size_t)r2->stride, cudaMemcpyHostToDevice, sh));
-            CK(cudaMemcpyAsync(F.l2.p, r2->len, n * 2, cudaMemcpyHostToDevice, sh));
+            CK(cudaMemcpyAsync(F.r1.p, r1->packed, n * (size_t)r1->stride, cudaMemcpyHostToDevice, sh));
+            CK(cudaMemcpyAsync(F.l1.p, r1->len, n * 2, cudaMemcpyHostToDevice, sh));
         }
-        io.r2 = ReadsDev{F.r2.as<uint8_t>(), F.l2.as<uint16_t>(), r2->stride, r2->words};
+        io.r1 = ReadsDev{F.r1.as<uint8_t>(), F.l1.as<uint16_t>(), r1->stride, r1->words};
+        io.r2 = io.r1;
+        if (r2) {
+            F.r2.ensure(n * (size_t)r2->stride + 64); F.l2.ensure(n * 2 + 16);
+            if (n) {
+                CK(cudaMemcpyAsync(F.r2.p, r2->packed, n * (size_t)r2->stride, cudaMemcpyHostToDevice, sh));
+                CK(cudaMemcpyAsync(F.l2.p, r2->len, n * 2, cudaMemcpyHostToDevice, sh));
+            }
+            io.r2 = ReadsDev{F.r2.as<uint8_t>(), F.l2.as<uint16_t>(), r2->stride, r2->words};
+        }
     }
     if (key) {
         F.key.ensure(n * 8 + 16); F.seg.ensure(5 * 8 * (size_t)n_libs);
@@ -1327,8 +1360,8 @@ void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_read
         const size_t L = (size_t)c->tx_wl.cb_len;
         F.cb.ensure(n * L + 16); F.cbq.ensure(n * L + 16);
         if (n) {
-            CK(cudaMemcpyAsync(F.cb.p, cb, n * L, cudaMemcpyHostToDevice, sh));
-            CK(cudaMemcpyAsync(F.cbq.p, cb_qual, n * L, cudaMemcpyHostToDevice, sh));
+            CK(cudaMemcpyAsync(F.cb.p, cb->cb, n * L, cudaMemcpyHostToDevice, sh));
+            CK(cudaMemcpyAsync(F.cbq.p, cb->qual, n * L, cudaMemcpyHostToDevice, sh));
         }
     }
     if (len1 && n) {      // per-library lengths: all up before the first kernel
@@ -1342,6 +1375,7 @@ void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_read
     CK(cudaEventRecord(F.h2d_done, sh));
     CK(cudaStreamWaitEvent(c->s_compute, F.h2d_done, 0));
     if (cb) lane_cb_slab(c, F, n);                  // the keys are final before any library's rows are appended
+    if (!n_libs) { CK(cudaEventRecord(F.done, c->s_compute)); CK(cudaStreamWaitEvent(sd, F.done, 0)); }   // (barcodes only)
     nb200_ctx::BatchBuf &B = c->bb[lane];
     const uint64_t nbmax = std::max<uint64_t>(n, 1);
     for (int li = 0; li < n_libs; li++) {
@@ -1392,8 +1426,9 @@ void lane_wait(nb200_ctx *c, int lane) {
                 S.hi_rows = std::max<uint64_t>(S.hi_rows, s[0] + s[1]);
                 S.hi_ids = std::max<uint64_t>(S.hi_ids, s[2] + s[3]);
             }
-        if (F.hcb) {
+        if (F.has_cb) {
             c->tx_hi = std::max<uint64_t>(c->tx_hi, F.h_cb.p[8]);
+            if (c->tx_cache) c->tx_miss_hi = std::max<uint64_t>(c->tx_miss_hi, F.h_cb.p[9]);
             // a pair fastq-to-bam writes (barcode corrected) that it or align on its BAM refuses: CbCounters::pad
             const unsigned long long bad = F.h_cb.p[7];
             if (bad & kTenxLongName) throw std::runtime_error("read name longer than 254 bytes");
@@ -1411,9 +1446,10 @@ void lane_wait(nb200_ctx *c, int lane) {
         const std::vector<nb200_read_result *> orr = F.out_res;
         const std::vector<int32_t *> of = F.out_feats;
         const std::vector<uint16_t *> h1 = F.hlen1, h2 = F.hlen2;
+        const CbSlab cb = F.hcb;
         lane_submit(c, lane, &r1, F.paired ? &r2 : nullptr, libs.data(), (int)libs.size(), orr.empty() ? nullptr : orr.data(),
                     of.empty() ? nullptr : of.data(), h1.empty() ? nullptr : h1.data(), h2.empty() ? nullptr : h2.data(), F.hkey,
-                    F.hcb, F.hcbq, F.seq);
+                    F.has_cb ? &cb : nullptr, F.seq);
     }
 }
 
@@ -1600,17 +1636,18 @@ static std::unique_ptr<DevWhitelist> build_whitelist(nb200_ctx *c, std::vector<s
     return W;
 }
 
-// ---- fastq-to-counts: the whitelist on every context, the cache rule over every context's log (slab_api.hpp) ----------
-// the multi-candidate log back to empty, its buffers, outgrown buffers and decisions freed (current device: c's)
+// ---- 10x mode: the whitelist on every context, the cache rule over every context's log (slab_api.hpp) ----------------
+// the logs back to empty, their buffers, outgrown buffers, decisions and hit flags freed (current device: c's)
 static void reset_cb_log(nb200_ctx *c) {
-    for (DevBuf *b : {&c->tx_key, &c->tx_ord, &c->tx_choice, &c->tx_dec}) b->release();
-    c->tx_old.clear();
-    c->tx_cap = c->tx_hi = 0;
+    for (DevBuf *b : {&c->tx_key, &c->tx_ord, &c->tx_choice, &c->tx_dec, &c->tx_hit, &c->tx_miss}) b->release();
+    c->tx_old.clear(); c->tx_miss_old.clear();
+    c->tx_cap = c->tx_hi = c->tx_miss_cap = c->tx_miss_hi = 0;
     c->tx_base.clear();
+    c->tx_cache = false;
 }
 
 void lane_cb_begin(const std::vector<nb200_ctx *> &ctxs, const std::vector<std::string> &whitelist, int cb_len,
-                   std::vector<uint32_t> *rank, std::vector<std::string> *cells) {
+                   std::vector<uint32_t> *rank, std::vector<std::string> *cells, bool cache_size) {
     uint64_t n_unique = 0;
     const std::vector<WlSlot> tab = wl_slots(whitelist, cb_len, &n_unique);
     for (nb200_ctx *c : ctxs) {
@@ -1621,6 +1658,14 @@ void lane_cb_begin(const std::vector<nb200_ctx *> &ctxs, const std::vector<std::
         c->tx_wl = WlDev{c->tx_table.as<WlSlot>(), tab.size() - 1, cb_len};
         c->tx_n.ensure(8);
         CK(cudaMemset(c->tx_n.p, 0, 8));
+        c->tx_cache = cache_size;
+        c->tx_entries = whitelist.size();
+        if (cache_size) {
+            c->tx_hit.ensure(whitelist.size() + 16);
+            CK(cudaMemset(c->tx_hit.p, 0, whitelist.size() + 16));
+            c->tx_miss_n.ensure(8);
+            CK(cudaMemset(c->tx_miss_n.p, 0, 8));
+        }
     }
     CK(cudaSetDevice(ctxs[0]->device));
     // cells: the distinct lines in byte order (= key order), pandas-NA tokens left out (report drops such a cell)
@@ -1687,6 +1732,59 @@ void lane_cb_resolve(const std::vector<nb200_ctx *> &ctxs) {
     cub_sort64(c, ord.as<uint64_t>(), sorted.as<uint64_t>(), perm.as<uint32_t>() + E, perm.as<uint32_t>(), (uint32_t)E, 64);
     cb_first_decides(c, perm.as<uint32_t>(), key.as<uint64_t>(), (uint32_t)E, c->tx_dec.as<int32_t>());
     CK(cudaStreamSynchronize(s));
+}
+
+uint64_t lane_cb_cache_size(const std::vector<nb200_ctx *> &ctxs) {
+    nb200_ctx *c = ctxs[0];
+    if (!c->tx_cache) throw std::runtime_error("cache size without lane_cb_begin(cache_size)");
+    std::vector<uint64_t> cnt(ctxs.size());
+    for (size_t d = 0; d < ctxs.size(); d++) {
+        CK(cudaSetDevice(ctxs[d]->device));
+        CK(cudaStreamSynchronize(ctxs[d]->s_compute));
+        CK(cudaMemcpy(&cnt[d], ctxs[d]->tx_miss_n.p, 8, cudaMemcpyDeviceToHost));
+    }
+    CK(cudaSetDevice(c->device));
+    uint64_t M = 0;
+    for (uint64_t x : cnt) M += x;
+    if (M > 0x7FFFFFF0ull) throw LimitError("more than 2^31 reads whose cell barcode is not on the whitelist (CUB item counts are int)");
+    enable_peers(ctxs);
+    cudaStream_t s = c->s_compute;
+    const uint64_t E = c->tx_entries;
+    DevBuf other, keys, sorted, num;
+    num.ensure(8);
+    CK(cudaMemsetAsync(num.p, 0, 8, s));
+    if (ctxs.size() > 1) other.ensure(E + 16);
+    uint64_t at = 0;
+    if (M) keys.ensure(M * 8);
+    for (size_t d = 0; d < ctxs.size(); d++) {      // every context's hit flags or-ed into the first's, every miss log gathered
+        const nb200_ctx *x = ctxs[d];
+        auto copy = [&](void *dst, const void *src, size_t bytes) {
+            if (!bytes) return;
+            if (x->device == c->device) CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, s));
+            else CK(cudaMemcpyPeerAsync(dst, c->device, src, x->device, bytes, s));
+        };
+        if (d && E) {
+            copy(other.p, x->tx_hit.p, E);
+            cb_or_flags_kernel<<<nblk(E, 256), 256, 0, s>>>(other.as<uint8_t>(), E, c->tx_hit.as<uint8_t>());
+        }
+        copy(keys.as<uint64_t>() + at, x->tx_miss.p, cnt[d] * 8);
+        at += cnt[d];
+    }
+    if (E) cb_count_flags_kernel<<<nblk(E, 256), 256, 0, s>>>(c->tx_hit.as<uint8_t>(), E, num.as<unsigned long long>());
+    if (M) {
+        sorted.ensure(M * 8);
+        size_t bytes = 0;
+        const int bits = std::min(64, 3 * c->tx_wl.cb_len);
+        CK(cub::DeviceRadixSort::SortKeys(nullptr, bytes, keys.as<uint64_t>(), sorted.as<uint64_t>(), (int)M, 0, bits, s));
+        c->cub_tmp.ensure(bytes);
+        CK(cub::DeviceRadixSort::SortKeys(c->cub_tmp.p, bytes, keys.as<uint64_t>(), sorted.as<uint64_t>(), (int)M, 0, bits, s));
+        cb_count_distinct_kernel<<<nblk(M, 256), 256, 0, s>>>(sorted.as<uint64_t>(), M, num.as<unsigned long long>());
+    }
+    CK(cudaGetLastError());
+    unsigned long long d = 0;
+    CK(cudaMemcpyAsync(&d, num.p, 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    return d;
 }
 
 void lane_cb_end(const std::vector<nb200_ctx *> &ctxs) {
@@ -2305,61 +2403,23 @@ int32_t nb200_align(nb200_ctx *c, int32_t lib_id, const nb200_reads *r1, const n
     API_END(c)
 }
 
-// reads in memory (the 10x one-pass route) -> per library: GPU path -> per-read TSV
-static void align_readset(nb200_ctx *c, const ReadSet &R, const int32_t *lib_ids, const char *const *outputs, int32_t n_libs,
-                          PhaseTimer &pt) {
-    const uint64_t n = R.r1.size();
-    auto pack = [&](const Arena &a, std::vector<uint8_t> &buf, std::vector<uint16_t> &len, nb200_reads &out) {
-        int64_t ml = 1;
-        for (uint64_t i = 0; i < n; i++) ml = std::max<int64_t>(ml, a.off[i + 1] - a.off[i]);
-        if (ml > NB200_MAX_READ_LEN) throw std::runtime_error("read longer than 500 bases");
-        uint32_t words, stride;
-        nb200_pack_layout((uint32_t)ml, &words, &stride);
-        buf.assign(n * (size_t)stride + 64, 0); len.assign(n + 1, 0);
-        if (n && nb200_pack_reads(c, a.data.data(), a.off.data(), n, words, stride, buf.data(), len.data()) != 0)
-            throw std::runtime_error(c->err);
-        out = nb200_reads{buf.data(), len.data(), n, stride, words};
-    };
-    std::vector<uint8_t> b1, b2;
-    std::vector<uint16_t> l1, l2;
-    nb200_reads p1{}, p2{};
-    pack(R.r1, b1, l1, p1);
-    pack(R.r2, b2, l2, p2);
-    pt.lap("2-bit pack");
-    for (int li = 0; li < n_libs; li++) {
-        DevLibrary &L = get_lib(c, lib_ids[li]);
-        const int mh = L.host.cfg.max_hits_to_report;
-        std::vector<nb200_read_result> res(n + 1);
-        std::vector<int32_t> feats((n + 1) * (size_t)mh);
-        nb200_counts counts{};
-        ensure_read_buffers(c, &p1, &p2, false);
-        HostInput hin{&p1, &p2, nullptr};
-        run_align(c, L, &hin, 0.05, 0, &counts);
-        c->resident = true;
-        pt.lap("GPU align");
-        if (n) {
-            CK(cudaMemcpy(res.data(), c->results.p, n * sizeof(nb200_read_result), cudaMemcpyDeviceToHost));
-            CK(cudaMemcpy(feats.data(), c->feats.p, n * (size_t)mh * 4, cudaMemcpyDeviceToHost));
-        }
-        pt.lap("fetch per-read results");
-        write_per_read_tsv(outputs[li], R, res.data(), feats.data(), mh, L.host.feature_names, c->host_threads);
-        pt.lap("write TSV");
-    }
-}
-
 // values per library in the out3 of the counting entries: rows used, count rows written, UMIs dropped (+ UMIs corrected)
 static int out3_per_lib(int32_t umi_flags) { return (umi_flags & NB200_UMI_CORRECT) ? 4 : 3; }
 
 // File-level entries: what the aligner process does between its argv and its exit code (nimble/__main__.py:177-196),
 // streaming (stream.cpp).  One pass over `inputs` on the contexts `ctxs`, whose libraries carry the same ids in the same
-// order; per library a per-read TSV (outputs) and/or a counts TSV (counts_outputs).  whitelist: the 10x mode of
-// fastq-to-counts (inputs = raw R1 and R2), null otherwise.
+// order; per library a per-read TSV (outputs) and/or a counts TSV (counts_outputs).  whitelist: the 10x mode (inputs =
+// raw R1 and R2; fastq-to-bam, align --map, fastq-to-counts), null otherwise; bam_output: fastq-to-bam's BAM (10x mode,
+// may be the only output: n_libs 0); cache_size: compute fastq-to-bam's "Correction cache size" (10x mode).
 static FileStats run_job(const std::vector<nb200_ctx *> &ctxs, const int32_t *lib_ids, int32_t n_libs, const char *const *inputs,
                          int32_t n_inputs, const char *const *outputs, const char *const *counts_outputs, double umi_threshold,
-                         int32_t disable_thresholding, const char *whitelist, int32_t cb_len, int32_t umi_len) {
+                         int32_t disable_thresholding, const char *whitelist, int32_t cb_len, int32_t umi_len,
+                         const char *bam_output = nullptr, bool cache_size = false) {
     FileJob job;
     std::vector<std::string> wl;
     if (whitelist) { read_whitelist_lines(whitelist, wl); job.whitelist = &wl; job.cb_len = cb_len; job.umi_len = umi_len; }
+    if (bam_output) job.bam_output = bam_output;
+    job.cache_size = cache_size;
     job.inputs.assign(inputs, inputs + n_inputs);
     job.ctxs = ctxs;
     job.lib_ids.assign(lib_ids, lib_ids + n_libs);
@@ -2396,7 +2456,7 @@ static int32_t files_multi(const int32_t *devices, int32_t n_devices, int32_t ho
                            const char *const *library_json, int32_t n_libs, const char *strand_filter, int32_t k, const char *trim,
                            const char *const *outputs, const char *const *counts_outputs, double umi_threshold, int32_t disable_thresholding,
                            uint64_t *out3, char *err, size_t err_cap, double *stats4, const char *whitelist = nullptr, int32_t cb_len = 16,
-                           int32_t umi_len = 12, nb200_cb_stats *cb_stats = nullptr);
+                           int32_t umi_len = 12, nb200_cb_stats *cb_stats = nullptr, bool cache_size = false);
 
 int32_t nb200_align_files_multi(const int32_t *devices, int32_t n_devices, int32_t host_threads, const char *const *inputs, int32_t n_inputs,
                                 const char *const *library_json, int32_t n_libs, const char *strand_filter, int32_t k,
@@ -2434,7 +2494,7 @@ static int32_t files_multi(const int32_t *devices, int32_t n_devices, int32_t ho
                            const char *const *library_json, int32_t n_libs, const char *strand_filter, int32_t k, const char *trim,
                            const char *const *outputs, const char *const *counts_outputs, double umi_threshold, int32_t disable_thresholding,
                            uint64_t *out3, char *err, size_t err_cap, double *stats4, const char *whitelist, int32_t cb_len,
-                           int32_t umi_len, nb200_cb_stats *cb_stats) {
+                           int32_t umi_len, nb200_cb_stats *cb_stats, bool cache_size) {
     auto fail = [&](int32_t rc, const std::string &w) { if (err && err_cap) { snprintf(err, err_cap, "%s", w.c_str()); } return rc; };
     if (!devices || n_devices < 1 || !inputs || n_inputs < 1 || n_inputs > 2 || !library_json || n_libs < 1 || (!outputs && !counts_outputs))
         return fail(NB200_EINVAL, "bad arguments");
@@ -2469,7 +2529,7 @@ static int32_t files_multi(const int32_t *devices, int32_t n_devices, int32_t ho
     if (rc == NB200_OK) {
         try {
             const FileStats st = run_job(ctxs, ids.data(), n_libs, inputs, n_inputs, outputs, counts_outputs, umi_threshold,
-                                         disable_thresholding, whitelist, cb_len, umi_len);
+                                         disable_thresholding, whitelist, cb_len, umi_len, nullptr, cache_size);
             if (stats4) { stats4[0] = (double)st.n_reads; stats4[1] = st.seconds; stats4[2] = (double)st.called; stats4[3] = (double)st.n_slabs; }
             if (out3) for (size_t i = 0; i < st.counts3.size(); i++) out3[i] = st.counts3[i];
             if (cb_stats) *cb_stats = st.cb;
@@ -2514,64 +2574,39 @@ int32_t nb200_fastq_to_counts_multi(const int32_t *devices, int32_t n_devices, i
                        umi_threshold, disable_thresholding, out3, err, err_cap, stats4, whitelist_path, cb_len, umi_len, stats);
 }
 
-// fastq-to-bam + align without the intermediate BAM: the pairs fastq_to_bam_with_barcodes would write
-// (corrected CB, raw UB, read 1 = R1 minus barcode+UMI, read 2 = R2) go straight to the aligner.
+// fastq-to-bam + align without the intermediate BAM, streaming (stream.cpp, 10x mode): the pairs
+// fastq_to_bam_with_barcodes would write (corrected CB, raw UB, read 1 = R1 minus barcode+UMI, read 2 = R2) go straight to
+// the aligner, slab by slab.
 int32_t nb200_align_10x_fastq(nb200_ctx *c, const char *r1_fastq, const char *r2_fastq, const char *whitelist_path, int32_t cb_len,
                               int32_t umi_len, const int32_t *lib_ids, const char *const *outputs, int32_t n_libs,
                               nb200_cb_stats *stats) {
     API_BEGIN(c)
     if (!r1_fastq || !r2_fastq || !whitelist_path || !lib_ids || !outputs || n_libs < 1 || cb_len < 1 || umi_len < 0)
         throw std::runtime_error("bad arguments");
-    PhaseTimer pt;
-    nb200_cb_stats st{};
-    std::vector<std::string> lines;
-    read_whitelist_lines(whitelist_path, lines);
-    std::unique_ptr<DevWhitelist> W = build_whitelist(c, std::move(lines), cb_len);
-    FastqQ A, B;
-    {
-        std::string err;
-        std::thread t([&] { try { load_fastq_qual(r2_fastq, B); } catch (const std::exception &e) { err = e.what(); } });
-        try { load_fastq_qual(r1_fastq, A); } catch (...) { t.join(); throw; }
-        t.join();
-        if (!err.empty()) throw IoError(err);
-    }
-    pt.lap("whitelist + FASTQ parse");
-    const size_t n = std::min(A.recs.size(), B.recs.size());
-    std::vector<uint8_t> cb(n * (size_t)cb_len + 16), qual(n * (size_t)cb_len + 16), elig(n + 16);
-    slice_barcodes(A, B, cb_len, umi_len, c->host_threads, cb.data(), qual.data(), elig.data(), st);
-    std::vector<int32_t> idx(n + 1);
-    std::vector<uint8_t> status(n + 1);
-    nb200_cb_stats dev{};
-    cb_upload(c, cb_len, (const char *)cb.data(), qual.data(), elig.data(), n, &dev);
-    cb_run(c, *W, &dev);
-    cb_fetch(c, idx.data(), status.data(), &dev);
-    c->ev_pool.clear();
-    c->cb_resident = false;
-    dev.total_pairs = st.total_pairs; dev.name_mismatch = st.name_mismatch; dev.too_short = st.too_short;
-    dev.no_remaining_seq = st.no_remaining_seq;
-    pt.lap("barcode correction");
-    ReadSet R;
-    const uint32_t bl = (uint32_t)(cb_len + umi_len);
-    uint64_t written = 0;
-    for (size_t i = 0; i < n; i++) {
-        if (status[i] != NB200_CB_PERFECT && status[i] != NB200_CB_CORRECTED) continue;
-        const FqRec &x = A.recs[i], &y = B.recs[i];
-        const char *t1 = A.text.data(), *t2 = B.text.data();
-        uint32_t nl = x.name_len;
-        if (nl >= 2 && t1[x.name + nl - 2] == '/' && t1[x.name + nl - 1] == '1') nl -= 2;
-        const std::string &cbs = W->entries[(size_t)idx[i]];
-        R.names.add(t1 + x.name, nl);
-        R.r1.add(t1 + x.seq + bl, x.len - bl);
-        R.r2.add(t2 + y.seq, y.len);
-        R.cb.add(cbs.data(), cbs.size());
-        R.ub.add(t1 + x.seq + cb_len, (size_t)umi_len);
-        written++;
-    }
-    dev.written_pairs = written;
-    pt.lap("build read set");
-    align_readset(c, R, lib_ids, outputs, n_libs, pt);
-    if (stats) *stats = dev;
+    if (stats) *stats = nb200_cb_stats{};
+    const char *inputs[2] = {r1_fastq, r2_fastq};
+    const FileStats st = run_job({c}, lib_ids, n_libs, inputs, 2, outputs, nullptr, 0.05, 0, whitelist_path, cb_len, umi_len, nullptr, true);
+    if (stats) *stats = st.cb;
     API_END(c)
+}
+
+int32_t nb200_align_10x_fastq_multi(const int32_t *devices, int32_t n_devices, int32_t host_threads, const char *r1_fastq,
+                                    const char *r2_fastq, const char *whitelist_path, int32_t cb_len, int32_t umi_len,
+                                    const char *const *library_json, int32_t n_libs, const char *strand_filter, int32_t k,
+                                    const char *trim, const char *const *per_read_outputs, const char *const *counts_outputs,
+                                    double umi_threshold, int32_t disable_thresholding, uint64_t *out3, nb200_cb_stats *stats,
+                                    char *err, size_t err_cap, double *stats4) {
+    if (stats) *stats = nb200_cb_stats{};
+    if (!r1_fastq || !r2_fastq || !whitelist_path || (!per_read_outputs && !counts_outputs) || cb_len < 1 || cb_len > kCbMaxLen ||
+        umi_len < 0) {
+        if (err && err_cap) snprintf(err, err_cap, "bad arguments");
+        return NB200_EINVAL;
+    }
+    const char *inputs[2] = {r1_fastq, r2_fastq};
+    // with counts outputs this is fastq-to-counts with a per-read TSV: cache_size stays 0, as nb200_fastq_to_counts keeps it
+    return files_multi(devices, n_devices, host_threads, inputs, 2, library_json, n_libs, strand_filter, k, trim, per_read_outputs,
+                       counts_outputs, umi_threshold, disable_thresholding, out3, err, err_cap, stats4, whitelist_path, cb_len, umi_len,
+                       stats, counts_outputs == nullptr);
 }
 
 int32_t nb200_umi_counts(nb200_ctx *c, int32_t lib_id, uint64_t n_rows, const uint64_t *key, const uint32_t *off,
@@ -2985,42 +3020,16 @@ int32_t nb200_correct_barcodes(nb200_ctx *c, int32_t wl_id, const char *cb, cons
     API_END(c)
 }
 
+// streaming (stream.cpp, 10x mode without a library): the barcodes of each slab are corrected on the device, the BAM
+// records are built and compressed on the host's pool and written in file order
 int32_t nb200_fastq_to_bam(nb200_ctx *c, const char *r1_fastq, const char *r2_fastq, const char *whitelist_path,
                            const char *output_bam, int32_t cb_len, int32_t umi_len, nb200_cb_stats *stats) {
     API_BEGIN(c)
     if (!r1_fastq || !r2_fastq || !whitelist_path || !output_bam || cb_len < 1 || umi_len < 0) throw std::runtime_error("bad arguments");
-    nb200_cb_stats st{};
-    std::vector<std::string> lines;
-    read_whitelist_lines(whitelist_path, lines);
-    std::unique_ptr<DevWhitelist> W = build_whitelist(c, std::move(lines), cb_len);
-    FastqQ A, B;
-    {
-        std::string err;
-        std::thread t([&] { try { load_fastq_qual(r2_fastq, B); } catch (const std::exception &e) { err = e.what(); } });
-        try { load_fastq_qual(r1_fastq, A); } catch (...) { t.join(); throw; }
-        t.join();
-        if (!err.empty()) throw IoError(err);
-    }
-    const size_t n = std::min(A.recs.size(), B.recs.size());
-    std::vector<uint8_t> cb(n * (size_t)cb_len + 16), qual(n * (size_t)cb_len + 16), elig(n + 16);
-    slice_barcodes(A, B, cb_len, umi_len, c->host_threads, cb.data(), qual.data(), elig.data(), st);
-    std::vector<int32_t> idx(n + 1);
-    std::vector<uint8_t> status(n + 1);
-    nb200_cb_stats dev{};
-    cudaEvent_t e0 = new_event(c), e1 = new_event(c);
-    CK(cudaEventRecord(e0, c->s_compute));
-    cb_upload(c, cb_len, (const char *)cb.data(), qual.data(), elig.data(), n, &dev);
-    cb_run(c, *W, &dev);
-    cb_fetch(c, idx.data(), status.data(), &dev);
-    CK(cudaEventRecord(e1, c->s_compute));
-    CK(cudaEventSynchronize(e1));
-    CK(cudaEventElapsedTime(&dev.total_ms, e0, e1));
-    c->ev_pool.clear();
-    dev.total_pairs = st.total_pairs; dev.name_mismatch = st.name_mismatch; dev.too_short = st.too_short;
-    dev.no_remaining_seq = st.no_remaining_seq;
-    write_10x_bam(output_bam, A, B, cb_len, umi_len, idx.data(), status.data(), W->entries, c->host_threads, dev);
-    c->cb_resident = false;
-    if (stats) *stats = dev;
+    if (stats) *stats = nb200_cb_stats{};
+    const char *inputs[2] = {r1_fastq, r2_fastq};
+    const FileStats st = run_job({c}, nullptr, 0, inputs, 2, nullptr, nullptr, 0.05, 0, whitelist_path, cb_len, umi_len, output_bam, true);
+    if (stats) *stats = st.cb;
     API_END(c)
 }
 

@@ -11,7 +11,7 @@
 namespace nb200 {
 
 constexpr int kFileLanes = 2;
-// fastq-to-counts, host key of a pair before correction: flags in the high half, the UMI (or kTenxNaUmi) in the low half
+// 10x mode, host key of a pair before correction: flags in the high half, the UMI (or kTenxNaUmi) in the low half
 constexpr uint64_t kTenxLongRead = 1, kTenxLongName = 2;   // a read over 500 bases after the cut / a name over 254 bytes
 constexpr uint32_t kTenxNaUmi = 0xFFFFFFFFu;               // (UMI ids stay below it: umi_code < 2^31, interned < 2^32 - 1)
 
@@ -25,14 +25,21 @@ void lane_bind_thread(nb200_ctx *c);
 // out_res / out_feats may be null (counts only: no per-read results come back).
 // key (counts mode, after lane_rows_begin): per read cell << 32 | umi or NB200_NO_BARCODE, PINNED; it goes up with the
 // reads and every library's rows that count are appended to that library's row store on the device.
-// cb / cb_qual (fastq-to-counts, after lane_cb_begin): per read the raw cell barcode and its phred values (n x cb_len,
-// PINNED); key then holds flags << 32 | umi (kTenx*: umi kTenxNaUmi for a pandas-NA UMI), the device corrects the barcodes
-// and fills the cell half (barcode.cuh: cb_key_kernel).  A flagged read whose barcode is corrected makes lane_wait throw
-// (the two-step route fails on exactly those pairs).  seq: the slab's place in the file (the cache rule's order).
+// cb (10x mode, after lane_cb_begin): the slab's raw cell barcodes; the device corrects them and copies each pair's
+// correction back into cb's PINNED out buffers (read them after lane_wait).  With key (counts mode) key holds flags << 32 |
+// umi on entry (kTenx*: umi kTenxNaUmi for a pandas-NA UMI) and the device fills the cell half (barcode.cuh:
+// cb_key_kernel); a flagged read whose barcode is corrected makes lane_wait throw (the two-step route fails on exactly
+// those pairs).  n_libs == 0 (fastq-to-bam): only the barcodes go up and are corrected, the reads are not uploaded.
+// seq: the slab's place in the file (the cache rule's order).
+struct CbSlab {
+    const uint8_t *cb = nullptr, *qual = nullptr;  // in: n x cb_len raw bases / phred values
+    int32_t *idx = nullptr;                        // out: whitelist line, or -1 (the device's own choice for a read with
+    uint8_t *status = nullptr;                     //      several candidates: the host's resolve step decides those)
+    uint8_t *multi = nullptr;                      // out: NB200_CB_* / 1 = several candidates
+};
 void lane_submit(nb200_ctx *c, int lane, const nb200_reads *r1, const nb200_reads *r2, const int32_t *lib_ids, int n_libs,
                  nb200_read_result *const *out_res, int32_t *const *out_feats, uint16_t *const *len1 = nullptr,
-                 uint16_t *const *len2 = nullptr, const uint64_t *key = nullptr, const uint8_t *cb = nullptr,
-                 const uint8_t *cb_qual = nullptr, uint64_t seq = 0);
+                 uint16_t *const *len2 = nullptr, const uint64_t *key = nullptr, const CbSlab *cb = nullptr, uint64_t seq = 0);
 // --trim setting of a library (nb200_library_set_trim); false = none
 bool lane_trim(nb200_ctx *c, int32_t lib_id, int *target, double *strictness);
 // Block until the slab of this lane is done and its outputs are in the host buffers (re-runs it with a larger
@@ -69,17 +76,20 @@ void lane_rows_count(const std::vector<nb200_ctx *> &ctxs, int li, int32_t lib_i
                      const std::vector<uint32_t> &cell_rank, double threshold, int umi_flags, nb200_counts *counts, uint64_t *rows,
                      bool tenx = false);
 
-// ---- fastq-to-counts: cell barcodes corrected slab by slab, the correction cache over the whole call ------------
+// ---- 10x mode: cell barcodes corrected slab by slab, the correction cache over the whole call ---------------------
 // Upload the whitelist table to every context and empty their logs of reads with several candidates.  rank[i] = rank
 // of whitelist line i among the distinct lines in byte order, ~0u for a line that can never match or is a pandas NA
-// token (report drops such a cell); cells[rank] = the line.
+// token (report drops such a cell); cells[rank] = the line.  cache_size: also keep what lane_cb_cache_size counts.
 void lane_cb_begin(const std::vector<nb200_ctx *> &ctxs, const std::vector<std::string> &whitelist, int cb_len,
-                   std::vector<uint32_t> *rank, std::vector<std::string> *cells);
+                   std::vector<uint32_t> *rank, std::vector<std::string> *cells, bool cache_size = false);
 // After lane_wait: the slab's perfect matches, corrections, no-corrections, exact misses, multi-candidate reads, probes.
 void lane_cb_counters(nb200_ctx *c, int lane, uint64_t *out6);
 // After the last slab: the first read (in file order) of each raw barcode among the logged ones decides for all of them
 // (the reference's correction_cache, DESIGN.md §2.8); the decisions stay on ctxs[0] for lane_rows_count.
 void lane_cb_resolve(const std::vector<nb200_ctx *> &ctxs);
+// After the last slab (lane_cb_begin with cache_size): distinct raw barcodes of the call made of ACGTN only = whitelist
+// entries hit exactly on any context + distinct raw barcodes among the exact misses of every context.
+uint64_t lane_cb_cache_size(const std::vector<nb200_ctx *> &ctxs);
 // Free the whitelist tables and logs of the call.
 void lane_cb_end(const std::vector<nb200_ctx *> &ctxs);
 

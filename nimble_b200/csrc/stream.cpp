@@ -10,11 +10,14 @@
 //                         slab's buffers (page-locked in the background, cached across calls), --trim lengths per library;
 //                         format task: per-read rows -> text (gzip member for .gz outputs)
 //   one thread per GPU    two slabs in flight (slab_api.hpp): H2D, kernels, D2H overlap across slabs
+//   resolver thread       10x mode: slabs in input order, the cell barcode of every pair final (resolve_slab)
 //   committer thread      writes the formatted slabs in input order, merges bulk tables, recycles slabs
 //
 // Memory is bounded by the slab pool and by the number of inflated chunks in flight, not by the file size.
-// 10x mode (nb200_fastq_to_counts): raw R1 / R2 FASTQ; the parse task keeps the pairs fastq-to-bam would correct
-// (tenx_select) and the GPU threads correct their barcodes slab by slab (slab_api.hpp: lane_cb_*).
+// 10x mode (fastq-to-bam, align --map, fastq-to-counts): raw R1 / R2 FASTQ; the parse task keeps the pairs fastq-to-bam
+// would correct (tenx_select), the GPU threads correct their barcodes slab by slab (slab_api.hpp: lane_cb_*), the
+// resolver applies the cache rule in file order, the format tasks write BAM records and per-read rows of the pairs
+// fastq-to-bam writes.  Neither the GPU threads nor the slab pool ever wait on the two ordered points.
 #include "stream.hpp"
 
 #include <zlib.h>
@@ -35,6 +38,7 @@
 #include <string_view>
 #include <thread>
 #include <unordered_map>
+#include <unordered_set>
 
 #include "fast_inflate.hpp"
 #include "ingest.hpp"
@@ -69,9 +73,14 @@ struct Abort {
     std::mutex m;
     std::string what;
     bool io = false;
+    std::function<void()> wake;                  // called once, when the flag goes up (a thread that waits for order)
     void set(const std::string &w, bool is_io = false) {
-        std::lock_guard<std::mutex> g(m);
-        if (!flag.exchange(true)) { what = w; io = is_io; }
+        bool first = false;
+        {
+            std::lock_guard<std::mutex> g(m);
+            if (!flag.exchange(true)) { what = w; io = is_io; first = true; }
+        }
+        if (first && wake) wake();
     }
 };
 
@@ -484,6 +493,17 @@ struct Slab {
     uint8_t *cbc = nullptr, *cbq = nullptr;
     uint64_t pairs = 0, name_mismatch = 0, too_short = 0, no_remaining_seq = 0;
     uint64_t cbn[6] = {0, 0, 0, 0, 0, 0};                                // lane_cb_counters
+    // 10x mode: per pair its correction (CbSlab's out buffers; cbi final after resolve_slab), the UMI (ub), the pairs
+    // fastq-to-bam writes; BAM output: R1 after barcode and UMI, its qualities, R2, its qualities back to back per pair
+    // (FASTQ text) and R1's length, then the slab's records in BGZF blocks; cache size: the raw barcodes with a byte
+    // outside ACGTN
+    int32_t *cbi = nullptr;
+    uint8_t *cbs = nullptr, *cbm = nullptr;
+    uint64_t written = 0;
+    StrCol rec;
+    std::vector<uint32_t> len1;
+    std::string bam;
+    std::vector<std::string> inval;
 };
 
 // ---- counts mode: CB / UB strings -> key = cell << 32 | umi -------------------------------------------------------
@@ -589,6 +609,8 @@ struct Task {
     const std::vector<TrimTable> *trims = nullptr;   // per library (--trim), or nullptr
     BarcodeDict *bc = nullptr;                   // counts mode
     int cb_len = 0, umi_len = 0;                 // 10x mode when cb_len > 0 (tenx_select)
+    bool libs = true;                            // 10x mode: reads go to libraries (else barcodes only: nothing packed)
+    bool bam_text = false, inval = false;        // 10x mode: keep what the BAM records need / non-ACGTN raw barcodes
     std::string qconv;                           // 10x mode with --trim: the qualities as fastq-to-bam's BAM stores them
 };
 
@@ -721,8 +743,9 @@ static void pack_ascii(const char *s, uint32_t L, uint8_t *rec, uint32_t words, 
 }
 
 // 10x mode, first step of the parse task: keep the pairs fastq-to-bam would hand to the barcode correction
-// (process_pair's rules, slice_barcodes) and turn each into what that BAM's records hold: raw CB + phred values into the
-// slab, the UMI into the key's low half, read 1 = R1 after barcode and UMI, read 2 = R2.  The rest is counted.
+// (process_pair's rules) and turn each into what that BAM's records hold: raw CB + phred values into the slab, the UMI
+// into the key's low half and the slab's UB column, the name without /1, read 1 = R1 after barcode and UMI, read 2 = R2.
+// The rest is counted.
 static void tenx_select(Task &t) {
     Slab &S = *t.slab;
     const uint32_t L = (uint32_t)t.cb_len, U = (uint32_t)t.umi_len, bl = L + U;
@@ -741,22 +764,38 @@ static void tenx_select(Task &t) {
         return (n && (uint8_t)t.qconv[at] == 0xFF) ? nullptr : t.qconv.data() + at;
     };
     S.pairs = t.e.size(); S.name_mismatch = S.too_short = S.no_remaining_seq = 0;
+    S.ub.reset(t.e.size());
+    S.inval.clear();
+    if (t.bam_text) { S.rec.reset(t.e.size()); S.len1.clear(); }
     size_t o = 0;
     for (size_t i = 0; i < t.e.size(); i++) {
         Entry e = t.e[i];
         if (!name_eq_stripped(e.name, e.ln, e.name2, e.ln2)) { S.name_mismatch++; continue; }
         if (e.la < bl) { S.too_short++; continue; }
         if (e.la == bl) { S.no_remaining_seq++; continue; }
-        // what writing the BAM (a name over 254 bytes) or aligning it (a read over 500 bases) refuses: the two steps fail
-        // only when the pair is written, i.e. its barcode gets a correction, so the device decides (cb_key_kernel).  The
-        // pair still takes part in the correction and its cache rule; an over-long read goes to the kernels empty.
-        uint32_t nl = e.ln;
-        if (nl >= 2 && e.name[nl - 2] == '/' && e.name[nl - 1] == '1') nl -= 2;
-        const uint64_t flags = (nl > 254 ? kTenxLongName : 0) | ((e.la - bl > NB200_MAX_READ_LEN || e.lb > NB200_MAX_READ_LEN) ? kTenxLongRead : 0);
+        // what writing the BAM (a name over 254 bytes) or aligning it (a read over 500 bases; fastq-to-bam alone writes any
+        // length) refuses: the steps fail only when the pair is written, i.e. its barcode gets a correction, so the
+        // resolve step decides (and in counts mode also cb_key_kernel).  The pair still takes part in the correction and
+        // its cache rule; an over-long read goes to the kernels empty.
+        if (e.ln >= 2 && e.name[e.ln - 2] == '/' && e.name[e.ln - 1] == '1') e.ln -= 2;
+        const bool long_read = t.libs && (e.la - bl > NB200_MAX_READ_LEN || e.lb > NB200_MAX_READ_LEN);
+        const uint64_t flags = (e.ln > 254 ? kTenxLongName : 0) | (long_read ? kTenxLongRead : 0);
         memcpy(S.cbc + o * L, e.a, L);
         for (uint32_t j = 0; j < L; j++) S.cbq[o * L + j] = (uint8_t)(e.qa[j] - 33);
+        if (t.inval)
+            for (uint32_t j = 0; j < L; j++)
+                if (!strchr("ACGTN", e.a[j]) || !e.a[j]) { S.inval.emplace_back(e.a, L); break; }
         const std::string_view umi(e.a + L, U);
-        S.key[o] = (flags << 32) | (pandas_na(umi) ? kTenxNaUmi : umi_id(umi, *t.bc, umis));
+        S.ub.add(umi.data(), U);
+        // the UMI half is read by the counts only (cb_key_kernel); without counts the UMI stays text (S.ub)
+        const uint32_t umi_key = !t.bc ? 0u : pandas_na(umi) ? kTenxNaUmi : umi_id(umi, *t.bc, umis);
+        S.key[o] = (flags << 32) | umi_key;
+        if (t.bam_text) {
+            S.rec.data.append(e.a + bl, e.la - bl); S.rec.data.append(e.qa + bl, e.la - bl);
+            S.rec.data.append(e.b, e.lb); S.rec.add(e.qb, e.lb);
+            S.len1.push_back(e.la - bl);
+            if (S.rec.data.size() > 0xFFFFFFFFull) throw std::runtime_error("reads of one slab longer than 4 GB in all");   // (StrCol offsets)
+        }
         if (want_q) { e.qa = bam_qual(e.qa + bl, e.la - bl); e.qb = bam_qual(e.qb, e.lb); }
         e.a += bl; e.la -= bl;
         if (flags & kTenxLongRead) { e.la = 0; e.lb = 0; }
@@ -770,11 +809,12 @@ static void parse_task(Task &t) {
     if (t.cb_len) tenx_select(t);
     Slab &S = *t.slab;
     const size_t n = t.segs.empty() ? t.e.size() : t.n_seg_records;
-    S.n = n; S.paired = t.paired; S.has_tags = t.bam;
+    S.n = n; S.paired = t.paired; S.has_tags = t.bam || t.cb_len;
     uint32_t w1 = std::max(1u, (t.max1 + 31) / 32), s1 = stride_for(t.max1), w2 = std::max(1u, (t.max2 + 31) / 32), s2 = stride_for(t.max2);
     S.r1 = nb200_reads{S.p1, S.l1, n, s1, w1};
     S.r2 = nb200_reads{S.p2, S.l2, n, s2, w2};
-    S.names.reset(n); S.cb.reset(n); S.ub.reset(n); S.ur.reset(n); S.gn.reset(n);
+    S.names.reset(n); S.cb.reset(n); S.ur.reset(n); S.gn.reset(n);
+    if (!t.cb_len) S.ub.reset(n);
     S.pos1.assign(n, -1); S.pos2.assign(n, -1);
     S.bases1 = S.bases2 = 0;
     const bool trimming = t.trims && !S.lt1.empty();
@@ -829,6 +869,7 @@ static void parse_task(Task &t) {
             }
         } else {
             S.names.add(e.name, e.ln);
+            if (!t.libs) continue;
             pack_ascii(e.a, e.la, S.p1 + i * (size_t)s1, w1, s1); S.l1[i] = (uint16_t)e.la; S.bases1 += e.la;
             if (t.paired) { pack_ascii(e.b, e.lb, S.p2 + i * (size_t)s2, w2, s2); S.l2[i] = (uint16_t)e.lb; S.bases2 += e.lb; }
         }
@@ -871,8 +912,11 @@ static inline void put_uint(std::string &o, uint64_t v) {
     while (n) o.push_back(b[--n]);
 }
 
-// rows of one slab for one library (runs on the pool)
-static void format_slab(Slab &S, size_t li, const LibOut &lo) {
+static inline bool tenx_written(const Slab &S, size_t i) { return S.cbs[i] == NB200_CB_PERFECT || S.cbs[i] == NB200_CB_CORRECTED; }
+
+// rows of one slab for one library (runs on the pool).  10x mode (wl: the whitelist lines): the pairs fastq-to-bam
+// writes, as align writes the rows of its BAM: corrected CB, raw UMI as UB, no UR, GN or positions.
+static void format_slab(Slab &S, size_t li, const LibOut &lo, const std::vector<std::string> *wl) {
     const size_t n = S.n;
     const nb200_read_result *res = S.res[li];
     const int32_t *feats = S.feats[li];
@@ -881,7 +925,7 @@ static void format_slab(Slab &S, size_t li, const LibOut &lo) {
     if (S.has_tags) {
         text.reserve(n * 48);
         for (size_t i = 0; i < n; i++) {
-            if (!res[i].n_feat) continue;
+            if (!res[i].n_feat || (wl && !tenx_written(S, i))) continue;
             S.called += li == 0;
             for (int j = 0; j < res[i].n_feat; j++) {
                 if (j) text += ',';
@@ -891,6 +935,13 @@ static void format_slab(Slab &S, size_t li, const LibOut &lo) {
             text += "\t1";
             for (int o = 0; o < 4; o++) { text += '\t'; put_uint(text, res[i].score[o]); }
             text += '\t'; text.append(S.names.ptr(i), S.names.len(i));
+            if (wl) {
+                const std::string &cb = (*wl)[(size_t)S.cbi[i]];
+                text += '\t'; text += cb;
+                text += '\t'; text.append(S.ub.ptr(i), S.ub.len(i));
+                text += "\t\t\t\t\n";
+                continue;
+            }
             text += '\t'; text.append(S.cb.ptr(i), S.cb.len(i));
             text += '\t'; text.append(S.ub.ptr(i), S.ub.len(i));
             text += '\t'; text.append(S.ur.ptr(i), S.ur.len(i));
@@ -911,6 +962,22 @@ static void format_slab(Slab &S, size_t li, const LibOut &lo) {
             m[key]++;
         }
     }
+}
+
+// 10x mode: the BAM records of the pairs of one slab that fastq-to-bam writes, in BGZF blocks (runs on the pool)
+static void format_bam(Slab &S, const std::vector<std::string> &wl, int umi_len) {
+    std::string raw;
+    const uint32_t U = (uint32_t)umi_len;
+    for (size_t i = 0; i < S.n; i++) {
+        if (!tenx_written(S, i)) continue;
+        const std::string &cb = wl[(size_t)S.cbi[i]];
+        const char *r = S.rec.ptr(i), *name = S.names.ptr(i), *umi = S.ub.ptr(i);
+        const uint32_t l1 = S.len1[i], l2 = (uint32_t)(S.rec.len(i) - 2 * (size_t)l1) / 2, nl = (uint32_t)S.names.len(i);
+        bam_record(raw, name, nl, 77, r, r + l1, l1, cb.data(), (uint32_t)cb.size(), umi, U);
+        bam_record(raw, name, nl, 141, r + 2 * (size_t)l1, r + 2 * (size_t)l1 + l2, l2, cb.data(), (uint32_t)cb.size(), umi, U);
+    }
+    S.bam.clear();
+    bgzf_blocks(raw, S.bam);
 }
 
 // ---- the pipeline -----------------------------------------------------------------------------------------
@@ -936,6 +1003,13 @@ struct Pipeline {
     bool counts = false;                           // counts TSVs: keys per read, rows kept on the devices
     bool tenx = false;                             // raw 10x R1 / R2 in, cell barcodes corrected on the devices (FileJob)
     BarcodeDict bc;
+    // 10x mode: the ordered resolve step (resolver thread), fastq-to-bam's BAM, the cache size's non-ACGTN barcodes
+    Channel<Slab *> to_resolve;
+    std::thread resolver;
+    std::unordered_map<uint64_t, int32_t> first_choice;      // raw barcode (3-bit code) with several candidates -> line
+    FILE *bam_f = nullptr;
+    std::string bam_tmp;
+    std::unordered_set<std::string> inval;
     std::mutex seg_m;
     std::vector<std::vector<RowSeg>> segs;         // counts mode, per library: the segments of every slab on every context
     uint64_t tagged = 0;
@@ -954,8 +1028,11 @@ struct Pipeline {
             S->res.push_back((nb200_read_result *)S->grab(kSlabReads * sizeof(nb200_read_result) + 64));
             S->feats.push_back((int32_t *)S->grab(kSlabReads * (size_t)libs[li].max_hits * 4 + 64));
         }
-        if (counts) S->key = (uint64_t *)S->grab(kSlabReads * 8 + 64);
-        if (tenx) { S->cbc = (uint8_t *)S->grab(kSlabReads * (size_t)job.cb_len + 64); S->cbq = (uint8_t *)S->grab(kSlabReads * (size_t)job.cb_len + 64); }
+        if (counts || tenx) S->key = (uint64_t *)S->grab(kSlabReads * 8 + 64);
+        if (tenx) {
+            S->cbc = (uint8_t *)S->grab(kSlabReads * (size_t)job.cb_len + 64); S->cbq = (uint8_t *)S->grab(kSlabReads * (size_t)job.cb_len + 64);
+            S->cbi = (int32_t *)S->grab(kSlabReads * 4 + 64); S->cbs = (uint8_t *)S->grab(kSlabReads + 64); S->cbm = (uint8_t *)S->grab(kSlabReads + 64);
+        }
         if (!trims.empty())
             for (size_t li = 0; li < n_libs; li++) S->lt1.push_back((uint16_t *)S->grab(kSlabReads * 2 + 64));
         S->out.resize(n_libs); S->bulk.resize(n_libs);
@@ -1017,17 +1094,69 @@ struct Pipeline {
 
     // a parsed slab goes to a GPU (or straight to the committer in a dry run)
     void after_parse(Slab *S) { if (dry) to_commit.push(S); else to_gpu.push(S); }
-    // a slab with results: format every library's rows on the pool, then commit
+    // a slab with results: (10x mode: through the resolve step first) format every library's rows and the BAM records on
+    // the pool, then commit
     void after_gpu(Slab *S) {
-        if (!per_read) { to_commit.push(S); return; }
-        auto left = std::make_shared<std::atomic<size_t>>(libs.size());
-        for (size_t li = 0; li < libs.size(); li++)
-            pool->push(Pool::FORMAT, [this, S, li, left] {
+        if (tenx) to_resolve.push(S); else format(S);
+    }
+    void format(Slab *S) {
+        const size_t nl = per_read ? libs.size() : 0, tasks = nl + (bam_f ? 1 : 0);
+        if (!tasks) { to_commit.push(S); return; }
+        auto left = std::make_shared<std::atomic<size_t>>(tasks);
+        for (size_t li = 0; li < tasks; li++)
+            pool->push(Pool::FORMAT, [this, S, li, nl, left] {
                 const double t_in = now_s();
-                try { if (!ab.flag) format_slab(*S, li, libs[li]); } catch (const std::exception &e) { ab.set(e.what()); }
+                try {
+                    if (!ab.flag) {
+                        if (li < nl) format_slab(*S, li, libs[li], job.whitelist);
+                        else format_bam(*S, *job.whitelist, job.umi_len);
+                    }
+                } catch (const std::exception &e) { ab.set(e.what()); }
                 g_ns_format += (uint64_t)((now_s() - t_in) * 1e9);
                 if (left->fetch_sub(1) == 1) to_commit.push(S);
             });
+    }
+
+    // 10x mode: each slab's pairs in file order.  A pair with several candidates takes the line the first such pair with
+    // its raw barcode took, in this call (DESIGN.md §2.8, §2.11); a pair fastq-to-bam writes that it or align on its BAM
+    // refuses fails the call.  The raw barcode of such a pair is ACGTN only and at most kCbMaxLen (21) bases: 3 bits a base.
+    void resolve_slab(Slab &S) {
+        static const struct Code { uint8_t c[256]; Code() { memset(c, 7, sizeof c); c['A'] = 0; c['C'] = 1; c['G'] = 2; c['N'] = 3; c['T'] = 4; } } code;
+        const size_t L = (size_t)job.cb_len;
+        S.written = 0;
+        for (size_t i = 0; i < S.n; i++) {
+            if (!tenx_written(S, i)) continue;
+            if (S.cbm[i]) {
+                uint64_t k = 0;
+                for (size_t j = 0; j < L; j++) k = (k << 3) | code.c[S.cbc[i * L + j]];
+                S.cbi[i] = first_choice.emplace(k, S.cbi[i]).first->second;
+            }
+            const uint64_t fl = S.key[i] >> 32;
+            if (fl & kTenxLongName) throw std::runtime_error("read name longer than 254 bytes");
+            if (fl & kTenxLongRead) throw std::runtime_error("read longer than 500 bases");
+            S.written++;
+        }
+    }
+    void resolve_main() {
+        std::map<uint64_t, Slab *> pending;
+        uint64_t next = 0;
+        Slab *S = nullptr;
+        while (to_resolve.pop(S)) {                       // (nullptr: the abort flag went up)
+            if (S) pending[S->seq] = S;
+            if (ab.flag) {                                // slabs of a failed call go back unordered
+                for (auto &kv : pending) to_commit.push(kv.second);
+                pending.clear();
+                continue;
+            }
+            while (!pending.empty() && pending.begin()->first == next) {
+                Slab *T = pending.begin()->second;
+                pending.erase(pending.begin());
+                next++;
+                try { resolve_slab(*T); } catch (const std::exception &e) { ab.set(e.what()); to_commit.push(T); continue; }
+                format(T);
+            }
+        }
+        for (auto &kv : pending) to_commit.push(kv.second);
     }
 
     void gpu_main(nb200_ctx *c, int ctx_index) {
@@ -1057,10 +1186,11 @@ struct Pipeline {
                 if (fly[lane]) finish(lane);
                 fly[lane] = S;
                 const double t_in = now_s();
+                const CbSlab cbs{S->cbc, S->cbq, S->cbi, S->cbs, S->cbm};
                 lane_submit(c, lane, &S->r1, S->paired ? &S->r2 : nullptr, job.lib_ids.data(), (int)job.lib_ids.size(),
                             S->res.empty() ? nullptr : S->res.data(), S->feats.empty() ? nullptr : S->feats.data(),
                             S->lt1.empty() ? nullptr : S->lt1.data(), (S->paired && !S->lt2.empty()) ? S->lt2.data() : nullptr,
-                            counts ? S->key : nullptr, tenx ? S->cbc : nullptr, tenx ? S->cbq : nullptr, S->seq);
+                            counts ? S->key : nullptr, tenx ? &cbs : nullptr, S->seq);
                 g_ns_gpu_submit += (uint64_t)((now_s() - t_in) * 1e9);
                 lane ^= 1;
             }
@@ -1107,6 +1237,13 @@ struct Pipeline {
                             }
                             std::string().swap(T->out[li]);
                         }
+                        if (bam_f && !T->bam.empty()) {
+                            const double t_in = now_s();
+                            if (fwrite(T->bam.data(), 1, T->bam.size(), bam_f) != T->bam.size()) throw IoError("write failed: " + bam_tmp);
+                            g_ns_write += (uint64_t)((now_s() - t_in) * 1e9);
+                        }
+                        std::string().swap(T->bam);
+                        for (std::string &x : T->inval) inval.insert(std::move(x));
                         stats.n_reads += T->n; stats.bases1 += T->bases1; stats.bases2 += T->bases2; stats.called += T->called;
                         stats.paired |= T->paired; stats.has_tags |= T->has_tags; stats.n_slabs++;
                         tagged += T->tagged;
@@ -1116,7 +1253,7 @@ struct Pipeline {
                             c.no_remaining_seq += T->no_remaining_seq;
                             c.cb_perfect_match += T->cbn[0]; c.cb_corrected += T->cbn[1]; c.cb_no_correction += T->cbn[2];
                             c.n_exact_miss += T->cbn[3]; c.n_multi += T->cbn[4]; c.probes += T->cbn[5];
-                            c.written_pairs += T->cbn[0] + T->cbn[1];
+                            c.written_pairs += T->written;
                         }
                         if (dry && !getenv("NB200_INGEST_NOSUM"))      // reader statistics (nb200_host_ingest_stats): FNV-1a over every field of every read
                             for (size_t i = 0; i < T->n; i++) {
@@ -1149,7 +1286,10 @@ struct Pipeline {
         t->slab = S;
         t->trims = trims.empty() ? nullptr : &trims;
         t->bc = counts ? &bc : nullptr;
-        if (tenx) { t->cb_len = job.cb_len; t->umi_len = job.umi_len; }
+        if (tenx) {
+            t->cb_len = job.cb_len; t->umi_len = job.umi_len;
+            t->libs = !job.lib_ids.empty(); t->bam_text = bam_f != nullptr; t->inval = job.cache_size;
+        }
         pool->push(Pool::PARSE, [this, t] {
             const double t_in = now_s();
             try { parse_task(*t); } catch (...) { to_commit.push(t->slab); throw; }
@@ -1432,9 +1572,10 @@ namespace nb200 {
 
 void run_file_pipeline(const FileJob &job, FileStats *stats_out) {
     if (job.inputs.empty() || job.inputs.size() > 2) throw std::runtime_error("expected one or two --input files");
-    const bool counts = !job.counts_outputs.empty();
-    if (!job.ctxs.empty() && (job.lib_ids.empty() || (!job.outputs.empty() && job.lib_ids.size() != job.outputs.size()) ||
-                              (job.outputs.empty() && !counts) || (counts && job.counts_outputs.size() != job.lib_ids.size())))
+    const bool counts = !job.counts_outputs.empty(), bam_out = !job.bam_output.empty();
+    const bool lib_out = !job.outputs.empty() || counts;       // libraries are aligned against iff they have an output
+    if (!job.ctxs.empty() && (job.lib_ids.empty() == lib_out || (!job.outputs.empty() && job.lib_ids.size() != job.outputs.size()) ||
+                              (counts && job.counts_outputs.size() != job.lib_ids.size()) || (!lib_out && !bam_out)))
         throw std::runtime_error("bad arguments");
     const auto t0 = std::chrono::steady_clock::now();
     Pipeline P(job);
@@ -1442,8 +1583,9 @@ void run_file_pipeline(const FileJob &job, FileStats *stats_out) {
     P.counts = counts && !P.dry;
     P.per_read = !job.outputs.empty();
     P.tenx = job.whitelist != nullptr;
-    if (P.tenx && (!P.counts || P.per_read || job.inputs.size() != 2 || job.umi_len < 0))
+    if ((P.tenx && (P.dry || job.inputs.size() != 2 || job.umi_len < 0)) || ((bam_out || job.cache_size) && !P.tenx))
         throw std::runtime_error("bad arguments");
+    P.ab.wake = [&P] { P.to_resolve.push(nullptr); };
     g_wait_block = g_wait_slab = 0.0;
     g_ns_inflate = 0; g_ns_parse = 0; g_ns_format = 0; g_ns_gpu_wait = 0; g_ns_gpu_submit = 0; g_ns_write = 0; g_ns_intern = 0;
     double t_alloc = 0.0, t_walk = 0.0, t_drain = 0.0, t_finish = 0.0, t_free = 0.0, t_counts = 0.0;
@@ -1460,7 +1602,7 @@ void run_file_pipeline(const FileJob &job, FileStats *stats_out) {
     std::vector<uint32_t> wl_rank;                     // 10x mode: whitelist line -> cell rank (lane_cb_begin)
     std::vector<std::string> wl_cells;
     struct CbEnd { const FileJob &j; bool on; ~CbEnd() { if (on) try { lane_cb_end(j.ctxs); } catch (...) {} } } cb_end{job, P.tenx};
-    if (P.tenx) lane_cb_begin(job.ctxs, *job.whitelist, job.cb_len, &wl_rank, &wl_cells);
+    if (P.tenx) lane_cb_begin(job.ctxs, *job.whitelist, job.cb_len, &wl_rank, &wl_cells, job.cache_size);
     // outputs
     for (size_t li = 0; li < (P.dry ? 0 : job.lib_ids.size()); li++) {
         LibOut lo;
@@ -1490,13 +1632,21 @@ void run_file_pipeline(const FileJob &job, FileStats *stats_out) {
             if (!P.per_read) break;
             lo.f = fopen(lo.tmp.c_str(), "wb");
             if (!lo.f) throw IoError("cannot write " + lo.tmp);
-            if (bam) {                                      // per-read TSV: the header leads (its own gzip member for .gz)
+            if (bam || P.tenx) {                            // per-read TSV: the header leads (its own gzip member for .gz)
                 std::string hdr(kPerReadHeader), z;
                 if (lo.gz) gzip_member(hdr, z);
                 const std::string &w = lo.gz ? z : hdr;
                 if (fwrite(w.data(), 1, w.size(), lo.f) != w.size()) throw IoError("write failed: " + lo.tmp);
             }
         }
+        if (bam_out) {                                      // fastq-to-bam's header leads
+            P.bam_tmp = job.bam_output + ".tmp";
+            P.bam_f = fopen(P.bam_tmp.c_str(), "wb");
+            if (!P.bam_f) throw IoError("cannot write " + P.bam_tmp);
+            const std::string hdr = bam_header_bgzf();
+            if (fwrite(hdr.data(), 1, hdr.size(), P.bam_f) != hdr.size()) throw IoError("write failed: " + P.bam_tmp);
+        }
+        if (P.tenx) P.resolver = std::thread([&P] { P.resolve_main(); });
         for (size_t d = 0; d < job.ctxs.size(); d++) P.gpu_threads.emplace_back([&P, &job, d] { P.gpu_main(job.ctxs[d], (int)d); });
         P.committer = std::thread([&P] { P.commit_main(); });
         std::string walk_err; bool walk_io = false;
@@ -1529,6 +1679,8 @@ void run_file_pipeline(const FileJob &job, FileStats *stats_out) {
         P.to_gpu.close();
         for (auto &t : P.gpu_threads) t.join();
         P.gpu_threads.clear();
+        P.to_resolve.close();
+        if (P.resolver.joinable()) P.resolver.join();
         P.to_commit.close();
         P.committer.join();
         P.pool->stop();
@@ -1536,16 +1688,25 @@ void run_file_pipeline(const FileJob &job, FileStats *stats_out) {
         const double t_fin0 = now_s();
         if (P.ab.flag) {
             for (LibOut &lo : P.libs) { if (lo.f) fclose(lo.f); lo.f = nullptr; remove(lo.tmp.c_str()); }
+            if (P.bam_f) { fclose(P.bam_f); P.bam_f = nullptr; remove(P.bam_tmp.c_str()); }
             P.free_all();
             if (P.ab.io) throw IoError(P.ab.what);
             throw std::runtime_error(P.ab.what);
         }
         if (P.counts && !P.tenx && P.stats.n_reads && !P.tagged)
             throw std::runtime_error("no read of " + job.inputs[0] + " carries a CB or UB tag: counts need cell barcodes and UMIs");
-        // finish the files: per-read outputs are complete, bulk tables are written now
+        if (job.cache_size) P.stats.cb.cache_size = lane_cb_cache_size(job.ctxs) + P.inval.size();   // (+ non-ACGTN strings)
+        // finish the files: per-read outputs are complete, bulk tables are written now, the BAM gets its end-of-file block
+        if (P.bam_f) {
+            const bool ok = fwrite(kBgzfEof, 1, sizeof kBgzfEof, P.bam_f) == sizeof kBgzfEof;
+            const bool closed = fclose(P.bam_f) == 0;
+            P.bam_f = nullptr;
+            if (!ok || !closed) throw IoError("write failed: " + P.bam_tmp);
+            if (rename(P.bam_tmp.c_str(), job.bam_output.c_str()) != 0) throw IoError("cannot rename " + P.bam_tmp);
+        }
         for (LibOut &lo : P.libs) {
             if (!lo.f) continue;
-            if (!bam) {
+            if (!bam && !P.tenx) {
                 // `features<TAB>count` for untagged input (nimble/parse.py:39-57), rows in ascending feature-string order
                 std::vector<std::pair<std::string, uint64_t>> rows;
                 rows.reserve(lo.bulk.size());
@@ -1612,10 +1773,13 @@ void run_file_pipeline(const FileJob &job, FileStats *stats_out) {
         P.stop_pinner();
         P.free_slabs.close(); P.to_gpu.close();
         for (auto &t : P.gpu_threads) if (t.joinable()) t.join();
+        P.to_resolve.close();
+        if (P.resolver.joinable()) P.resolver.join();
         P.to_commit.close();
         if (P.committer.joinable()) P.committer.join();
         if (P.pool) P.pool->stop();
         for (LibOut &lo : P.libs) if (lo.f) { fclose(lo.f); remove(lo.tmp.c_str()); }
+        if (P.bam_f) { fclose(P.bam_f); P.bam_f = nullptr; remove(P.bam_tmp.c_str()); }
         P.free_all();
         throw;
     }

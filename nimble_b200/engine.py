@@ -353,7 +353,8 @@ class Engine:
         return int(out[0]), int(out[1])
 
     def align_10x_fastq(self, r1_fastq, r2_fastq, whitelist_path, libs, outputs, cb_length=16, umi_length=12):
-        """fastq-to-bam + align in one call, no intermediate BAM (nb200_align_10x_fastq).  Returns the barcode statistics."""
+        """fastq-to-bam + align in one streaming pass, no intermediate BAM (nb200_align_10x_fastq).  Returns the barcode
+        statistics (fastq_to_bam's, cache_size included)."""
         ids = (ct.c_int32 * len(libs))(*[l.id for l in libs])
         outs = (ct.c_char_p * len(outputs))(*[os.fspath(p).encode() for p in outputs])
         st = CbStats()

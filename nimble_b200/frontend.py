@@ -311,24 +311,63 @@ PER_READ_COLUMNS = ["nimble_features", "nimble_score", "r1_forward_score", "r1_r
                     "r2_reverse_score", "r1_QNAME", "r1_CB", "r1_UB", "r1_UR", "r1_GN", "r1_POS", "r2_POS"]
 
 
+def _devices(gpus):
+    """gpus (a count, or a list of device indices) -> the device list."""
+    return list(range(int(gpus))) if isinstance(gpus, int) else [int(g) for g in gpus]
+
+
+def _align_10x_multi(devs, num_cores, r1_fastq, r2_fastq, cb_whitelist_file, library_list, strand_filter, k, trim, cb_length,
+                     umi_length, outs, cnts=None, threshold=0.05, umi_flags=0):
+    """One nb200_align_10x_fastq_multi call: per-read TSVs (outs) and / or counts TSVs (cnts) over the devices devs.
+    Returns (barcode statistics, out3 per library or None); raises NimbleB200Error."""
+    import ctypes as ct
+    from . import _lib
+    L = _lib.load()
+    d = (ct.c_int32 * len(devs))(*devs)
+    libs = (ct.c_char_p * len(library_list))(*[os.fspath(p).encode() for p in library_list])
+    out_c = (ct.c_char_p * len(outs))(*[os.fspath(p).encode() for p in outs]) if outs else None
+    cnt_c = (ct.c_char_p * len(cnts))(*[os.fspath(p).encode() for p in cnts]) if cnts else None
+    w = 4 if umi_flags & _lib.UMI_CORRECT else 3
+    out3 = (ct.c_uint64 * (w * len(library_list)))()
+    cst = _lib.CbStats()
+    err = ct.create_string_buffer(1024)
+    st4 = (ct.c_double * 4)()
+    rc = L.nb200_align_10x_fastq_multi(d, len(devs), int(num_cores or 0), os.fspath(r1_fastq).encode(), os.fspath(r2_fastq).encode(),
+                                       os.fspath(cb_whitelist_file).encode(), int(cb_length), int(umi_length), libs, len(library_list),
+                                       strand_filter.encode(), int(k or 0), (trim or "").encode(), out_c, cnt_c, float(threshold),
+                                       int(umi_flags), out3, ct.byref(cst), err, len(err), st4)
+    if rc != 0:
+        raise _lib.NimbleB200Error(rc, err.value.decode(errors="replace"))
+    st = {f: getattr(cst, f) for f, _ in _lib.CbStats._fields_}
+    return st, ([tuple(out3[w * i:w * (i + 1)]) for i in range(len(library_list))] if cnts else None)
+
+
 def align_10x(reference, output, r1_fastq, r2_fastq, cb_whitelist_file, num_cores=1, strand_filter="unstranded", cb_length=16,
-              umi_length=12, k=None, engine=None):
-    """`fastq-to-bam` + `align` in one pass over raw 10x FASTQs, without the BAM in between (an extension: the
-    reference needs both commands).  Output = the per-read TSV(s) `align` would write for that BAM."""
+              umi_length=12, k=None, engine=None, gpus=None):
+    """`fastq-to-bam` + `align` in one streaming pass over raw 10x FASTQs, without the BAM in between (an extension: the
+    reference needs both commands).  Output = the per-read TSV(s) `align` would write for that BAM.  gpus (also
+    $NB200_GPUS): a count or a list of devices, as for fastq_to_counts."""
     from .engine import Engine
     from ._lib import NimbleB200Error
+    if gpus is None and os.environ.get("NB200_GPUS"):
+        gpus = int(os.environ["NB200_GPUS"])
     own = engine is None
     try:
-        eng = engine or Engine(int(os.environ.get("LOCAL_RANK", 0)), int(num_cores or 0))
         library_list = reference.split(",")
-        outs = [append_path_string(output, "." + os.path.splitext(os.path.basename(l))[0] if len(library_list) > 1 else "")
-                for l in library_list]
-        libs = [eng.load_library(l, strand_filter=strand_filter, k=k) for l in library_list]
-        st = eng.align_10x_fastq(r1_fastq, r2_fastq, cb_whitelist_file, libs, outs, cb_length, umi_length)
+        outs = _per_library_paths(output, library_list)
+        if gpus and engine is None and (not isinstance(gpus, int) or gpus > 1):
+            st, _ = _align_10x_multi(_devices(gpus), num_cores, r1_fastq, r2_fastq, cb_whitelist_file, library_list, strand_filter, k,
+                                     "", cb_length, umi_length, outs)
+        else:
+            eng = engine or Engine(int(os.environ.get("LOCAL_RANK", 0)), int(num_cores or 0))
+            try:
+                libs = [eng.load_library(l, strand_filter=strand_filter, k=k) for l in library_list]
+                st = eng.align_10x_fastq(r1_fastq, r2_fastq, cb_whitelist_file, libs, outs, cb_length, umi_length)
+            finally:
+                if own:
+                    eng.close()
         print("nimble_b200: %d pairs, %d with a valid cell barcode (%d corrected) -> %s"
               % (st["total_pairs"], st["written_pairs"], st["cb_corrected"], ", ".join(outs)))
-        if own:
-            eng.close()
         return 0
     except NimbleB200Error as e:
         print("nimble_b200 aligner error: %s" % e, file=sys.stderr)
@@ -392,7 +431,7 @@ def align_multi_gpu(reference, output, input, num_cores, strand_filter, k, gpus,
     import ctypes as ct
     from . import _lib
     L = _lib.load()
-    devs = list(range(int(gpus))) if isinstance(gpus, int) else [int(g) for g in gpus]
+    devs = _devices(gpus)
     library_list = reference.split(",")
     outs = _per_library_paths(output, library_list)
     cnts = _per_library_paths(counts, library_list)
@@ -762,26 +801,35 @@ def _print_pair_stats(st):
 
 def fastq_to_counts(reference, r1_fastq, r2_fastq, cb_whitelist_file, counts, num_cores=1, strand_filter="unstranded", trim="",
                     k=None, gpus=None, cb_length=16, umi_length=12, threshold=0.05, disable_thresholding=False, engine=None,
-                    correct_umis=False):
+                    correct_umis=False, output=None):
     """`fastq-to-bam`, then `align --counts` on its BAM, in one streaming pass without the BAM (an extension: the reference
     needs fastq-to-bam, align and report).  Raw 10x R1 / R2 FASTQ(.gz) + whitelist in, the counts TSV `report` would
     write out, one per library (named like align's outputs).  gpus (also $NB200_GPUS): a count or a list of devices.
     correct_umis (extension): merge UMIs one substitution away from a better-supported UMI of the same cell before the UMI
-    stage (DESIGN.md §2.12).  Returns 0 on success, 1 on an error (with a message on stderr), 2 without a CUDA device."""
+    stage (DESIGN.md §2.12).  output (extension): also write the per-read TSV align --map writes, in the same pass (named like
+    align's outputs; runs through nb200_align_10x_fastq_multi, so not with an engine).  Returns 0 on success, 1 on an
+    error (with a message on stderr), 2 without a CUDA device."""
     import ctypes as ct
     from . import _lib
     from .engine import Engine
     from ._lib import NimbleB200Error
     library_list = reference.split(",")
     cnts = _per_library_paths(counts, library_list)
+    outs = _per_library_paths(output, library_list)
     if gpus is None and os.environ.get("NB200_GPUS"):
         gpus = int(os.environ["NB200_GPUS"])
     own = engine is None
     try:
         trims = parse_trim(trim, len(library_list))
-        if gpus and engine is None and (not isinstance(gpus, int) or gpus > 1):
+        if outs is not None:
+            if engine is not None:
+                raise ValueError("a per-read output with the counts needs the multi-device entry: call without an engine")
+            devs = _devices(gpus) if gpus else [int(os.environ.get("LOCAL_RANK", 0))]
+            st, o3 = _align_10x_multi(devs, num_cores, r1_fastq, r2_fastq, cb_whitelist_file, library_list, strand_filter, k, trim,
+                                      cb_length, umi_length, outs, cnts, threshold, _lib.umi_flags(disable_thresholding, correct_umis))
+        elif gpus and engine is None and (not isinstance(gpus, int) or gpus > 1):
             L = _lib.load()
-            devs = list(range(int(gpus))) if isinstance(gpus, int) else [int(g) for g in gpus]
+            devs = _devices(gpus)
             d = (ct.c_int32 * len(devs))(*devs)
             libs = (ct.c_char_p * len(library_list))(*[os.fspath(p).encode() for p in library_list])
             cnt_c = (ct.c_char_p * len(cnts))(*[os.fspath(p).encode() for p in cnts])
@@ -821,5 +869,7 @@ def fastq_to_counts(reference, r1_fastq, r2_fastq, cb_whitelist_file, counts, nu
         print("nimble_b200: no pair written: every R1 that passed the name and length checks is exactly --cb-length + --umi-length "
               "(%d) bases long, so no read 1 is left after the barcode and UMI (fastq-to-bam drops such pairs)"
               % (int(cb_length) + int(umi_length)), file=sys.stderr)
+    for o in outs or []:
+        print("nimble_b200: wrote %s" % o)
     _print_counts_summary(cnts, o3)
     return 0
